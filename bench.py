@@ -3,6 +3,7 @@
 
   python bench.py --gpus N --steps K --warmup W            # this repo's CUDA planner
   python bench.py --impl reference --gpus N --steps K ...  # the reference's CPU planner (oracle port)
+  python bench.py ... --dump-outputs bench_outputs         # also save the last timed plan's outputs (.npy)
 
 A "step" is ONE planning call (policy.generate_action: 5 CEM iterations of sample -> fused ensemble
 rollout + scoring -> score-reduce -> select -> refit) at BASELINE configs[1] (C1 dims: 5-member
@@ -128,11 +129,12 @@ def _cpu_planners(c, objective='penalty'):
             "torch": lambda st, z, eps, zf: pt.do_generate_action(st, z, eps, zf)[2]}
 
 
-def time_cpu_planner(c, budget_s=20.0, max_plans=12, label="C1"):
+def time_cpu_planner(c, budget_s=20.0, max_plans=12, label="C1", steps=None, warmup=0):
     """Times the CPU restatements of the reference planner on this box's host cores: whole plans with
     the normal draws pre-generated outside the timed region. Both restatements (numpy and torch-CPU,
     cross-checked against each other and against fixtures produced by the unmodified reference code) get
-    two plans each; the faster one is the baseline and gets the rest of the budget."""
+    two plans each; the faster one is the baseline and gets the rest of the budget. With `steps`, the
+    faster one instead runs `warmup` untimed plans and then exactly `steps` timed ones, with no budget."""
     from simba_b200 import synthetic
     z, eps, zf = synthetic.make_draws(c['I'], 1, c['N'], c['H'], c['A'], c['P'], c['O'], seed=2)
     z, eps, zf = z[:, 0], eps[:, 0], zf[0]
@@ -156,6 +158,10 @@ def time_cpu_planner(c, budget_s=20.0, max_plans=12, label="C1"):
             break
     best_name = min(probe, key=probe.get)
     fn, times = planners[best_name], [probe[best_name]]
+    if steps is not None:
+        for _ in range(warmup):
+            fn(c['state'], z, eps, zf)
+        times, max_plans, budget_s = [], steps, float('inf')
     while len(times) < max_plans and time.perf_counter() - t_start < budget_s:
         t0 = time.perf_counter()
         n = fn(c['state'], z, eps, zf)
@@ -181,7 +187,7 @@ def run_reference(args):
         return
     from simba_b200 import synthetic
     c = synthetic.make_workload('c1')
-    cb = time_cpu_planner(c, budget_s=15.0 * max(1, args.steps) / 5.0, max_plans=max(2, args.steps + args.warmup))
+    cb = time_cpu_planner(c, steps=args.steps, warmup=args.warmup)
     line = {"impl": "reference", "metric": METRIC, "value": cb["value"], "unit": UNIT, "n_gpus": args.gpus,
             "steps": args.steps, "warmup": args.warmup, "ms_per_step": cb["ms_per_plan_median"],
             "higher_is_better": True, "scaling": "weak", "vs_baseline": None, "dtype": "f32",
@@ -205,8 +211,15 @@ def main():
     ap.add_argument('--precision', default='bf16', choices=['bf16', 'fp32'])
     ap.add_argument('--extras', default=None, help="comma list of: c3, c4, c5, fp32, train, none (default: c3,c4 when N > 1, fp32,c4,c3,c5,train when N == 1)")
     ap.add_argument('--no-cpu-baseline', action='store_true')
+    ap.add_argument('--dump-outputs', metavar='DIR', default=None,
+                    help="write what the last timed plan returned (device plan: action, score, iterations; "
+                         "end to end: action) as DIR/<name>.npy in float32, for comparing two builds")
     args = ap.parse_args()
+    if args.steps < 1:
+        ap.error("--steps must be at least 1")
     if args.impl == 'reference':
+        if args.dump_outputs:
+            ap.error("--dump-outputs applies to the b200 arm")
         return run_reference(args)
 
     import torch
@@ -223,7 +236,7 @@ def main():
     if world > 1:
         dist.init_process_group('nccl', device_id=torch.device('cuda', local_rank))
     lib = _lib.load()
-    W, K = max(3, args.warmup), max(1, args.steps)
+    W, K = max(3, args.warmup), args.steps
 
     c = synthetic.make_workload('c1')
     precision = args.precision
@@ -262,6 +275,8 @@ def main():
     sync_all()
     t_wall = time.perf_counter() - t_wall0
     ms = np.array([a.elapsed_time(b) for a, b in ev])
+    last_plan = {"plan_action": out_a.cpu().numpy(), "plan_score": out_s.cpu().numpy(),
+                 "plan_iterations": out_i.cpu().numpy()}
     iters_total = int(out_i.cpu()[0])
     t_rank = torch.tensor([ms.sum() / 1e3], dtype=torch.float64, device='cuda')
     if world > 1:
@@ -282,6 +297,8 @@ def main():
         a = pol.generate_action(states_np[k % n_pool])
         t_e2e += time.perf_counter() - t0
     assert np.all(np.isfinite(a))
+    if args.dump_outputs:
+        dump_outputs(args.dump_outputs, dict(last_plan, e2e_action=a), '_rank%d' % rank if world > 1 else '')
     t_e = torch.tensor([t_e2e], dtype=torch.float64, device='cuda')
     if world > 1:
         dist.all_reduce(t_e, op=dist.ReduceOp.MAX)
@@ -398,6 +415,13 @@ def main():
         print(json.dumps(line))
     if world > 1:
         dist.destroy_process_group()
+
+
+def dump_outputs(out_dir, arrays, suffix=''):
+    """Each array as <out_dir>/<name><suffix>.npy in float32 (iteration counts are exact in float32)."""
+    os.makedirs(out_dir, exist_ok=True)
+    for name, x in arrays.items():
+        np.save(os.path.join(out_dir, name + suffix + '.npy'), np.asarray(x, dtype=np.float32))
 
 
 def committed_traffic(key):
