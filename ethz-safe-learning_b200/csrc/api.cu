@@ -102,12 +102,10 @@ struct simba_model {
   void* d_w_bf16 = nullptr;
   void* d_w_wide = nullptr;     // wide-model tcgen05 weight stream (rollout_tc_wide.cu)
   int64_t w_wide_member_bytes = 0;
-  float* d_bias_tc = nullptr;
   void* d_bias_k16 = nullptr;   // per member, per layer: UMMA B tile [128 n][16 k] (no swizzle) holding the bias as bf16 hi + lo
   float tc_scale_a[64] = {0}, tc_scale_b[64] = {0};
   float* d_smin = nullptr;
   float* d_sdelta = nullptr;
-  float* d_sinv = nullptr;
   int n_chunks = 0, bias_stride = 0, act_rows = 0;
   int64_t w_bf16_member_bytes = 0;
   // scratch for the model-level entry points (tile lists are rebuilt per call size)
@@ -143,12 +141,10 @@ extern "C" int simba_model_create(const simba_model_config_t* cfg, simba_model_t
 }
 
 static void model_free_device(simba_model* m) {
-  cudaFree(m->d_w_f32); cudaFree(m->d_bias_f32); cudaFree(m->d_w_bf16); cudaFree(m->d_bias_tc); cudaFree(m->d_bias_k16);
-  cudaFree(m->d_w_wide); m->d_w_wide = nullptr;
-  m->d_bias_tc = nullptr; m->d_bias_k16 = nullptr;
-  cudaFree(m->d_smin); cudaFree(m->d_sdelta); cudaFree(m->d_sinv);
-  m->d_w_f32 = m->d_bias_f32 = m->d_smin = m->d_sdelta = m->d_sinv = nullptr;
-  m->d_w_bf16 = nullptr;
+  cudaFree(m->d_w_f32); cudaFree(m->d_bias_f32); cudaFree(m->d_w_bf16); cudaFree(m->d_bias_k16); cudaFree(m->d_w_wide);
+  cudaFree(m->d_smin); cudaFree(m->d_sdelta);
+  m->d_w_f32 = m->d_bias_f32 = m->d_smin = m->d_sdelta = nullptr;
+  m->d_w_bf16 = m->d_bias_k16 = m->d_w_wide = nullptr;
 }
 
 extern "C" int simba_model_destroy(simba_model_t* m) {
@@ -214,17 +210,181 @@ extern "C" int simba_model_set_scaler(simba_model_t* m, const float* mn, const f
   return SIMBA_OK;
 }
 
-// bf16 image of one member for the tcgen05 kernel: for every layer the UMMA B operand
-// B[n][k] = W[k][n], K-major, SWIZZLE_128B: per 64-wide K atom a [N_pad rows][128 bytes] slab,
-// 16-byte chunk c of row n stored at chunk (c ^ (n & 7)). Heads: mu -> rows [0, O),
-// var -> rows [64, 64 + O) of a 128-row tile.
+// bf16 (hi, lo) split of a bias, hi = bf16(v), lo = bf16(v - hi): the kernels multiply both by a constant 1
+static void split_bf16(float v, uint16_t& hi, uint16_t& lo) {
+  hi = f32_to_bf16_rne(v);
+  lo = f32_to_bf16_rne(v - bf16_to_f32(hi));
+}
+
+// byte offset of element (n, k), 0 <= k < 64, in a K-major SWIZZLE_128B tile: row n is 128 bytes, and its
+// 16-byte chunk c is stored at chunk c ^ (n & 7)
+static int64_t sw128_offset(int n, int k) { return (int64_t)n * 128 + ((k / 8) ^ (n & 7)) * 16 + (k % 8) * 2; }
+
+// first commit: allocate; later commits overwrite in place (the sizes are fixed by the model config)
+template <class D, class T>
+static cudaError_t upload(D*& dst, const std::vector<T>& host) {
+  const size_t bytes = host.size() * sizeof(T);
+  const cudaError_t e = dst ? cudaSuccess : cudaMalloc(&dst, bytes);
+  return e != cudaSuccess ? e : cudaMemcpy(dst, host.data(), bytes, cudaMemcpyHostToDevice);
+}
+
+// fp32 chunk stream of the fp32 kernel, per member: layer -> column block (128) -> k chunk (16), heads fused
+// as N = 2*O; the biases per layer, padded to whole column blocks (layout in m->n_chunks, m->bias_stride)
+static void pack_f32_image(const simba_model* m, std::vector<float>& w, std::vector<float>& b) {
+  const auto& c = m->cfg;
+  const int L = c.n_layers, E = c.ensemble_size, U = c.units, O = c.obs_dim, IN = c.obs_dim + c.act_dim;
+  const int KC = kF32ChunkRows, NB = kF32ChunkCols;
+  w.assign((size_t)E * m->n_chunks * KC * NB, 0.0f);
+  b.assign((size_t)E * m->bias_stride, 0.0f);
+  for (int e = 0; e < E; ++e) {
+    const std::vector<float>* kern = &m->kernels[e * (L + 2)];
+    const std::vector<float>* bias = &m->biases[e * (L + 2)];
+    size_t chunk = (size_t)e * m->n_chunks;
+    int boff = 0;
+    for (int l = 0; l <= L; ++l) {
+      const int K = l == 0 ? IN : U, N = l == L ? 2 * O : U;
+      const int Kp = round_up(K, KC), Np = round_up(N, NB);
+      auto weight = [&](int k, int n) -> float {
+        if (k >= K || n >= N) return 0.0f;
+        if (l < L) return kern[l][(size_t)k * U + n];
+        if (n < O) return kern[L][(size_t)k * O + n];            // mu head
+        return kern[L + 1][(size_t)k * O + (n - O)];             // var head
+      };
+      for (int nb = 0; nb < Np; nb += NB)
+        for (int kc = 0; kc < Kp; kc += KC, ++chunk)
+          for (int kk = 0; kk < KC; ++kk)
+            for (int n = 0; n < NB; ++n)
+              w[(chunk * KC + kk) * NB + n] = weight(kc + kk, nb + n);
+      for (int n = 0; n < N; ++n)
+        b[(size_t)e * m->bias_stride + boff + n] = l < L ? bias[l][n] : n < O ? bias[L][n] : bias[L + 1][n - O];
+      boff += Np;
+    }
+  }
+}
+
 static int64_t bf16_layer_bytes(int K) { return (int64_t)round_up(K, 64) / 64 * (128 * 128); }
+
+// bf16 image of the tcgen05 kernel, per member and layer the UMMA B operand B[n][k] = W[k][n], K-major SWIZZLE_128B:
+// one [128 rows][128 bytes] slab per 64-wide K atom; hidden and head layers occupy K = 128 (zero-padded). Heads: mu
+// -> rows [0, O), var -> rows [64, 64 + O), the raw-variance head pre-scaled by log2(e) (the kernels evaluate softplus
+// as ln2 * lg2(1 + ex2(x log2 e)) and get x log2 e out of the GEMM). Layer 0 carries its bias in the K padding (the
+// kernel feeds the constant 1 at k = IN, IN + 1). `bias_k16`: every layer's bias as one more K = 16 block of its GEMM,
+// B[n][0] = hi, B[n][1] = lo, K-major SWIZZLE_NONE: 8-row x 16-byte core matrices, the two K halves 128 B apart
+// (leading byte offset), 8-row groups 256 B apart (stride byte offset) -> 4 KB per layer. Returns a member's bytes.
+static int64_t pack_bf16_image(const simba_model* m, std::vector<uint16_t>& img, std::vector<uint16_t>& bias_k16) {
+  const auto& c = m->cfg;
+  const int L = c.n_layers, E = c.ensemble_size, U = c.units, O = c.obs_dim, IN = c.obs_dim + c.act_dim;
+  int64_t member_bytes = 0;
+  for (int l = 0; l <= L; ++l) member_bytes += bf16_layer_bytes(l == 0 ? IN : 128);
+  img.assign((size_t)E * member_bytes / 2, 0);
+  bias_k16.assign((size_t)E * (L + 1) * 2048, 0);
+  for (int e = 0; e < E; ++e) {
+    const std::vector<float>* kern = &m->kernels[e * (L + 2)];
+    const std::vector<float>* bias = &m->biases[e * (L + 2)];
+    int64_t off = (int64_t)e * member_bytes;
+    for (int l = 0; l <= L; ++l) {
+      const int K = l == 0 ? IN : U;
+      auto weight = [&](int k, int n) -> uint16_t {     // n = tile row (output feature)
+        if (l == 0 && IN + 2 <= 64 && (k == IN || k == IN + 1) && n < U) {
+          uint16_t hi, lo;
+          split_bf16(bias[0][n], hi, lo);
+          return k == IN ? hi : lo;
+        }
+        if (k >= K) return 0;
+        if (l < L) return n < U ? f32_to_bf16_rne(kern[l][(size_t)k * U + n]) : 0;
+        if (n < O) return f32_to_bf16_rne(kern[L][(size_t)k * O + n]);
+        if (n >= 64 && n < 64 + O) return f32_to_bf16_rne(kLog2e * kern[L + 1][(size_t)k * O + (n - 64)]);
+        return 0;
+      };
+      const int Kp = l == 0 ? IN : 128;
+      for (int at = 0; at < round_up(Kp, 64) / 64; ++at)
+        for (int n = 0; n < 128; ++n)
+          for (int kk = 0; kk < 64; ++kk)
+            img[(off + (int64_t)at * 128 * 128 + sw128_offset(n, kk)) / 2] = weight(at * 64 + kk, n);
+      off += bf16_layer_bytes(Kp);
+      for (int n = 0; n < 128; ++n) {
+        float bv = 0.0f;
+        if (l < L) bv = n < U ? bias[l][n] : 0.0f;
+        else if (n < O) bv = bias[L][n];
+        else if (n >= 64 && n < 64 + O) bv = kLog2e * bias[L + 1][n - 64];
+        uint16_t* bk = &bias_k16[((size_t)e * (L + 1) + l) * 2048 + (size_t)(n / 8) * 128 + (size_t)(n % 8) * 8];
+        split_bf16(bv, bk[0], bk[1]);
+      }
+    }
+  }
+  return member_bytes;
+}
+
+// wide-model tcgen05 weight stream: per member the tiles of one rollout step in consumption order — layer 0:
+// one [UP x 64] tile; layers 1..L-1: KA tiles [UP x 64]; heads: KA tiles [128 x 64] (mu rows [0, O), var rows
+// [64, 64 + O), var pre-scaled by log2(e) as above); each tile K-major SWIZZLE_128B. UP is U zero-padded to a
+// multiple of 16. The bias of a layer sits in k rows KB (hi) and KB + 1 (lo), which the kernel multiplies by
+// constant ones in the A tile. Returns the bytes of one member's stream.
+static int64_t pack_wide_image(const simba_model* m, std::vector<uint16_t>& img) {
+  const auto& c = m->cfg;
+  const int L = c.n_layers, E = c.ensemble_size, U = c.units, O = c.obs_dim, IN = c.obs_dim + c.act_dim;
+  const int UP = rollout_tc_wide_units(U);
+  const int KA = (UP + 2 + 63) / 64;
+  const int64_t member_bytes = rollout_tc_wide_member_bytes(L, UP);
+  img.assign((size_t)E * member_bytes / 2, 0);
+  for (int e = 0; e < E; ++e) {
+    int64_t off = (int64_t)e * member_bytes;
+    for (int l = 0; l <= L; ++l) {
+      const int K = l == 0 ? IN : U;                     // real input width
+      const int KB = l == 0 ? IN : UP;                   // the A tile holds the constant ones at k = KB, KB + 1
+      const int rows = l < L ? UP : 128;                 // tile rows = output features
+      const int tiles = l == 0 ? 1 : KA;
+      auto weight = [&](int k, int n) -> uint16_t {
+        int layer = l, col = n;                          // Keras layer index and output column
+        if (l == L) {
+          if (n < O) { layer = L; col = n; }
+          else if (n >= 64 && n < 64 + O) { layer = L + 1; col = n - 64; }
+          else return 0;
+        } else if (n >= U) {
+          return 0;                                      // padded hidden unit: weights and bias 0
+        }
+        const int width = l < L ? U : O;
+        const float pre = layer == L + 1 ? kLog2e : 1.0f;
+        if (k < K) return f32_to_bf16_rne(pre * m->kernels[e * (L + 2) + layer][(size_t)k * width + col]);
+        if (k == KB || k == KB + 1) {
+          uint16_t hi, lo;
+          split_bf16(pre * m->biases[e * (L + 2) + layer][col], hi, lo);
+          return k == KB ? hi : lo;
+        }
+        return 0;
+      };
+      for (int tI = 0; tI < tiles; ++tI) {
+        for (int n = 0; n < rows; ++n)
+          for (int kk = 0; kk < 64; ++kk) img[(off + sw128_offset(n, kk)) / 2] = weight(tI * 64 + kk, n);
+        off += (int64_t)rows * 128;
+      }
+    }
+  }
+  return member_bytes;
+}
+
+// scaler: delta = max - min, 1.01 where delta < 1e-5 (transition_model.py:85-86), for the fp32 kernel and
+// simba_scale; the bf16 kernels take it as x_scaled = fma(x, a, b) (m->tc_scale_a, m->tc_scale_b)
+static std::vector<float> pack_scaler(simba_model* m) {
+  const int IN = m->cfg.obs_dim + m->cfg.act_dim;
+  std::vector<float> delta(IN), inv(IN);
+  for (int k = 0; k < IN; ++k) {
+    volatile float d = m->smax[k] - m->smin[k];
+    if (d < 1e-5f) d = 1.01f;
+    delta[k] = d;
+    inv[k] = 1.0f / d;
+  }
+  for (int k = 0; k < 64; ++k) {
+    m->tc_scale_a[k] = k < IN ? (m->scale_on ? inv[k] : 1.0f) : 0.0f;
+    m->tc_scale_b[k] = k < IN ? (m->scale_on ? -m->smin[k] * inv[k] : 0.0f) : 0.0f;
+  }
+  return delta;
+}
 
 extern "C" int simba_model_commit(simba_model_t* m) {
   if (!m) return fail(SIMBA_ERR_BAD_CONFIG, "null argument");
   const auto& c = m->cfg;
-  const int L = c.n_layers, E = c.ensemble_size, U = c.units, O = c.obs_dim;
-  const int IN = c.obs_dim + c.act_dim;
+  const int L = c.n_layers, U = c.units, O = c.obs_dim, IN = c.obs_dim + c.act_dim;
   for (size_t i = 0; i < m->layer_set.size(); ++i)
     if (!m->layer_set[i])
       return fail(SIMBA_ERR_NOT_READY, "member %zu layer %zu has no weights", i / (L + 2),
@@ -236,8 +396,6 @@ extern "C" int simba_model_commit(simba_model_t* m) {
   // pointers when the weights or the scaler change (e.g. after every model.fit of the agent loop).
   // The copies below are synchronous, so they are ordered after earlier launches on any stream
   // only by the caller's own synchronisation (generate_action is synchronous).
-
-  // ---- fp32 chunk stream: layer -> column block (128) -> k chunk (16), heads fused as N = 2*O ---
   const int KC = kF32ChunkRows, NB = kF32ChunkCols;
   int n_chunks = 0, bias_stride = 0, act_rows = round_up(IN, KC);
   for (int l = 0; l <= L; ++l) {
@@ -257,191 +415,27 @@ extern "C" int simba_model_commit(simba_model_t* m) {
       return fail(SIMBA_ERR_UNSUPPORTED, "units %d: the rollout kernels keep a row tile's activations in "
                   "shared memory, which holds at most ~780 hidden units", U);
   }
-  std::vector<float> w((size_t)E * n_chunks * KC * NB, 0.0f), b((size_t)E * bias_stride, 0.0f);
-  for (int e = 0; e < E; ++e) {
-    size_t chunk = (size_t)e * n_chunks;
-    int boff = 0;
-    for (int l = 0; l <= L; ++l) {
-      const int K = l == 0 ? IN : U, N = l == L ? 2 * O : U;
-      const int Kp = round_up(K, KC), Np = round_up(N, NB);
-      auto weight = [&](int k, int n) -> float {
-        if (k >= K || n >= N) return 0.0f;
-        if (l < L) return m->kernels[e * (L + 2) + l][(size_t)k * U + n];
-        if (n < O) return m->kernels[e * (L + 2) + L][(size_t)k * O + n];            // mu head
-        return m->kernels[e * (L + 2) + L + 1][(size_t)k * O + (n - O)];             // var head
-      };
-      for (int nb = 0; nb < Np; nb += NB)
-        for (int kc = 0; kc < Kp; kc += KC, ++chunk)
-          for (int kk = 0; kk < KC; ++kk)
-            for (int n = 0; n < NB; ++n)
-              w[(chunk * KC + kk) * NB + n] = weight(kc + kk, nb + n);
-      for (int n = 0; n < N; ++n) {
-        float bv;
-        if (l < L) bv = m->biases[e * (L + 2) + l][n];
-        else bv = n < O ? m->biases[e * (L + 2) + L][n] : m->biases[e * (L + 2) + L + 1][n - O];
-        b[(size_t)e * bias_stride + boff + n] = bv;
-      }
-      boff += Np;
-    }
-  }
+  std::vector<float> w, b;
+  pack_f32_image(m, w, b);
   CUDA_TRY(cudaDeviceSynchronize());
-  if (!m->d_w_f32) CUDA_TRY(cudaMalloc(&m->d_w_f32, w.size() * sizeof(float)));
-  CUDA_TRY(cudaMemcpy(m->d_w_f32, w.data(), w.size() * sizeof(float), cudaMemcpyHostToDevice));
-  if (!m->d_bias_f32) CUDA_TRY(cudaMalloc(&m->d_bias_f32, b.size() * sizeof(float)));
-  CUDA_TRY(cudaMemcpy(m->d_bias_f32, b.data(), b.size() * sizeof(float), cudaMemcpyHostToDevice));
-
-  // ---- bf16 UMMA image (only the shapes the tcgen05 kernel covers) -------------------------------
+  CUDA_TRY(upload(m->d_w_f32, w));
+  CUDA_TRY(upload(m->d_bias_f32, b));
+  // bf16 images only for the shapes a tcgen05 kernel covers
   m->w_bf16_member_bytes = 0;
   if (rollout_tc_supported(O, c.act_dim, L, U, 1)) {
-    int64_t member_bytes = 0;
-    // hidden / head layers always occupy K = 128 (two atoms): narrower models are zero-padded
-    for (int l = 0; l <= L; ++l) member_bytes += bf16_layer_bytes(l == 0 ? IN : 128);
-    std::vector<uint16_t> img((size_t)E * member_bytes / 2, 0);
-    for (int e = 0; e < E; ++e) {
-      int64_t off = (int64_t)e * member_bytes;
-      for (int l = 0; l <= L; ++l) {
-        const int K = l == 0 ? IN : U;
-        auto weight = [&](int k, int n) -> float {     // n = tile row (output feature)
-          if (l == 0 && IN + 2 <= 64 && (k == IN || k == IN + 1) && n < U) {
-            // layer 0 carries its bias in the K padding: the kernel feeds the constant 1 at k = IN, IN + 1
-            const float bv = m->biases[e * (L + 2)][n];
-            const float hi = bf16_to_f32(f32_to_bf16_rne(bv));
-            return k == IN ? hi : bv - hi;             // rounded to bf16 below: bf16(b), bf16(b - hi)
-          }
-          if (k >= K) return 0.0f;
-          if (l < L) return n < U ? m->kernels[e * (L + 2) + l][(size_t)k * U + n] : 0.0f;
-          if (n < O) return m->kernels[e * (L + 2) + L][(size_t)k * O + n];
-          // the raw-variance head is pre-scaled by log2(e): the kernels evaluate softplus as
-          // ln2 * lg2(1 + ex2(x log2 e)) and get x log2 e straight out of the GEMM
-          if (n >= 64 && n < 64 + O) return kLog2e * m->kernels[e * (L + 2) + L + 1][(size_t)k * O + (n - 64)];
-          return 0.0f;
-        };
-        const int Kp = l == 0 ? IN : 128;
-        const int atoms = round_up(Kp, 64) / 64;
-        for (int at = 0; at < atoms; ++at)
-          for (int n = 0; n < 128; ++n)
-            for (int kk = 0; kk < 64; ++kk) {
-              const int chunk16 = kk / 8, within = kk % 8;
-              const int64_t byte = off + (int64_t)at * 128 * 128 + (int64_t)n * 128 +
-                                   ((chunk16 ^ (n & 7)) * 16) + within * 2;
-              img[byte / 2] = f32_to_bf16_rne(weight(at * 64 + kk, n));
-            }
-        off += bf16_layer_bytes(Kp);
-      }
-    }
-    m->w_bf16_member_bytes = member_bytes;
-    if (!m->d_w_bf16) CUDA_TRY(cudaMalloc(&m->d_w_bf16, img.size() * 2));
-    CUDA_TRY(cudaMemcpy(m->d_w_bf16, img.data(), img.size() * 2, cudaMemcpyHostToDevice));
-    std::vector<float> bt((size_t)E * (L + 1) * 128, 0.0f);
-    for (int e = 0; e < E; ++e) {
-      for (int l = 0; l < L; ++l)
-        for (int n = 0; n < U; ++n) bt[((size_t)e * (L + 1) + l) * 128 + n] = m->biases[e * (L + 2) + l][n];
-      for (int n = 0; n < O; ++n) {
-        bt[((size_t)e * (L + 1) + L) * 128 + n] = m->biases[e * (L + 2) + L][n];
-        bt[((size_t)e * (L + 1) + L) * 128 + 64 + n] = kLog2e * m->biases[e * (L + 2) + L + 1][n];   // (see above)
-      }
-    }
-    if (!m->d_bias_tc) CUDA_TRY(cudaMalloc(&m->d_bias_tc, bt.size() * sizeof(float)));
-    CUDA_TRY(cudaMemcpy(m->d_bias_tc, bt.data(), bt.size() * sizeof(float), cudaMemcpyHostToDevice));
-    // bias as one more K = 16 block of every layer's GEMM: B[n][0] = bf16(b[n]), B[n][1] = bf16(b[n] - hi),
-    // K-major, SWIZZLE_NONE canonical layout: 8-row x 16-byte core matrices, the two K halves 128 B apart
-    // (leading byte offset), 8-row groups 256 B apart (stride byte offset) -> 4 KB per layer
-    std::vector<uint16_t> bk((size_t)E * (L + 1) * 2048, 0);
-    for (int e = 0; e < E; ++e)
-      for (int l = 0; l <= L; ++l)
-        for (int n = 0; n < 128; ++n) {
-          const float bv = bt[((size_t)e * (L + 1) + l) * 128 + n];
-          const uint16_t hi = f32_to_bf16_rne(bv);
-          uint32_t hb = (uint32_t)hi << 16;
-          float hf;
-          memcpy(&hf, &hb, 4);
-          const uint16_t lo = f32_to_bf16_rne(bv - hf);
-          const size_t base = ((size_t)e * (L + 1) + l) * 2048 + (size_t)(n / 8) * 128 + (size_t)(n % 8) * 8;
-          bk[base + 0] = hi;
-          bk[base + 1] = lo;
-        }
-    if (!m->d_bias_k16) CUDA_TRY(cudaMalloc(&m->d_bias_k16, bk.size() * 2));
-    CUDA_TRY(cudaMemcpy(m->d_bias_k16, bk.data(), bk.size() * 2, cudaMemcpyHostToDevice));
+    std::vector<uint16_t> img, bias_k16;
+    m->w_bf16_member_bytes = pack_bf16_image(m, img, bias_k16);
+    CUDA_TRY(upload(m->d_w_bf16, img));
+    CUDA_TRY(upload(m->d_bias_k16, bias_k16));
   }
-
-  // ---- wide-model tcgen05 weight stream: per member the tiles of one rollout step in consumption
-  //      order — layer 0: one [U x 64] tile; layers 1..L-1: KA tiles [U x 64]; heads: KA tiles
-  //      [128 x 64] (mu rows [0, O), var rows [64, 64 + O)); each tile K-major SWIZZLE_128B. The bias
-  //      of a layer sits in k rows K_real (bf16 hi) and K_real + 1 (bf16 of the remainder), which the
-  //      kernel multiplies by constant ones in the A tile. -----------------------------------------
   m->w_wide_member_bytes = 0;
   if (rollout_tc_wide_supported(O, c.act_dim, L, U, 1)) {
-    const int UP = rollout_tc_wide_units(U);               // kernel width: U zero-padded to 16
-    const int KA = (UP + 2 + 63) / 64;
-    const int64_t member_bytes = rollout_tc_wide_member_bytes(L, UP);
-    std::vector<uint16_t> img((size_t)E * member_bytes / 2, 0);
-    auto split_bias = [&](float bv, uint16_t& hi, uint16_t& lo) {
-      hi = f32_to_bf16_rne(bv);
-      uint32_t hb = (uint32_t)hi << 16;
-      float hf;
-      memcpy(&hf, &hb, 4);
-      lo = f32_to_bf16_rne(bv - hf);
-    };
-    for (int e = 0; e < E; ++e) {
-      int64_t off = (int64_t)e * member_bytes;
-      for (int l = 0; l <= L; ++l) {
-        const int K = l == 0 ? IN : U;                     // real input width
-        const int KB = l == 0 ? IN : UP;                   // the A tile holds the constant ones at k = KB, KB + 1
-        const int rows = l < L ? UP : 128;                 // tile rows = output features
-        const int tiles = l == 0 ? 1 : KA;
-        auto weight = [&](int k, int n) -> uint16_t {
-          int layer = l, col = n;                          // Keras layer index and output column
-          if (l == L) {
-            if (n < O) { layer = L; col = n; }
-            else if (n >= 64 && n < 64 + O) { layer = L + 1; col = n - 64; }
-            else return 0;
-          } else if (n >= U) {
-            return 0;                                      // padded hidden unit: weights and bias 0
-          }
-          const int width = l < L ? U : O;
-          const float pre = layer == L + 1 ? kLog2e : 1.0f;   // raw-variance head pre-scaled by log2(e)
-          if (k < K) return f32_to_bf16_rne(pre * m->kernels[e * (L + 2) + layer][(size_t)k * width + col]);
-          if (k == KB || k == KB + 1) {
-            uint16_t hi, lo;
-            split_bias(pre * m->biases[e * (L + 2) + layer][col], hi, lo);
-            return k == KB ? hi : lo;
-          }
-          return 0;
-        };
-        for (int tI = 0; tI < tiles; ++tI) {
-          for (int n = 0; n < rows; ++n)
-            for (int kk = 0; kk < 64; ++kk) {
-              const int chunk16 = kk / 8, within = kk % 8;
-              const int64_t byte = off + (int64_t)n * 128 + ((chunk16 ^ (n & 7)) * 16) + within * 2;
-              img[byte / 2] = weight(tI * 64 + kk, n);
-            }
-          off += (int64_t)rows * 128;
-        }
-      }
-    }
-    m->w_wide_member_bytes = member_bytes;
-    if (!m->d_w_wide) CUDA_TRY(cudaMalloc(&m->d_w_wide, img.size() * 2));
-    CUDA_TRY(cudaMemcpy(m->d_w_wide, img.data(), img.size() * 2, cudaMemcpyHostToDevice));
+    std::vector<uint16_t> img;
+    m->w_wide_member_bytes = pack_wide_image(m, img);
+    CUDA_TRY(upload(m->d_w_wide, img));
   }
-
-  // ---- scaler: delta = max - min, 1.01 where delta < 1e-5 (transition_model.py:85-86) ----------
-  std::vector<float> delta(IN), inv(IN);
-  for (int k = 0; k < IN; ++k) {
-    volatile float d = m->smax[k] - m->smin[k];
-    if (d < 1e-5f) d = 1.01f;
-    delta[k] = d;
-    inv[k] = 1.0f / d;
-  }
-  for (int k = 0; k < 64; ++k) {
-    m->tc_scale_a[k] = k < IN ? (m->scale_on ? inv[k] : 1.0f) : 0.0f;
-    m->tc_scale_b[k] = k < IN ? (m->scale_on ? -m->smin[k] * inv[k] : 0.0f) : 0.0f;
-  }
-  if (!m->d_smin) CUDA_TRY(cudaMalloc(&m->d_smin, IN * sizeof(float)));
-  if (!m->d_sdelta) CUDA_TRY(cudaMalloc(&m->d_sdelta, IN * sizeof(float)));
-  if (!m->d_sinv) CUDA_TRY(cudaMalloc(&m->d_sinv, IN * sizeof(float)));
-  CUDA_TRY(cudaMemcpy(m->d_smin, m->smin.data(), IN * sizeof(float), cudaMemcpyHostToDevice));
-  CUDA_TRY(cudaMemcpy(m->d_sdelta, delta.data(), IN * sizeof(float), cudaMemcpyHostToDevice));
-  CUDA_TRY(cudaMemcpy(m->d_sinv, inv.data(), IN * sizeof(float), cudaMemcpyHostToDevice));
+  CUDA_TRY(upload(m->d_smin, m->smin));
+  CUDA_TRY(upload(m->d_sdelta, pack_scaler(m)));
   m->committed = true;
   ++m->generation;
   return SIMBA_OK;
@@ -459,14 +453,11 @@ static void fill_model_params(const simba_model* m, RolloutParams& prm) {
   prm.w_bf16_member_bytes = m->w_bf16_member_bytes;
   prm.w_wide = m->d_w_wide;
   prm.w_wide_member_bytes = m->w_wide_member_bytes;
-  prm.bias_tc = m->d_bias_tc;
   prm.bias_k16 = m->d_bias_k16;
   memcpy(prm.tc_scale_a, m->tc_scale_a, sizeof(prm.tc_scale_a));
   memcpy(prm.tc_scale_b, m->tc_scale_b, sizeof(prm.tc_scale_b));
-  prm.tc_tiles_per_cta = 1;
   prm.smin = m->d_smin;
   prm.sdelta = m->d_sdelta;
-  prm.sinv = m->d_sinv;
   prm.scale_on = m->scale_on;
 }
 
@@ -543,6 +534,37 @@ static void split_tail_items(std::vector<Tile>& tiles, int sms) {
   }
 }
 
+// The rollout kernel of a planner and the tile list it walks, from the shapes, the precision and the SM count.
+// The diagnostic switches SIMBA_B200_NO_TAIL_SPLIT and SIMBA_B200_NO_PAIR are read here and nowhere else.
+static int choose_rollout(const simba_model_config_t& mc, const simba_planner_config_t& cfg, const RowGeom& g,
+                          int sms, RolloutKernel& kernel, std::vector<Tile>& tiles) {
+  const int O = mc.obs_dim, A = mc.act_dim, L = mc.n_layers, U = mc.units, H = cfg.horizon, nc = cfg.scorer.n_constraints;
+  kernel = RolloutKernel::kF32;
+  build_tiles(g, cfg.precision == SIMBA_PREC_FP32 ? kF32TileRows : kTcTileRows, tiles);
+  if (cfg.precision == SIMBA_PREC_FP32) return SIMBA_OK;
+  if (rollout_tc_supported(O, A, L, U, H)) {
+    kernel = RolloutKernel::kTcOneCta;
+    if ((int)tiles.size() > sms && rollout_tc_two_tiles_fit(L, nc)) {
+      // more tiles than SMs: two tiles per CTA so one tile's MMAs overlap the other's epilogue
+      kernel = RolloutKernel::kTcTwoTile;
+      build_tiles(g, kTcTileRows, tiles, 2);
+      if (getenv("SIMBA_B200_NO_TAIL_SPLIT") == nullptr) split_tail_items(tiles, sms);
+    } else if ((int)tiles.size() * 2 <= sms && rollout_tc_pair_fits(L, nc) && getenv("SIMBA_B200_NO_PAIR") == nullptr) {
+      // few tiles (a single plan): two SMs per tile, the head pass split between them
+      kernel = RolloutKernel::kTcPair;
+    }
+    return SIMBA_OK;
+  }
+  if (rollout_tc_wide_supported(O, A, L, U, H) && rollout_tc_wide_fits(L, U, nc)) {
+    kernel = RolloutKernel::kTcWide;
+    return SIMBA_OK;
+  }
+  return fail(SIMBA_ERR_UNSUPPORTED,
+              "bf16 tcgen05 rollout covers units <= 128 (obs_dim <= 60, obs_dim+act_dim <= 64, <= 5 layers) and "
+              "wide models with 128 < units <= ~416 (less with several constrained lidars; obs_dim+act_dim <= 62); "
+              "use precision fp32 for this shape");
+}
+
 // ---------------------------------------------------------------------------------------------
 // NCCL, loaded lazily so that a process that already holds torch's bundled libnccl reuses it
 // ---------------------------------------------------------------------------------------------
@@ -603,11 +625,9 @@ struct simba_planner {
   simba_planner_config_t cfg{};
   int device = 0;
   RowGeom geom{};
-  std::vector<Tile> tiles;
+  RolloutKernel kernel = RolloutKernel::kF32;
+  std::vector<Tile> tiles;     // the two-tile kernel's work item i is tiles [2i, 2i + 1]
   Tile* d_tiles = nullptr;
-  int tile_rows = 0;
-  int tiles_per_cta = 1;
-  int tc_pair = 0;
   int n_sms = 0;
 
   bool use_pdl = false;        // programmatic dependent launch between rollout and fused update kernels
@@ -726,14 +746,6 @@ extern "C" int simba_planner_create(simba_model_t* model, const simba_planner_co
     return fail(SIMBA_ERR_BAD_CONFIG, "objective %d unknown", cfg->objective);
   if (cfg->precision != SIMBA_PREC_FP32 && cfg->precision != SIMBA_PREC_BF16_TC)
     return fail(SIMBA_ERR_BAD_CONFIG, "precision %d unknown", cfg->precision);
-  if (cfg->precision == SIMBA_PREC_BF16_TC &&
-      !rollout_tc_supported(mc.obs_dim, mc.act_dim, mc.n_layers, mc.units, cfg->horizon) &&
-      !(rollout_tc_wide_supported(mc.obs_dim, mc.act_dim, mc.n_layers, mc.units, cfg->horizon) &&
-        rollout_tc_wide_fits(mc.n_layers, mc.units, cfg->scorer.n_constraints)))
-    return fail(SIMBA_ERR_UNSUPPORTED,
-                "bf16 tcgen05 rollout covers units <= 128 (obs_dim <= 60, obs_dim+act_dim <= 64, <= 5 layers) and "
-                "wide models with 128 < units <= ~416 (less with several constrained lidars; obs_dim+act_dim <= 62); "
-                "use precision fp32 for this shape");
   int rc = validate_scorer(cfg->scorer, mc.obs_dim);
   if (rc != SIMBA_OK) return rc;
   if ((long)cfg->n_states * cfg->particles * cfg->n_samples > 0x7fffffffL / 2)
@@ -748,26 +760,10 @@ extern "C" int simba_planner_create(simba_model_t* model, const simba_planner_co
   rc = build_geom(cfg->n_states, cfg->particles, cfg->n_samples, cfg->world_size, cfg->rank,
                   cfg->horizon, mc.obs_dim, mc.act_dim, mc.ensemble_size, cfg->member_map, p->geom);
   if (rc != SIMBA_OK) { delete p; return rc; }
-  p->tile_rows = cfg->precision == SIMBA_PREC_BF16_TC ? kTcTileRows : kF32TileRows;
-  build_tiles(p->geom, p->tile_rows, p->tiles);
-  if (cfg->precision == SIMBA_PREC_BF16_TC && mc.units <= 128 && p->tiles.size() > 148 &&
-      rollout_tc_two_tiles_fit(mc.n_layers, cfg->scorer.n_constraints)) {
-    // more tiles than SMs: two tiles per CTA so one tile's MMAs overlap the other's epilogue
-    p->tiles_per_cta = 2;
-    build_tiles(p->geom, p->tile_rows, p->tiles, 2);
-    int sms_now = 0;
-    cudaDeviceGetAttribute(&sms_now, cudaDevAttrMultiProcessorCount, p->device);
-    if (getenv("SIMBA_B200_NO_TAIL_SPLIT") == nullptr) split_tail_items(p->tiles, sms_now);
-  }
-  {
-    // few tiles (a single plan): two SMs per tile, the head pass split between them (rollout_tc.cu, PAIR)
-    int sms = 0;
-    cudaDeviceGetAttribute(&sms, cudaDevAttrMultiProcessorCount, p->device);
-    p->n_sms = sms;
-    p->tc_pair = cfg->precision == SIMBA_PREC_BF16_TC && mc.units <= 128 && p->tiles_per_cta == 1 &&
-                 (int)p->tiles.size() * 2 <= sms && rollout_tc_pair_fits(mc.n_layers, cfg->scorer.n_constraints) &&
-                 getenv("SIMBA_B200_NO_PAIR") == nullptr;
-  }
+  ce = cudaDeviceGetAttribute(&p->n_sms, cudaDevAttrMultiProcessorCount, p->device);
+  if (ce != cudaSuccess) { delete p; return fail(SIMBA_ERR_CUDA, "SM count: %s", cudaGetErrorString(ce)); }
+  rc = choose_rollout(mc, *cfg, p->geom, p->n_sms, p->kernel, p->tiles);
+  if (rc != SIMBA_OK) { delete p; return rc; }
 
   p->fused_update = cfg->world_size == 1 && cfg->n_samples <= 1024 && getenv("SIMBA_B200_NO_FUSE") == nullptr;
   p->use_pdl = p->fused_update && cfg->precision == SIMBA_PREC_BF16_TC && getenv("SIMBA_B200_NO_PDL") == nullptr;
@@ -839,6 +835,13 @@ extern "C" int simba_planner_set_external_draws(simba_planner_t* p, const float*
 extern "C" int simba_planner_count_threshold(simba_planner_t* p, int32_t* out) {
   if (!p || !out) return fail(SIMBA_ERR_BAD_CONFIG, "null argument");
   *out = p->c_max;
+  return SIMBA_OK;
+}
+
+extern "C" int simba_planner_rollout_kernel(simba_planner_t* p, int32_t* kernel, int32_t* work_items) {
+  if (!p || !kernel || !work_items) return fail(SIMBA_ERR_BAD_CONFIG, "null argument");
+  *kernel = (int32_t)p->kernel;
+  *work_items = (int32_t)p->tiles.size() / (p->kernel == RolloutKernel::kTcTwoTile ? 2 : 1);
   return SIMBA_OK;
 }
 
@@ -926,8 +929,7 @@ static int do_rollout_score(simba_planner_t* p, const float* states, const float
   prm.objective = p->cfg.objective;
   prm.active = active;
   prm.row_return = row_return; prm.row_costmask = row_costmask; prm.row_costsum = row_costsum;
-  prm.tc_tiles_per_cta = p->tiles_per_cta;
-  prm.tc_pair = p->tc_pair;
+  prm.kernel = p->kernel;
   prm.n_sms = p->n_sms;
   prm.pdl = pdl ? 1 : 0;
 #ifdef SIMBA_TC_TIMELINE
@@ -935,15 +937,11 @@ static int do_rollout_score(simba_planner_t* p, const float* states, const float
   if (const char* tlp = getenv("SIMBA_TC_TIMELINE_PTR"))
     prm.timeline = reinterpret_cast<long long*>(strtoull(tlp, nullptr, 10));
 #endif
-  if (p->cfg.precision == SIMBA_PREC_BF16_TC) {
-    if (p->model->cfg.units <= 128) {
-      CUDA_TRY(launch_rollout_tc(prm, prm.n_tiles, (cudaStream_t)stream));
-    } else {
-      prm.U = rollout_tc_wide_units(p->model->cfg.units);          // zero-padded width
-      CUDA_TRY(launch_rollout_tc_wide(prm, prm.n_tiles, (cudaStream_t)stream));
-    }
-  } else
-    CUDA_TRY(launch_rollout_f32(prm, prm.n_tiles, (cudaStream_t)stream));
+  switch (p->kernel) {
+    case RolloutKernel::kF32: CUDA_TRY(launch_rollout_f32(prm, prm.n_tiles, (cudaStream_t)stream)); break;
+    case RolloutKernel::kTcWide: CUDA_TRY(launch_rollout_tc_wide(prm, prm.n_tiles, (cudaStream_t)stream)); break;
+    default: CUDA_TRY(launch_rollout_tc(prm, prm.n_tiles, (cudaStream_t)stream));
+  }
   return SIMBA_OK;
 }
 

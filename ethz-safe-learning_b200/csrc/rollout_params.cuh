@@ -9,6 +9,15 @@ constexpr int kF32ChunkCols = 128;   // weight chunk = [16 k-rows][128 cols] fp3
 constexpr int kF32ChunkRows = 16;
 constexpr int kTcTileRows = 128;     // rows per tile of the tcgen05 kernel (UMMA_M)
 
+// The rollout kernel a planner launches; simba_planner_rollout_kernel reports it with these values.
+enum class RolloutKernel : int32_t {
+  kF32 = SIMBA_ROLLOUT_FP32,                // rollout_f32.cu, 32-row tiles
+  kTcOneCta = SIMBA_ROLLOUT_TC_ONE_CTA,     // rollout_tc.cu <1,4>: one CTA per 128-row tile
+  kTcPair = SIMBA_ROLLOUT_TC_PAIR,          // <1,4,pair>: a cluster of two CTAs per tile splits the head pass
+  kTcTwoTile = SIMBA_ROLLOUT_TC_TWO_TILE,   // <2,2>: persistent CTAs, two tiles per work item (MMA / epilogue ping-pong)
+  kTcWide = SIMBA_ROLLOUT_TC_WIDE,          // rollout_tc_wide.cu: 128 < units <= ~416
+};
+
 struct RolloutParams {
   RowGeom g;
   simba_scorer_t scorer;
@@ -19,18 +28,16 @@ struct RolloutParams {
   const float* w_f32;
   const float* bias_f32;
   int32_t n_chunks, bias_stride, act_rows;
-  // bf16 image: per member, per layer pre-swizzled UMMA B tiles (see pack_bf16 in api.cu)
+  // bf16 image: per member, per layer pre-swizzled UMMA B tiles (see pack_bf16_image in api.cu)
   const void* w_bf16;
   int64_t w_bf16_member_bytes;
   // wide models (128 < units <= 440): per member the per-step stream of UMMA weight tiles in
   // consumption order, biases in the K padding (see rollout_tc_wide.cu)
   const void* w_wide;
   int64_t w_wide_member_bytes;
-  const void* bias_k16;       // [E][L+1][4096 B] bias K-blocks (see simba_model_commit)
-  const float* bias_tc;       // [E][L+1][128] fp32 (heads: mu bias at [0, O), var bias at [64, 64+O))
-  int32_t tc_tiles_per_cta;   // 1 (latency: small populations) or 2 (MMA / epilogue ping-pong)
+  const void* bias_k16;       // [E][L+1][4096 B] bias K-blocks (see pack_bf16_image in api.cu)
+  RolloutKernel kernel;       // which launch_rollout_* runs and, for rollout_tc.cu, which variant
   int32_t n_sms;              // SMs of the planner's device (grid of the persistent tcgen05 kernels)
-  int32_t tc_pair;            // one-tile variant only: a cluster of two CTAs per tile splits the head pass
   int32_t pdl;                // launch with programmatic stream serialization (fused plan path)
   float tc_scale_a[64];       // bf16 path: x_scaled[k] = fma(x[k], a[k], b[k]); zero beyond O + A
   float tc_scale_b[64];
@@ -38,7 +45,6 @@ struct RolloutParams {
   // where max - min < 1e-5
   const float* smin;
   const float* sdelta;
-  const float* sinv;          // 1 / sdelta (bf16 path multiplies)
   int32_t scale_on;
   // inputs
   const float* states;        // [S, O] (or per row when state_per_row)
@@ -66,11 +72,11 @@ struct RolloutParams {
 
 size_t rollout_f32_smem_bytes(const RolloutParams& prm);
 cudaError_t launch_rollout_f32(const RolloutParams& prm, int n_tiles, cudaStream_t stream);
-cudaError_t launch_rollout_tc(const RolloutParams& prm, int n_tiles, cudaStream_t stream);
+cudaError_t launch_rollout_tc(const RolloutParams& prm, int n_tiles, cudaStream_t stream);   // prm.kernel: kTc{OneCta,Pair,TwoTile}
 bool rollout_tc_supported(int O, int A, int L, int U, int H);
 bool rollout_tc_two_tiles_fit(int L, int n_constraints);
 bool rollout_tc_pair_fits(int L, int n_constraints);
-cudaError_t launch_rollout_tc_wide(const RolloutParams& prm, int n_tiles, cudaStream_t stream);
+cudaError_t launch_rollout_tc_wide(const RolloutParams& prm, int n_tiles, cudaStream_t stream);   // prm.U: the model's units
 bool rollout_tc_wide_supported(int O, int A, int L, int U, int H);
 bool rollout_tc_wide_fits(int L, int U, int n_constraints);
 int rollout_tc_wide_units(int U);                  // U rounded up to a multiple of 16

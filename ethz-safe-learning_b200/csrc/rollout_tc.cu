@@ -798,9 +798,12 @@ static cudaError_t launch_variant(const RolloutParams& prm, int n_tiles, cudaStr
 
 cudaError_t launch_rollout_tc(const RolloutParams& prm, int n_tiles, cudaStream_t stream) {
   if (n_tiles == 0) return cudaSuccess;
-  if (prm.tc_tiles_per_cta == 2) return launch_variant<2, 2, false>(prm, n_tiles, stream);
-  if (prm.tc_pair) return launch_variant<1, 4, true>(prm, n_tiles, stream);
-  return launch_variant<1, 4, false>(prm, n_tiles, stream);
+  switch (prm.kernel) {
+    case RolloutKernel::kTcOneCta: return launch_variant<1, 4, false>(prm, n_tiles, stream);
+    case RolloutKernel::kTcPair: return launch_variant<1, 4, true>(prm, n_tiles, stream);
+    case RolloutKernel::kTcTwoTile: return launch_variant<2, 2, false>(prm, n_tiles, stream);
+    default: return cudaErrorInvalidValue;
+  }
 }
 
 }  // namespace simba

@@ -494,8 +494,10 @@ static size_t wide_smem_bytes(int L, int U, int nparts) {
   return b + 1024;                                                 // alignment slack
 }
 
-cudaError_t launch_rollout_tc_wide(const RolloutParams& prm, int n_tiles, cudaStream_t stream) {
+cudaError_t launch_rollout_tc_wide(const RolloutParams& model_prm, int n_tiles, cudaStream_t stream) {
   if (n_tiles == 0) return cudaSuccess;
+  RolloutParams prm = model_prm;
+  prm.U = rollout_tc_wide_units(prm.U);                            // the kernel runs the zero-padded width
   const size_t smem = wide_smem_bytes(prm.L, prm.U, 1 + prm.scorer.n_constraints);
   // set on every launch: the attribute is per device and per function, and launches happen only at
   // graph capture or in the non-graph entry points, never on the replayed hot path

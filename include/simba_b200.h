@@ -218,6 +218,17 @@ int simba_planner_copy_buffer(simba_planner_t* p, int32_t which, void* dst_devic
 int simba_planner_launches_per_plan(simba_planner_t* p, int32_t* out);
 /* Beta-posterior count threshold c_max used for the safety test (safe_cem_mpc.py:110-120) */
 int simba_planner_count_threshold(simba_planner_t* p, int32_t* out);
+/* the rollout kernel a planner launches, chosen at creation from the shapes, the precision and the
+ * device's SM count */
+typedef enum simba_rollout_kernel {
+  SIMBA_ROLLOUT_FP32 = 0,          /* fp32 SIMT, 32-row tiles                                        */
+  SIMBA_ROLLOUT_TC_ONE_CTA = 1,    /* bf16 tcgen05, one CTA per 128-row tile                         */
+  SIMBA_ROLLOUT_TC_PAIR = 2,       /* bf16 tcgen05, a cluster of two CTAs per tile (at most SMs / 2 tiles) */
+  SIMBA_ROLLOUT_TC_TWO_TILE = 3,   /* bf16 tcgen05, persistent CTAs, two tiles per work item (more tiles than SMs) */
+  SIMBA_ROLLOUT_TC_WIDE = 4        /* bf16 tcgen05 weight-streaming kernel, 128 < units <= ~416      */
+} simba_rollout_kernel;
+/* -> *kernel (simba_rollout_kernel) and *work_items, the number of work items one launch walks */
+int simba_planner_rollout_kernel(simba_planner_t* p, int32_t* kernel, int32_t* work_items);
 
 /* multi-GPU plumbing: the communicator for simba_allgather_scores. unique_id is NCCL's
  * 128-byte ncclUniqueId, produced on rank 0 and broadcast by the caller (torch.distributed). */

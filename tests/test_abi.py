@@ -37,23 +37,31 @@ def test_library_loads_and_exports_every_declared_symbol():
     assert b'sm_100a' in lib.simba_version()
 
 
-def test_header_is_plain_c_and_struct_sizes_match_ctypes():
-    from simba_b200 import _lib
-    prog = r'''
-#include <stdio.h>
-#include "simba_b200.h"
-int main(void) {
-  printf("%zu %zu %zu\n", sizeof(simba_model_config_t), sizeof(simba_scorer_t), sizeof(simba_planner_config_t));
-  return 0;
-}'''
+def _print_from_c(fmt, *args):
+    """Compile and run `printf(fmt, args...)` as a C99 program that includes the header -> the integers printed."""
+    prog = '#include <stdio.h>\n#include "simba_b200.h"\nint main(void) { printf("%s\\n", %s); return 0; }\n' % (
+        fmt, ', '.join(args))
     with tempfile.TemporaryDirectory() as d:
         src = os.path.join(d, 't.c')
         open(src, 'w').write(prog)
         exe = os.path.join(d, 't')
         subprocess.check_call(['gcc', '-std=c99', '-Wall', '-Werror', '-I', os.path.join(ROOT, 'include'),
                                src, '-o', exe])
-        sizes = [int(v) for v in subprocess.check_output([exe]).split()]
+        return [int(v) for v in subprocess.check_output([exe]).split()]
+
+
+def test_header_is_plain_c_and_struct_sizes_match_ctypes():
+    from simba_b200 import _lib
+    sizes = _print_from_c('%zu %zu %zu', 'sizeof(simba_model_config_t)', 'sizeof(simba_scorer_t)',
+                          'sizeof(simba_planner_config_t)')
     assert sizes == [C.sizeof(_lib.ModelConfig), C.sizeof(_lib.Scorer), C.sizeof(_lib.PlannerConfig)]
+
+
+def test_rollout_kernel_constants_match_ctypes():
+    from simba_b200 import _lib
+    names = ('FP32', 'TC_ONE_CTA', 'TC_PAIR', 'TC_TWO_TILE', 'TC_WIDE')
+    values = _print_from_c(' '.join(['%d'] * len(names)), *['(int)SIMBA_ROLLOUT_' + n for n in names])
+    assert values == [getattr(_lib, 'ROLLOUT_' + n) for n in names]
 
 
 def test_no_cpu_fallback_without_gpu():

@@ -1,10 +1,12 @@
 """Kernel variants the host selects by shape, each held to a reference it must equal.
 
-`simba_planner_create` picks the two-tile persistent rollout (and splits its last round) above 148 tiles,
-the two-CTA pair kernel for few tiles, and the trainer picks 4-, 8- or 16-row chain tiles from the batch.
-Production shapes (C4, C3, batches above 128 rows) run these variants; the other tests mostly run the small
-ones. Every test here first restates the host's choice in Python and asserts that the variant it claims to
-test is the one that runs, so no test can pass because the host took a different path.
+`simba_planner_create` picks the two-tile persistent rollout (and splits its last round) when there are more
+tiles than SMs, the two-CTA pair kernel for few tiles, and the trainer picks 4-, 8- or 16-row chain tiles from
+the batch. Production shapes (C4, C3, batches above 128 rows) run these variants; the other tests mostly run the
+small ones. The rollout tests restate the host's choice in Python, which picks shapes without a planner per
+candidate and documents the rule, and ask the library (simba_planner_rollout_kernel) whether the kernel and the
+number of work items they claim to test are the ones it runs, so no test can pass because the host took a
+different path.
 
   A  two-tile rollout (more items than SMs, split tail, padding tiles): per-row outputs bit-identical to
      the same rows through the pair kernel, one state at a time, and with the tail split switched off
@@ -14,6 +16,8 @@ test is the one that runs, so no test can pass because the host took a different
      wrong-counter controls that must come out at least 10x worse
   D  trainer steps with 8- and 16-row chain tiles against oracle/train_oracle.py
 """
+import ctypes as C
+
 import numpy as np
 import pytest
 
@@ -35,28 +39,28 @@ def _sms():
     return torch.cuda.get_device_properties(0).multi_processor_count
 
 
-def _tiles(c, group=1):
+def _tiles(c, group=1, rows=128):
     """build_tiles (csrc/api.cu): each member's S * rows_per_state rows (tf.split map, one rank: P*N/E rows
-    per state) cut into 128-row tiles (kTcTileRows), the run padded with empty tiles to a multiple of
-    `group`. -> [(member, k0, count)]"""
+    per state) cut into 128-row tiles (kTcTileRows; the fp32 kernel: 32), the run padded with empty tiles to
+    a multiple of `group`. -> [(member, k0, count)]"""
     m = c['P'] * c['N'] // c['E']
     tiles = []
     for e in range(c['E']):
         total = c['S'] * m
-        tiles += [(e, k0, min(128, total - k0)) for k0 in range(0, total, 128)]
+        tiles += [(e, k0, min(rows, total - k0)) for k0 in range(0, total, rows)]
         while len(tiles) % group:
             tiles.append((e, 0, 0))
     return tiles
 
 
 def _tc_variant(c, sms, tail_split=True):
-    """simba_planner_create + split_tail_items (csrc/api.cu) for units <= 128 at most four layers (where
+    """choose_rollout + split_tail_items (csrc/api.cu) for units <= 128 at most four layers (where
     rollout_tc_two_tiles_fit and rollout_tc_pair_fits hold with one constrained lidar) -> dict:
     kernel 'two' / 'pair' / 'one', items (work items of the launch), split (the tail split fired),
     pad_in_tail (an empty padding tile sat in the round that was split)."""
     assert c['U'] <= 128 and c['L'] <= 4
     tiles = _tiles(c)
-    if len(tiles) <= 148:
+    if len(tiles) <= sms:
         return dict(kernel='pair' if 2 * len(tiles) <= sms else 'one', items=len(tiles), split=False,
                     pad_in_tail=False)
     tiles = _tiles(c, 2)
@@ -80,8 +84,24 @@ def _pick_S(c, want, start, tail_split=True):
     for S in range(start, start + 96):
         v = _tc_variant(dict(c, S=S), sms, tail_split)
         if want(v):
+            switches = () if tail_split else ('SIMBA_B200_NO_TAIL_SPLIT',)
+            assert _library_choice(dict(c, S=S), switches=switches) == (v['kernel'], v['items']), (S, v)
             return S, v
     pytest.skip("no S in [%d, %d) produces this variant on %d SMs" % (start, start + 96, sms))
+
+
+def _library_choice(c, precision='bf16', switches=()):
+    """simba_planner_rollout_kernel of a fresh planner for c, created with the given diagnostic switches set
+    -> (kernel: 'fp32' / 'one' / 'pair' / 'two' / 'wide', work items of one launch)."""
+    from simba_b200 import _lib
+    names = {_lib.ROLLOUT_FP32: 'fp32', _lib.ROLLOUT_TC_ONE_CTA: 'one', _lib.ROLLOUT_TC_PAIR: 'pair',
+             _lib.ROLLOUT_TC_TWO_TILE: 'two', _lib.ROLLOUT_TC_WIDE: 'wide'}
+    kernel, items = C.c_int32(-1), C.c_int32(-1)
+    with pytest.MonkeyPatch.context() as mp:
+        _set_switches(mp, *switches)
+        pol = helpers.cuda_policy(c, 'penalty', precision=precision)       # owns the planner handle
+        _lib.check(_lib.load().simba_planner_rollout_kernel(pol._ensure_planner(), C.byref(kernel), C.byref(items)))
+    return names[kernel.value], items.value
 
 
 def _chain_tile_rows(E, rows):
@@ -142,6 +162,32 @@ def _assert_rows_close_to_oracle(c, got, acts, eps):
     assert cand.max() < 2e-2
 
 
+# ---- the rollout kernels of the benchmark's shapes -----------------------------------------------------------
+BENCH_SHAPES = {              # (workload, overrides, precision, kernel)
+    'c1': ('c1', dict(), 'bf16', 'pair'),                 # the headline plan: one state, 25 tiles
+    'c1-16-states': ('c1', dict(S=16), 'bf16', 'two'),    # 375 tiles, the last round split
+    'c4': ('c4', dict(), 'bf16', 'two'),                  # 1024 states per call
+    'c5': ('c5', dict(), 'bf16', 'wide'),
+    'c1-fp32': ('c1', dict(), 'fp32', 'fp32'),
+}
+
+
+@pytest.mark.parametrize("shape", list(BENCH_SHAPES))
+def test_benchmark_shapes_run_the_expected_rollout_kernel(shape):
+    cfg, over, precision, kernel = BENCH_SHAPES[shape]
+    c = helpers.workload(cfg, **over)
+    got = _library_choice(c, precision)
+    if kernel == 'fp32':
+        assert got == ('fp32', len(_tiles(c, rows=32)))
+    elif kernel == 'wide':
+        assert got == ('wide', len(_tiles(c)))
+    else:
+        v = _tc_variant(c, _sms())
+        assert v['kernel'] == kernel and got == (kernel, v['items'])
+        if shape == 'c1-16-states':
+            assert v['split'] and got[1] > _library_choice(c, switches=('SIMBA_B200_NO_TAIL_SPLIT',))[1]
+
+
 # ---- A: two-tile persistent rollout, per row, bit for bit ---------------------------------------------------
 CASES_A = {
     # C1 dims: more work items than SMs, and the last round split into single tiles (375 tiles at S = 16)
@@ -162,8 +208,10 @@ def test_two_tile_rollout_rows_equal_pair_kernel_rows(case, monkeypatch):
     S, v = _pick_S(helpers.workload('c1', **over), want, start)
     c = helpers.workload('c1', S=S, **over)
     sms = _sms()
-    assert _tc_variant(dict(c, S=1), sms)['kernel'] == 'pair'
-    assert _tc_variant(c, sms, tail_split=False)['kernel'] == 'two'
+    one, whole = _tc_variant(dict(c, S=1), sms), _tc_variant(c, sms, tail_split=False)
+    assert one['kernel'] == 'pair' and whole['kernel'] == 'two'
+    assert _library_choice(dict(c, S=1)) == ('pair', one['items'])
+    assert _library_choice(c, switches=('SIMBA_B200_NO_TAIL_SPLIT',)) == ('two', whole['items'])
     print("%s: S=%d %s" % (case, S, v))
     B, H, O = c['P'] * c['N'], c['H'], c['O']
     rng = np.random.default_rng(21)
@@ -251,7 +299,10 @@ def test_plans_without_programmatic_dependent_launch_are_bit_identical(cfg, monk
     streaming kernel over three states."""
     c = helpers.workload('c1') if cfg == 'c1' else helpers.workload('tiny', U=400, L=2, S=3)
     if cfg == 'c1':
-        assert _tc_variant(c, _sms())['kernel'] == 'pair'
+        v = _tc_variant(c, _sms())
+        assert v['kernel'] == 'pair' and _library_choice(c) == ('pair', v['items'])
+    else:
+        assert _library_choice(c) == ('wide', len(_tiles(c)))
     base = _plan(c, monkeypatch, seed=SEED64)
     plain = _plan(c, monkeypatch, ('SIMBA_B200_NO_PDL',), seed=SEED64)
     _assert_plans_equal(base, plain)
@@ -264,6 +315,7 @@ def test_wide_batched_plans_equal_per_state_plans(monkeypatch):
     c = helpers.workload('tiny', U=400, L=2, S=3)
     draws = synthetic.make_draws(c['I'], 3, c['N'], c['H'], c['A'], c['P'], c['O'], seed=6)
     tiles = _tiles(c)
+    assert _library_choice(c) == ('wide', len(tiles))
     assert any(k0 // (c['P'] * c['N'] // c['E']) != (k0 + n - 1) // (c['P'] * c['N'] // c['E'])
                for _, k0, n in tiles)                         # a tile holds rows of two states
     base = _plan(c, monkeypatch, draws=draws)
@@ -301,6 +353,9 @@ def _path_workload(path):
         expect = {'pair-latency': 'pair', 'two-tile': 'two'}.get(path, 'one')
         got = 'one' if (v['kernel'] == 'pair' and switches) else v['kernel']
         assert got == expect, (path, v)
+        assert _library_choice(c, switches=switches) == (got, v['items']), (path, v)
+    else:
+        assert _library_choice(c, switches=switches) == ('wide', len(_tiles(c))), path
     assert c['S'] >= 2
     return c, switches
 
