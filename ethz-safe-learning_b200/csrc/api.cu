@@ -100,10 +100,10 @@ struct simba_model {
   float* d_w_f32 = nullptr;
   float* d_bias_f32 = nullptr;
   void* d_w_bf16 = nullptr;
-  void* d_w_wide = nullptr;     // wide-model tcgen05 weight stream (rollout_tc_wide.cu)
+  void* d_w_wide = nullptr;     // weight stream of rollout_tc_wide.cu (of the variant the shape selects)
   int64_t w_wide_member_bytes = 0;
   void* d_bias_k16 = nullptr;   // per member, per layer: UMMA B tile [128 n][16 k] (no swizzle) holding the bias as bf16 hi + lo
-  float tc_scale_a[64] = {0}, tc_scale_b[64] = {0};
+  float tc_scale_a[128] = {0}, tc_scale_b[128] = {0};
   float* d_smin = nullptr;
   float* d_sdelta = nullptr;
   int n_chunks = 0, bias_stride = 0, act_rows = 0;
@@ -315,30 +315,31 @@ static int64_t pack_bf16_image(const simba_model* m, std::vector<uint16_t>& img,
   return member_bytes;
 }
 
-// wide-model tcgen05 weight stream: per member the tiles of one rollout step in consumption order — layer 0:
-// one [UP x 64] tile; layers 1..L-1: KA tiles [UP x 64]; heads: KA tiles [128 x 64] (mu rows [0, O), var rows
-// [64, 64 + O), var pre-scaled by log2(e) as above); each tile K-major SWIZZLE_128B. UP is U zero-padded to a
-// multiple of 16. The bias of a layer sits in k rows KB (hi) and KB + 1 (lo), which the kernel multiplies by
-// constant ones in the A tile. Returns the bytes of one member's stream.
-static int64_t pack_wide_image(const simba_model* m, std::vector<uint16_t>& img) {
+// weight stream of rollout_tc_wide.cu's variant with state width sw (64 or 128): per member the tiles of one
+// rollout step in consumption order — layer 0: sw / 64 tiles [UP x 64]; layers 1..L-1: KA tiles [UP x 64];
+// heads: KA tiles [2 sw x 64] (mu rows [0, O), var rows [sw, sw + O), var pre-scaled by log2(e) as above); each
+// tile K-major SWIZZLE_128B. UP is U zero-padded as rollout_tc_wide_units says. The bias of a layer sits in k
+// rows KB (hi) and KB + 1 (lo), which the kernel multiplies by constant ones in the A tile. Returns the bytes
+// of one member's stream.
+static int64_t pack_wide_image(const simba_model* m, int sw, std::vector<uint16_t>& img) {
   const auto& c = m->cfg;
   const int L = c.n_layers, E = c.ensemble_size, U = c.units, O = c.obs_dim, IN = c.obs_dim + c.act_dim;
-  const int UP = rollout_tc_wide_units(U);
+  const int UP = rollout_tc_wide_units(sw, U);
   const int KA = (UP + 2 + 63) / 64;
-  const int64_t member_bytes = rollout_tc_wide_member_bytes(L, UP);
+  const int64_t member_bytes = rollout_tc_wide_member_bytes(sw, L, UP);
   img.assign((size_t)E * member_bytes / 2, 0);
   for (int e = 0; e < E; ++e) {
     int64_t off = (int64_t)e * member_bytes;
     for (int l = 0; l <= L; ++l) {
       const int K = l == 0 ? IN : U;                     // real input width
       const int KB = l == 0 ? IN : UP;                   // the A tile holds the constant ones at k = KB, KB + 1
-      const int rows = l < L ? UP : 128;                 // tile rows = output features
-      const int tiles = l == 0 ? 1 : KA;
+      const int rows = l < L ? UP : 2 * sw;              // tile rows = output features
+      const int tiles = l == 0 ? sw / 64 : KA;
       auto weight = [&](int k, int n) -> uint16_t {
         int layer = l, col = n;                          // Keras layer index and output column
         if (l == L) {
           if (n < O) { layer = L; col = n; }
-          else if (n >= 64 && n < 64 + O) { layer = L + 1; col = n - 64; }
+          else if (n >= sw && n < sw + O) { layer = L + 1; col = n - sw; }
           else return 0;
         } else if (n >= U) {
           return 0;                                      // padded hidden unit: weights and bias 0
@@ -374,11 +375,17 @@ static std::vector<float> pack_scaler(simba_model* m) {
     delta[k] = d;
     inv[k] = 1.0f / d;
   }
-  for (int k = 0; k < 64; ++k) {
+  for (int k = 0; k < 128; ++k) {
     m->tc_scale_a[k] = k < IN ? (m->scale_on ? inv[k] : 1.0f) : 0.0f;
     m->tc_scale_b[k] = k < IN ? (m->scale_on ? -m->smin[k] * inv[k] : 0.0f) : 0.0f;
   }
   return delta;
+}
+
+// rollout_tc_wide.cu's 128-column variant runs only the bf16 shapes that every other tcgen05 kernel rejects
+static bool wide_obs_selected(int O, int A, int L, int U, int H) {
+  return !rollout_tc_supported(O, A, L, U, H) && !rollout_tc_wide_supported(64, O, A, L, U, H) &&
+         rollout_tc_wide_supported(128, O, A, L, U, H);
 }
 
 extern "C" int simba_model_commit(simba_model_t* m) {
@@ -429,9 +436,11 @@ extern "C" int simba_model_commit(simba_model_t* m) {
     CUDA_TRY(upload(m->d_bias_k16, bias_k16));
   }
   m->w_wide_member_bytes = 0;
-  if (rollout_tc_wide_supported(O, c.act_dim, L, U, 1)) {
+  const int wide_sw = rollout_tc_wide_supported(64, O, c.act_dim, L, U, 1) ? 64
+                      : wide_obs_selected(O, c.act_dim, L, U, 1)            ? 128 : 0;
+  if (wide_sw != 0) {
     std::vector<uint16_t> img;
-    m->w_wide_member_bytes = pack_wide_image(m, img);
+    m->w_wide_member_bytes = pack_wide_image(m, wide_sw, img);
     CUDA_TRY(upload(m->d_w_wide, img));
   }
   CUDA_TRY(upload(m->d_smin, m->smin));
@@ -555,13 +564,19 @@ static int choose_rollout(const simba_model_config_t& mc, const simba_planner_co
     }
     return SIMBA_OK;
   }
-  if (rollout_tc_wide_supported(O, A, L, U, H) && rollout_tc_wide_fits(L, U, nc)) {
+  if (rollout_tc_wide_supported(64, O, A, L, U, H) && rollout_tc_wide_fits(64, L, U, nc)) {
     kernel = RolloutKernel::kTcWide;
     return SIMBA_OK;
   }
+  if (wide_obs_selected(O, A, L, U, H) && rollout_tc_wide_fits(128, L, U, nc)) {
+    kernel = RolloutKernel::kTcWideObs;
+    return SIMBA_OK;
+  }
   return fail(SIMBA_ERR_UNSUPPORTED,
-              "bf16 tcgen05 rollout covers units <= 128 (obs_dim <= 60, obs_dim+act_dim <= 64, <= 5 layers) and "
-              "wide models with 128 < units <= ~416 (less with several constrained lidars; obs_dim+act_dim <= 62); "
+              "bf16 tcgen05 rollout covers units <= 128 (obs_dim <= 60, obs_dim+act_dim <= 64, <= 5 layers), "
+              "wide models with 128 < units <= ~416 (less with several constrained lidars; obs_dim+act_dim <= 62) "
+              "and, for other shapes, obs_dim+act_dim <= 126 with obs_dim <= 124, act_dim <= 4, units <= 384 and "
+              "<= 6 layers; "
               "use precision fp32 for this shape");
 }
 
@@ -939,7 +954,8 @@ static int do_rollout_score(simba_planner_t* p, const float* states, const float
 #endif
   switch (p->kernel) {
     case RolloutKernel::kF32: CUDA_TRY(launch_rollout_f32(prm, prm.n_tiles, (cudaStream_t)stream)); break;
-    case RolloutKernel::kTcWide: CUDA_TRY(launch_rollout_tc_wide(prm, prm.n_tiles, (cudaStream_t)stream)); break;
+    case RolloutKernel::kTcWide:
+    case RolloutKernel::kTcWideObs: CUDA_TRY(launch_rollout_tc_wide(prm, prm.n_tiles, (cudaStream_t)stream)); break;
     default: CUDA_TRY(launch_rollout_tc(prm, prm.n_tiles, (cudaStream_t)stream));
   }
   return SIMBA_OK;

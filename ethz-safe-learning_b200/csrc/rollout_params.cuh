@@ -15,7 +15,8 @@ enum class RolloutKernel : int32_t {
   kTcOneCta = SIMBA_ROLLOUT_TC_ONE_CTA,     // rollout_tc.cu <1,4>: one CTA per 128-row tile
   kTcPair = SIMBA_ROLLOUT_TC_PAIR,          // <1,4,pair>: a cluster of two CTAs per tile splits the head pass
   kTcTwoTile = SIMBA_ROLLOUT_TC_TWO_TILE,   // <2,2>: persistent CTAs, two tiles per work item (MMA / epilogue ping-pong)
-  kTcWide = SIMBA_ROLLOUT_TC_WIDE,          // rollout_tc_wide.cu: 128 < units <= ~416
+  kTcWide = SIMBA_ROLLOUT_TC_WIDE,          // rollout_tc_wide.cu <64>: 128 < units <= ~416
+  kTcWideObs = SIMBA_ROLLOUT_TC_WIDE_OBS,   // rollout_tc_wide.cu <128>: obs_dim + act_dim + 2 <= 128, obs_dim <= 124, units <= 384
 };
 
 struct RolloutParams {
@@ -31,16 +32,16 @@ struct RolloutParams {
   // bf16 image: per member, per layer pre-swizzled UMMA B tiles (see pack_bf16_image in api.cu)
   const void* w_bf16;
   int64_t w_bf16_member_bytes;
-  // wide models (128 < units <= 440): per member the per-step stream of UMMA weight tiles in
-  // consumption order, biases in the K padding (see rollout_tc_wide.cu)
+  // wide models (128 < units <= 440) and wide observations: per member the per-step stream of UMMA
+  // weight tiles in consumption order, biases in the K padding (see rollout_tc_wide.cu)
   const void* w_wide;
   int64_t w_wide_member_bytes;
   const void* bias_k16;       // [E][L+1][4096 B] bias K-blocks (see pack_bf16_image in api.cu)
   RolloutKernel kernel;       // which launch_rollout_* runs and, for rollout_tc.cu, which variant
   int32_t n_sms;              // SMs of the planner's device (grid of the persistent tcgen05 kernels)
   int32_t pdl;                // launch with programmatic stream serialization (fused plan path)
-  float tc_scale_a[64];       // bf16 path: x_scaled[k] = fma(x[k], a[k], b[k]); zero beyond O + A
-  float tc_scale_b[64];
+  float tc_scale_a[128];      // bf16 path: x_scaled[k] = fma(x[k], a[k], b[k]); zero beyond O + A
+  float tc_scale_b[128];
   // scaler (transition_model.py:79-87): x_scaled = (x - smin) / sdelta, sdelta already holds 1.01
   // where max - min < 1e-5
   const float* smin;
@@ -76,10 +77,11 @@ cudaError_t launch_rollout_tc(const RolloutParams& prm, int n_tiles, cudaStream_
 bool rollout_tc_supported(int O, int A, int L, int U, int H);
 bool rollout_tc_two_tiles_fit(int L, int n_constraints);
 bool rollout_tc_pair_fits(int L, int n_constraints);
+// The weight-streaming kernel comes in two state widths `sw`: 64 (prm.kernel kTcWide) and 128 (kTcWideObs).
 cudaError_t launch_rollout_tc_wide(const RolloutParams& prm, int n_tiles, cudaStream_t stream);   // prm.U: the model's units
-bool rollout_tc_wide_supported(int O, int A, int L, int U, int H);
-bool rollout_tc_wide_fits(int L, int U, int n_constraints);
-int rollout_tc_wide_units(int U);                  // U rounded up to a multiple of 16
-int64_t rollout_tc_wide_member_bytes(int L, int U);   // U = padded units
+bool rollout_tc_wide_supported(int sw, int O, int A, int L, int U, int H);
+bool rollout_tc_wide_fits(int sw, int L, int U, int n_constraints);
+int rollout_tc_wide_units(int sw, int U);                     // the padded width the kernel runs
+int64_t rollout_tc_wide_member_bytes(int sw, int L, int UP);   // UP = padded units
 
 }  // namespace simba

@@ -24,6 +24,16 @@
 //   * biases ride in the K padding: the A tile holds constant ones at k = K_real, K_real + 1 and
 //     the weight tiles hold bf16(b) and bf16(b - hi) in those two k rows, so no epilogue touches
 //     a bias (K_real = 62 -> 64 for layer 0, 400 -> 448 for the others).
+//
+// The state width kSW is a template parameter. kSW = 64 is the wide-model kernel described above (TMEM
+// state columns [448, 512), heads N = 128: mu in rows [0, O), raw var in rows [64, 64 + O)). kSW = 128
+// runs observations up to obs_dim + act_dim + 2 = 128 for any hidden width up to 384: layer 0 spans two
+// K atoms, the state sits in TMEM columns [384, 512), the heads are one N = 256 MMA per K-step (mu in rows
+// [0, O), raw var in rows [128, 128 + O)) and each epilogue thread owns 32 outputs (4 Philox blocks per
+// step; obs_dim <= 124, so that the four action columns at O stay inside the state). Its hidden widths are padded
+// to at least 128, so the hidden layers' constant ones (k = U, U + 1)
+// lie beyond the layer-0 input that the head pass rewrites every step (k < 128).
+#include <algorithm>
 #include <cstdlib>
 #include <type_traits>
 
@@ -54,41 +64,56 @@ constexpr int kWideThreads = kEpiThreads + 64;   // + producer warp + MMA warp
 constexpr int kAtomBytes = 128 * 128;         // one 64-wide K atom of a 128-row tile (bf16, SW128)
 constexpr int kStages = 2;
 constexpr int kBarEpi = 1, kBarAcc = 2, kBarA = 3, kBarScore = 4;   // named barrier ids
-constexpr int kStateCol = 448;                // TMEM: accumulator columns [0, units), state [448, 512)
 constexpr int kTmemCols = 512;
-constexpr int OW = 64 / kQ;                   // head outputs / state dims / layer-0 K elements per thread
-constexpr int NB = OW / 8;                    // Philox blocks / 8-wide chunks per thread and step
 
-constexpr int kHeadGroup = 3;                 // head K-blocks (16 KB each) fetched per TMA tile
+// Layout constants of the variant with state width kSW (64 or 128)
+template <int kSW>
+struct WideCfg {
+  static constexpr int kStateCol = kTmemCols - kSW;   // TMEM: accumulator columns [0, units), state [kStateCol, 512)
+  static constexpr int OW = kSW / kQ;                 // head outputs / state dims / layer-0 K elements per thread
+  static constexpr int NB = OW / 8;                   // Philox blocks / 8-wide chunks per thread and step
+  static constexpr int kL0Atoms = kSW / 64;           // K-blocks of layer 0
+  static constexpr int kHeadN = 2 * kSW;              // head rows: mu at [0, O), raw var at [kSW, kSW + O)
+  // head K-blocks ([kHeadN x 64] bf16: 16 or 32 KB) fetched per TMA tile. At kSW = 128 a block alone is as
+  // large as three of the narrow variant's, and two per stage would not leave room for a 320-unit A tile.
+  static constexpr int kHeadGroup = kSW == 64 ? 3 : 1;
+  static constexpr int kMinUnits = kSW == 64 ? 0 : 128;   // see the file comment
+  static constexpr int kMaxUnits = kSW == 64 ? 448 - 2 : kStateCol;
+};
 
 struct WideShape {
   int U, KA, L;
   uint32_t hid_tile_bytes;      // [U x 64] bf16
-  uint32_t head_tile_bytes;     // [128 x 64] bf16 (one K-block; kHeadGroup of them travel together)
+  uint32_t head_tile_bytes;     // [kHeadN x 64] bf16 (one K-block; kHeadGroup of them travel together)
   int head_tiles;               // ceil(KA / kHeadGroup)
   int tiles_per_step;
 };
 
+template <int kSW>
 __host__ __device__ inline WideShape wide_shape(int U, int L) {
+  using C = WideCfg<kSW>;
   WideShape s;
   s.U = U; s.L = L;
   s.KA = (U + 2 + 63) / 64;
   s.hid_tile_bytes = (uint32_t)U * 128u;
-  s.head_tile_bytes = 128u * 128u;
-  s.head_tiles = (s.KA + kHeadGroup - 1) / kHeadGroup;
-  s.tiles_per_step = 1 + (L - 1) * s.KA + s.head_tiles;
+  s.head_tile_bytes = (uint32_t)C::kHeadN * 128u;
+  s.head_tiles = (s.KA + C::kHeadGroup - 1) / C::kHeadGroup;
+  s.tiles_per_step = C::kL0Atoms + (L - 1) * s.KA + s.head_tiles;
   return s;
 }
 
+template <int kSW>
 __host__ __device__ inline uint32_t wide_stage_bytes(const WideShape& s) {
-  const uint32_t head = (uint32_t)kHeadGroup * s.head_tile_bytes;
+  const uint32_t head = (uint32_t)WideCfg<kSW>::kHeadGroup * s.head_tile_bytes;
   const uint32_t big = s.hid_tile_bytes > head ? s.hid_tile_bytes : head;
   return (big + 1023u) & ~1023u;
 }
 
 // source offset / size of tile `i` of the per-step stream
+template <int kSW>
 __device__ __forceinline__ void wide_tile(const WideShape& s, int i, uint32_t& off, uint32_t& bytes) {
-  const int n_hid = 1 + (s.L - 1) * s.KA;
+  constexpr int kHeadGroup = WideCfg<kSW>::kHeadGroup;
+  const int n_hid = WideCfg<kSW>::kL0Atoms + (s.L - 1) * s.KA;
   if (i < n_hid) { off = (uint32_t)i * s.hid_tile_bytes; bytes = s.hid_tile_bytes; return; }
   // the heads' K-blocks are small (16 KB), so kHeadGroup consecutive ones travel as one tile: with
   // one block per tile the two-stage ring was latency-bound there (4.9 k cycles for 2.6 k of MMAs)
@@ -104,24 +129,27 @@ struct TileInfoW {
 
 }  // namespace
 
+template <int kSW>
 __global__ void __launch_bounds__(kWideThreads, 1) rollout_tc_wide_kernel(const RolloutParams prm) {
+  using C = WideCfg<kSW>;
+  constexpr int kStateCol = C::kStateCol, OW = C::OW, NB = C::NB, kHeadGroup = C::kHeadGroup;
   extern __shared__ __align__(1024) uint8_t smem_raw[];
   const RowGeom& g = prm.g;
   const int L = prm.L, U = prm.U;
   const int H = g.H;
   const int O = g.O, A = g.A;
   const int warp = threadIdx.x >> 5, lane = threadIdx.x & 31;
-  const WideShape ws = wide_shape(U, L);
+  const WideShape ws = wide_shape<kSW>(U, L);
   const int KA = ws.KA;
 
   // ---- shared memory carve-up (base is 1024-aligned: required by SWIZZLE_128B) -------------------
   uint8_t* a_smem = smem_raw;                                              // [KA][128 x 64] bf16 SW128
   uint8_t* b_smem = a_smem + (size_t)KA * kAtomBytes;                      // [kStages][U x 64] bf16 SW128
-  const uint32_t stage_bytes = wide_stage_bytes(ws);
-  float* scale_smem = reinterpret_cast<float*>(b_smem + (size_t)kStages * stage_bytes);   // [2][64]
-  float* pen_smem = scale_smem + 128;                                      // [kParts][64]
+  const uint32_t stage_bytes = wide_stage_bytes<kSW>(ws);
+  float* scale_smem = reinterpret_cast<float*>(b_smem + (size_t)kStages * stage_bytes);   // [2][kSW]
+  float* pen_smem = scale_smem + 2 * kSW;                                  // [kParts][kSW]
   const int nparts = 1 + prm.scorer.n_constraints;
-  float* part_smem = pen_smem + kHeadParts * 64;                               // [kQ][nparts][128]
+  float* part_smem = pen_smem + kHeadParts * kSW;                              // [kQ][nparts][128]
   // running objective of every rollout row (RowScore fields, field-major), see rollout_tc.cu
   uint32_t* rs_smem = reinterpret_cast<uint32_t*>(part_smem + kQ * nparts * 128);   // [8][128]
   uint64_t* bars = reinterpret_cast<uint64_t*>(rs_smem + 8 * 128);
@@ -175,7 +203,7 @@ __global__ void __launch_bounds__(kWideThreads, 1) rollout_tc_wide_kernel(const 
           const int s = i % kStages;
           if (i >= kStages) mbar_wait(bar_empty[s], ((i / kStages) - 1) & 1);
           uint32_t off, bytes;
-          wide_tile(ws, in_step, off, bytes);
+          wide_tile<kSW>(ws, in_step, off, bytes);
           mbar_expect_tx(bar_full[s], bytes);
           bulk_g2s(smem_u32(b_smem + (size_t)s * stage_bytes), wsrc + off, bytes, bar_full[s]);
           if (++in_step == ws.tiles_per_step) in_step = 0;
@@ -185,7 +213,7 @@ __global__ void __launch_bounds__(kWideThreads, 1) rollout_tc_wide_kernel(const 
       // ===================== MMA warp: one elected thread issues every tcgen05.mma ================
       const int N1 = ((U / 2 + 15) / 16) * 16, N2 = U - N1;        // two N halves, multiples of 16
       const uint32_t idesc1 = umma_idesc_n((uint32_t)N1), idesc2 = umma_idesc_n((uint32_t)N2);
-      const uint32_t idesc_head = umma_idesc_n(128u);
+      const uint32_t idesc_head = umma_idesc_n((uint32_t)C::kHeadN);
       const uint32_t a_base = smem_u32(a_smem);
       int tile0 = 0;                                               // ring position at the start of the layer
       uint32_t acc_ph = 0;
@@ -193,11 +221,11 @@ __global__ void __launch_bounds__(kWideThreads, 1) rollout_tc_wide_kernel(const 
         for (int layer = 0; layer <= L; ++layer) {
           named_bar_sync<kEpiThreads + 32>(kBarA);                 // this layer's A tile is complete
           tc_fence_after();
-          const int n_tiles_layer = layer < L ? (layer == 0 ? 1 : KA) : ws.head_tiles;
+          const int n_tiles_layer = layer < L ? (layer == 0 ? C::kL0Atoms : KA) : ws.head_tiles;
           if (elect_one()) {
             int tile = tile0;                                      // running index into the ring
             if (layer < L) {
-              const int kblocks = layer == 0 ? 1 : KA;
+              const int kblocks = layer == 0 ? C::kL0Atoms : KA;
               for (int kb = 0; kb < kblocks; ++kb, ++tile) {
                 const int s = tile % kStages;
                 mbar_wait(bar_full[s], (tile / kStages) & 1);
@@ -250,8 +278,8 @@ __global__ void __launch_bounds__(kWideThreads, 1) rollout_tc_wide_kernel(const 
       const int r = (wl & 3) * 32 + lane;                   // row in tile == TMEM lane
       // scaler / penalty tables, zeroed A tile with the constant ones of the bias rows
       {
-        head_tables_init(scale_smem, pen_smem, prm.tc_scale_a, prm.tc_scale_b, prm.scorer, O + A, threadIdx.x,
-                         kEpiThreads);
+        head_tables_init<kSW>(scale_smem, pen_smem, prm.tc_scale_a, prm.tc_scale_b, prm.scorer, O + A, threadIdx.x,
+                              kEpiThreads);
         uint32_t* a32 = reinterpret_cast<uint32_t*>(a_smem);
         for (int i = threadIdx.x; i < KA * kAtomBytes / 4; i += kEpiThreads) a32[i] = 0u;
         named_bar_sync<kEpiThreads>(kBarEpi);
@@ -292,11 +320,14 @@ __global__ void __launch_bounds__(kWideThreads, 1) rollout_tc_wide_kernel(const 
       auto a_chunk = [&](int c8) -> uint32_t {
         return a_row + (uint32_t)(c8 >> 3) * kAtomBytes + ((((uint32_t)c8 & 7u) ^ rsw) << 4);
       };
-      // A operand in shared memory: K elements [k0, k0 + 8) of this thread's row = one 16-byte chunk of atom 0
+      // A operand in shared memory: K elements [k0, k0 + 8) of this thread's row = one 16-byte chunk of the
+      // layer-0 input (atom 0, and atom 1 for k0 >= 64 at kSW = 128)
       struct AStoreSmem {
         uint32_t a_row, rsw;
         __device__ __forceinline__ void store8(int k0, uint32_t p0, uint32_t p1, uint32_t p2, uint32_t p3) const {
-          st_shared_v4(a_row + ((((uint32_t)(k0 >> 3) & 7u) ^ rsw) << 4), p0, p1, p2, p3);
+          uint32_t a = a_row + ((((uint32_t)(k0 >> 3) & 7u) ^ rsw) << 4);
+          if (C::kL0Atoms > 1) a += (uint32_t)(k0 >> 6) * kAtomBytes;
+          st_shared_v4(a, p0, p1, p2, p3);
         }
       };
       const AStoreSmem astore{a_row, rsw};
@@ -312,9 +343,13 @@ __global__ void __launch_bounds__(kWideThreads, 1) rollout_tc_wide_kernel(const 
       };
 
       const bool owns_actions = (O >= hc.o_base) && (O < hc.o_base + OW);
+      // a_0 goes into the state columns [O, O + A) of whichever slices hold them (head_first_pass); at kSW = 128
+      // they may straddle two slices (O = 63, A = 2), so every thread whose slice meets them fetches a_0. Later
+      // actions come from the owner alone (head_store_actions writes all four columns).
+      const bool needs_a0 = kSW == 64 ? owns_actions : (O < hc.o_base + OW) && (O + A > hc.o_base);
       float act_pf[4] = {0.f, 0.f, 0.f, 0.f};
-      auto prefetch_actions = [&](int tn) {
-        if (owns_actions && row_ok && tn < H) {
+      auto prefetch_actions = [&](int tn, bool mine) {
+        if (mine && row_ok && tn < H) {
 #pragma unroll
           for (int a = 0; a < 4; ++a)
             if (a < A) act_pf[a] = act_ptr[tn * A + a];
@@ -353,9 +388,9 @@ __global__ void __launch_bounds__(kWideThreads, 1) rollout_tc_wide_kernel(const 
       };
 
       uint32_t* my_rs = rs_smem + r;                      // cum, costsum, cmask lo / hi, dist, cost, done
-      prefetch_actions(0);
-      head_first_pass<OW>(hc, astore, s0_ptr, row_ok, act_pf);
-      prefetch_actions(1);
+      prefetch_actions(0, needs_a0);
+      head_first_pass<OW, kSW>(hc, astore, s0_ptr, row_ok, act_pf);
+      prefetch_actions(1, owns_actions);
       tmem_st_wait();
       publish_a();                                       // layer-0 input of step 0
       named_bar_sync<kEpiThreads>(kBarScore);            // partial minima of s_0 visible to the scorers
@@ -381,7 +416,7 @@ __global__ void __launch_bounds__(kWideThreads, 1) rollout_tc_wide_kernel(const 
 #endif
         TLW(0);
         if (owns_actions) head_store_actions(hc, act_pf);   // a_{t+1}, fetched during step t - 1
-        prefetch_actions(t + 2);
+        prefetch_actions(t + 2, owns_actions);
         // ---- hidden layers: TMEM -> ReLU -> bf16 -> swizzled A tile (bias is in the accumulator) ----
         for (int l = 0; l < L; ++l) {
           wait_accumulator();
@@ -412,16 +447,25 @@ __global__ void __launch_bounds__(kWideThreads, 1) rollout_tc_wide_kernel(const 
           publish_a();
           TLW(3 + l * 4);
           if (prm.sampling_propagation) {
-            // the NB = 2 Philox blocks of the step ride in the shadow of the first two hidden layers' MMAs
+            // the NB (2 or 4) Philox blocks of the step ride in the shadow of the hidden layers' MMAs: block b
+            // after layer b, the blocks beyond the last layer after that one
             if (l == 0) make_noise(std::integral_constant<int, 0>{}, t);
             if (l == (L > 1 ? 1 : 0)) make_noise(std::integral_constant<int, 1>{}, t);
+            if constexpr (NB > 2) {
+              if (l == (L > 2 ? 2 : L - 1)) make_noise(std::integral_constant<int, 2>{}, t);
+              if (l == (L > 3 ? 3 : L - 1)) make_noise(std::integral_constant<int, 3>{}, t);
+            }
           }
         }
         // ---- Gaussian heads + state update + next input + partial minima (tc_head.cuh) -----------------
         wait_accumulator();
         TLW(40);
-        if (prm.sampling_propagation) head_step_pass<OW, true>(hc, noise, astore, t + 1 < H);
-        else head_step_pass<OW, false>(hc, noise, astore, t + 1 < H);
+        if constexpr (kSW == 128) {
+          // 96 registers: re-derive the slice predicates every step instead of holding them (no spills)
+          asm volatile("mov.b32 %0, %0;" : "+r"(hc.slice_bits));
+        }
+        if (prm.sampling_propagation) head_step_pass<OW, true, kSW, kSW>(hc, noise, astore, t + 1 < H);
+        else head_step_pass<OW, false, kSW, kSW>(hc, noise, astore, t + 1 < H);
         TLW(41);
         tmem_st_wait();
         if (t + 1 < H) publish_a();
@@ -462,47 +506,59 @@ __global__ void __launch_bounds__(kWideThreads, 1) rollout_tc_wide_kernel(const 
 }
 
 // ---- host side ------------------------------------------------------------------------------------
-static size_t wide_smem_bytes(int L, int U, int nparts);
-
-// widths that are not a multiple of 16 run zero-padded to the next one (rollout_tc_wide_units)
-int rollout_tc_wide_units(int U) { return (U + 15) / 16 * 16; }
-
-// shape check used when the weight images are packed (no scorer yet: one constraint slot assumed)
-bool rollout_tc_wide_supported(int O, int A, int L, int U, int H) {
-  return U > 128 && rollout_tc_wide_units(U) <= 448 - 2 && O >= 1 && O <= 60 && O + A + 2 <= 64 && A <= 4 &&
-         L >= 1 && L <= 6 && H >= 1 && H <= 64 && wide_smem_bytes(L, rollout_tc_wide_units(U), 1) <= 227 * 1024;
-}
-
-// the A tile, the two-stage weight ring and the per-constraint exchange buffers must share 227 KB
-bool rollout_tc_wide_fits(int L, int U, int n_constraints) {
-  return wide_smem_bytes(L, rollout_tc_wide_units(U), 1 + n_constraints) <= 227 * 1024;
-}
-
-int64_t rollout_tc_wide_member_bytes(int L, int U) {
-  const WideShape ws = wide_shape(U, L);
-  return (int64_t)(1 + (L - 1) * ws.KA) * ws.hid_tile_bytes + (int64_t)ws.KA * ws.head_tile_bytes;
-}
-
+template <int kSW>
 static size_t wide_smem_bytes(int L, int U, int nparts) {
-  const WideShape ws = wide_shape(U, L);
+  const WideShape ws = wide_shape<kSW>(U, L);
   size_t b = (size_t)ws.KA * kAtomBytes;
-  b += (size_t)kStages * wide_stage_bytes(ws);
-  b += 128 * sizeof(float) + kHeadParts * 64 * sizeof(float);
+  b += (size_t)kStages * wide_stage_bytes<kSW>(ws);
+  b += 2 * kSW * sizeof(float) + kHeadParts * kSW * sizeof(float);
   b += (size_t)kQ * nparts * 128 * sizeof(float);
   b += (size_t)8 * 128 * sizeof(uint32_t);                          // per-row running objective
   b += 6 * sizeof(uint64_t) + 2 * sizeof(uint32_t) + sizeof(TileInfoW);
   return b + 1024;                                                 // alignment slack
 }
 
-cudaError_t launch_rollout_tc_wide(const RolloutParams& model_prm, int n_tiles, cudaStream_t stream) {
-  if (n_tiles == 0) return cudaSuccess;
+static size_t wide_smem_bytes(int sw, int L, int UP, int nparts) {
+  return sw == 64 ? wide_smem_bytes<64>(L, UP, nparts) : wide_smem_bytes<128>(L, UP, nparts);
+}
+
+// widths that are not a multiple of 16 run zero-padded to the next one; the 128-column variant pads to at
+// least 128 (file comment)
+int rollout_tc_wide_units(int sw, int U) {
+  const int UP = (U + 15) / 16 * 16;
+  return sw == 64 ? UP : std::max(UP, WideCfg<128>::kMinUnits);
+}
+
+// shape check used when the weight images are packed (no scorer yet: one constraint slot assumed). The layer-0
+// input needs O + A + 2 K elements; head_store_actions writes four state columns from O, so O + 4 <= kSW as well
+// (the <64> variant's O <= 60 implies it).
+bool rollout_tc_wide_supported(int sw, int O, int A, int L, int U, int H) {
+  const int UP = rollout_tc_wide_units(sw, U);
+  const bool shape = sw == 64 ? U > 128 && UP <= WideCfg<64>::kMaxUnits && O <= 60 && O + A + 2 <= 64
+                              : UP <= WideCfg<128>::kMaxUnits && O + A + 2 <= 128 && O + 4 <= 128;
+  return shape && O >= 1 && A <= 4 && L >= 1 && L <= 6 && H >= 1 && H <= 64 &&
+         wide_smem_bytes(sw, L, UP, 1) <= 227 * 1024;
+}
+
+// the A tile, the two-stage weight ring and the per-constraint exchange buffers must share 227 KB
+bool rollout_tc_wide_fits(int sw, int L, int U, int n_constraints) {
+  return wide_smem_bytes(sw, L, rollout_tc_wide_units(sw, U), 1 + n_constraints) <= 227 * 1024;
+}
+
+int64_t rollout_tc_wide_member_bytes(int sw, int L, int UP) {
+  const WideShape ws = sw == 64 ? wide_shape<64>(UP, L) : wide_shape<128>(UP, L);
+  return (int64_t)(ws.tiles_per_step - ws.head_tiles) * ws.hid_tile_bytes + (int64_t)ws.KA * ws.head_tile_bytes;
+}
+
+template <int kSW>
+static cudaError_t launch_wide(const RolloutParams& model_prm, int n_tiles, cudaStream_t stream) {
   RolloutParams prm = model_prm;
-  prm.U = rollout_tc_wide_units(prm.U);                            // the kernel runs the zero-padded width
-  const size_t smem = wide_smem_bytes(prm.L, prm.U, 1 + prm.scorer.n_constraints);
+  prm.U = rollout_tc_wide_units(kSW, prm.U);                       // the kernel runs the zero-padded width
+  const size_t smem = wide_smem_bytes<kSW>(prm.L, prm.U, 1 + prm.scorer.n_constraints);
   // set on every launch: the attribute is per device and per function, and launches happen only at
   // graph capture or in the non-graph entry points, never on the replayed hot path
   {
-    cudaError_t e = cudaFuncSetAttribute(rollout_tc_wide_kernel, cudaFuncAttributeMaxDynamicSharedMemorySize,
+    cudaError_t e = cudaFuncSetAttribute(rollout_tc_wide_kernel<kSW>, cudaFuncAttributeMaxDynamicSharedMemorySize,
                                          (int)smem);
     if (e != cudaSuccess) return e;
   }
@@ -516,7 +572,16 @@ cudaError_t launch_rollout_tc_wide(const RolloutParams& model_prm, int n_tiles, 
   attr[0].val.programmaticStreamSerializationAllowed = 1;
   cfg.attrs = attr;
   cfg.numAttrs = prm.pdl ? 1 : 0;
-  return cudaLaunchKernelEx(&cfg, rollout_tc_wide_kernel, prm);
+  return cudaLaunchKernelEx(&cfg, rollout_tc_wide_kernel<kSW>, prm);
+}
+
+cudaError_t launch_rollout_tc_wide(const RolloutParams& prm, int n_tiles, cudaStream_t stream) {
+  if (n_tiles == 0) return cudaSuccess;
+  switch (prm.kernel) {
+    case RolloutKernel::kTcWide: return launch_wide<64>(prm, n_tiles, stream);
+    case RolloutKernel::kTcWideObs: return launch_wide<128>(prm, n_tiles, stream);
+    default: return cudaErrorInvalidValue;
+  }
 }
 
 }  // namespace simba

@@ -88,17 +88,20 @@ __device__ __forceinline__ uint4 external_noise8_bf16(const float* ep, int o0, i
 //                             1 that multiplies the bias rows riding in the K padding of layer 0
 //   pen[p][o]: 0 where state dim o belongs to part p's lidar slice, +inf elsewhere, so that
 //              min_o (s[o] + pen[p][o]) is the slice minimum (part 0: goal lidar or the goal_dist dim)
+// Both tables are kTW entries wide per row: the kernel's state width (64, or 128 for rollout_tc_wide.cu's
+// wide-observation variant); sa / sb hold at least kTW entries.
+template <int kTW = 64>
 __device__ __forceinline__ void head_tables_init(float* scale_smem, float* pen_smem, const float* sa,
                                                  const float* sb, const simba_scorer_t& sc, int ones_at,
                                                  int tid, int nthreads) {
-  for (int i = tid; i < 64; i += nthreads) {
+  for (int i = tid; i < kTW; i += nthreads) {
     const bool one = ones_at >= 0 && (i == ones_at || i == ones_at + 1);
     scale_smem[i] = one ? 0.0f : sa[i];
-    scale_smem[64 + i] = one ? 1.0f : sb[i];
+    scale_smem[kTW + i] = one ? 1.0f : sb[i];
     const bool in_goal = sc.goal_dist_index >= 0 ? (i == sc.goal_dist_index) : (i >= sc.goal_begin && i < sc.goal_end);
     pen_smem[i] = in_goal ? 0.0f : INFINITY;
     for (int q = 0; q < SIMBA_MAX_CONSTRAINTS; ++q)
-      pen_smem[(1 + q) * 64 + i] =
+      pen_smem[(1 + q) * kTW + i] =
           (q < sc.n_constraints && i >= sc.con_begin[q] && i < sc.con_end[q]) ? 0.0f : INFINITY;
   }
 }
@@ -120,13 +123,14 @@ __device__ __forceinline__ uint32_t head_slice_bits(const simba_scorer_t& sc, in
 }
 
 struct HeadCtx {
-  uint32_t t_acc;        // TMEM address of this row's head accumulators: mu at + o, raw var at + 64 + o
+  uint32_t t_acc;        // TMEM address of this row's head accumulators: mu at + o, raw var at + kVar + o
+                         // (kVar = the head stride of head_step_pass: 64, or 128 for wide observations)
   uint32_t t_state;      // TMEM address of this row's fp32 state columns
   int o_base;            // first output / state dim of this thread
   int O, A;
   uint32_t slice_bits;   // head_slice_bits
   int n_constraints;
-  const float* scale_smem;
+  const float* scale_smem;   // head_tables_init tables, kTW entries per row
   const float* pen_smem;
   float* part;           // this thread's slot of the partial-minima exchange: part p at part[p * 128]
   // two-CTA variant of rollout_tc.cu, CTA 1: the slot lives in CTA 0 (shared::cluster address of part p = 0,
@@ -160,7 +164,7 @@ __device__ __forceinline__ float slice_min8(const float (&v)[8], const float* pe
 // scoring + next-step input of one chunk, given the new state values sv[8] of dims [oc, oc + 8). The
 // action a_{t+1} sits in state columns [O, O + A) (head_store_actions), so x = scale([s, a]) needs no
 // special case here.
-template <class AStore>
+template <int kTW, class AStore>
 __device__ __forceinline__ void head_chunk_tail(const HeadCtx& c, const AStore& astore, int oc, uint32_t bits,
                                                 const float (&sv)[8], bool write_next, float& gmin,
                                                 float (&cmin)[SIMBA_MAX_CONSTRAINTS]) {
@@ -169,14 +173,14 @@ __device__ __forceinline__ void head_chunk_tail(const HeadCtx& c, const AStore& 
     if (bits >> 1) {
 #pragma unroll
       for (int q = 0; q < SIMBA_MAX_CONSTRAINTS; ++q)
-        if ((bits >> (1 + q)) & 1u) cmin[q] = slice_min8(sv, c.pen_smem + (1 + q) * 64 + oc, cmin[q]);
+        if ((bits >> (1 + q)) & 1u) cmin[q] = slice_min8(sv, c.pen_smem + (1 + q) * kTW + oc, cmin[q]);
     }
   }
   if (write_next) {
     const ulonglong2 a0 = *reinterpret_cast<const ulonglong2*>(c.scale_smem + oc);
     const ulonglong2 a1 = *reinterpret_cast<const ulonglong2*>(c.scale_smem + oc + 4);
-    const ulonglong2 b0 = *reinterpret_cast<const ulonglong2*>(c.scale_smem + 64 + oc);
-    const ulonglong2 b1 = *reinterpret_cast<const ulonglong2*>(c.scale_smem + 64 + oc + 4);
+    const ulonglong2 b0 = *reinterpret_cast<const ulonglong2*>(c.scale_smem + kTW + oc);
+    const ulonglong2 b1 = *reinterpret_cast<const ulonglong2*>(c.scale_smem + kTW + oc + 4);
     float x[8];
     f2_unpack(f2_fma(f2_pack(sv[0], sv[1]), a0.x, b0.x), x[0], x[1]);
     f2_unpack(f2_fma(f2_pack(sv[2], sv[3]), a0.y, b0.y), x[2], x[3]);
@@ -211,7 +215,7 @@ __device__ __forceinline__ void head_publish(const HeadCtx& c, float gmin, const
 }
 
 // s_0 from global memory: state -> TMEM, x_0 -> A operand, partial minima (once per launch)
-template <int OW, class AStore>
+template <int OW, int kTW = 64, class AStore>
 __device__ __forceinline__ void head_first_pass(const HeadCtx& c, const AStore& astore, const float* s0_ptr,
                                                 bool row_ok, const float (&act0)[4]) {
   float gmin = INFINITY, cmin[SIMBA_MAX_CONSTRAINTS];
@@ -231,7 +235,7 @@ __device__ __forceinline__ void head_first_pass(const HeadCtx& c, const AStore& 
       st[i] = __float_as_uint(sv[i]);
     }
     tmem_st<8>(c.t_state + oc, st);
-    head_chunk_tail(c, astore, oc, (c.slice_bits >> (ch * 5)) & 31u, sv, true, gmin, cmin);
+    head_chunk_tail<kTW>(c, astore, oc, (c.slice_bits >> (ch * 5)) & 31u, sv, true, gmin, cmin);
   }
   head_publish(c, gmin, cmin);
 }
@@ -256,14 +260,15 @@ __device__ __forceinline__ void head_first_pass_vals(const HeadCtx& c, const ASt
     st[i] = __float_as_uint(sv[i]);
   }
   tmem_st<8>(c.t_state + oc, st);
-  head_chunk_tail(c, astore, oc, c.slice_bits & 31u, sv, true, gmin, cmin);
+  head_chunk_tail<64>(c, astore, oc, c.slice_bits & 31u, sv, true, gmin, cmin);
   head_publish(c, gmin, cmin);
 }
 
 // Step t: s_{t+1} = s_t + mu (+ sqrt(softplus(raw var) + 1e-4) * eps), state back to TMEM, scaled bf16
 // x_{t+1} into the A operand, partial lidar minima of s_{t+1} published. Padded outputs (o >= O) have
-// zero weights, zero bias and zero noise, so their delta is exactly 0 and needs no mask.
-template <int OW, bool kSample, class Noise, class AStore>
+// zero weights, zero bias and zero noise, so their delta is exactly 0 and needs no mask. kVar: TMEM column
+// offset of the raw-variance head from the mu head; kTW: width of the tables (both = the state width).
+template <int OW, bool kSample, int kVar = 64, int kTW = 64, class Noise, class AStore>
 __device__ __forceinline__ void head_step_pass(const HeadCtx& c, const Noise& noise, const AStore& astore,
                                                bool write_next) {
   constexpr int NCH = OW / 8;
@@ -272,7 +277,7 @@ __device__ __forceinline__ void head_step_pass(const HeadCtx& c, const Noise& no
   for (int q = 0; q < SIMBA_MAX_CONSTRAINTS; ++q) cmin[q] = INFINITY;
   uint32_t vm[2][8], vv[2][8], st[2][8];
   tmem_ld<8>(c.t_acc + c.o_base, vm[0]);
-  if (kSample) tmem_ld<8>(c.t_acc + 64 + c.o_base, vv[0]);
+  if (kSample) tmem_ld<8>(c.t_acc + kVar + c.o_base, vv[0]);
   tmem_ld<8>(c.t_state + c.o_base, st[0]);
 #pragma unroll
   for (int ch = 0; ch < NCH; ++ch) {
@@ -281,7 +286,7 @@ __device__ __forceinline__ void head_step_pass(const HeadCtx& c, const Noise& no
     tmem_ld_wait();
     if (ch + 1 < NCH) {                                    // next chunk's loads fly during this chunk's math
       tmem_ld<8>(c.t_acc + oc + 8, vm[nxt]);
-      if (kSample) tmem_ld<8>(c.t_acc + 64 + oc + 8, vv[nxt]);
+      if (kSample) tmem_ld<8>(c.t_acc + kVar + oc + 8, vv[nxt]);
       tmem_ld<8>(c.t_state + oc + 8, st[nxt]);
     }
     float sv[8];
@@ -318,7 +323,7 @@ __device__ __forceinline__ void head_step_pass(const HeadCtx& c, const Noise& no
       for (int i = 0; i < 8; ++i) so[i] = __float_as_uint(sv[i]);
       tmem_st<8>(c.t_state + oc, so);
     }
-    head_chunk_tail(c, astore, oc, (c.slice_bits >> (ch * 5)) & 31u, sv, write_next, gmin, cmin);
+    head_chunk_tail<kTW>(c, astore, oc, (c.slice_bits >> (ch * 5)) & 31u, sv, write_next, gmin, cmin);
   }
   head_publish(c, gmin, cmin);
 }

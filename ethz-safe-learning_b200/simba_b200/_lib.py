@@ -18,7 +18,8 @@ MAP_SPLIT, MAP_PARTICLE = 0, 1
 (BUF_ACTIONS, BUF_ROW_RETURN, BUF_ROW_COSTMASK, BUF_ROW_COSTSUM, BUF_PAIRS_LOCAL, BUF_PAIRS_ALL,
  BUF_ELITE, BUF_MU, BUF_SIGMA, BUF_BEST_ACTION, BUF_BEST_SCORE, BUF_ACTIVE, BUF_SCORES) = range(13)
 
-(ROLLOUT_FP32, ROLLOUT_TC_ONE_CTA, ROLLOUT_TC_PAIR, ROLLOUT_TC_TWO_TILE, ROLLOUT_TC_WIDE) = range(5)
+(ROLLOUT_FP32, ROLLOUT_TC_ONE_CTA, ROLLOUT_TC_PAIR, ROLLOUT_TC_TWO_TILE, ROLLOUT_TC_WIDE,
+ ROLLOUT_TC_WIDE_OBS) = range(6)
 
 PRECISIONS = {'fp32': PREC_FP32, 'bf16': PREC_BF16_TC}
 MEMBER_MAPS = {'split': MAP_SPLIT, 'particle': MAP_PARTICLE}

@@ -225,7 +225,9 @@ typedef enum simba_rollout_kernel {
   SIMBA_ROLLOUT_TC_ONE_CTA = 1,    /* bf16 tcgen05, one CTA per 128-row tile                         */
   SIMBA_ROLLOUT_TC_PAIR = 2,       /* bf16 tcgen05, a cluster of two CTAs per tile (at most SMs / 2 tiles) */
   SIMBA_ROLLOUT_TC_TWO_TILE = 3,   /* bf16 tcgen05, persistent CTAs, two tiles per work item (more tiles than SMs) */
-  SIMBA_ROLLOUT_TC_WIDE = 4        /* bf16 tcgen05 weight-streaming kernel, 128 < units <= ~416      */
+  SIMBA_ROLLOUT_TC_WIDE = 4,       /* bf16 tcgen05 weight-streaming kernel, 128 < units <= ~416      */
+  SIMBA_ROLLOUT_TC_WIDE_OBS = 5    /* the same with 128 state columns: obs_dim + act_dim + 2 <= 128, obs_dim <= 124,
+                                      units <= 384, for bf16 shapes the kernels above reject           */
 } simba_rollout_kernel;
 /* -> *kernel (simba_rollout_kernel) and *work_items, the number of work items one launch walks */
 int simba_planner_rollout_kernel(simba_planner_t* p, int32_t* kernel, int32_t* work_items);
