@@ -1277,9 +1277,9 @@ extern "C" int simba_planner_init_nccl(simba_planner_t* p, const void* uid) {
 }
 
 // ---- model-level entry points -----------------------------------------------------------------------
-static int model_tiles(simba_model* m, const RowGeom& g, int* n_tiles) {
-  std::vector<Tile> tiles;
-  build_tiles(g, kF32TileRows, tiles);
+// The model keeps one device tile list for its entry points. It is overwritten only after a device-wide
+// synchronise, so a launch of any entry point still in flight on another stream never sees it change.
+static int model_upload_tiles(simba_model* m, const std::vector<Tile>& tiles, int* n_tiles) {
   if ((int)tiles.size() > m->tiles_cap) {
     cudaFree(m->d_tiles);
     m->d_tiles = nullptr;
@@ -1292,6 +1292,70 @@ static int model_tiles(simba_model* m, const RowGeom& g, int* n_tiles) {
   CUDA_TRY(cudaMemcpy(m->d_tiles, tiles.data(), tiles.size() * sizeof(Tile), cudaMemcpyHostToDevice));
   *n_tiles = (int)tiles.size();
   return SIMBA_OK;
+}
+
+static int model_tiles(simba_model* m, const RowGeom& g, int* n_tiles) {
+  std::vector<Tile> tiles;
+  build_tiles(g, kF32TileRows, tiles);
+  return model_upload_tiles(m, tiles, n_tiles);
+}
+
+// The tcgen05 kernel of a bf16 unfold (simba_unfold_tc) and its tile list: 128-row tiles of the tf.split member
+// map, the same shape predicates as choose_rollout with no constraints (no scorer), and the same image the model
+// commit packed. The trajectory forms have no per-row cost mask, so the horizon is bounded by the Philox step
+// counter alone (65535, as for the fp32 kernel); the predicates see at most the planner's bound.
+static int choose_unfold(const simba_model_config_t& mc, const RowGeom& g, int sms, RolloutKernel& kernel,
+                         std::vector<Tile>& tiles) {
+  const int O = mc.obs_dim, A = mc.act_dim, L = mc.n_layers, U = mc.units, H = std::min(g.H, SIMBA_MAX_HORIZON);
+  build_tiles(g, kTcTileRows, tiles);
+  if (rollout_tc_supported(O, A, L, U, H)) {
+    kernel = RolloutKernel::kTcOneCta;
+    if ((int)tiles.size() > sms && rollout_tc_two_tiles_fit(L, 0)) {
+      kernel = RolloutKernel::kTcTwoTile;
+      build_tiles(g, kTcTileRows, tiles, 2);
+      split_tail_items(tiles, sms);
+    }
+    return SIMBA_OK;
+  }
+  if (rollout_tc_wide_supported(64, O, A, L, U, H) && rollout_tc_wide_fits(64, L, U, 0)) {
+    kernel = RolloutKernel::kTcWide;
+    return SIMBA_OK;
+  }
+  if (wide_obs_selected(O, A, L, U, H) && rollout_tc_wide_fits(128, L, U, 0)) {
+    kernel = RolloutKernel::kTcWideObs;
+    return SIMBA_OK;
+  }
+  return fail(SIMBA_ERR_UNSUPPORTED,
+              "no bf16 tcgen05 kernel covers obs_dim %d, act_dim %d, %d x %d units: they cover units <= 128 "
+              "(obs_dim <= 60, obs_dim+act_dim <= 64, <= 5 layers), 128 < units <= ~416 (obs_dim+act_dim <= 62) and, "
+              "for other shapes, obs_dim+act_dim <= 126 with obs_dim <= 124, act_dim <= 4, units <= 384 and <= 6 "
+              "layers; use simba_unfold (fp32) for this shape", O, A, L, U);
+}
+
+// the device check of the bf16 unfold entry points, per call: one attribute query (cudaGetDeviceProperties, which
+// simba_device_check uses, costs milliseconds)
+static int unfold_tc_device_check(const simba_model* m) {
+  int dev = 0;
+  if (m) dev = m->device;
+  else CUDA_TRY(cudaGetDevice(&dev));
+  int major = 0;
+  CUDA_TRY(cudaDeviceGetAttribute(&major, cudaDevAttrComputeCapabilityMajor, dev));
+  if (major != 10) return fail(SIMBA_ERR_ARCH, "device %d is sm_%d*; the tcgen05 kernels need sm_100a", dev, major);
+  return SIMBA_OK;
+}
+
+// shared checks of the two bf16 unfold entry points -> geometry, SM count, kernel and tile list
+static int unfold_tc_plan(simba_model* m, int32_t batch, int32_t horizon, RowGeom& g, int& sms,
+                          RolloutKernel& kernel, std::vector<Tile>& tiles) {
+  if (!m->committed) return fail(SIMBA_ERR_NOT_READY, "model not committed");
+  if (horizon < 1 || horizon > 65535 || batch < 1)
+    return fail(SIMBA_ERR_BAD_CONFIG, "batch %d / horizon %d out of range", batch, horizon);
+  CUDA_TRY(cudaSetDevice(m->device));
+  int rc = build_geom(1, 1, batch, 1, 0, horizon, m->cfg.obs_dim, m->cfg.act_dim, m->cfg.ensemble_size,
+                      SIMBA_MAP_SPLIT, g);
+  if (rc != SIMBA_OK) return rc;
+  CUDA_TRY(cudaDeviceGetAttribute(&sms, cudaDevAttrMultiProcessorCount, m->device));
+  return choose_unfold(m->cfg, g, sms, kernel, tiles);
 }
 
 static void null_scorer(simba_scorer_t& sc) {
@@ -1325,6 +1389,51 @@ extern "C" int simba_unfold(simba_model_t* m, const float* s0, const float* acti
   prm.objective = SIMBA_OBJ_REWARD;
   prm.traj_out = out_traj;
   CUDA_TRY(launch_rollout_f32(prm, n_tiles, (cudaStream_t)stream));
+  return SIMBA_OK;
+}
+
+extern "C" int simba_unfold_tc(simba_model_t* m, const float* s0, const float* actions,
+                               const float* eps, uint64_t seed, int32_t batch, int32_t horizon,
+                               int32_t sampling_propagation, float* out_traj, void* stream) {
+  int rc = unfold_tc_device_check(m);
+  if (rc != SIMBA_OK) return rc;
+  if (!m || !s0 || !actions || !out_traj) return fail(SIMBA_ERR_BAD_CONFIG, "null argument");
+  RolloutParams prm{};
+  int sms = 0;
+  std::vector<Tile> tiles;
+  rc = unfold_tc_plan(m, batch, horizon, prm.g, sms, prm.kernel, tiles);
+  if (rc != SIMBA_OK) return rc;
+  int n_tiles = 0;
+  rc = model_upload_tiles(m, tiles, &n_tiles);
+  if (rc != SIMBA_OK) return rc;
+  prm.tiles = m->d_tiles; prm.n_tiles = n_tiles;   // prm.scorer stays zero: the trajectory forms score nothing
+  fill_model_params(m, prm);
+  prm.n_sms = sms;
+  prm.states = s0; prm.state_stride = m->cfg.obs_dim; prm.state_per_row = 1;
+  prm.actions = actions; prm.action_stride = (int64_t)horizon * m->cfg.act_dim;
+  prm.eps = eps; prm.seed = seed; prm.iteration = 0;
+  prm.sampling_propagation = sampling_propagation;
+  prm.objective = SIMBA_OBJ_REWARD;
+  prm.traj_out = out_traj;
+  const bool wide = prm.kernel == RolloutKernel::kTcWide || prm.kernel == RolloutKernel::kTcWideObs;
+  CUDA_TRY(wide ? launch_unfold_tc_wide(prm, n_tiles, (cudaStream_t)stream)
+                : launch_unfold_tc(prm, n_tiles, (cudaStream_t)stream));
+  return SIMBA_OK;
+}
+
+extern "C" int simba_unfold_tc_kernel(simba_model_t* m, int32_t batch, int32_t horizon, int32_t* kernel,
+                                      int32_t* work_items) {
+  int rc = unfold_tc_device_check(m);
+  if (rc != SIMBA_OK) return rc;
+  if (!m || !kernel || !work_items) return fail(SIMBA_ERR_BAD_CONFIG, "null argument");
+  RowGeom g;
+  int sms = 0;
+  RolloutKernel k = RolloutKernel::kF32;
+  std::vector<Tile> tiles;
+  rc = unfold_tc_plan(m, batch, horizon, g, sms, k, tiles);
+  if (rc != SIMBA_OK) return rc;
+  *kernel = (int32_t)k;
+  *work_items = (int32_t)tiles.size() / (k == RolloutKernel::kTcTwoTile ? 2 : 1);
   return SIMBA_OK;
 }
 

@@ -77,8 +77,11 @@ cudaError_t launch_rollout_tc(const RolloutParams& prm, int n_tiles, cudaStream_
 bool rollout_tc_supported(int O, int A, int L, int U, int H);
 bool rollout_tc_two_tiles_fit(int L, int n_constraints);
 bool rollout_tc_pair_fits(int L, int n_constraints);
+// the trajectory form of rollout_tc.cu (simba_unfold_tc): prm.kernel kTcOneCta or kTcTwoTile, prm.traj_out set
+cudaError_t launch_unfold_tc(const RolloutParams& prm, int n_tiles, cudaStream_t stream);
 // The weight-streaming kernel comes in two state widths `sw`: 64 (prm.kernel kTcWide) and 128 (kTcWideObs).
 cudaError_t launch_rollout_tc_wide(const RolloutParams& prm, int n_tiles, cudaStream_t stream);   // prm.U: the model's units
+cudaError_t launch_unfold_tc_wide(const RolloutParams& prm, int n_tiles, cudaStream_t stream);   // trajectory form
 bool rollout_tc_wide_supported(int sw, int O, int A, int L, int U, int H);
 bool rollout_tc_wide_fits(int sw, int L, int U, int n_constraints);
 int rollout_tc_wide_units(int sw, int U);                     // the padded width the kernel runs

@@ -135,9 +135,16 @@ struct AStorePair {
 // written only after the peer has sent all of step t + 1, which it does after consuming step t, so two
 // suffice (and a barrier is re-armed for step t + 2 long before that step's bytes can arrive; were they
 // early, a negative transaction count is legal and the pending arm keeps the phase open).
-template <int NTILES, int Q, bool PAIR>
-__global__ void __launch_bounds__(kBoundThreads, 1) rollout_tc_kernel(const RolloutParams prm) {
+//
+// TRAJ (simba_unfold_tc): the trajectory form. The epilogue threads write s_0 and every s_{t+1} of their
+// valid rows to prm.traj_out [B, H + 1, O] (tc_head.cuh TrajSink) and score nothing: the scorer warps
+// idle, no partial minima are published, the scorer struct is not read. Each thread whose column slice
+// meets the action block stores its own action columns (head_store_own_actions). H is bounded only by
+// the 16 bits of the Philox step counter.
+template <int NTILES, int Q, bool PAIR, bool TRAJ>
+__device__ __forceinline__ void rollout_tc_body(const RolloutParams& prm) {
   static_assert(!PAIR || (NTILES == 1 && Q == 4), "the pair variant is the one-tile latency configuration");
+  static_assert(!(PAIR && TRAJ), "the trajectory form has no pair variant");
   constexpr int kTileThreads = Q * 128;
   constexpr int kTileWarps = Q * 4;
   constexpr int kEpiThreads = NTILES * kTileThreads;
@@ -179,7 +186,7 @@ __global__ void __launch_bounds__(kBoundThreads, 1) rollout_tc_kernel(const Roll
   uint8_t* ones_smem = biask_smem + (L + 1) * 4096;                        // [4096]: A operand of the bias K-step
   float* scale_smem = reinterpret_cast<float*>(ones_smem + 4096);          // [2][64]: a, b of x*a+b
   float* pen_smem = scale_smem + 128;                                      // [kHeadParts][64]
-  const int nparts = 1 + prm.scorer.n_constraints;                         // goal + constrained lidars
+  const int nparts = TRAJ ? 1 : 1 + prm.scorer.n_constraints;              // goal + constrained lidars
   float* part_smem = pen_smem + kHeadParts * 64;                           // [1 or 2 (PAIR)][NTILES][NSL][nparts][128]
   const int part_buf_floats = NTILES * NSL * nparts * 128;
   uint4* xch_smem = reinterpret_cast<uint4*>(part_smem + (PAIR ? 2 : 1) * part_buf_floats);   // PAIR: [2][Q][128] x 16 B
@@ -270,8 +277,13 @@ __global__ void __launch_bounds__(kBoundThreads, 1) rollout_tc_kernel(const Roll
       reinterpret_cast<uint32_t*>(ones_smem)[i] = first ? 0x3F803F80u : 0u;
     }
     fence_proxy_async();                                // generic-proxy writes -> visible to the MMA
-    head_tables_init(scale_smem, pen_smem, prm.tc_scale_a, prm.tc_scale_b, prm.scorer,
-                     l0_pad_bias ? O + A : -1, threadIdx.x, kEpiThreads);
+    if constexpr (TRAJ) {                               // the penalty table is never read
+      head_tables_init(scale_smem, pen_smem, prm.tc_scale_a, prm.tc_scale_b, simba_scorer_t{},
+                       l0_pad_bias ? O + A : -1, threadIdx.x, kEpiThreads);
+    } else {
+      head_tables_init(scale_smem, pen_smem, prm.tc_scale_a, prm.tc_scale_b, prm.scorer,
+                       l0_pad_bias ? O + A : -1, threadIdx.x, kEpiThreads);
+    }
   }
   if (PAIR && threadIdx.x == 0) {
     // arm the exchange barriers for s_0 (step -1, barrier 1) and step 0 (barrier 0); see the scorer warps
@@ -359,7 +371,7 @@ __global__ void __launch_bounds__(kBoundThreads, 1) rollout_tc_kernel(const Roll
           if (lane == 0 && xbytes(ts + 2) != 0u) mbar_expect_tx(xbar + 8u * ((uint32_t)ts & 1u), xbytes(ts + 2));
         }
       }
-      if (tis.valid && crank == 0) {                                       // PAIR: CTA 0 keeps the objective
+      if (!TRAJ && tis.valid && crank == 0) {                              // PAIR: CTA 0 keeps the objective
         const simba_scorer_t& sc = prm.scorer;
         const bool done_first = objective_done_first(prm.objective);
         // the objective of the lane's four rows is parked in shared memory (field-major), so the row
@@ -494,8 +506,8 @@ __global__ void __launch_bounds__(kBoundThreads, 1) rollout_tc_kernel(const Roll
         hc.t_state = lane_base + (uint32_t)(NTILES * 128 + j * 64);
         hc.o_base = (PAIR ? (int)crank * 32 : 0) + cgp * OW;
         hc.O = O; hc.A = A;
-        hc.slice_bits = head_slice_bits<OW>(sc, hc.o_base);
-        hc.n_constraints = sc.n_constraints;
+        hc.slice_bits = TRAJ ? 0u : head_slice_bits<OW>(sc, hc.o_base);
+        hc.n_constraints = TRAJ ? 0 : sc.n_constraints;
         hc.scale_smem = scale_smem;
         hc.pen_smem = pen_smem;
         // partial minima: slice crank * Q + cgp of the buffer the scorer warp (PAIR: of CTA 0) reads
@@ -505,7 +517,7 @@ __global__ void __launch_bounds__(kBoundThreads, 1) rollout_tc_kernel(const Roll
         astore.t_a = t_a;
         const uint32_t my_xbar = smem_u32(&bars[1 + NTILES]);                 // PAIR: [2] mbarriers, 8 bytes apart
         const uint32_t peer_xbar = PAIR ? cluster_map_u32(my_xbar, crank ^ 1u) : 0u;
-        const bool keeps_score = !PAIR || crank == 0;                         // this CTA's scorer warp is the live one
+        const bool keeps_score = !TRAJ && (!PAIR || crank == 0);              // this CTA's scorer warp is the live one
         const uint32_t part_remote0 = (PAIR && crank != 0) ? cluster_map_u32(smem_u32(part_slot0), 0u) : 0u;
         if constexpr (PAIR) {
           astore.peer_slot = cluster_map_u32(smem_u32(xch_smem + cgp * 128 + r), crank ^ 1u);
@@ -530,6 +542,12 @@ __global__ void __launch_bounds__(kBoundThreads, 1) rollout_tc_kernel(const Roll
           }
         };
         const float* s0_ptr = prm.states + (prm.state_per_row ? id.r_global : (int64_t)id.s) * prm.state_stride;
+        // TRAJ: this row's s_t in traj_out, advanced by one step before every head pass
+        typename std::conditional<TRAJ, TrajSink, NoTraj>::type sink{};
+        if constexpr (TRAJ) {
+          sink.row = row_ok ? prm.traj_out + id.out * (int64_t)(H + 1) * O : nullptr;
+          sink.O = O;
+        }
 
 #ifdef SIMBA_TC_TIMELINE
         const int tl_who = (j == 0 && lane == 0) ? (wl == 0 ? 0 : (wl == kTileWarps - 1 ? 1 : -1)) : -1;
@@ -552,8 +570,10 @@ __global__ void __launch_bounds__(kBoundThreads, 1) rollout_tc_kernel(const Roll
 
         // the thread whose column slice holds state column O prefetches a_{t+1} one step ahead (the L2
         // latency is off the critical path) and parks it in state columns [O, O + A) of its row
-        // (tc_head.cuh head_store_actions; A <= 4 on this path)
-        const bool owns_actions = (O >= hc.o_base) && (O < hc.o_base + OW);
+        // (tc_head.cuh head_store_actions; A <= 4 on this path). TRAJ: every thread whose slice meets
+        // [O, O + A) fetches the actions and stores its own columns of them (head_store_own_actions).
+        const bool owns_actions = TRAJ ? (O < hc.o_base + OW) && (O + A > hc.o_base)
+                                       : (O >= hc.o_base) && (O < hc.o_base + OW);
         float act_pf[4] = {0.f, 0.f, 0.f, 0.f};
         auto prefetch_actions = [&](int tn) {
           if (owns_actions && row_ok && tn < H) {
@@ -616,7 +636,7 @@ __global__ void __launch_bounds__(kBoundThreads, 1) rollout_tc_kernel(const Roll
         if (live) {
         prefetch_actions(0);
         if constexpr (PAIR) head_first_pass_vals(hc, astore, s0v, act_pf);
-        else head_first_pass<OW>(hc, astore, s0_ptr, row_ok, act_pf);
+        else head_first_pass<OW>(hc, astore, s0_ptr, row_ok, act_pf, sink);
         prefetch_actions(1);
         exchange(-1, true);
         publish_a();                                        // layer-0 input of step 0
@@ -629,7 +649,10 @@ __global__ void __launch_bounds__(kBoundThreads, 1) rollout_tc_kernel(const Roll
           tl_t = t;
 #endif
           TL(0);
-          if (owns_actions) head_store_actions(hc, act_pf);   // a_{t+1}, fetched during step t - 1
+          if (owns_actions) {                                 // a_{t+1}, fetched during step t - 1
+            if constexpr (TRAJ) head_store_own_actions<OW>(hc, act_pf);
+            else head_store_actions(hc, act_pf);
+          }
           prefetch_actions(t + 2);
           // ---- hidden layers: TMEM accumulator (bias included) -> ReLU -> bf16 -> next A operand ------
           for (int l = 0; l < L; ++l) {
@@ -692,8 +715,11 @@ __global__ void __launch_bounds__(kBoundThreads, 1) rollout_tc_kernel(const Roll
               hc.part_mbar = astore.peer_bar;
             }
           }
-          if (prm.sampling_propagation) head_step_pass<OW, true>(hc, noise, astore, t + 1 < H);
-          else head_step_pass<OW, false>(hc, noise, astore, t + 1 < H);
+          if constexpr (TRAJ) {
+            if (sink.row != nullptr) sink.row += O;
+          }
+          if (prm.sampling_propagation) head_step_pass<OW, true>(hc, noise, astore, t + 1 < H, sink);
+          else head_step_pass<OW, false>(hc, noise, astore, t + 1 < H, sink);
           TL(41);
           exchange(t, t + 1 < H);
           if (t + 1 < H) publish_a();                       // next step's layer 0 goes out
@@ -721,6 +747,17 @@ __global__ void __launch_bounds__(kBoundThreads, 1) rollout_tc_kernel(const Roll
   TLK(4);
   if (warp == 0) tmem_dealloc(tmem_base, kTmemCols);
   TLK(5);
+}
+
+template <int NTILES, int Q, bool PAIR>
+__global__ void __launch_bounds__(kBoundThreads, 1) rollout_tc_kernel(const RolloutParams prm) {
+  rollout_tc_body<NTILES, Q, PAIR, false>(prm);
+}
+
+// the trajectory form (simba_unfold_tc): <1, 4> and the persistent two-tile <2, 2>
+template <int NTILES, int Q>
+__global__ void __launch_bounds__(kBoundThreads, 1) unfold_tc_kernel(const RolloutParams prm) {
+  rollout_tc_body<NTILES, Q, false, true>(prm);
 }
 
 // ---- host side ------------------------------------------------------------------------------------
@@ -757,14 +794,15 @@ bool rollout_tc_pair_fits(int L, int n_constraints) {
   return tc_smem_bytes(L, 1, 4, 1 + n_constraints, true) + 1024 <= kMaxSmem;
 }
 
-template <int NTILES, int Q, bool PAIR>
+template <int NTILES, int Q, bool PAIR, bool TRAJ = false>
 static cudaError_t launch_variant(const RolloutParams& prm, int n_tiles, cudaStream_t stream) {
-  const size_t smem = tc_smem_bytes(prm.L, NTILES, Q, 1 + prm.scorer.n_constraints, PAIR);
+  void (*kern)(const RolloutParams) = rollout_tc_kernel<NTILES, Q, PAIR>;
+  if constexpr (TRAJ) kern = unfold_tc_kernel<NTILES, Q>;
+  const size_t smem = tc_smem_bytes(prm.L, NTILES, Q, TRAJ ? 1 : 1 + prm.scorer.n_constraints, PAIR);
   // set on every launch: the attribute is per device and per function, and launches happen only at
   // graph capture or in the non-graph entry points, never on the replayed hot path
   {
-    cudaError_t e = cudaFuncSetAttribute(rollout_tc_kernel<NTILES, Q, PAIR>,
-                                         cudaFuncAttributeMaxDynamicSharedMemorySize, (int)smem);
+    cudaError_t e = cudaFuncSetAttribute(kern, cudaFuncAttributeMaxDynamicSharedMemorySize, (int)smem);
     if (e != cudaSuccess) return e;
   }
   const int n_items = (n_tiles + NTILES - 1) / NTILES;
@@ -793,7 +831,7 @@ static cudaError_t launch_variant(const RolloutParams& prm, int n_tiles, cudaStr
   }
   cfg.attrs = attr;
   cfg.numAttrs = na;
-  return cudaLaunchKernelEx(&cfg, rollout_tc_kernel<NTILES, Q, PAIR>, prm);
+  return cudaLaunchKernelEx(&cfg, kern, prm);
 }
 
 cudaError_t launch_rollout_tc(const RolloutParams& prm, int n_tiles, cudaStream_t stream) {
@@ -802,6 +840,15 @@ cudaError_t launch_rollout_tc(const RolloutParams& prm, int n_tiles, cudaStream_
     case RolloutKernel::kTcOneCta: return launch_variant<1, 4, false>(prm, n_tiles, stream);
     case RolloutKernel::kTcPair: return launch_variant<1, 4, true>(prm, n_tiles, stream);
     case RolloutKernel::kTcTwoTile: return launch_variant<2, 2, false>(prm, n_tiles, stream);
+    default: return cudaErrorInvalidValue;
+  }
+}
+
+cudaError_t launch_unfold_tc(const RolloutParams& prm, int n_tiles, cudaStream_t stream) {
+  if (n_tiles == 0) return cudaSuccess;
+  switch (prm.kernel) {
+    case RolloutKernel::kTcOneCta: return launch_variant<1, 4, false, true>(prm, n_tiles, stream);
+    case RolloutKernel::kTcTwoTile: return launch_variant<2, 2, false, true>(prm, n_tiles, stream);
     default: return cudaErrorInvalidValue;
   }
 }

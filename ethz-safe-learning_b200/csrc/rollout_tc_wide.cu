@@ -129,8 +129,12 @@ struct TileInfoW {
 
 }  // namespace
 
-template <int kSW>
-__global__ void __launch_bounds__(kWideThreads, 1) rollout_tc_wide_kernel(const RolloutParams prm) {
+// TRAJ (simba_unfold_tc): the trajectory form. The epilogue threads write s_0 and every s_{t+1} of their valid
+// rows to prm.traj_out [B, H + 1, O] (tc_head.cuh TrajSink) and score nothing (no partial minima, no objective,
+// no scorer struct read). Each thread whose column slice meets the action block stores its own action columns
+// (head_store_own_actions). H is bounded only by the 16 bits of the Philox step counter.
+template <int kSW, bool TRAJ>
+__device__ __forceinline__ void rollout_tc_wide_body(const RolloutParams& prm) {
   using C = WideCfg<kSW>;
   constexpr int kStateCol = C::kStateCol, OW = C::OW, NB = C::NB, kHeadGroup = C::kHeadGroup;
   extern __shared__ __align__(1024) uint8_t smem_raw[];
@@ -148,7 +152,7 @@ __global__ void __launch_bounds__(kWideThreads, 1) rollout_tc_wide_kernel(const 
   const uint32_t stage_bytes = wide_stage_bytes<kSW>(ws);
   float* scale_smem = reinterpret_cast<float*>(b_smem + (size_t)kStages * stage_bytes);   // [2][kSW]
   float* pen_smem = scale_smem + 2 * kSW;                                  // [kParts][kSW]
-  const int nparts = 1 + prm.scorer.n_constraints;
+  const int nparts = TRAJ ? 1 : 1 + prm.scorer.n_constraints;
   float* part_smem = pen_smem + kHeadParts * kSW;                              // [kQ][nparts][128]
   // running objective of every rollout row (RowScore fields, field-major), see rollout_tc.cu
   uint32_t* rs_smem = reinterpret_cast<uint32_t*>(part_smem + kQ * nparts * 128);   // [8][128]
@@ -278,8 +282,12 @@ __global__ void __launch_bounds__(kWideThreads, 1) rollout_tc_wide_kernel(const 
       const int r = (wl & 3) * 32 + lane;                   // row in tile == TMEM lane
       // scaler / penalty tables, zeroed A tile with the constant ones of the bias rows
       {
-        head_tables_init<kSW>(scale_smem, pen_smem, prm.tc_scale_a, prm.tc_scale_b, prm.scorer, O + A, threadIdx.x,
-                              kEpiThreads);
+        if constexpr (TRAJ)                                  // the penalty table is never read
+          head_tables_init<kSW>(scale_smem, pen_smem, prm.tc_scale_a, prm.tc_scale_b, simba_scorer_t{}, O + A,
+                                threadIdx.x, kEpiThreads);
+        else
+          head_tables_init<kSW>(scale_smem, pen_smem, prm.tc_scale_a, prm.tc_scale_b, prm.scorer, O + A, threadIdx.x,
+                                kEpiThreads);
         uint32_t* a32 = reinterpret_cast<uint32_t*>(a_smem);
         for (int i = threadIdx.x; i < KA * kAtomBytes / 4; i += kEpiThreads) a32[i] = 0u;
         named_bar_sync<kEpiThreads>(kBarEpi);
@@ -301,6 +309,12 @@ __global__ void __launch_bounds__(kWideThreads, 1) rollout_tc_wide_kernel(const 
       const bool done_first = objective_done_first(prm.objective);
       const simba_scorer_t& sc = prm.scorer;
       const float* s0_ptr = prm.states + (prm.state_per_row ? id.r_global : (int64_t)id.s) * prm.state_stride;
+      // TRAJ: this row's s_t in traj_out, advanced by one step before every head pass
+      typename std::conditional<TRAJ, TrajSink, NoTraj>::type sink{};
+      if constexpr (TRAJ) {
+        sink.row = row_ok ? prm.traj_out + id.out * (int64_t)(H + 1) * O : nullptr;
+        sink.O = O;
+      }
       const uint32_t a_row = smem_u32(a_smem) + (uint32_t)(r >> 3) * 1024u + (uint32_t)(r & 7) * 128u;
       const uint32_t rsw = (uint32_t)(r & 7);
 
@@ -309,8 +323,8 @@ __global__ void __launch_bounds__(kWideThreads, 1) rollout_tc_wide_kernel(const 
       hc.t_state = t_lane + (uint32_t)kStateCol;
       hc.o_base = cgp * OW;
       hc.O = O; hc.A = A;
-      hc.slice_bits = head_slice_bits<OW>(sc, hc.o_base);
-      hc.n_constraints = sc.n_constraints;
+      hc.slice_bits = TRAJ ? 0u : head_slice_bits<OW>(sc, hc.o_base);
+      hc.n_constraints = TRAJ ? 0 : sc.n_constraints;
       hc.scale_smem = scale_smem;
       hc.pen_smem = pen_smem;
       hc.part = part_smem + (cgp * nparts) * 128 + r;
@@ -342,11 +356,13 @@ __global__ void __launch_bounds__(kWideThreads, 1) rollout_tc_wide_kernel(const 
         tc_fence_after();
       };
 
-      const bool owns_actions = (O >= hc.o_base) && (O < hc.o_base + OW);
+      // TRAJ: every thread whose slice meets [O, O + A) fetches and stores its own action columns, every step
+      const bool meets_actions = (O < hc.o_base + OW) && (O + A > hc.o_base);
+      const bool owns_actions = TRAJ ? meets_actions : (O >= hc.o_base) && (O < hc.o_base + OW);
       // a_0 goes into the state columns [O, O + A) of whichever slices hold them (head_first_pass); at kSW = 128
       // they may straddle two slices (O = 63, A = 2), so every thread whose slice meets them fetches a_0. Later
       // actions come from the owner alone (head_store_actions writes all four columns).
-      const bool needs_a0 = kSW == 64 ? owns_actions : (O < hc.o_base + OW) && (O + A > hc.o_base);
+      const bool needs_a0 = (kSW == 64 && !TRAJ) ? owns_actions : meets_actions;
       float act_pf[4] = {0.f, 0.f, 0.f, 0.f};
       auto prefetch_actions = [&](int tn, bool mine) {
         if (mine && row_ok && tn < H) {
@@ -389,12 +405,12 @@ __global__ void __launch_bounds__(kWideThreads, 1) rollout_tc_wide_kernel(const 
 
       uint32_t* my_rs = rs_smem + r;                      // cum, costsum, cmask lo / hi, dist, cost, done
       prefetch_actions(0, needs_a0);
-      head_first_pass<OW, kSW>(hc, astore, s0_ptr, row_ok, act_pf);
+      head_first_pass<OW, kSW>(hc, astore, s0_ptr, row_ok, act_pf, sink);
       prefetch_actions(1, owns_actions);
       tmem_st_wait();
       publish_a();                                       // layer-0 input of step 0
-      named_bar_sync<kEpiThreads>(kBarScore);            // partial minima of s_0 visible to the scorers
-      if (cgp == 0) {
+      if constexpr (!TRAJ) named_bar_sync<kEpiThreads>(kBarScore);   // partial minima of s_0 visible to the scorers
+      if (!TRAJ && cgp == 0) {
         float d0, c0;
         head_combine<kQ>(sc, part_row, nparts, d0, c0);
         my_rs[0] = 0u; my_rs[128] = 0u; my_rs[256] = 0u; my_rs[384] = 0u;
@@ -415,7 +431,10 @@ __global__ void __launch_bounds__(kWideThreads, 1) rollout_tc_wide_kernel(const 
         tl_t = t;
 #endif
         TLW(0);
-        if (owns_actions) head_store_actions(hc, act_pf);   // a_{t+1}, fetched during step t - 1
+        if (owns_actions) {                                 // a_{t+1}, fetched during step t - 1
+          if constexpr (TRAJ) head_store_own_actions<OW>(hc, act_pf);
+          else head_store_actions(hc, act_pf);
+        }
         prefetch_actions(t + 2, owns_actions);
         // ---- hidden layers: TMEM -> ReLU -> bf16 -> swizzled A tile (bias is in the accumulator) ----
         for (int l = 0; l < L; ++l) {
@@ -460,18 +479,21 @@ __global__ void __launch_bounds__(kWideThreads, 1) rollout_tc_wide_kernel(const 
         // ---- Gaussian heads + state update + next input + partial minima (tc_head.cuh) -----------------
         wait_accumulator();
         TLW(40);
-        if constexpr (kSW == 128) {
+        if constexpr (kSW == 128 && !TRAJ) {
           // 96 registers: re-derive the slice predicates every step instead of holding them (no spills)
           asm volatile("mov.b32 %0, %0;" : "+r"(hc.slice_bits));
         }
-        if (prm.sampling_propagation) head_step_pass<OW, true, kSW, kSW>(hc, noise, astore, t + 1 < H);
-        else head_step_pass<OW, false, kSW, kSW>(hc, noise, astore, t + 1 < H);
+        if constexpr (TRAJ) {
+          if (sink.row != nullptr) sink.row += O;
+        }
+        if (prm.sampling_propagation) head_step_pass<OW, true, kSW, kSW>(hc, noise, astore, t + 1 < H, sink);
+        else head_step_pass<OW, false, kSW, kSW>(hc, noise, astore, t + 1 < H, sink);
         TLW(41);
         tmem_st_wait();
         if (t + 1 < H) publish_a();
         TLW(42);
-        named_bar_sync<kEpiThreads>(kBarScore);            // partial minima of s_{t+1} visible to the scorers
-        if (cgp == 0) {
+        if constexpr (!TRAJ) named_bar_sync<kEpiThreads>(kBarScore);   // partial minima of s_{t+1} visible to the scorers
+        if (!TRAJ && cgp == 0) {
           float next_dist, next_cost;
           head_combine<kQ>(sc, part_row, nparts, next_dist, next_cost);
           RowScore rs;
@@ -492,7 +514,7 @@ __global__ void __launch_bounds__(kWideThreads, 1) rollout_tc_wide_kernel(const 
         }
         TLW(43);
       }
-      if (cgp == 0 && row_ok && prm.row_return != nullptr) {
+      if (!TRAJ && cgp == 0 && row_ok && prm.row_return != nullptr) {
         prm.row_return[id.out] = __uint_as_float(my_rs[0]);
         prm.row_costmask[id.out] = (uint64_t)my_rs[256] | ((uint64_t)my_rs[384] << 32);
         prm.row_costsum[id.out] = __uint_as_float(my_rs[128]);
@@ -503,6 +525,17 @@ __global__ void __launch_bounds__(kWideThreads, 1) rollout_tc_wide_kernel(const 
   tc_fence_before();
   __syncthreads();
   if (warp == 0) tmem_dealloc(tmem_base, kTmemCols);
+}
+
+template <int kSW>
+__global__ void __launch_bounds__(kWideThreads, 1) rollout_tc_wide_kernel(const RolloutParams prm) {
+  rollout_tc_wide_body<kSW, false>(prm);
+}
+
+// the trajectory form (simba_unfold_tc)
+template <int kSW>
+__global__ void __launch_bounds__(kWideThreads, 1) unfold_tc_wide_kernel(const RolloutParams prm) {
+  rollout_tc_wide_body<kSW, true>(prm);
 }
 
 // ---- host side ------------------------------------------------------------------------------------
@@ -550,16 +583,17 @@ int64_t rollout_tc_wide_member_bytes(int sw, int L, int UP) {
   return (int64_t)(ws.tiles_per_step - ws.head_tiles) * ws.hid_tile_bytes + (int64_t)ws.KA * ws.head_tile_bytes;
 }
 
-template <int kSW>
+template <int kSW, bool TRAJ = false>
 static cudaError_t launch_wide(const RolloutParams& model_prm, int n_tiles, cudaStream_t stream) {
   RolloutParams prm = model_prm;
   prm.U = rollout_tc_wide_units(kSW, prm.U);                       // the kernel runs the zero-padded width
-  const size_t smem = wide_smem_bytes<kSW>(prm.L, prm.U, 1 + prm.scorer.n_constraints);
+  void (*kern)(const RolloutParams) = rollout_tc_wide_kernel<kSW>;
+  if constexpr (TRAJ) kern = unfold_tc_wide_kernel<kSW>;
+  const size_t smem = wide_smem_bytes<kSW>(prm.L, prm.U, TRAJ ? 1 : 1 + prm.scorer.n_constraints);
   // set on every launch: the attribute is per device and per function, and launches happen only at
   // graph capture or in the non-graph entry points, never on the replayed hot path
   {
-    cudaError_t e = cudaFuncSetAttribute(rollout_tc_wide_kernel<kSW>, cudaFuncAttributeMaxDynamicSharedMemorySize,
-                                         (int)smem);
+    cudaError_t e = cudaFuncSetAttribute(kern, cudaFuncAttributeMaxDynamicSharedMemorySize, (int)smem);
     if (e != cudaSuccess) return e;
   }
   cudaLaunchConfig_t cfg{};
@@ -572,7 +606,7 @@ static cudaError_t launch_wide(const RolloutParams& model_prm, int n_tiles, cuda
   attr[0].val.programmaticStreamSerializationAllowed = 1;
   cfg.attrs = attr;
   cfg.numAttrs = prm.pdl ? 1 : 0;
-  return cudaLaunchKernelEx(&cfg, rollout_tc_wide_kernel<kSW>, prm);
+  return cudaLaunchKernelEx(&cfg, kern, prm);
 }
 
 cudaError_t launch_rollout_tc_wide(const RolloutParams& prm, int n_tiles, cudaStream_t stream) {
@@ -580,6 +614,15 @@ cudaError_t launch_rollout_tc_wide(const RolloutParams& prm, int n_tiles, cudaSt
   switch (prm.kernel) {
     case RolloutKernel::kTcWide: return launch_wide<64>(prm, n_tiles, stream);
     case RolloutKernel::kTcWideObs: return launch_wide<128>(prm, n_tiles, stream);
+    default: return cudaErrorInvalidValue;
+  }
+}
+
+cudaError_t launch_unfold_tc_wide(const RolloutParams& prm, int n_tiles, cudaStream_t stream) {
+  if (n_tiles == 0) return cudaSuccess;
+  switch (prm.kernel) {
+    case RolloutKernel::kTcWide: return launch_wide<64, true>(prm, n_tiles, stream);
+    case RolloutKernel::kTcWideObs: return launch_wide<128, true>(prm, n_tiles, stream);
     default: return cudaErrorInvalidValue;
   }
 }

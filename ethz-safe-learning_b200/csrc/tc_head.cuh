@@ -214,10 +214,54 @@ __device__ __forceinline__ void head_publish(const HeadCtx& c, float gmin, const
     if (q < c.n_constraints) c.part[(1 + q) * 128] = cmin[q];
 }
 
+// Where the state values of a head pass go besides TMEM. The planning kernels keep nothing (NoTraj: the pass
+// scores the states). The trajectory form of the kernels (simba_unfold_tc) writes them to its row of
+// traj_out [B, H + 1, O] (TrajSink) and skips the scoring: no slice minima, nothing published.
+struct NoTraj {
+  static constexpr bool kScore = true;
+  __device__ __forceinline__ void put8(int, const float (&)[8]) const {}
+};
+struct TrajSink {
+  static constexpr bool kScore = false;
+  float* row;   // this row's state of the current step in traj_out, null for a padding row
+  int O;
+  // outputs [oc, oc + 8) below O: 16-byte stores where the address allows (row offsets are not 16-byte
+  // aligned for odd O), streaming (the trajectories are written once and read by the caller)
+  __device__ __forceinline__ void put8(int oc, const float (&v)[8]) const {
+    if (row == nullptr || oc >= O) return;
+    float* p = row + oc;
+    if (oc + 8 <= O && (reinterpret_cast<uintptr_t>(p) & 15u) == 0) {
+      __stcs(reinterpret_cast<float4*>(p), make_float4(v[0], v[1], v[2], v[3]));
+      __stcs(reinterpret_cast<float4*>(p + 4), make_float4(v[4], v[5], v[6], v[7]));
+    } else if (oc + 8 <= O && (reinterpret_cast<uintptr_t>(p) & 7u) == 0) {
+#pragma unroll
+      for (int i = 0; i < 8; i += 2) __stcs(reinterpret_cast<float2*>(p + i), make_float2(v[i], v[i + 1]));
+    } else {
+#pragma unroll
+      for (int i = 0; i < 8; ++i)
+        if (oc + i < O) __stcs(p + i, v[i]);
+    }
+  }
+};
+
+// Trajectory form: every thread whose slice [o_base, o_base + OW) meets the action columns [O, O + A) stores
+// its own columns of a_{t+1}, so that no column is written by two warps and an action block that crosses
+// into the next slice (O = 47, A = 2) is carried whole (head_store_actions writes all four from the owner).
+template <int OW>
+__device__ __forceinline__ void head_store_own_actions(const HeadCtx& c, const float (&act)[4]) {
+#pragma unroll
+  for (int a = 0; a < 4; ++a) {
+    if (a < c.A && c.O + a >= c.o_base && c.O + a < c.o_base + OW) {   // warp-uniform
+      const uint32_t v[1] = {__float_as_uint(act[a])};
+      tmem_st<1>(c.t_state + (uint32_t)(c.O + a), v);
+    }
+  }
+}
+
 // s_0 from global memory: state -> TMEM, x_0 -> A operand, partial minima (once per launch)
-template <int OW, int kTW = 64, class AStore>
+template <int OW, int kTW = 64, class AStore, class Sink = NoTraj>
 __device__ __forceinline__ void head_first_pass(const HeadCtx& c, const AStore& astore, const float* s0_ptr,
-                                                bool row_ok, const float (&act0)[4]) {
+                                                bool row_ok, const float (&act0)[4], const Sink& sink = Sink()) {
   float gmin = INFINITY, cmin[SIMBA_MAX_CONSTRAINTS];
 #pragma unroll
   for (int q = 0; q < SIMBA_MAX_CONSTRAINTS; ++q) cmin[q] = INFINITY;
@@ -235,9 +279,10 @@ __device__ __forceinline__ void head_first_pass(const HeadCtx& c, const AStore& 
       st[i] = __float_as_uint(sv[i]);
     }
     tmem_st<8>(c.t_state + oc, st);
-    head_chunk_tail<kTW>(c, astore, oc, (c.slice_bits >> (ch * 5)) & 31u, sv, true, gmin, cmin);
+    sink.put8(oc, sv);                                      // s_0 as read: the action columns lie beyond O
+    head_chunk_tail<kTW>(c, astore, oc, Sink::kScore ? (c.slice_bits >> (ch * 5)) & 31u : 0u, sv, true, gmin, cmin);
   }
-  head_publish(c, gmin, cmin);
+  if constexpr (Sink::kScore) head_publish(c, gmin, cmin);
 }
 
 // The same for a thread that owns one 8-wide chunk and already holds its eight s_0 values (zero beyond O or
@@ -268,9 +313,9 @@ __device__ __forceinline__ void head_first_pass_vals(const HeadCtx& c, const ASt
 // x_{t+1} into the A operand, partial lidar minima of s_{t+1} published. Padded outputs (o >= O) have
 // zero weights, zero bias and zero noise, so their delta is exactly 0 and needs no mask. kVar: TMEM column
 // offset of the raw-variance head from the mu head; kTW: width of the tables (both = the state width).
-template <int OW, bool kSample, int kVar = 64, int kTW = 64, class Noise, class AStore>
+template <int OW, bool kSample, int kVar = 64, int kTW = 64, class Noise, class AStore, class Sink = NoTraj>
 __device__ __forceinline__ void head_step_pass(const HeadCtx& c, const Noise& noise, const AStore& astore,
-                                               bool write_next) {
+                                               bool write_next, const Sink& sink = Sink()) {
   constexpr int NCH = OW / 8;
   float gmin = INFINITY, cmin[SIMBA_MAX_CONSTRAINTS];
 #pragma unroll
@@ -323,9 +368,11 @@ __device__ __forceinline__ void head_step_pass(const HeadCtx& c, const Noise& no
       for (int i = 0; i < 8; ++i) so[i] = __float_as_uint(sv[i]);
       tmem_st<8>(c.t_state + oc, so);
     }
-    head_chunk_tail<kTW>(c, astore, oc, (c.slice_bits >> (ch * 5)) & 31u, sv, write_next, gmin, cmin);
+    sink.put8(oc, sv);                                     // s_{t+1} as stored to TMEM
+    head_chunk_tail<kTW>(c, astore, oc, Sink::kScore ? (c.slice_bits >> (ch * 5)) & 31u : 0u, sv, write_next,
+                         gmin, cmin);
   }
-  head_publish(c, gmin, cmin);
+  if constexpr (Sink::kScore) head_publish(c, gmin, cmin);
 }
 
 // closest_distance (safety_gym.py:188-192) of a slice from its raw minimum m = min_b s[b]:

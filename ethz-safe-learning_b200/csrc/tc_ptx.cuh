@@ -120,7 +120,9 @@ __device__ __forceinline__ void tmem_ld(uint32_t taddr, uint32_t (&v)[N]) {
 }
 template <int N>
 __device__ __forceinline__ void tmem_st(uint32_t taddr, const uint32_t (&v)[N]) {
-  static_assert(N == 4 || N == 8 || N == 16, "unsupported TMEM store width");
+  static_assert(N == 1 || N == 4 || N == 8 || N == 16, "unsupported TMEM store width");
+  if constexpr (N == 1)
+    asm volatile("tcgen05.st.sync.aligned.32x32b.x1.b32 [%0], {%1};" :: "r"(taddr), "r"(v[0]) : "memory");
   if constexpr (N == 4)
     asm volatile("tcgen05.st.sync.aligned.32x32b.x4.b32 [%0], {%1, %2, %3, %4};"
                  :: "r"(taddr), "r"(v[0]), "r"(v[1]), "r"(v[2]), "r"(v[3]) : "memory");

@@ -100,6 +100,8 @@ _SIGNATURES = {
     'simba_nccl_unique_id': [_vp],
     'simba_planner_init_nccl': [_vp, _vp],
     'simba_unfold': [_vp, _vp, _vp, _vp, _u64, _i32, _i32, _i32, _vp, _vp],
+    'simba_unfold_tc': [_vp, _vp, _vp, _vp, _u64, _i32, _i32, _i32, _vp, _vp],
+    'simba_unfold_tc_kernel': [_vp, _i32, _i32, _P(_i32), _P(_i32)],
     'simba_ensemble_forward': [_vp, _vp, _vp, _i32, _vp, _vp, _vp, _vp],
     'simba_scale': [_vp, _vp, _i32, _vp, _vp],
     'simba_score_trajectories': [_vp, _vp, _vp, _vp, _vp],

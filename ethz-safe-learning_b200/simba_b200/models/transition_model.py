@@ -1,7 +1,9 @@
 """TransitionModel — mirrors simba/models/transition_model.py for the inference methods.
 
 `unfold_sequences` (transition_model.py:64-77), `scale` (:79-87), `predict` (:52-56) and
-`simulate_trajectories` (:58-62) run on the GPU through libsimba_b200.so. `fit` (:34-40) fits the
+`simulate_trajectories` (:58-62) run on the GPU through libsimba_b200.so. The rollout methods take
+`precision='fp32'` (fp32 SIMT kernel, simba_unfold) or `precision='bf16'`: the bf16 tensor-core kernels
+a bf16 CemMpc plans with (simba_unfold_tc), so the trajectories are the ones that planner scores. `fit` (:34-40) fits the
 scaler statistics (`_fit_statistics`, :42-50) and trains the ensemble on scaled inputs and
 observation deltas with the device trainer (MlpEnsemble.fit).
 """
@@ -75,22 +77,33 @@ class TransitionModel(BaseModel):
         next_observations = np.asarray(targets, dtype=np.float32)
         return self.model.fit(self.scale(inputs), (next_observations - observations).astype(np.float32))
 
-    def predict(self, inputs):
-        """transition_model.py:52-56 -> np[B, 2, O]."""
+    def predict(self, inputs, *, precision='fp32'):
+        """transition_model.py:52-56 -> np[B, 2, O]. `precision` as in unfold_sequences."""
         inputs = np.asarray(inputs, dtype=np.float32)
         return self.simulate_trajectories(
             current_state=inputs[..., :self.observation_space_dim],
-            action_sequences=np.expand_dims(inputs[..., -self.action_space_dim:], axis=1))
+            action_sequences=np.expand_dims(inputs[..., -self.action_space_dim:], axis=1),
+            precision=precision)
 
-    def simulate_trajectories(self, current_state, action_sequences, eps=None, seed=0):
+    def simulate_trajectories(self, current_state, action_sequences, eps=None, seed=0, *, precision='fp32'):
+        """transition_model.py:58-62 -> np[B, H+1, O]. `precision` as in unfold_sequences."""
         out = self.unfold_sequences(np.asarray(current_state, dtype=np.float32),
-                                    np.asarray(action_sequences, dtype=np.float32), eps=eps, seed=seed)
+                                    np.asarray(action_sequences, dtype=np.float32), eps=eps, seed=seed,
+                                    precision=precision)
         return out if isinstance(out, np.ndarray) else out.cpu().numpy()
 
-    def unfold_sequences(self, s_0, action_sequences, eps=None, seed=0):
+    def unfold_sequences(self, s_0, action_sequences, eps=None, seed=0, *, precision='fp32'):
         """transition_model.py:64-77. s_0 [B, O], action_sequences [B, H, A] -> [B, H+1, O].
         eps [H, B, O]: the N(0,1) draws of the per-step Normal.sample(); if None they come from
-        the Philox NOISE stream with `seed` (row = batch index)."""
+        the Philox NOISE stream with `seed` (row = batch index).
+
+        precision='fp32' runs the fp32 SIMT kernel. precision='bf16' runs the bf16 tcgen05 kernel that a
+        bf16 CemMpc plans with (weights, activations and draws rounded to bf16, states in fp32; s_0 is
+        returned bit for bit): the same draws and actions give the trajectories that planner scores.
+        Shapes no tcgen05 kernel covers raise SimbaError (code -6); there is no fp32 fall-back."""
+        if precision not in ('fp32', 'bf16'):
+            raise ValueError("precision must be 'fp32' or 'bf16', not %r" % (precision,))
+        entry = self._lib.simba_unfold if precision == 'fp32' else self._lib.simba_unfold_tc
         s0, kind = _device.to_device(s_0)
         acts, _ = _device.to_device(action_sequences)
         b, horizon = acts.shape[0], acts.shape[1]
@@ -101,9 +114,9 @@ class TransitionModel(BaseModel):
         traj = torch.empty((b, horizon + 1, self.observation_space_dim), dtype=torch.float32,
                            device=s0.device)
         h = self.model._ensure_handle()
-        _lib.check(self._lib.simba_unfold(h, _device.ptr(s0), _device.ptr(acts), _device.ptr(e),
-                                          int(seed), b, horizon, int(bool(self.sampling_propagation)),
-                                          _device.ptr(traj), _device.stream_ptr()))
+        _lib.check(entry(h, _device.ptr(s0), _device.ptr(acts), _device.ptr(e),
+                         int(seed), b, horizon, int(bool(self.sampling_propagation)),
+                         _device.ptr(traj), _device.stream_ptr()))
         return _device.like_input(traj, kind)
 
     def scale(self, inputs):

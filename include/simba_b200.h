@@ -239,10 +239,23 @@ int simba_planner_init_nccl(simba_planner_t* p, const void* unique_id_128_bytes_
 
 /* ---- model-level entry points (the other public methods of the reference's model interface) -- */
 /* TransitionModel.unfold_sequences — transition_model.py:64-77. s0 [B, O]; actions [B, H, A];
- * eps_or_null [H, B, O]; out_traj [B, H+1, O]. member map = tf.split (B % E == 0). fp32 path. */
+ * eps_or_null [H, B, O]; out_traj [B, H+1, O] (s_0, then s_1 .. s_H). member map = tf.split (B % E == 0).
+ * fp32 SIMT kernel (rollout_f32_kernel), 1 <= H <= 65535. Noise: eps_or_null, else Philox NOISE stream with
+ * row = batch index, iteration 0, state 0. DEVICE pointers, asynchronous on stream. */
 int simba_unfold(simba_model_t* m, const float* s0, const float* actions, const float* eps_or_null,
                  uint64_t seed, int32_t batch, int32_t horizon, int32_t sampling_propagation,
                  float* out_traj, void* stream);
+/* The same on the bf16 tcgen05 rollout kernels of a bf16 planner (the trajectory form of the kernel
+ * simba_unfold_tc_kernel reports): same arguments, layouts and noise contract, with weights, activations and
+ * normal draws rounded to bf16 as the planner's rollouts are; states stay fp32. s_0 is copied bit for bit.
+ * SIMBA_ERR_UNSUPPORTED for shapes no tcgen05 kernel covers (no fp32 fall-back). */
+int simba_unfold_tc(simba_model_t* m, const float* s0, const float* actions, const float* eps_or_null,
+                    uint64_t seed, int32_t batch, int32_t horizon, int32_t sampling_propagation,
+                    float* out_traj, void* stream);
+/* -> *kernel (simba_rollout_kernel) and *work_items that simba_unfold_tc would launch for this batch and
+ * horizon on the current device */
+int simba_unfold_tc_kernel(simba_model_t* m, int32_t batch, int32_t horizon, int32_t* kernel,
+                           int32_t* work_items);
 /* MlpEnsemble.forward / __call__ — mlp_ensemble.py:122-132,189-193. x [B, O+A] is used as given
  * (already scaled); out_mu, out_var [B, O]; out_sample_or_null = mu + sqrt(var) * eps. */
 int simba_ensemble_forward(simba_model_t* m, const float* x, const float* eps_or_null,
