@@ -22,16 +22,6 @@ using namespace simba;
 // ---------------------------------------------------------------------------------------------
 static thread_local std::string g_last_error;
 
-static int fail(int code, const char* fmt, ...) {
-  char buf[512];
-  va_list ap;
-  va_start(ap, fmt);
-  vsnprintf(buf, sizeof(buf), fmt, ap);
-  va_end(ap);
-  g_last_error = buf;
-  return code;
-}
-
 int simba::set_error(int code, const char* fmt, ...) {
   char buf[512];
   va_list ap;
@@ -42,25 +32,17 @@ int simba::set_error(int code, const char* fmt, ...) {
   return code;
 }
 
-#define CUDA_TRY(expr)                                                                    \
-  do {                                                                                    \
-    cudaError_t _e = (expr);                                                              \
-    if (_e != cudaSuccess)                                                                \
-      return fail(SIMBA_ERR_CUDA, "%s failed: %s (%s:%d)", #expr, cudaGetErrorString(_e), \
-                  __FILE__, __LINE__);                                                    \
-  } while (0)
-
 extern "C" const char* simba_last_error(void) { return g_last_error.c_str(); }
 extern "C" const char* simba_version(void) { return "simba_b200 0.1 (sm_100a)"; }
 
 extern "C" int simba_device_check(void) {
   int dev = 0;
-  CUDA_TRY(cudaGetDevice(&dev));
+  SIMBA_CUDA_TRY(cudaGetDevice(&dev));
   cudaDeviceProp prop;
-  CUDA_TRY(cudaGetDeviceProperties(&prop, dev));
+  SIMBA_CUDA_TRY(cudaGetDeviceProperties(&prop, dev));
   if (prop.major != 10)
-    return fail(SIMBA_ERR_ARCH, "device %d is sm_%d%d; this library is built for sm_100a only", dev,
-                prop.major, prop.minor);
+    return set_error(SIMBA_ERR_ARCH, "device %d is sm_%d%d; this library is built for sm_100a only", dev,
+                     prop.major, prop.minor);
   return SIMBA_OK;
 }
 
@@ -117,16 +99,16 @@ struct simba_model {
 };
 
 extern "C" int simba_model_create(const simba_model_config_t* cfg, simba_model_t** out) {
-  if (!cfg || !out) return fail(SIMBA_ERR_BAD_CONFIG, "null argument");
+  if (!cfg || !out) return set_error(SIMBA_ERR_BAD_CONFIG, "null argument");
   if (cfg->obs_dim < 1 || cfg->act_dim < 1 || cfg->act_dim > SIMBA_MAX_ACT)
-    return fail(SIMBA_ERR_BAD_CONFIG, "obs_dim %d / act_dim %d out of range (act_dim <= %d)",
-                cfg->obs_dim, cfg->act_dim, SIMBA_MAX_ACT);
+    return set_error(SIMBA_ERR_BAD_CONFIG, "obs_dim %d / act_dim %d out of range (act_dim <= %d)",
+                     cfg->obs_dim, cfg->act_dim, SIMBA_MAX_ACT);
   if (cfg->ensemble_size < 1 || cfg->ensemble_size > SIMBA_MAX_MEMBERS)
-    return fail(SIMBA_ERR_BAD_CONFIG, "ensemble_size %d out of range [1, %d]", cfg->ensemble_size,
-                SIMBA_MAX_MEMBERS);
+    return set_error(SIMBA_ERR_BAD_CONFIG, "ensemble_size %d out of range [1, %d]", cfg->ensemble_size,
+                     SIMBA_MAX_MEMBERS);
   if (cfg->n_layers < 1 || cfg->n_layers > 16 || cfg->units < 1 || cfg->units > 4096)
-    return fail(SIMBA_ERR_BAD_CONFIG, "n_layers %d / units %d out of range", cfg->n_layers,
-                cfg->units);
+    return set_error(SIMBA_ERR_BAD_CONFIG, "n_layers %d / units %d out of range", cfg->n_layers,
+                     cfg->units);
   int rc = simba_device_check();
   if (rc != SIMBA_OK) return rc;
   simba_model* m = new simba_model();
@@ -158,10 +140,10 @@ extern "C" int simba_model_destroy(simba_model_t* m) {
 
 extern "C" int simba_model_set_layer(simba_model_t* m, int32_t member, int32_t layer,
                                      const float* kernel, const float* bias) {
-  if (!m || !kernel || !bias) return fail(SIMBA_ERR_BAD_CONFIG, "null argument");
+  if (!m || !kernel || !bias) return set_error(SIMBA_ERR_BAD_CONFIG, "null argument");
   const int L = m->cfg.n_layers;
   if (member < 0 || member >= m->cfg.ensemble_size || layer < 0 || layer >= L + 2)
-    return fail(SIMBA_ERR_BAD_CONFIG, "member %d / layer %d out of range", member, layer);
+    return set_error(SIMBA_ERR_BAD_CONFIG, "member %d / layer %d out of range", member, layer);
   const int K = m->layer_in(layer), N = m->layer_out(layer);
   const int idx = member * (L + 2) + layer;
   m->kernels[idx].assign(kernel, kernel + (size_t)K * N);
@@ -173,13 +155,13 @@ extern "C" int simba_model_set_layer(simba_model_t* m, int32_t member, int32_t l
 
 extern "C" int simba_model_get_layer(simba_model_t* m, int32_t member, int32_t layer,
                                      float* kernel_out, float* bias_out) {
-  if (!m || !kernel_out || !bias_out) return fail(SIMBA_ERR_BAD_CONFIG, "null argument");
+  if (!m || !kernel_out || !bias_out) return set_error(SIMBA_ERR_BAD_CONFIG, "null argument");
   const int L = m->cfg.n_layers;
   if (member < 0 || member >= m->cfg.ensemble_size || layer < 0 || layer >= L + 2)
-    return fail(SIMBA_ERR_BAD_CONFIG, "member %d / layer %d out of range", member, layer);
+    return set_error(SIMBA_ERR_BAD_CONFIG, "member %d / layer %d out of range", member, layer);
   const int idx = member * (L + 2) + layer;
   if (!m->layer_set[idx])
-    return fail(SIMBA_ERR_NOT_READY, "member %d layer %d has no weights", member, layer);
+    return set_error(SIMBA_ERR_NOT_READY, "member %d layer %d has no weights", member, layer);
   memcpy(kernel_out, m->kernels[idx].data(), m->kernels[idx].size() * sizeof(float));
   memcpy(bias_out, m->biases[idx].data(), m->biases[idx].size() * sizeof(float));
   return SIMBA_OK;
@@ -189,16 +171,16 @@ const simba_model_config_t* simba::model_config(const simba_model_t* m) { return
 
 extern "C" int simba_model_set_scaler(simba_model_t* m, const float* mn, const float* mx,
                                       int32_t scale_features) {
-  if (!m) return fail(SIMBA_ERR_BAD_CONFIG, "null argument");
+  if (!m) return set_error(SIMBA_ERR_BAD_CONFIG, "null argument");
   const int IN = m->cfg.obs_dim + m->cfg.act_dim;
   m->scale_on = scale_features ? 1 : 0;
   if (m->scale_on) {
-    if (!mn || !mx) return fail(SIMBA_ERR_BAD_CONFIG, "scale_features set but bounds are null");
+    if (!mn || !mx) return set_error(SIMBA_ERR_BAD_CONFIG, "scale_features set but bounds are null");
     for (int k = 0; k < IN; ++k)
       if (!std::isfinite(mn[k]) || !std::isfinite(mx[k]))
-        return fail(SIMBA_ERR_NONFINITE,
-                    "inputs_min/max[%d] is not finite: the reference's scale() would produce NaN "
-                    "(transition_model.py:85-87); fit statistics first", k);
+        return set_error(SIMBA_ERR_NONFINITE,
+                         "inputs_min/max[%d] is not finite: the reference's scale() would produce NaN "
+                         "(transition_model.py:85-87); fit statistics first", k);
     m->smin.assign(mn, mn + IN);
     m->smax.assign(mx, mx + IN);
   } else {
@@ -382,22 +364,28 @@ static std::vector<float> pack_scaler(simba_model* m) {
   return delta;
 }
 
-// rollout_tc_wide.cu's 128-column variant runs only the bf16 shapes that every other tcgen05 kernel rejects
-static bool wide_obs_selected(int O, int A, int L, int U, int H) {
-  return !rollout_tc_supported(O, A, L, U, H) && !rollout_tc_wide_supported(64, O, A, L, U, H) &&
-         rollout_tc_wide_supported(128, O, A, L, U, H);
+// The one shape rule of the tcgen05 kernels: the family that runs a model, from its config alone. kTcOneCta stands
+// for rollout_tc.cu (whose variant choose_rollout picks), kTcWide and kTcWideObs for rollout_tc_wide.cu <64> and
+// <128>, kF32 for none. Each family runs every shape an earlier one rejects, and none other. simba_model_commit packs
+// the weight image of this family alone, so the kernel choose_rollout picks always finds its image.
+static RolloutKernel tc_family(const simba_model_config_t& c) {
+  const int O = c.obs_dim, A = c.act_dim, L = c.n_layers, U = c.units;
+  if (rollout_tc_supported(O, A, L, U)) return RolloutKernel::kTcOneCta;
+  if (rollout_tc_wide_supported(64, O, A, L, U)) return RolloutKernel::kTcWide;
+  if (rollout_tc_wide_supported(128, O, A, L, U)) return RolloutKernel::kTcWideObs;
+  return RolloutKernel::kF32;
 }
 
 extern "C" int simba_model_commit(simba_model_t* m) {
-  if (!m) return fail(SIMBA_ERR_BAD_CONFIG, "null argument");
+  if (!m) return set_error(SIMBA_ERR_BAD_CONFIG, "null argument");
   const auto& c = m->cfg;
   const int L = c.n_layers, U = c.units, O = c.obs_dim, IN = c.obs_dim + c.act_dim;
   for (size_t i = 0; i < m->layer_set.size(); ++i)
     if (!m->layer_set[i])
-      return fail(SIMBA_ERR_NOT_READY, "member %zu layer %zu has no weights", i / (L + 2),
-                  i % (L + 2));
-  if (!m->scaler_set) return fail(SIMBA_ERR_NOT_READY, "scaler not set");
-  CUDA_TRY(cudaSetDevice(m->device));
+      return set_error(SIMBA_ERR_NOT_READY, "member %zu layer %zu has no weights", i / (L + 2),
+                       i % (L + 2));
+  if (!m->scaler_set) return set_error(SIMBA_ERR_NOT_READY, "scaler not set");
+  SIMBA_CUDA_TRY(cudaSetDevice(m->device));
   // Device images are allocated on the first commit and updated IN PLACE afterwards (their sizes
   // are fixed by the immutable model config): planners that captured a CUDA graph keep valid
   // pointers when the weights or the scaler change (e.g. after every model.fit of the agent loop).
@@ -419,32 +407,31 @@ extern "C" int simba_model_commit(simba_model_t* m) {
     RolloutParams probe{};
     probe.g.O = O; probe.g.A = c.act_dim; probe.act_rows = act_rows;
     if (rollout_f32_smem_bytes(probe) > 227 * 1024)
-      return fail(SIMBA_ERR_UNSUPPORTED, "units %d: the rollout kernels keep a row tile's activations in "
-                  "shared memory, which holds at most ~780 hidden units", U);
+      return set_error(SIMBA_ERR_UNSUPPORTED, "units %d: the rollout kernels keep a row tile's activations in "
+                       "shared memory, which holds at most ~780 hidden units", U);
   }
   std::vector<float> w, b;
   pack_f32_image(m, w, b);
-  CUDA_TRY(cudaDeviceSynchronize());
-  CUDA_TRY(upload(m->d_w_f32, w));
-  CUDA_TRY(upload(m->d_bias_f32, b));
-  // bf16 images only for the shapes a tcgen05 kernel covers
+  SIMBA_CUDA_TRY(cudaDeviceSynchronize());
+  SIMBA_CUDA_TRY(upload(m->d_w_f32, w));
+  SIMBA_CUDA_TRY(upload(m->d_bias_f32, b));
+  // the bf16 image of the tcgen05 family that runs this shape, if any
+  const RolloutKernel family = tc_family(c);
   m->w_bf16_member_bytes = 0;
-  if (rollout_tc_supported(O, c.act_dim, L, U, 1)) {
+  if (family == RolloutKernel::kTcOneCta) {
     std::vector<uint16_t> img, bias_k16;
     m->w_bf16_member_bytes = pack_bf16_image(m, img, bias_k16);
-    CUDA_TRY(upload(m->d_w_bf16, img));
-    CUDA_TRY(upload(m->d_bias_k16, bias_k16));
+    SIMBA_CUDA_TRY(upload(m->d_w_bf16, img));
+    SIMBA_CUDA_TRY(upload(m->d_bias_k16, bias_k16));
   }
   m->w_wide_member_bytes = 0;
-  const int wide_sw = rollout_tc_wide_supported(64, O, c.act_dim, L, U, 1) ? 64
-                      : wide_obs_selected(O, c.act_dim, L, U, 1)            ? 128 : 0;
-  if (wide_sw != 0) {
+  if (family == RolloutKernel::kTcWide || family == RolloutKernel::kTcWideObs) {
     std::vector<uint16_t> img;
-    m->w_wide_member_bytes = pack_wide_image(m, wide_sw, img);
-    CUDA_TRY(upload(m->d_w_wide, img));
+    m->w_wide_member_bytes = pack_wide_image(m, family == RolloutKernel::kTcWide ? 64 : 128, img);
+    SIMBA_CUDA_TRY(upload(m->d_w_wide, img));
   }
-  CUDA_TRY(upload(m->d_smin, m->smin));
-  CUDA_TRY(upload(m->d_sdelta, pack_scaler(m)));
+  SIMBA_CUDA_TRY(upload(m->d_smin, m->smin));
+  SIMBA_CUDA_TRY(upload(m->d_sdelta, pack_scaler(m)));
   m->committed = true;
   ++m->generation;
   return SIMBA_OK;
@@ -475,20 +462,20 @@ static void fill_model_params(const simba_model* m, RolloutParams& prm) {
 // ---------------------------------------------------------------------------------------------
 static int build_geom(int S, int P, int N, int world, int rank, int H, int O, int A, int E,
                       int member_map, RowGeom& g) {
-  if (N % world) return fail(SIMBA_ERR_SHAPE, "n_samples %d not divisible by world_size %d", N, world);
+  if (N % world) return set_error(SIMBA_ERR_SHAPE, "n_samples %d not divisible by world_size %d", N, world);
   memset(&g, 0, sizeof(g));
   g.S = S; g.P = P; g.N = N; g.N_local = N / world; g.cand0 = rank * g.N_local;
   g.H = H; g.O = O; g.A = A; g.E = E;
   const long B = (long)P * N;
   if (member_map == SIMBA_MAP_SPLIT) {
     if (B % E)
-      return fail(SIMBA_ERR_SHAPE,
-                  "tf.split needs particles*n_samples (%ld) divisible by ensemble_size (%d) "
-                  "(mlp_ensemble.py:123); use member_map=PARTICLE", B, E);
+      return set_error(SIMBA_ERR_SHAPE,
+                       "tf.split needs particles*n_samples (%ld) divisible by ensemble_size (%d) "
+                       "(mlp_ensemble.py:123); use member_map=PARTICLE", B, E);
     if (world > 1 && P % E)
-      return fail(SIMBA_ERR_SHAPE,
-                  "member_map=SPLIT with world_size > 1 needs ensemble_size (%d) to divide "
-                  "particles (%d)", E, P);
+      return set_error(SIMBA_ERR_SHAPE,
+                       "member_map=SPLIT with world_size > 1 needs ensemble_size (%d) to divide "
+                       "particles (%d)", E, P);
     if (world == 1) {
       for (int e = 0; e < E; ++e) { g.lr_lo[e] = (int)(e * (B / E)); g.rows_per_state[e] = (int)(B / E); }
       return SIMBA_OK;
@@ -543,41 +530,53 @@ static void split_tail_items(std::vector<Tile>& tiles, int sms) {
   }
 }
 
-// The rollout kernel of a planner and the tile list it walks, from the shapes, the precision and the SM count.
-// The diagnostic switches SIMBA_B200_NO_TAIL_SPLIT and SIMBA_B200_NO_PAIR are read here and nowhere else.
-static int choose_rollout(const simba_model_config_t& mc, const simba_planner_config_t& cfg, const RowGeom& g,
-                          int sms, RolloutKernel& kernel, std::vector<Tile>& tiles) {
-  const int O = mc.obs_dim, A = mc.act_dim, L = mc.n_layers, U = mc.units, H = cfg.horizon, nc = cfg.scorer.n_constraints;
+// The rollout kernel and the tile list it walks, for a planner (nc constraints) or a trajectory call (traj, nc = 0),
+// from the precision, the row geometry and the SM count. fp32 runs rollout_f32_kernel on 32-row tiles; bf16 runs the
+// tcgen05 family tc_family names on 128-row tiles, or fails. The diagnostic switches SIMBA_B200_NO_TAIL_SPLIT and
+// SIMBA_B200_NO_PAIR are read here and nowhere else.
+static int choose_rollout(const simba_model_config_t& mc, int precision, const RowGeom& g, int nc, bool traj, int sms,
+                          RolloutKernel& kernel, std::vector<Tile>& tiles) {
+  const int L = mc.n_layers, U = mc.units;
   kernel = RolloutKernel::kF32;
-  build_tiles(g, cfg.precision == SIMBA_PREC_FP32 ? kF32TileRows : kTcTileRows, tiles);
-  if (cfg.precision == SIMBA_PREC_FP32) return SIMBA_OK;
-  if (rollout_tc_supported(O, A, L, U, H)) {
-    kernel = RolloutKernel::kTcOneCta;
+  build_tiles(g, precision == SIMBA_PREC_FP32 ? kF32TileRows : kTcTileRows, tiles);
+  if (precision == SIMBA_PREC_FP32) return SIMBA_OK;
+  kernel = tc_family(mc);
+  if (kernel == RolloutKernel::kTcOneCta) {
     if ((int)tiles.size() > sms && rollout_tc_two_tiles_fit(L, nc)) {
       // more tiles than SMs: two tiles per CTA so one tile's MMAs overlap the other's epilogue
       kernel = RolloutKernel::kTcTwoTile;
       build_tiles(g, kTcTileRows, tiles, 2);
       if (getenv("SIMBA_B200_NO_TAIL_SPLIT") == nullptr) split_tail_items(tiles, sms);
-    } else if ((int)tiles.size() * 2 <= sms && rollout_tc_pair_fits(L, nc) && getenv("SIMBA_B200_NO_PAIR") == nullptr) {
+    } else if (!traj && (int)tiles.size() * 2 <= sms && rollout_tc_pair_fits(L, nc) &&
+               getenv("SIMBA_B200_NO_PAIR") == nullptr) {
       // few tiles (a single plan): two SMs per tile, the head pass split between them
       kernel = RolloutKernel::kTcPair;
     }
     return SIMBA_OK;
   }
-  if (rollout_tc_wide_supported(64, O, A, L, U, H) && rollout_tc_wide_fits(64, L, U, nc)) {
-    kernel = RolloutKernel::kTcWide;
-    return SIMBA_OK;
+  if (kernel == RolloutKernel::kTcWide && rollout_tc_wide_fits(64, L, U, nc)) return SIMBA_OK;
+  if (kernel == RolloutKernel::kTcWideObs && rollout_tc_wide_fits(128, L, U, nc)) return SIMBA_OK;
+  return set_error(SIMBA_ERR_UNSUPPORTED,
+                   "no bf16 tcgen05 kernel covers obs_dim %d, act_dim %d, %d x %d units with %d constraints: they "
+                   "cover units <= 128 (obs_dim <= 60, obs_dim+act_dim <= 64, <= 5 layers), 128 < units <= ~416 (less "
+                   "with several constrained lidars; obs_dim+act_dim <= 62) and, for other shapes, obs_dim+act_dim <= "
+                   "126 with obs_dim <= 124, act_dim <= 4, units <= 384 and <= 6 layers; use fp32 for this shape",
+                   mc.obs_dim, mc.act_dim, L, U, nc);
+}
+
+// the work items of a launch: the two-tile kernel's item i is tiles [2i, 2i + 1]
+static int32_t n_work_items(RolloutKernel kernel, const std::vector<Tile>& tiles) {
+  return (int32_t)tiles.size() / (kernel == RolloutKernel::kTcTwoTile ? 2 : 1);
+}
+
+cudaError_t simba::launch_rollout(const RolloutParams& prm, cudaStream_t stream) {
+  if (prm.n_tiles == 0) return cudaSuccess;
+  switch (prm.kernel) {
+    case RolloutKernel::kF32: return launch_rollout_f32(prm, stream);
+    case RolloutKernel::kTcWide:
+    case RolloutKernel::kTcWideObs: return launch_rollout_tc_wide(prm, stream);
+    default: return launch_rollout_tc(prm, stream);
   }
-  if (wide_obs_selected(O, A, L, U, H) && rollout_tc_wide_fits(128, L, U, nc)) {
-    kernel = RolloutKernel::kTcWideObs;
-    return SIMBA_OK;
-  }
-  return fail(SIMBA_ERR_UNSUPPORTED,
-              "bf16 tcgen05 rollout covers units <= 128 (obs_dim <= 60, obs_dim+act_dim <= 64, <= 5 layers), "
-              "wide models with 128 < units <= ~416 (less with several constrained lidars; obs_dim+act_dim <= 62) "
-              "and, for other shapes, obs_dim+act_dim <= 126 with obs_dim <= 124, act_dim <= 4, units <= 384 and "
-              "<= 6 layers; "
-              "use precision fp32 for this shape");
 }
 
 // ---------------------------------------------------------------------------------------------
@@ -612,14 +611,14 @@ int nccl_load() {
     if (g_nccl.lib) break;
     g_nccl.lib = dlopen(n, RTLD_NOW);
   }
-  if (!g_nccl.lib) return fail(SIMBA_ERR_NCCL, "cannot load libnccl.so.2: %s", dlerror());
+  if (!g_nccl.lib) return set_error(SIMBA_ERR_NCCL, "cannot load libnccl.so.2: %s", dlerror());
   g_nccl.get_unique_id = (nccl_get_unique_id_t)dlsym(g_nccl.lib, "ncclGetUniqueId");
   g_nccl.comm_init_rank = (nccl_comm_init_rank_t)dlsym(g_nccl.lib, "ncclCommInitRank");
   g_nccl.all_gather = (nccl_all_gather_t)dlsym(g_nccl.lib, "ncclAllGather");
   g_nccl.comm_destroy = (nccl_comm_destroy_t)dlsym(g_nccl.lib, "ncclCommDestroy");
   g_nccl.get_error_string = (nccl_get_error_string_t)dlsym(g_nccl.lib, "ncclGetErrorString");
   if (!g_nccl.get_unique_id || !g_nccl.comm_init_rank || !g_nccl.all_gather || !g_nccl.comm_destroy)
-    return fail(SIMBA_ERR_NCCL, "libnccl is missing a required symbol");
+    return set_error(SIMBA_ERR_NCCL, "libnccl is missing a required symbol");
   return SIMBA_OK;
 }
 }  // namespace
@@ -628,8 +627,8 @@ int nccl_load() {
   do {                                                                                     \
     int _r = (expr);                                                                       \
     if (_r != 0)                                                                           \
-      return fail(SIMBA_ERR_NCCL, "%s failed: %s", #expr,                                  \
-                  g_nccl.get_error_string ? g_nccl.get_error_string(_r) : "nccl error");   \
+      return set_error(SIMBA_ERR_NCCL, "%s failed: %s", #expr,                             \
+                       g_nccl.get_error_string ? g_nccl.get_error_string(_r) : "nccl error");\
   } while (0)
 
 // ---------------------------------------------------------------------------------------------
@@ -698,20 +697,20 @@ static int beta_count_threshold(int P, float thr, float mu, float sigma) {
 }
 
 static int validate_scorer(const simba_scorer_t& s, int O) {
-  if (s.goal_dist_index >= O) return fail(SIMBA_ERR_BAD_CONFIG, "goal_dist_index out of range");
+  if (s.goal_dist_index >= O) return set_error(SIMBA_ERR_BAD_CONFIG, "goal_dist_index out of range");
   if (s.goal_dist_index < 0 &&
       (s.goal_begin < 0 || s.goal_end > O || s.goal_begin >= s.goal_end))
-    return fail(SIMBA_ERR_BAD_CONFIG, "goal lidar slice [%d, %d) invalid for obs_dim %d",
-                s.goal_begin, s.goal_end, O);
+    return set_error(SIMBA_ERR_BAD_CONFIG, "goal lidar slice [%d, %d) invalid for obs_dim %d",
+                     s.goal_begin, s.goal_end, O);
   if (s.n_constraints < 0 || s.n_constraints > SIMBA_MAX_CONSTRAINTS)
-    return fail(SIMBA_ERR_BAD_CONFIG, "n_constraints %d out of range", s.n_constraints);
+    return set_error(SIMBA_ERR_BAD_CONFIG, "n_constraints %d out of range", s.n_constraints);
   for (int j = 0; j < s.n_constraints; ++j)
     if (s.con_begin[j] < 0 || s.con_end[j] > O || s.con_begin[j] >= s.con_end[j])
-      return fail(SIMBA_ERR_BAD_CONFIG, "constraint slice %d invalid", j);
+      return set_error(SIMBA_ERR_BAD_CONFIG, "constraint slice %d invalid", j);
   if (!s.constrain_indicator && s.n_constraints > 1)
-    return fail(SIMBA_ERR_UNSUPPORTED,
-                "constrain_indicator=False with more than one constrained object class is not "
-                "offered on the fused path (per-step cost must fit one bit)");
+    return set_error(SIMBA_ERR_UNSUPPORTED,
+                     "constrain_indicator=False with more than one constrained object class is not "
+                     "offered on the fused path (per-step cost must fit one bit)");
   return SIMBA_OK;
 }
 
@@ -739,45 +738,45 @@ extern "C" int simba_planner_destroy(simba_planner_t* p) {
 
 extern "C" int simba_planner_create(simba_model_t* model, const simba_planner_config_t* cfg,
                                     simba_planner_t** out) {
-  if (!model || !cfg || !out) return fail(SIMBA_ERR_BAD_CONFIG, "null argument");
-  if (!model->committed) return fail(SIMBA_ERR_NOT_READY, "model not committed");
+  if (!model || !cfg || !out) return set_error(SIMBA_ERR_BAD_CONFIG, "null argument");
+  if (!model->committed) return set_error(SIMBA_ERR_NOT_READY, "model not committed");
   const auto& mc = model->cfg;
   if (cfg->horizon < 1 || cfg->horizon > SIMBA_MAX_HORIZON)
-    return fail(SIMBA_ERR_BAD_CONFIG, "horizon %d out of range [1, %d]", cfg->horizon,
-                SIMBA_MAX_HORIZON);
+    return set_error(SIMBA_ERR_BAD_CONFIG, "horizon %d out of range [1, %d]", cfg->horizon,
+                     SIMBA_MAX_HORIZON);
   if (cfg->horizon * mc.act_dim > 1024)
-    return fail(SIMBA_ERR_BAD_CONFIG, "horizon*act_dim %d > 1024", cfg->horizon * mc.act_dim);
+    return set_error(SIMBA_ERR_BAD_CONFIG, "horizon*act_dim %d > 1024", cfg->horizon * mc.act_dim);
   if (cfg->iterations < 1 || cfg->iterations > 65535)
-    return fail(SIMBA_ERR_BAD_CONFIG, "iterations %d out of range", cfg->iterations);
+    return set_error(SIMBA_ERR_BAD_CONFIG, "iterations %d out of range", cfg->iterations);
   if (cfg->n_samples < 1 || cfg->n_elite < 1 || cfg->n_elite > cfg->n_samples)
-    return fail(SIMBA_ERR_BAD_CONFIG, "need 1 <= n_elite (%d) <= n_samples (%d)", cfg->n_elite,
-                cfg->n_samples);
+    return set_error(SIMBA_ERR_BAD_CONFIG, "need 1 <= n_elite (%d) <= n_samples (%d)", cfg->n_elite,
+                     cfg->n_samples);
   if (cfg->particles < 1 || cfg->particles > 255)
-    return fail(SIMBA_ERR_BAD_CONFIG, "particles %d out of range [1, 255]", cfg->particles);
-  if (cfg->n_states < 1) return fail(SIMBA_ERR_BAD_CONFIG, "n_states %d < 1", cfg->n_states);
+    return set_error(SIMBA_ERR_BAD_CONFIG, "particles %d out of range [1, 255]", cfg->particles);
+  if (cfg->n_states < 1) return set_error(SIMBA_ERR_BAD_CONFIG, "n_states %d < 1", cfg->n_states);
   if (cfg->world_size < 1 || cfg->rank < 0 || cfg->rank >= cfg->world_size)
-    return fail(SIMBA_ERR_BAD_CONFIG, "rank %d / world_size %d invalid", cfg->rank, cfg->world_size);
+    return set_error(SIMBA_ERR_BAD_CONFIG, "rank %d / world_size %d invalid", cfg->rank, cfg->world_size);
   if (cfg->objective < 0 || cfg->objective > 3)
-    return fail(SIMBA_ERR_BAD_CONFIG, "objective %d unknown", cfg->objective);
+    return set_error(SIMBA_ERR_BAD_CONFIG, "objective %d unknown", cfg->objective);
   if (cfg->precision != SIMBA_PREC_FP32 && cfg->precision != SIMBA_PREC_BF16_TC)
-    return fail(SIMBA_ERR_BAD_CONFIG, "precision %d unknown", cfg->precision);
+    return set_error(SIMBA_ERR_BAD_CONFIG, "precision %d unknown", cfg->precision);
   int rc = validate_scorer(cfg->scorer, mc.obs_dim);
   if (rc != SIMBA_OK) return rc;
   if ((long)cfg->n_states * cfg->particles * cfg->n_samples > 0x7fffffffL / 2)
-    return fail(SIMBA_ERR_BAD_CONFIG, "n_states*particles*n_samples too large");
+    return set_error(SIMBA_ERR_BAD_CONFIG, "n_states*particles*n_samples too large");
 
   simba_planner* p = new simba_planner();
   p->model = model;
   p->cfg = *cfg;
   p->device = model->device;
   cudaError_t ce = cudaSetDevice(p->device);
-  if (ce != cudaSuccess) { delete p; return fail(SIMBA_ERR_CUDA, "cudaSetDevice: %s", cudaGetErrorString(ce)); }
+  if (ce != cudaSuccess) { delete p; return set_error(SIMBA_ERR_CUDA, "cudaSetDevice: %s", cudaGetErrorString(ce)); }
   rc = build_geom(cfg->n_states, cfg->particles, cfg->n_samples, cfg->world_size, cfg->rank,
                   cfg->horizon, mc.obs_dim, mc.act_dim, mc.ensemble_size, cfg->member_map, p->geom);
   if (rc != SIMBA_OK) { delete p; return rc; }
   ce = cudaDeviceGetAttribute(&p->n_sms, cudaDevAttrMultiProcessorCount, p->device);
-  if (ce != cudaSuccess) { delete p; return fail(SIMBA_ERR_CUDA, "SM count: %s", cudaGetErrorString(ce)); }
-  rc = choose_rollout(mc, *cfg, p->geom, p->n_sms, p->kernel, p->tiles);
+  if (ce != cudaSuccess) { delete p; return set_error(SIMBA_ERR_CUDA, "SM count: %s", cudaGetErrorString(ce)); }
+  rc = choose_rollout(mc, cfg->precision, p->geom, cfg->scorer.n_constraints, false, p->n_sms, p->kernel, p->tiles);
   if (rc != SIMBA_OK) { delete p; return rc; }
 
   p->fused_update = cfg->world_size == 1 && cfg->n_samples <= 1024 && getenv("SIMBA_B200_NO_FUSE") == nullptr;
@@ -793,8 +792,8 @@ extern "C" int simba_planner_create(simba_model_t* model, const simba_planner_co
     cudaError_t _e = cudaMalloc((void**)&(ptr), (bytes));                                 \
     if (_e != cudaSuccess) {                                                              \
       planner_free(p); delete p;                                                          \
-      return fail(SIMBA_ERR_CUDA, "cudaMalloc(%zu) failed: %s", (size_t)(bytes),          \
-                  cudaGetErrorString(_e));                                                \
+      return set_error(SIMBA_ERR_CUDA, "cudaMalloc(%zu) failed: %s", (size_t)(bytes),     \
+                       cudaGetErrorString(_e));                                           \
     }                                                                                     \
   } while (0)
   PL_ALLOC(p->d_tiles, std::max<size_t>(1, p->tiles.size()) * sizeof(Tile));
@@ -831,8 +830,8 @@ extern "C" int simba_planner_create(simba_model_t* model, const simba_planner_co
       cudaStreamCreateWithFlags(&p->own_stream, cudaStreamNonBlocking) != cudaSuccess ||
       cudaEventCreateWithFlags(&p->plan_done, cudaEventDisableTiming) != cudaSuccess) {
     planner_free(p); delete p;
-    return fail(SIMBA_ERR_CUDA, "planner staging allocation failed: %s",
-                cudaGetErrorString(cudaGetLastError()));
+    return set_error(SIMBA_ERR_CUDA, "planner staging allocation failed: %s",
+                     cudaGetErrorString(cudaGetLastError()));
   }
   *out = p;
   return SIMBA_OK;
@@ -840,7 +839,7 @@ extern "C" int simba_planner_create(simba_model_t* model, const simba_planner_co
 
 extern "C" int simba_planner_set_external_draws(simba_planner_t* p, const float* z_actions,
                                                 const float* eps, const float* z_final) {
-  if (!p) return fail(SIMBA_ERR_BAD_CONFIG, "null argument");
+  if (!p) return set_error(SIMBA_ERR_BAD_CONFIG, "null argument");
   p->ext_z_actions = z_actions; p->ext_eps = eps; p->ext_z_final = z_final;
   if (p->graph_exec) { cudaGraphExecDestroy(p->graph_exec); p->graph_exec = nullptr; }
   if (p->graph) { cudaGraphDestroy(p->graph); p->graph = nullptr; }
@@ -848,21 +847,21 @@ extern "C" int simba_planner_set_external_draws(simba_planner_t* p, const float*
 }
 
 extern "C" int simba_planner_count_threshold(simba_planner_t* p, int32_t* out) {
-  if (!p || !out) return fail(SIMBA_ERR_BAD_CONFIG, "null argument");
+  if (!p || !out) return set_error(SIMBA_ERR_BAD_CONFIG, "null argument");
   *out = p->c_max;
   return SIMBA_OK;
 }
 
 extern "C" int simba_planner_rollout_kernel(simba_planner_t* p, int32_t* kernel, int32_t* work_items) {
-  if (!p || !kernel || !work_items) return fail(SIMBA_ERR_BAD_CONFIG, "null argument");
+  if (!p || !kernel || !work_items) return set_error(SIMBA_ERR_BAD_CONFIG, "null argument");
   *kernel = (int32_t)p->kernel;
-  *work_items = (int32_t)p->tiles.size() / (p->kernel == RolloutKernel::kTcTwoTile ? 2 : 1);
+  *work_items = n_work_items(p->kernel, p->tiles);
   return SIMBA_OK;
 }
 
 extern "C" int simba_planner_buffer(simba_planner_t* p, int32_t which, void** out_ptr,
                                     uint64_t* out_bytes) {
-  if (!p || !out_ptr || !out_bytes) return fail(SIMBA_ERR_BAD_CONFIG, "null argument");
+  if (!p || !out_ptr || !out_bytes) return set_error(SIMBA_ERR_BAD_CONFIG, "null argument");
   const auto& c = p->cfg; const auto& mc = p->model->cfg;
   const uint64_t S = c.n_states, N = c.n_samples, Nl = p->geom.N_local, P = c.particles;
   const uint64_t HA = (uint64_t)c.horizon * mc.act_dim, A = mc.act_dim, W = c.world_size;
@@ -880,7 +879,7 @@ extern "C" int simba_planner_buffer(simba_planner_t* p, int32_t which, void** ou
     case SIMBA_BUF_BEST_SCORE: *out_ptr = p->best_score; *out_bytes = S * 4; break;
     case SIMBA_BUF_ACTIVE: *out_ptr = p->active; *out_bytes = S * 4; break;
     case SIMBA_BUF_SCORES: *out_ptr = p->scores; *out_bytes = S * N * 4; break;
-    default: return fail(SIMBA_ERR_BAD_CONFIG, "unknown buffer %d", which);
+    default: return set_error(SIMBA_ERR_BAD_CONFIG, "unknown buffer %d", which);
   }
   return SIMBA_OK;
 }
@@ -890,8 +889,8 @@ extern "C" int simba_planner_copy_buffer(simba_planner_t* p, int32_t which, void
   uint64_t bytes = 0;
   int rc = simba_planner_buffer(p, which, &src, &bytes);
   if (rc != SIMBA_OK) return rc;
-  if (!dst) return fail(SIMBA_ERR_BAD_CONFIG, "null argument");
-  CUDA_TRY(cudaMemcpyAsync(dst, src, bytes, cudaMemcpyDeviceToDevice, (cudaStream_t)stream));
+  if (!dst) return set_error(SIMBA_ERR_BAD_CONFIG, "null argument");
+  SIMBA_CUDA_TRY(cudaMemcpyAsync(dst, src, bytes, cudaMemcpyDeviceToDevice, (cudaStream_t)stream));
   return SIMBA_OK;
 }
 
@@ -912,9 +911,9 @@ static SampleParams make_sample_params(simba_planner_t* p, const float* mu, cons
 static int do_sample_actions(simba_planner_t* p, const float* mu, const float* sigma,
                              const float* z, uint64_t seed, const uint64_t* seed_ptr,
                              int32_t iteration, const int32_t* active, float* out, void* stream) {
-  if (!p || !mu || !sigma || !out) return fail(SIMBA_ERR_BAD_CONFIG, "null argument");
+  if (!p || !mu || !sigma || !out) return set_error(SIMBA_ERR_BAD_CONFIG, "null argument");
   const SampleParams sp = make_sample_params(p, mu, sigma, z, seed, seed_ptr, iteration, active, out);
-  CUDA_TRY(launch_sample_actions(sp, (cudaStream_t)stream));
+  SIMBA_CUDA_TRY(launch_sample_actions(sp, (cudaStream_t)stream));
   return SIMBA_OK;
 }
 
@@ -929,7 +928,7 @@ static int do_rollout_score(simba_planner_t* p, const float* states, const float
                             int32_t iteration, const int32_t* active, float* row_return,
                             uint64_t* row_costmask, float* row_costsum, void* stream, bool pdl = false) {
   if (!p || !states || !actions || !row_return || !row_costmask || !row_costsum)
-    return fail(SIMBA_ERR_BAD_CONFIG, "null argument");
+    return set_error(SIMBA_ERR_BAD_CONFIG, "null argument");
   RolloutParams prm{};
   prm.seed_ptr = seed_ptr;
   prm.g = p->geom;
@@ -952,12 +951,7 @@ static int do_rollout_score(simba_planner_t* p, const float* states, const float
   if (const char* tlp = getenv("SIMBA_TC_TIMELINE_PTR"))
     prm.timeline = reinterpret_cast<long long*>(strtoull(tlp, nullptr, 10));
 #endif
-  switch (p->kernel) {
-    case RolloutKernel::kF32: CUDA_TRY(launch_rollout_f32(prm, prm.n_tiles, (cudaStream_t)stream)); break;
-    case RolloutKernel::kTcWide:
-    case RolloutKernel::kTcWideObs: CUDA_TRY(launch_rollout_tc_wide(prm, prm.n_tiles, (cudaStream_t)stream)); break;
-    default: CUDA_TRY(launch_rollout_tc(prm, prm.n_tiles, (cudaStream_t)stream));
-  }
+  SIMBA_CUDA_TRY(launch_rollout(prm, (cudaStream_t)stream));
   return SIMBA_OK;
 }
 
@@ -1019,23 +1013,23 @@ extern "C" int simba_score_reduce(simba_planner_t* p, const float* row_return,
                                   const uint64_t* row_costmask, const float* row_costsum,
                                   const int32_t* active, float* out_pairs_local, void* stream) {
   if (!p || !row_return || !row_costmask || !row_costsum || !out_pairs_local)
-    return fail(SIMBA_ERR_BAD_CONFIG, "null argument");
+    return set_error(SIMBA_ERR_BAD_CONFIG, "null argument");
   const ReduceParams rp = make_reduce_params(p, row_return, row_costmask, row_costsum, active, out_pairs_local);
-  CUDA_TRY(launch_score_reduce(rp, (cudaStream_t)stream));
+  SIMBA_CUDA_TRY(launch_score_reduce(rp, (cudaStream_t)stream));
   return SIMBA_OK;
 }
 
 extern "C" int simba_allgather_scores(simba_planner_t* p, const float* pairs_local,
                                       float* out_pairs_all, void* stream) {
-  if (!p || !pairs_local || !out_pairs_all) return fail(SIMBA_ERR_BAD_CONFIG, "null argument");
+  if (!p || !pairs_local || !out_pairs_all) return set_error(SIMBA_ERR_BAD_CONFIG, "null argument");
   const size_t count = (size_t)p->cfg.n_states * p->geom.N_local * 2;
   if (p->cfg.world_size == 1) {
     if (pairs_local != out_pairs_all)
-      CUDA_TRY(cudaMemcpyAsync(out_pairs_all, pairs_local, count * 4, cudaMemcpyDeviceToDevice,
+      SIMBA_CUDA_TRY(cudaMemcpyAsync(out_pairs_all, pairs_local, count * 4, cudaMemcpyDeviceToDevice,
                                (cudaStream_t)stream));
     return SIMBA_OK;
   }
-  if (!p->comm) return fail(SIMBA_ERR_NOT_READY, "world_size > 1 but simba_planner_init_nccl was not called");
+  if (!p->comm) return set_error(SIMBA_ERR_NOT_READY, "world_size > 1 but simba_planner_init_nccl was not called");
   NCCL_TRY(g_nccl.all_gather(pairs_local, out_pairs_all, count, kNcclFloat, p->comm,
                              (cudaStream_t)stream));
   return SIMBA_OK;
@@ -1045,27 +1039,27 @@ extern "C" int simba_select_elites(simba_planner_t* p, const float* pairs_all, c
                                    const int32_t* active, int32_t* out_elite, float* out_scores,
                                    float* best_action, float* best_score, void* stream) {
   if (!p || !pairs_all || !actions || !out_elite || !best_action || !best_score)
-    return fail(SIMBA_ERR_BAD_CONFIG, "null argument");
+    return set_error(SIMBA_ERR_BAD_CONFIG, "null argument");
   const SelectParams sp = make_select_params(p, pairs_all, actions, active, out_elite, out_scores,
                                              best_action, best_score);
-  CUDA_TRY(launch_select_elites(sp, (cudaStream_t)stream));
+  SIMBA_CUDA_TRY(launch_select_elites(sp, (cudaStream_t)stream));
   return SIMBA_OK;
 }
 
 extern "C" int simba_refit(simba_planner_t* p, const float* actions, const int32_t* elite, float* mu,
                            float* sigma, int32_t* active, int32_t* iterations_run, void* stream) {
-  if (!p || !actions || !elite || !mu || !sigma) return fail(SIMBA_ERR_BAD_CONFIG, "null argument");
+  if (!p || !actions || !elite || !mu || !sigma) return set_error(SIMBA_ERR_BAD_CONFIG, "null argument");
   const RefitParams rp = make_refit_params(p, actions, elite, mu, sigma, active, iterations_run);
-  CUDA_TRY(launch_refit(rp, (cudaStream_t)stream));
+  SIMBA_CUDA_TRY(launch_refit(rp, (cudaStream_t)stream));
   return SIMBA_OK;
 }
 
 static int do_finalize_action(simba_planner_t* p, const float* best_action, const float* z,
                               uint64_t seed, const uint64_t* seed_ptr, float* out_action,
                               void* stream) {
-  if (!p || !best_action || !out_action) return fail(SIMBA_ERR_BAD_CONFIG, "null argument");
+  if (!p || !best_action || !out_action) return set_error(SIMBA_ERR_BAD_CONFIG, "null argument");
   const FinalizeParams fp = make_finalize_params(p, best_action, z, seed, seed_ptr, out_action);
-  CUDA_TRY(launch_finalize(fp, (cudaStream_t)stream));
+  SIMBA_CUDA_TRY(launch_finalize(fp, (cudaStream_t)stream));
   return SIMBA_OK;
 }
 
@@ -1094,12 +1088,12 @@ static int enqueue_plan(simba_planner* p, cudaStream_t st, int* n_launches) {
   ip.active = p->active; ip.iterations_run = p->iters;
   const bool multi = c.world_size > 1;
   float* pairs_all = multi ? p->pairs_all : p->pairs_local;
-  if (!p->fused_update) { CUDA_TRY(launch_plan_init(ip, st)); ++launches; }
+  if (!p->fused_update) { SIMBA_CUDA_TRY(launch_plan_init(ip, st)); ++launches; }
   if (p->fused_update) {
     // small population on one rank: init + sample(0) in one launch, then per iteration rollout + one fused update kernel
     const float* z0 = p->ext_z_actions;
     const SampleParams sp0 = make_sample_params(p, p->mu, p->sigma, z0, 0, sp, 0, p->active, p->actions);
-    CUDA_TRY(launch_plan_begin(ip, sp0, st)); ++launches;
+    SIMBA_CUDA_TRY(launch_plan_begin(ip, sp0, st)); ++launches;
     int rc = SIMBA_OK;
     for (int it = 0; it < c.iterations; ++it) {
       const float* eps = p->ext_eps ? p->ext_eps + (size_t)it * S * c.horizon * B * O : nullptr;
@@ -1126,7 +1120,7 @@ static int enqueue_plan(simba_planner* p, cudaStream_t st, int* n_launches) {
       if (const char* tlp = getenv("SIMBA_TC_TIMELINE_PTR"))
         u.timeline = reinterpret_cast<long long*>(strtoull(tlp, nullptr, 10)) + (3 * 64 + 1 + it) * 64;
 #endif
-      CUDA_TRY(launch_cem_update(u, st)); ++launches;
+      SIMBA_CUDA_TRY(launch_cem_update(u, st)); ++launches;
     }
     if (n_launches) *n_launches = launches;
     return SIMBA_OK;
@@ -1138,7 +1132,7 @@ static int enqueue_plan(simba_planner* p, cudaStream_t st, int* n_launches) {
     // recompute the elite rows the other ranks sampled (SURVEY.md section 8 e)
     SampleParams smp = make_sample_params(p, p->mu, p->sigma, z, 0, sp, it, p->active, p->actions);
     if (multi) { smp.cand0 = p->geom.cand0; smp.n_cand = p->geom.N_local; }
-    CUDA_TRY(launch_sample_actions(smp, st)); ++launches;
+    SIMBA_CUDA_TRY(launch_sample_actions(smp, st)); ++launches;
     int rc = do_rollout_score(p, p->d_states, p->actions, eps, 0, sp, it, p->active, p->row_ret,
                               p->row_cmask, p->row_csum, st);
     if (rc) return rc; ++launches;
@@ -1152,33 +1146,33 @@ static int enqueue_plan(simba_planner* p, cudaStream_t st, int* n_launches) {
                                           p->best_action, p->best_score);
     RefitParams rfp = make_refit_params(p, p->actions, p->elite, p->mu, p->sigma, p->active, p->iters);
     if (multi) { slp.regen = 1; slp.sample = smp; rfp.regen = 1; rfp.sample = smp; }
-    CUDA_TRY(launch_select_elites(slp, st)); ++launches;
-    CUDA_TRY(launch_refit(rfp, st)); ++launches;
+    SIMBA_CUDA_TRY(launch_select_elites(slp, st)); ++launches;
+    SIMBA_CUDA_TRY(launch_refit(rfp, st)); ++launches;
   }
   int rc = do_finalize_action(p, p->best_action, p->ext_z_final, 0, sp, p->d_out_action, st);
   if (rc) return rc; ++launches;
-  CUDA_TRY(launch_plan_output(p->best_score, p->iters, p->d_out_score, p->d_out_iters, c.n_states, st));
+  SIMBA_CUDA_TRY(launch_plan_output(p->best_score, p->iters, p->d_out_score, p->d_out_iters, c.n_states, st));
   ++launches;
   if (n_launches) *n_launches = launches;
   return SIMBA_OK;
 }
 
 static int ensure_graph(simba_planner* p) {
-  if (!p->model->committed) return fail(SIMBA_ERR_NOT_READY, "model has uncommitted changes");
+  if (!p->model->committed) return set_error(SIMBA_ERR_NOT_READY, "model has uncommitted changes");
   if (p->graph_exec && p->graph_generation == p->model->generation) return SIMBA_OK;
   // kernel parameters (scaler constants, flags) are baked into the graph nodes: a re-committed
   // model needs a fresh capture (weights themselves are updated in place and would not)
   if (p->graph_exec) { cudaGraphExecDestroy(p->graph_exec); p->graph_exec = nullptr; }
   if (p->graph) { cudaGraphDestroy(p->graph); p->graph = nullptr; }
-  CUDA_TRY(cudaStreamBeginCapture(p->own_stream, cudaStreamCaptureModeThreadLocal));
+  SIMBA_CUDA_TRY(cudaStreamBeginCapture(p->own_stream, cudaStreamCaptureModeThreadLocal));
   int launches = 0;
   int rc = enqueue_plan(p, p->own_stream, &launches);
   cudaGraph_t g = nullptr;
   cudaError_t ce = cudaStreamEndCapture(p->own_stream, &g);
   if (rc != SIMBA_OK) { if (g) cudaGraphDestroy(g); return rc; }
-  if (ce != cudaSuccess) return fail(SIMBA_ERR_CUDA, "graph capture failed: %s", cudaGetErrorString(ce));
+  if (ce != cudaSuccess) return set_error(SIMBA_ERR_CUDA, "graph capture failed: %s", cudaGetErrorString(ce));
   p->graph = g;
-  CUDA_TRY(cudaGraphInstantiate(&p->graph_exec, p->graph, 0));
+  SIMBA_CUDA_TRY(cudaGraphInstantiate(&p->graph_exec, p->graph, 0));
   p->launches_per_plan = launches;
   p->graph_generation = p->model->generation;
   return SIMBA_OK;
@@ -1190,12 +1184,12 @@ static int ensure_graph(simba_planner* p) {
 static int upload_seed(simba_planner* p, uint64_t seed, cudaStream_t st) {
   uint64_t* slot = p->h_seed_ring + (p->seed_slot++ & 63);
   *slot = seed;
-  CUDA_TRY(cudaMemcpyAsync(p->d_seed, slot, 8, cudaMemcpyHostToDevice, st));
+  SIMBA_CUDA_TRY(cudaMemcpyAsync(p->d_seed, slot, 8, cudaMemcpyHostToDevice, st));
   return SIMBA_OK;
 }
 
 extern "C" int simba_planner_launches_per_plan(simba_planner_t* p, int32_t* out) {
-  if (!p || !out) return fail(SIMBA_ERR_BAD_CONFIG, "null argument");
+  if (!p || !out) return set_error(SIMBA_ERR_BAD_CONFIG, "null argument");
   const int per_iter = 5 + (p->cfg.world_size > 1 ? 1 : 0);
   *out = p->fused_update ? 1 + 2 * p->cfg.iterations : 1 + per_iter * p->cfg.iterations + 2;
   return SIMBA_OK;
@@ -1203,51 +1197,51 @@ extern "C" int simba_planner_launches_per_plan(simba_planner_t* p, int32_t* out)
 
 extern "C" int simba_plan(simba_planner_t* p, const float* states, uint64_t seed, float* out_action,
                           float* out_score, int32_t* out_iterations, void* stream) {
-  if (!p || !states || !out_action || !out_score) return fail(SIMBA_ERR_BAD_CONFIG, "null argument");
-  CUDA_TRY(cudaSetDevice(p->device));
+  if (!p || !states || !out_action || !out_score) return set_error(SIMBA_ERR_BAD_CONFIG, "null argument");
+  SIMBA_CUDA_TRY(cudaSetDevice(p->device));
   cudaStream_t st = (cudaStream_t)stream;
   const size_t S = p->cfg.n_states, O = p->model->cfg.obs_dim, A = p->model->cfg.act_dim;
   int rc = ensure_graph(p);
   if (rc != SIMBA_OK) return rc;
   // a planner owns ONE workspace (seed, states, mu / sigma, actions, outputs): plans issued on different
   // streams are serialised behind each other here (a no-op when the caller keeps to one stream)
-  if (p->plan_done) CUDA_TRY(cudaStreamWaitEvent(st, p->plan_done, 0));
+  if (p->plan_done) SIMBA_CUDA_TRY(cudaStreamWaitEvent(st, p->plan_done, 0));
   rc = upload_seed(p, seed, st);
   if (rc != SIMBA_OK) return rc;
   if (states != p->d_states)
-    CUDA_TRY(cudaMemcpyAsync(p->d_states, states, S * O * 4, cudaMemcpyDeviceToDevice, st));
-  CUDA_TRY(cudaGraphLaunch(p->graph_exec, st));
+    SIMBA_CUDA_TRY(cudaMemcpyAsync(p->d_states, states, S * O * 4, cudaMemcpyDeviceToDevice, st));
+  SIMBA_CUDA_TRY(cudaGraphLaunch(p->graph_exec, st));
   if (out_action != p->d_out_action)
-    CUDA_TRY(cudaMemcpyAsync(out_action, p->d_out_action, S * A * 4, cudaMemcpyDeviceToDevice, st));
+    SIMBA_CUDA_TRY(cudaMemcpyAsync(out_action, p->d_out_action, S * A * 4, cudaMemcpyDeviceToDevice, st));
   if (out_score != p->d_out_score)
-    CUDA_TRY(cudaMemcpyAsync(out_score, p->d_out_score, S * 4, cudaMemcpyDeviceToDevice, st));
+    SIMBA_CUDA_TRY(cudaMemcpyAsync(out_score, p->d_out_score, S * 4, cudaMemcpyDeviceToDevice, st));
   if (out_iterations && out_iterations != p->d_out_iters)
-    CUDA_TRY(cudaMemcpyAsync(out_iterations, p->d_out_iters, S * 4, cudaMemcpyDeviceToDevice, st));
-  if (p->plan_done) CUDA_TRY(cudaEventRecord(p->plan_done, st));
+    SIMBA_CUDA_TRY(cudaMemcpyAsync(out_iterations, p->d_out_iters, S * 4, cudaMemcpyDeviceToDevice, st));
+  if (p->plan_done) SIMBA_CUDA_TRY(cudaEventRecord(p->plan_done, st));
   return SIMBA_OK;
 }
 
 extern "C" int simba_plan_host(simba_planner_t* p, const float* states_host, uint64_t seed,
                                float* out_action_host, float* out_score_host,
                                int32_t* out_iterations_host) {
-  if (!p || !states_host || !out_action_host) return fail(SIMBA_ERR_BAD_CONFIG, "null argument");
-  CUDA_TRY(cudaSetDevice(p->device));
+  if (!p || !states_host || !out_action_host) return set_error(SIMBA_ERR_BAD_CONFIG, "null argument");
+  SIMBA_CUDA_TRY(cudaSetDevice(p->device));
   const size_t S = p->cfg.n_states, O = p->model->cfg.obs_dim, A = p->model->cfg.act_dim;
   cudaStream_t st = p->own_stream;
   int rc = ensure_graph(p);
   if (rc != SIMBA_OK) return rc;
-  if (p->plan_done) CUDA_TRY(cudaStreamWaitEvent(st, p->plan_done, 0));    // behind a plan_device() on another stream
+  if (p->plan_done) SIMBA_CUDA_TRY(cudaStreamWaitEvent(st, p->plan_done, 0));    // behind a plan_device() on another stream
   // seed + states staged in pinned memory: one host-to-device copy (the call is synchronous, so one staging
   // block is enough), the graph, one device-to-host copy of the three results
   memcpy(p->h_in, &seed, sizeof(seed));
   memcpy(p->h_in + 16, states_host, S * O * 4);
-  CUDA_TRY(cudaMemcpyAsync(p->d_in, p->h_in, 16 + S * O * 4, cudaMemcpyHostToDevice, st));
-  CUDA_TRY(cudaGraphLaunch(p->graph_exec, st));
+  SIMBA_CUDA_TRY(cudaMemcpyAsync(p->d_in, p->h_in, 16 + S * O * 4, cudaMemcpyHostToDevice, st));
+  SIMBA_CUDA_TRY(cudaGraphLaunch(p->graph_exec, st));
   float* h_act = p->h_out;
   float* h_score = p->h_out + S * A;
   int32_t* h_iters = reinterpret_cast<int32_t*>(p->h_out + S * A + S);
-  CUDA_TRY(cudaMemcpyAsync(p->h_out, p->d_out, S * (A + 2) * 4, cudaMemcpyDeviceToHost, st));
-  CUDA_TRY(cudaStreamSynchronize(st));
+  SIMBA_CUDA_TRY(cudaMemcpyAsync(p->h_out, p->d_out, S * (A + 2) * 4, cudaMemcpyDeviceToHost, st));
+  SIMBA_CUDA_TRY(cudaStreamSynchronize(st));
   memcpy(out_action_host, h_act, S * A * 4);
   if (out_score_host) memcpy(out_score_host, h_score, S * 4);
   if (out_iterations_host) memcpy(out_iterations_host, h_iters, S * 4);
@@ -1256,7 +1250,7 @@ extern "C" int simba_plan_host(simba_planner_t* p, const float* states_host, uin
 
 // ---- NCCL plumbing ---------------------------------------------------------------------------------
 extern "C" int simba_nccl_unique_id(void* out) {
-  if (!out) return fail(SIMBA_ERR_BAD_CONFIG, "null argument");
+  if (!out) return set_error(SIMBA_ERR_BAD_CONFIG, "null argument");
   int rc = nccl_load();
   if (rc != SIMBA_OK) return rc;
   NcclUniqueId id;
@@ -1266,10 +1260,10 @@ extern "C" int simba_nccl_unique_id(void* out) {
 }
 
 extern "C" int simba_planner_init_nccl(simba_planner_t* p, const void* uid) {
-  if (!p || !uid) return fail(SIMBA_ERR_BAD_CONFIG, "null argument");
+  if (!p || !uid) return set_error(SIMBA_ERR_BAD_CONFIG, "null argument");
   int rc = nccl_load();
   if (rc != SIMBA_OK) return rc;
-  CUDA_TRY(cudaSetDevice(p->device));
+  SIMBA_CUDA_TRY(cudaSetDevice(p->device));
   NcclUniqueId id;
   memcpy(&id, uid, sizeof(id));
   NCCL_TRY(g_nccl.comm_init_rank(&p->comm, p->cfg.world_size, id, p->cfg.rank));
@@ -1279,57 +1273,18 @@ extern "C" int simba_planner_init_nccl(simba_planner_t* p, const void* uid) {
 // ---- model-level entry points -----------------------------------------------------------------------
 // The model keeps one device tile list for its entry points. It is overwritten only after a device-wide
 // synchronise, so a launch of any entry point still in flight on another stream never sees it change.
-static int model_upload_tiles(simba_model* m, const std::vector<Tile>& tiles, int* n_tiles) {
+static int model_upload_tiles(simba_model* m, const std::vector<Tile>& tiles) {
   if ((int)tiles.size() > m->tiles_cap) {
     cudaFree(m->d_tiles);
     m->d_tiles = nullptr;
     m->tiles_cap = 0;
-    CUDA_TRY(cudaMalloc((void**)&m->d_tiles, tiles.size() * sizeof(Tile)));
+    SIMBA_CUDA_TRY(cudaMalloc((void**)&m->d_tiles, tiles.size() * sizeof(Tile)));
     m->tiles_cap = (int)tiles.size();
   }
   // synchronous copy: orders after any earlier kernel that still reads the old list
-  CUDA_TRY(cudaDeviceSynchronize());
-  CUDA_TRY(cudaMemcpy(m->d_tiles, tiles.data(), tiles.size() * sizeof(Tile), cudaMemcpyHostToDevice));
-  *n_tiles = (int)tiles.size();
+  SIMBA_CUDA_TRY(cudaDeviceSynchronize());
+  SIMBA_CUDA_TRY(cudaMemcpy(m->d_tiles, tiles.data(), tiles.size() * sizeof(Tile), cudaMemcpyHostToDevice));
   return SIMBA_OK;
-}
-
-static int model_tiles(simba_model* m, const RowGeom& g, int* n_tiles) {
-  std::vector<Tile> tiles;
-  build_tiles(g, kF32TileRows, tiles);
-  return model_upload_tiles(m, tiles, n_tiles);
-}
-
-// The tcgen05 kernel of a bf16 unfold (simba_unfold_tc) and its tile list: 128-row tiles of the tf.split member
-// map, the same shape predicates as choose_rollout with no constraints (no scorer), and the same image the model
-// commit packed. The trajectory forms have no per-row cost mask, so the horizon is bounded by the Philox step
-// counter alone (65535, as for the fp32 kernel); the predicates see at most the planner's bound.
-static int choose_unfold(const simba_model_config_t& mc, const RowGeom& g, int sms, RolloutKernel& kernel,
-                         std::vector<Tile>& tiles) {
-  const int O = mc.obs_dim, A = mc.act_dim, L = mc.n_layers, U = mc.units, H = std::min(g.H, SIMBA_MAX_HORIZON);
-  build_tiles(g, kTcTileRows, tiles);
-  if (rollout_tc_supported(O, A, L, U, H)) {
-    kernel = RolloutKernel::kTcOneCta;
-    if ((int)tiles.size() > sms && rollout_tc_two_tiles_fit(L, 0)) {
-      kernel = RolloutKernel::kTcTwoTile;
-      build_tiles(g, kTcTileRows, tiles, 2);
-      split_tail_items(tiles, sms);
-    }
-    return SIMBA_OK;
-  }
-  if (rollout_tc_wide_supported(64, O, A, L, U, H) && rollout_tc_wide_fits(64, L, U, 0)) {
-    kernel = RolloutKernel::kTcWide;
-    return SIMBA_OK;
-  }
-  if (wide_obs_selected(O, A, L, U, H) && rollout_tc_wide_fits(128, L, U, 0)) {
-    kernel = RolloutKernel::kTcWideObs;
-    return SIMBA_OK;
-  }
-  return fail(SIMBA_ERR_UNSUPPORTED,
-              "no bf16 tcgen05 kernel covers obs_dim %d, act_dim %d, %d x %d units: they cover units <= 128 "
-              "(obs_dim <= 60, obs_dim+act_dim <= 64, <= 5 layers), 128 < units <= ~416 (obs_dim+act_dim <= 62) and, "
-              "for other shapes, obs_dim+act_dim <= 126 with obs_dim <= 124, act_dim <= 4, units <= 384 and <= 6 "
-              "layers; use simba_unfold (fp32) for this shape", O, A, L, U);
 }
 
 // the device check of the bf16 unfold entry points, per call: one attribute query (cudaGetDeviceProperties, which
@@ -1337,161 +1292,136 @@ static int choose_unfold(const simba_model_config_t& mc, const RowGeom& g, int s
 static int unfold_tc_device_check(const simba_model* m) {
   int dev = 0;
   if (m) dev = m->device;
-  else CUDA_TRY(cudaGetDevice(&dev));
+  else SIMBA_CUDA_TRY(cudaGetDevice(&dev));
   int major = 0;
-  CUDA_TRY(cudaDeviceGetAttribute(&major, cudaDevAttrComputeCapabilityMajor, dev));
-  if (major != 10) return fail(SIMBA_ERR_ARCH, "device %d is sm_%d*; the tcgen05 kernels need sm_100a", dev, major);
+  SIMBA_CUDA_TRY(cudaDeviceGetAttribute(&major, cudaDevAttrComputeCapabilityMajor, dev));
+  if (major != 10) return set_error(SIMBA_ERR_ARCH, "device %d is sm_%d*; the tcgen05 kernels need sm_100a", dev, major);
   return SIMBA_OK;
 }
 
-// shared checks of the two bf16 unfold entry points -> geometry, SM count, kernel and tile list
-static int unfold_tc_plan(simba_model* m, int32_t batch, int32_t horizon, RowGeom& g, int& sms,
-                          RolloutKernel& kernel, std::vector<Tile>& tiles) {
-  if (!m->committed) return fail(SIMBA_ERR_NOT_READY, "model not committed");
+// The rows of the model's own entry points: `batch` rows of one state under the tf.split member map, each from its
+// own s_0, scored by nothing. Checks the call and sets prm.g, prm.kernel and prm.n_sms; `tiles` is the kernel's list.
+// The trajectory forms have no per-row cost mask, so the horizon is bounded by the Philox step counter alone.
+static int model_rollout_choice(simba_model* m, int precision, int32_t batch, int32_t horizon, RolloutParams& prm,
+                                std::vector<Tile>& tiles) {
+  if (!m->committed) return set_error(SIMBA_ERR_NOT_READY, "model not committed");
   if (horizon < 1 || horizon > 65535 || batch < 1)
-    return fail(SIMBA_ERR_BAD_CONFIG, "batch %d / horizon %d out of range", batch, horizon);
-  CUDA_TRY(cudaSetDevice(m->device));
+    return set_error(SIMBA_ERR_BAD_CONFIG, "batch %d / horizon %d out of range", batch, horizon);
+  SIMBA_CUDA_TRY(cudaSetDevice(m->device));
   int rc = build_geom(1, 1, batch, 1, 0, horizon, m->cfg.obs_dim, m->cfg.act_dim, m->cfg.ensemble_size,
-                      SIMBA_MAP_SPLIT, g);
+                      SIMBA_MAP_SPLIT, prm.g);
   if (rc != SIMBA_OK) return rc;
-  CUDA_TRY(cudaDeviceGetAttribute(&sms, cudaDevAttrMultiProcessorCount, m->device));
-  return choose_unfold(m->cfg, g, sms, kernel, tiles);
+  SIMBA_CUDA_TRY(cudaDeviceGetAttribute(&prm.n_sms, cudaDevAttrMultiProcessorCount, m->device));
+  return choose_rollout(m->cfg, precision, prm.g, 0, true, prm.n_sms, prm.kernel, tiles);
 }
 
-static void null_scorer(simba_scorer_t& sc) {
-  memset(&sc, 0, sizeof(sc));
-  sc.goal_dist_index = 0;      // any in-range read; results are discarded
-  sc.lidar_max_dist = 1.0f;
+// model_rollout_choice, the tile upload and the model side of prm
+static int model_rollout_params(simba_model* m, int precision, int32_t batch, int32_t horizon, RolloutParams& prm) {
+  std::vector<Tile> tiles;
+  int rc = model_rollout_choice(m, precision, batch, horizon, prm, tiles);
+  if (rc != SIMBA_OK) return rc;
+  rc = model_upload_tiles(m, tiles);
+  if (rc != SIMBA_OK) return rc;
+  memset(&prm.scorer, 0, sizeof(prm.scorer));
+  prm.scorer.goal_dist_index = 0;      // any in-range read; results are discarded
+  prm.scorer.lidar_max_dist = 1.0f;
+  prm.tiles = m->d_tiles;
+  prm.n_tiles = (int)tiles.size();
+  fill_model_params(m, prm);
+  prm.objective = SIMBA_OBJ_REWARD;
+  return SIMBA_OK;
+}
+
+static int unfold(int precision, simba_model_t* m, const float* s0, const float* actions, const float* eps,
+                  uint64_t seed, int32_t batch, int32_t horizon, int32_t sampling_propagation, float* out_traj,
+                  void* stream) {
+  if (precision != SIMBA_PREC_FP32) {
+    int rc = unfold_tc_device_check(m);
+    if (rc != SIMBA_OK) return rc;
+  }
+  if (!m || !s0 || !actions || !out_traj) return set_error(SIMBA_ERR_BAD_CONFIG, "null argument");
+  RolloutParams prm{};
+  int rc = model_rollout_params(m, precision, batch, horizon, prm);
+  if (rc != SIMBA_OK) return rc;
+  prm.states = s0; prm.state_stride = m->cfg.obs_dim; prm.state_per_row = 1;
+  prm.actions = actions; prm.action_stride = (int64_t)horizon * m->cfg.act_dim;
+  prm.eps = eps; prm.seed = seed;
+  prm.sampling_propagation = sampling_propagation;
+  prm.traj_out = out_traj;
+  SIMBA_CUDA_TRY(launch_rollout(prm, (cudaStream_t)stream));
+  return SIMBA_OK;
 }
 
 extern "C" int simba_unfold(simba_model_t* m, const float* s0, const float* actions,
                             const float* eps, uint64_t seed, int32_t batch, int32_t horizon,
                             int32_t sampling_propagation, float* out_traj, void* stream) {
-  if (!m || !s0 || !actions || !out_traj) return fail(SIMBA_ERR_BAD_CONFIG, "null argument");
-  if (!m->committed) return fail(SIMBA_ERR_NOT_READY, "model not committed");
-  if (horizon < 1 || horizon > 65535 || batch < 1)
-    return fail(SIMBA_ERR_BAD_CONFIG, "batch %d / horizon %d out of range", batch, horizon);
-  CUDA_TRY(cudaSetDevice(m->device));
-  RolloutParams prm{};
-  int rc = build_geom(1, 1, batch, 1, 0, horizon, m->cfg.obs_dim, m->cfg.act_dim,
-                      m->cfg.ensemble_size, SIMBA_MAP_SPLIT, prm.g);
-  if (rc != SIMBA_OK) return rc;
-  int n_tiles = 0;
-  rc = model_tiles(m, prm.g, &n_tiles);
-  if (rc != SIMBA_OK) return rc;
-  null_scorer(prm.scorer);
-  prm.tiles = m->d_tiles; prm.n_tiles = n_tiles;
-  fill_model_params(m, prm);
-  prm.states = s0; prm.state_stride = m->cfg.obs_dim; prm.state_per_row = 1;
-  prm.actions = actions; prm.action_stride = (int64_t)horizon * m->cfg.act_dim;
-  prm.eps = eps; prm.seed = seed; prm.iteration = 0;
-  prm.sampling_propagation = sampling_propagation;
-  prm.objective = SIMBA_OBJ_REWARD;
-  prm.traj_out = out_traj;
-  CUDA_TRY(launch_rollout_f32(prm, n_tiles, (cudaStream_t)stream));
-  return SIMBA_OK;
+  return unfold(SIMBA_PREC_FP32, m, s0, actions, eps, seed, batch, horizon, sampling_propagation, out_traj, stream);
 }
 
 extern "C" int simba_unfold_tc(simba_model_t* m, const float* s0, const float* actions,
                                const float* eps, uint64_t seed, int32_t batch, int32_t horizon,
                                int32_t sampling_propagation, float* out_traj, void* stream) {
-  int rc = unfold_tc_device_check(m);
-  if (rc != SIMBA_OK) return rc;
-  if (!m || !s0 || !actions || !out_traj) return fail(SIMBA_ERR_BAD_CONFIG, "null argument");
-  RolloutParams prm{};
-  int sms = 0;
-  std::vector<Tile> tiles;
-  rc = unfold_tc_plan(m, batch, horizon, prm.g, sms, prm.kernel, tiles);
-  if (rc != SIMBA_OK) return rc;
-  int n_tiles = 0;
-  rc = model_upload_tiles(m, tiles, &n_tiles);
-  if (rc != SIMBA_OK) return rc;
-  prm.tiles = m->d_tiles; prm.n_tiles = n_tiles;   // prm.scorer stays zero: the trajectory forms score nothing
-  fill_model_params(m, prm);
-  prm.n_sms = sms;
-  prm.states = s0; prm.state_stride = m->cfg.obs_dim; prm.state_per_row = 1;
-  prm.actions = actions; prm.action_stride = (int64_t)horizon * m->cfg.act_dim;
-  prm.eps = eps; prm.seed = seed; prm.iteration = 0;
-  prm.sampling_propagation = sampling_propagation;
-  prm.objective = SIMBA_OBJ_REWARD;
-  prm.traj_out = out_traj;
-  const bool wide = prm.kernel == RolloutKernel::kTcWide || prm.kernel == RolloutKernel::kTcWideObs;
-  CUDA_TRY(wide ? launch_unfold_tc_wide(prm, n_tiles, (cudaStream_t)stream)
-                : launch_unfold_tc(prm, n_tiles, (cudaStream_t)stream));
-  return SIMBA_OK;
+  return unfold(SIMBA_PREC_BF16_TC, m, s0, actions, eps, seed, batch, horizon, sampling_propagation, out_traj,
+                stream);
 }
 
 extern "C" int simba_unfold_tc_kernel(simba_model_t* m, int32_t batch, int32_t horizon, int32_t* kernel,
                                       int32_t* work_items) {
   int rc = unfold_tc_device_check(m);
   if (rc != SIMBA_OK) return rc;
-  if (!m || !kernel || !work_items) return fail(SIMBA_ERR_BAD_CONFIG, "null argument");
-  RowGeom g;
-  int sms = 0;
-  RolloutKernel k = RolloutKernel::kF32;
+  if (!m || !kernel || !work_items) return set_error(SIMBA_ERR_BAD_CONFIG, "null argument");
+  RolloutParams prm{};
   std::vector<Tile> tiles;
-  rc = unfold_tc_plan(m, batch, horizon, g, sms, k, tiles);
+  rc = model_rollout_choice(m, SIMBA_PREC_BF16_TC, batch, horizon, prm, tiles);
   if (rc != SIMBA_OK) return rc;
-  *kernel = (int32_t)k;
-  *work_items = (int32_t)tiles.size() / (k == RolloutKernel::kTcTwoTile ? 2 : 1);
+  *kernel = (int32_t)prm.kernel;
+  *work_items = n_work_items(prm.kernel, tiles);
   return SIMBA_OK;
 }
 
 extern "C" int simba_ensemble_forward(simba_model_t* m, const float* x, const float* eps,
                                       int32_t batch, float* out_mu, float* out_var,
                                       float* out_sample, void* stream) {
-  if (!m || !x || !out_mu || !out_var) return fail(SIMBA_ERR_BAD_CONFIG, "null argument");
-  if (!m->committed) return fail(SIMBA_ERR_NOT_READY, "model not committed");
-  if (batch < 1) return fail(SIMBA_ERR_BAD_CONFIG, "batch %d < 1", batch);
-  CUDA_TRY(cudaSetDevice(m->device));
-  const int O = m->cfg.obs_dim, IN = O + m->cfg.act_dim;
+  if (!m || !x || !out_mu || !out_var) return set_error(SIMBA_ERR_BAD_CONFIG, "null argument");
   RolloutParams prm{};
-  int rc = build_geom(1, 1, batch, 1, 0, 1, O, m->cfg.act_dim, m->cfg.ensemble_size,
-                      SIMBA_MAP_SPLIT, prm.g);
+  int rc = model_rollout_params(m, SIMBA_PREC_FP32, batch, 1, prm);
   if (rc != SIMBA_OK) return rc;
-  int n_tiles = 0;
-  rc = model_tiles(m, prm.g, &n_tiles);
-  if (rc != SIMBA_OK) return rc;
-  null_scorer(prm.scorer);
-  prm.tiles = m->d_tiles; prm.n_tiles = n_tiles;
-  fill_model_params(m, prm);
+  const int O = m->cfg.obs_dim, IN = O + m->cfg.act_dim;
   prm.scale_on = 0;                               // x is used as given (mlp_ensemble.py:190)
   prm.states = x; prm.state_stride = IN; prm.state_per_row = 1;
   prm.actions = x + O; prm.action_stride = IN;
-  prm.eps = eps; prm.seed = 0; prm.iteration = 0;
-  prm.sampling_propagation = 0;
-  prm.objective = SIMBA_OBJ_REWARD;
+  prm.eps = eps;
   prm.mu_out = out_mu; prm.var_out = out_var; prm.sample_out = out_sample;
-  if (out_sample && !eps) return fail(SIMBA_ERR_BAD_CONFIG, "out_sample needs eps");
-  CUDA_TRY(launch_rollout_f32(prm, n_tiles, (cudaStream_t)stream));
+  if (out_sample && !eps) return set_error(SIMBA_ERR_BAD_CONFIG, "out_sample needs eps");
+  SIMBA_CUDA_TRY(launch_rollout(prm, (cudaStream_t)stream));
   return SIMBA_OK;
 }
 
 extern "C" int simba_scale(simba_model_t* m, const float* x, int32_t batch, float* out, void* stream) {
-  if (!m || !x || !out) return fail(SIMBA_ERR_BAD_CONFIG, "null argument");
-  if (!m->committed) return fail(SIMBA_ERR_NOT_READY, "model not committed");
-  CUDA_TRY(cudaSetDevice(m->device));
-  CUDA_TRY(launch_scale(x, m->d_smin, m->d_sdelta, m->scale_on, batch,
+  if (!m || !x || !out) return set_error(SIMBA_ERR_BAD_CONFIG, "null argument");
+  if (!m->committed) return set_error(SIMBA_ERR_NOT_READY, "model not committed");
+  SIMBA_CUDA_TRY(cudaSetDevice(m->device));
+  SIMBA_CUDA_TRY(launch_scale(x, m->d_smin, m->d_sdelta, m->scale_on, batch,
                         m->cfg.obs_dim + m->cfg.act_dim, out, (cudaStream_t)stream));
   return SIMBA_OK;
 }
 
 extern "C" int simba_score_trajectories(simba_planner_t* p, const float* traj, float* out_scores,
                                         float* out_pairs, void* stream) {
-  if (!p || !traj || !out_scores) return fail(SIMBA_ERR_BAD_CONFIG, "null argument");
+  if (!p || !traj || !out_scores) return set_error(SIMBA_ERR_BAD_CONFIG, "null argument");
   if (p->cfg.n_states != 1 || p->cfg.world_size != 1)
-    return fail(SIMBA_ERR_UNSUPPORTED, "score_trajectories needs n_states == 1 and world_size == 1");
-  CUDA_TRY(cudaSetDevice(p->device));
+    return set_error(SIMBA_ERR_UNSUPPORTED, "score_trajectories needs n_states == 1 and world_size == 1");
+  SIMBA_CUDA_TRY(cudaSetDevice(p->device));
   cudaStream_t st = (cudaStream_t)stream;
   const int rows = p->cfg.particles * p->cfg.n_samples;
-  CUDA_TRY(launch_score_traj_rows(p->cfg.scorer, traj, rows, p->cfg.horizon, p->model->cfg.obs_dim,
+  SIMBA_CUDA_TRY(launch_score_traj_rows(p->cfg.scorer, traj, rows, p->cfg.horizon, p->model->cfg.obs_dim,
                                   p->cfg.objective, p->row_ret, p->row_cmask, p->row_csum, st));
   int rc = simba_score_reduce(p, p->row_ret, p->row_cmask, p->row_csum, nullptr, p->pairs_local, st);
   if (rc != SIMBA_OK) return rc;
-  CUDA_TRY(launch_pairs_to_scores(p->pairs_local, p->cfg.n_samples, p->cfg.objective,
+  SIMBA_CUDA_TRY(launch_pairs_to_scores(p->pairs_local, p->cfg.n_samples, p->cfg.objective,
                                   (float)p->c_max, out_scores, st));
   if (out_pairs)
-    CUDA_TRY(cudaMemcpyAsync(out_pairs, p->pairs_local, (size_t)p->cfg.n_samples * 8,
+    SIMBA_CUDA_TRY(cudaMemcpyAsync(out_pairs, p->pairs_local, (size_t)p->cfg.n_samples * 8,
                              cudaMemcpyDeviceToDevice, st));
   return SIMBA_OK;
 }
@@ -1499,31 +1429,31 @@ extern "C" int simba_score_trajectories(simba_planner_t* p, const float* traj, f
 extern "C" int simba_scorer_eval(const simba_scorer_t* sc, const float* obs, const float* next_obs,
                                  int32_t batch, int32_t obs_dim, float* out_reward,
                                  int32_t* out_done, float* out_cost, void* stream) {
-  if (!sc || !obs) return fail(SIMBA_ERR_BAD_CONFIG, "null argument");
+  if (!sc || !obs) return set_error(SIMBA_ERR_BAD_CONFIG, "null argument");
   int rc = validate_scorer(*sc, obs_dim);
   if (rc != SIMBA_OK) return rc;
-  CUDA_TRY(launch_scorer_eval(*sc, obs, next_obs, batch, obs_dim, out_reward, out_done, out_cost,
+  SIMBA_CUDA_TRY(launch_scorer_eval(*sc, obs, next_obs, batch, obs_dim, out_reward, out_done, out_cost,
                               (cudaStream_t)stream));
   return SIMBA_OK;
 }
 
 // ---- RNG probes ----------------------------------------------------------------------------------------
 extern "C" int simba_philox_raw(const uint32_t counter[4], const uint32_t key[2], uint32_t out[4]) {
-  if (!counter || !key || !out) return fail(SIMBA_ERR_BAD_CONFIG, "null argument");
+  if (!counter || !key || !out) return set_error(SIMBA_ERR_BAD_CONFIG, "null argument");
   uint32_t* d = nullptr;
-  CUDA_TRY(cudaMalloc((void**)&d, 16));
+  SIMBA_CUDA_TRY(cudaMalloc((void**)&d, 16));
   cudaError_t e = launch_philox_raw(counter, key, d, nullptr);
   if (e == cudaSuccess) e = cudaMemcpy(out, d, 16, cudaMemcpyDeviceToHost);
   cudaFree(d);
-  CUDA_TRY(e);
+  SIMBA_CUDA_TRY(e);
   return SIMBA_OK;
 }
 
 extern "C" int simba_philox_normals(uint64_t seed, int32_t rng_stream, int32_t iteration, int32_t t,
                                     int32_t state_index, int32_t first_row, int32_t n_rows,
                                     int32_t n_elems, int32_t fast_math, float* out, void* stream) {
-  if (!out || n_rows < 1 || n_elems < 1) return fail(SIMBA_ERR_BAD_CONFIG, "bad argument");
-  CUDA_TRY(launch_philox_normals(seed, rng_stream, iteration, t, state_index, first_row, n_rows,
+  if (!out || n_rows < 1 || n_elems < 1) return set_error(SIMBA_ERR_BAD_CONFIG, "bad argument");
+  SIMBA_CUDA_TRY(launch_philox_normals(seed, rng_stream, iteration, t, state_index, first_row, n_rows,
                                  n_elems, fast_math, out, (cudaStream_t)stream));
   return SIMBA_OK;
 }

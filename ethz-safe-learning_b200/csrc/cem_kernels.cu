@@ -5,6 +5,7 @@
 #include <cooperative_groups.h>
 
 #include "cem_kernels.cuh"
+#include "internal.h"
 
 namespace cg = cooperative_groups;
 
@@ -612,31 +613,11 @@ static bool use_cluster_path(int N) {
   return N >= kSelClusterMinN && (N + kSelClusterSize - 1) / kSelClusterSize <= kSelClusterMaxSlice;
 }
 
-template <typename Kernel, typename... Args>
-static cudaError_t launch_cluster(Kernel kernel, int n_states, int threads, size_t smem, cudaStream_t st,
-                                  Args... args) {
-  cudaError_t e = cudaFuncSetAttribute(kernel, cudaFuncAttributeMaxDynamicSharedMemorySize, (int)smem);
-  if (e != cudaSuccess) return e;
-  cudaLaunchConfig_t cfg = {};
-  cfg.gridDim = dim3(n_states * kSelClusterSize);
-  cfg.blockDim = dim3(threads);
-  cfg.dynamicSmemBytes = smem;
-  cfg.stream = st;
-  cudaLaunchAttribute attr[1];
-  attr[0].id = cudaLaunchAttributeClusterDimension;
-  attr[0].val.clusterDim.x = kSelClusterSize;
-  attr[0].val.clusterDim.y = 1;
-  attr[0].val.clusterDim.z = 1;
-  cfg.attrs = attr;
-  cfg.numAttrs = 1;
-  return cudaLaunchKernelEx(&cfg, kernel, args...);
-}
-
 cudaError_t launch_select_elites(const SelectParams& p, cudaStream_t st) {
   if (use_cluster_path(p.N)) {
     const int slice = (p.N + kSelClusterSize - 1) / kSelClusterSize;
-    return launch_cluster(select_elites_cluster_kernel, p.S, kSelectThreads,
-                          (size_t)slice * sizeof(unsigned long long), st, p, slice);
+    return launch_kernel(select_elites_cluster_kernel, p.S * kSelClusterSize, kSelectThreads,
+                         (size_t)slice * sizeof(unsigned long long), st, kSelClusterSize, false, p, slice);
   }
   select_elites_kernel<<<p.S, kSelectThreads, 0, st>>>(p);
   return cudaGetLastError();
@@ -963,7 +944,7 @@ cudaError_t launch_refit(const RefitParams& p_in, cudaStream_t st) {
     if ((long)p.N * HA > 0x7fffffffL) return cudaErrorInvalidValue;   // 32-bit element offsets in the kernel
     const size_t smem = (size_t)(groups * HA + 3 * HA) * sizeof(float) +
                         (size_t)((p.K + kSelClusterSize - 1) / kSelClusterSize) * sizeof(int);
-    return launch_cluster(refit_cluster_kernel, p.S, kRefitThreads, smem, st, p);
+    return launch_kernel(refit_cluster_kernel, p.S * kSelClusterSize, kRefitThreads, smem, st, kSelClusterSize, false, p);
   }
   const size_t smem = (size_t)(groups * HA + 2 * HA) * sizeof(float);
   refit_kernel<<<p.S, kRefitThreads, smem, st>>>(p);
@@ -1365,21 +1346,8 @@ cudaError_t launch_cem_update(const UpdateParams& u_in, cudaStream_t st) {
   const size_t stage = update_stage_bytes(u.reduce.P, u.select.N, HA);
   u.stage = (smem + stage + 1024 <= 200 * 1024 && u.select.N <= kRefitThreads) ? 1 : 0;
   if (u.stage) smem += stage;
-  {
-    cudaError_t e = cudaFuncSetAttribute(cem_update_kernel<true>, cudaFuncAttributeMaxDynamicSharedMemorySize, 200 * 1024);
-    if (e != cudaSuccess) return e;
-  }
-  cudaLaunchConfig_t cfg{};
-  cfg.gridDim = dim3(u.refit.S);
-  cfg.blockDim = dim3(kRefitThreads);
-  cfg.dynamicSmemBytes = smem;
-  cfg.stream = st;
-  cudaLaunchAttribute attr[1];
-  attr[0].id = cudaLaunchAttributeProgrammaticStreamSerialization;
-  attr[0].val.programmaticStreamSerializationAllowed = 1;
-  cfg.attrs = attr;
-  cfg.numAttrs = u.pdl ? 1 : 0;
-  return u.stage ? cudaLaunchKernelEx(&cfg, cem_update_kernel<true>, u) : cudaLaunchKernelEx(&cfg, cem_update_kernel<false>, u);
+  return launch_kernel(u.stage ? cem_update_kernel<true> : cem_update_kernel<false>, u.refit.S, kRefitThreads, smem, st,
+                       1, u.pdl != 0, u);
 }
 
 // plan bookkeeping: reset mu/sigma/best/active at the start of a plan (cem_mpc.py:36-42)

@@ -272,8 +272,7 @@ size_t rollout_f32_smem_bytes(const RolloutParams& prm) {
   return floats * sizeof(float) + 5 * TM * sizeof(int64_t) + 16;
 }
 
-cudaError_t launch_rollout_f32(const RolloutParams& prm, int n_tiles, cudaStream_t stream) {
-  if (n_tiles == 0) return cudaSuccess;
+cudaError_t launch_rollout_f32(const RolloutParams& prm, cudaStream_t stream) {
   const size_t smem = rollout_f32_smem_bytes(prm);
   // set on every launch: the attribute is per device and per function, and launches happen only at
   // graph capture or in the non-graph entry points, never on the replayed hot path
@@ -282,7 +281,7 @@ cudaError_t launch_rollout_f32(const RolloutParams& prm, int n_tiles, cudaStream
                                          cudaFuncAttributeMaxDynamicSharedMemorySize, (int)smem);
     if (e != cudaSuccess) return e;
   }
-  rollout_f32_kernel<<<n_tiles, NT, smem, stream>>>(prm);
+  rollout_f32_kernel<<<prm.n_tiles, NT, smem, stream>>>(prm);
   return cudaGetLastError();
 }
 

@@ -37,7 +37,7 @@ struct RolloutParams {
   const void* w_wide;
   int64_t w_wide_member_bytes;
   const void* bias_k16;       // [E][L+1][4096 B] bias K-blocks (see pack_bf16_image in api.cu)
-  RolloutKernel kernel;       // which launch_rollout_* runs and, for rollout_tc.cu, which variant
+  RolloutKernel kernel;       // the kernel launch_rollout runs
   int32_t n_sms;              // SMs of the planner's device (grid of the persistent tcgen05 kernels)
   int32_t pdl;                // launch with programmatic stream serialization (fused plan path)
   float tc_scale_a[128];      // bf16 path: x_scaled[k] = fma(x[k], a[k], b[k]); zero beyond O + A
@@ -71,18 +71,22 @@ struct RolloutParams {
   long long* timeline;        // clock64 stamps of CTA 0 (-DSIMBA_TC_TIMELINE builds only, else null)
 };
 
+// Launches the kernel prm.kernel names over prm.tiles: the trajectory form of a tcgen05 kernel when prm.traj_out is
+// set, its planning form otherwise (the fp32 kernel takes both from prm at run time). Defined in api.cu, next to
+// choose_rollout, which picks prm.kernel and the tile list.
+cudaError_t launch_rollout(const RolloutParams& prm, cudaStream_t stream);
+// the branches of launch_rollout, one per kernel file
+cudaError_t launch_rollout_f32(const RolloutParams& prm, cudaStream_t stream);
+cudaError_t launch_rollout_tc(const RolloutParams& prm, cudaStream_t stream);        // kTc{OneCta,Pair,TwoTile}
+cudaError_t launch_rollout_tc_wide(const RolloutParams& prm, cudaStream_t stream);   // kTcWide{,Obs}; prm.U: the model's units
+
 size_t rollout_f32_smem_bytes(const RolloutParams& prm);
-cudaError_t launch_rollout_f32(const RolloutParams& prm, int n_tiles, cudaStream_t stream);
-cudaError_t launch_rollout_tc(const RolloutParams& prm, int n_tiles, cudaStream_t stream);   // prm.kernel: kTc{OneCta,Pair,TwoTile}
-bool rollout_tc_supported(int O, int A, int L, int U, int H);
+// Shape rules of the tcgen05 kernels, from the model alone (api.cu's tc_family combines them). rollout_tc.cu:
+bool rollout_tc_supported(int O, int A, int L, int U);
 bool rollout_tc_two_tiles_fit(int L, int n_constraints);
 bool rollout_tc_pair_fits(int L, int n_constraints);
-// the trajectory form of rollout_tc.cu (simba_unfold_tc): prm.kernel kTcOneCta or kTcTwoTile, prm.traj_out set
-cudaError_t launch_unfold_tc(const RolloutParams& prm, int n_tiles, cudaStream_t stream);
 // The weight-streaming kernel comes in two state widths `sw`: 64 (prm.kernel kTcWide) and 128 (kTcWideObs).
-cudaError_t launch_rollout_tc_wide(const RolloutParams& prm, int n_tiles, cudaStream_t stream);   // prm.U: the model's units
-cudaError_t launch_unfold_tc_wide(const RolloutParams& prm, int n_tiles, cudaStream_t stream);   // trajectory form
-bool rollout_tc_wide_supported(int sw, int O, int A, int L, int U, int H);
+bool rollout_tc_wide_supported(int sw, int O, int A, int L, int U);
 bool rollout_tc_wide_fits(int sw, int L, int U, int n_constraints);
 int rollout_tc_wide_units(int sw, int U);                     // the padded width the kernel runs
 int64_t rollout_tc_wide_member_bytes(int sw, int L, int UP);   // UP = padded units

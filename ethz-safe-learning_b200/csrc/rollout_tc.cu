@@ -45,6 +45,7 @@
 #include <type_traits>
 
 #include "common.cuh"
+#include "internal.h"
 #include "rollout_params.cuh"
 #include "tc_head.cuh"
 #include "tc_ptx.cuh"
@@ -777,10 +778,10 @@ static size_t tc_smem_bytes(int L, int ntiles, int q, int nparts, bool pair = fa
 
 constexpr size_t kMaxSmem = 227 * 1024;
 
-bool rollout_tc_supported(int O, int A, int L, int U, int H) {
+bool rollout_tc_supported(int O, int A, int L, int U) {
   // narrower hidden layers run zero-padded to 128 units (simba_model_commit pads the images); the
   // member's whole weight set must fit in shared memory next to the one-tile variant's buffers
-  return U >= 1 && U <= kU && O >= 1 && O <= kMaxO && O + A <= 64 && A <= 4 && L >= 1 && H >= 1 && H <= 64 &&
+  return U >= 1 && U <= kU && O >= 1 && O <= kMaxO && O + A <= 64 && A <= 4 && L >= 1 &&
          tc_smem_bytes(L, 1, 4, kHeadParts) + 1024 <= kMaxSmem;
 }
 
@@ -794,61 +795,32 @@ bool rollout_tc_pair_fits(int L, int n_constraints) {
   return tc_smem_bytes(L, 1, 4, 1 + n_constraints, true) + 1024 <= kMaxSmem;
 }
 
-template <int NTILES, int Q, bool PAIR, bool TRAJ = false>
-static cudaError_t launch_variant(const RolloutParams& prm, int n_tiles, cudaStream_t stream) {
+template <int NTILES, int Q, bool PAIR, bool TRAJ>
+static cudaError_t launch_variant(const RolloutParams& prm, cudaStream_t stream) {
   void (*kern)(const RolloutParams) = rollout_tc_kernel<NTILES, Q, PAIR>;
   if constexpr (TRAJ) kern = unfold_tc_kernel<NTILES, Q>;
   const size_t smem = tc_smem_bytes(prm.L, NTILES, Q, TRAJ ? 1 : 1 + prm.scorer.n_constraints, PAIR);
-  // set on every launch: the attribute is per device and per function, and launches happen only at
-  // graph capture or in the non-graph entry points, never on the replayed hot path
-  {
-    cudaError_t e = cudaFuncSetAttribute(kern, cudaFuncAttributeMaxDynamicSharedMemorySize, (int)smem);
-    if (e != cudaSuccess) return e;
-  }
-  const int n_items = (n_tiles + NTILES - 1) / NTILES;
+  const int n_items = (prm.n_tiles + NTILES - 1) / NTILES;
   const int sms = prm.n_sms;
   if (sms <= 0) return cudaErrorInvalidValue;
   // persistent CTAs (one per SM, 1 CTA / SM by shared memory and TMEM); the pair variant runs one item per cluster
   const int grid = PAIR ? 2 * n_items : (n_items < sms ? n_items : sms);
-  cudaLaunchConfig_t cfg{};
-  cfg.gridDim = dim3(grid);
-  cfg.blockDim = dim3(NTILES * Q * 128 + 64 * NTILES);             // epilogue warps + an issuer and a scorer warp per tile
-  cfg.dynamicSmemBytes = smem;
-  cfg.stream = stream;
-  cudaLaunchAttribute attr[2];
-  int na = 0;
-  if (PAIR) {
-    attr[na].id = cudaLaunchAttributeClusterDimension;
-    attr[na].val.clusterDim.x = 2;
-    attr[na].val.clusterDim.y = 1;
-    attr[na].val.clusterDim.z = 1;
-    ++na;
-  }
-  if (prm.pdl) {
-    attr[na].id = cudaLaunchAttributeProgrammaticStreamSerialization;
-    attr[na].val.programmaticStreamSerializationAllowed = 1;
-    ++na;
-  }
-  cfg.attrs = attr;
-  cfg.numAttrs = na;
-  return cudaLaunchKernelEx(&cfg, kern, prm);
+  // epilogue warps + an issuer and a scorer warp per tile
+  return launch_kernel(kern, grid, NTILES * Q * 128 + 64 * NTILES, smem, stream, PAIR ? 2 : 1, prm.pdl, prm);
 }
 
-cudaError_t launch_rollout_tc(const RolloutParams& prm, int n_tiles, cudaStream_t stream) {
-  if (n_tiles == 0) return cudaSuccess;
-  switch (prm.kernel) {
-    case RolloutKernel::kTcOneCta: return launch_variant<1, 4, false>(prm, n_tiles, stream);
-    case RolloutKernel::kTcPair: return launch_variant<1, 4, true>(prm, n_tiles, stream);
-    case RolloutKernel::kTcTwoTile: return launch_variant<2, 2, false>(prm, n_tiles, stream);
-    default: return cudaErrorInvalidValue;
+cudaError_t launch_rollout_tc(const RolloutParams& prm, cudaStream_t stream) {
+  if (prm.traj_out == nullptr) {
+    switch (prm.kernel) {
+      case RolloutKernel::kTcOneCta: return launch_variant<1, 4, false, false>(prm, stream);
+      case RolloutKernel::kTcPair: return launch_variant<1, 4, true, false>(prm, stream);
+      case RolloutKernel::kTcTwoTile: return launch_variant<2, 2, false, false>(prm, stream);
+      default: return cudaErrorInvalidValue;
+    }
   }
-}
-
-cudaError_t launch_unfold_tc(const RolloutParams& prm, int n_tiles, cudaStream_t stream) {
-  if (n_tiles == 0) return cudaSuccess;
-  switch (prm.kernel) {
-    case RolloutKernel::kTcOneCta: return launch_variant<1, 4, false, true>(prm, n_tiles, stream);
-    case RolloutKernel::kTcTwoTile: return launch_variant<2, 2, false, true>(prm, n_tiles, stream);
+  switch (prm.kernel) {   // the trajectory form has no pair variant
+    case RolloutKernel::kTcOneCta: return launch_variant<1, 4, false, true>(prm, stream);
+    case RolloutKernel::kTcTwoTile: return launch_variant<2, 2, false, true>(prm, stream);
     default: return cudaErrorInvalidValue;
   }
 }

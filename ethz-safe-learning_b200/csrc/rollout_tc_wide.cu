@@ -38,6 +38,7 @@
 #include <type_traits>
 
 #include "common.cuh"
+#include "internal.h"
 #include "rollout_params.cuh"
 #include "tc_head.cuh"
 #include "tc_ptx.cuh"
@@ -565,11 +566,11 @@ int rollout_tc_wide_units(int sw, int U) {
 // shape check used when the weight images are packed (no scorer yet: one constraint slot assumed). The layer-0
 // input needs O + A + 2 K elements; head_store_actions writes four state columns from O, so O + 4 <= kSW as well
 // (the <64> variant's O <= 60 implies it).
-bool rollout_tc_wide_supported(int sw, int O, int A, int L, int U, int H) {
+bool rollout_tc_wide_supported(int sw, int O, int A, int L, int U) {
   const int UP = rollout_tc_wide_units(sw, U);
   const bool shape = sw == 64 ? U > 128 && UP <= WideCfg<64>::kMaxUnits && O <= 60 && O + A + 2 <= 64
                               : UP <= WideCfg<128>::kMaxUnits && O + A + 2 <= 128 && O + 4 <= 128;
-  return shape && O >= 1 && A <= 4 && L >= 1 && L <= 6 && H >= 1 && H <= 64 &&
+  return shape && O >= 1 && A <= 4 && L >= 1 && L <= 6 &&
          wide_smem_bytes(sw, L, UP, 1) <= 227 * 1024;
 }
 
@@ -583,46 +584,27 @@ int64_t rollout_tc_wide_member_bytes(int sw, int L, int UP) {
   return (int64_t)(ws.tiles_per_step - ws.head_tiles) * ws.hid_tile_bytes + (int64_t)ws.KA * ws.head_tile_bytes;
 }
 
-template <int kSW, bool TRAJ = false>
-static cudaError_t launch_wide(const RolloutParams& model_prm, int n_tiles, cudaStream_t stream) {
+template <int kSW, bool TRAJ>
+static cudaError_t launch_wide(const RolloutParams& model_prm, cudaStream_t stream) {
   RolloutParams prm = model_prm;
   prm.U = rollout_tc_wide_units(kSW, prm.U);                       // the kernel runs the zero-padded width
   void (*kern)(const RolloutParams) = rollout_tc_wide_kernel<kSW>;
   if constexpr (TRAJ) kern = unfold_tc_wide_kernel<kSW>;
   const size_t smem = wide_smem_bytes<kSW>(prm.L, prm.U, TRAJ ? 1 : 1 + prm.scorer.n_constraints);
-  // set on every launch: the attribute is per device and per function, and launches happen only at
-  // graph capture or in the non-graph entry points, never on the replayed hot path
-  {
-    cudaError_t e = cudaFuncSetAttribute(kern, cudaFuncAttributeMaxDynamicSharedMemorySize, (int)smem);
-    if (e != cudaSuccess) return e;
-  }
-  cudaLaunchConfig_t cfg{};
-  cfg.gridDim = dim3(n_tiles);
-  cfg.blockDim = dim3(kWideThreads);
-  cfg.dynamicSmemBytes = smem;
-  cfg.stream = stream;
-  cudaLaunchAttribute attr[1];
-  attr[0].id = cudaLaunchAttributeProgrammaticStreamSerialization;
-  attr[0].val.programmaticStreamSerializationAllowed = 1;
-  cfg.attrs = attr;
-  cfg.numAttrs = prm.pdl ? 1 : 0;
-  return cudaLaunchKernelEx(&cfg, kern, prm);
+  return launch_kernel(kern, prm.n_tiles, kWideThreads, smem, stream, 1, prm.pdl, prm);
 }
 
-cudaError_t launch_rollout_tc_wide(const RolloutParams& prm, int n_tiles, cudaStream_t stream) {
-  if (n_tiles == 0) return cudaSuccess;
-  switch (prm.kernel) {
-    case RolloutKernel::kTcWide: return launch_wide<64>(prm, n_tiles, stream);
-    case RolloutKernel::kTcWideObs: return launch_wide<128>(prm, n_tiles, stream);
-    default: return cudaErrorInvalidValue;
+cudaError_t launch_rollout_tc_wide(const RolloutParams& prm, cudaStream_t stream) {
+  if (prm.traj_out == nullptr) {
+    switch (prm.kernel) {
+      case RolloutKernel::kTcWide: return launch_wide<64, false>(prm, stream);
+      case RolloutKernel::kTcWideObs: return launch_wide<128, false>(prm, stream);
+      default: return cudaErrorInvalidValue;
+    }
   }
-}
-
-cudaError_t launch_unfold_tc_wide(const RolloutParams& prm, int n_tiles, cudaStream_t stream) {
-  if (n_tiles == 0) return cudaSuccess;
   switch (prm.kernel) {
-    case RolloutKernel::kTcWide: return launch_wide<64, true>(prm, n_tiles, stream);
-    case RolloutKernel::kTcWideObs: return launch_wide<128, true>(prm, n_tiles, stream);
+    case RolloutKernel::kTcWide: return launch_wide<64, true>(prm, stream);
+    case RolloutKernel::kTcWideObs: return launch_wide<128, true>(prm, stream);
     default: return cudaErrorInvalidValue;
   }
 }
