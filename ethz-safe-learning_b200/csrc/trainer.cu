@@ -1,7 +1,9 @@
 // Ensemble training step on the device (include/simba_b200.h "ensemble training step"):
 // replaces MlpEnsemble.training_step / validation_step / fit's inner loop
 // (simba/models/mlp_ensemble.py:134-187). fp32 throughout — the reference trains in fp32 and the
-// planner's fp32 and bf16 weight images are both derived from these master weights.
+// planner's fp32 and bf16 weight images are both derived from these master weights. With
+// precision = SIMBA_PREC_BF16_TC the handle below runs trainer_tc.cu's tcgen05 kernels instead, on the
+// same master weights, Adam state, buffers and graphs.
 //
 // Shape of the work: E members x batch 64 x a 4x128 MLP is 28 MFLOP per member-step — nothing a
 // launch can hide — so the step is latency-bound and the design minimises dependent launches and
@@ -31,6 +33,7 @@
 
 #include "common.cuh"
 #include "internal.h"
+#include "train_common.cuh"
 
 using namespace simba;
 
@@ -48,44 +51,6 @@ constexpr int kRowsU = 64;       // update kernel: batch rows per staged chunk
 constexpr int kThreadsU = 256;
 constexpr int kMaxTrainLayers = 18;
 constexpr int kGraphSteps = 16;  // fit(): steps per CUDA-graph launch
-
-struct TrainState {
-  int iterations;        // optimizer.iterations
-  int fit_step;          // step index inside the running fit()
-  float lr_t;            // lr(iterations) * sqrt(1 - beta2^t) / (1 - beta1^t) of the current step
-  float loss;
-  unsigned nll_ticket;
-};
-
-struct FitDesc {
-  const float* inputs;
-  const float* targets;
-  const int* batch_index;   // [steps, E, bmax]
-  const int* batch_rows;    // [steps] or null
-  float* losses;            // [steps] or null
-  int bmax;
-};
-
-struct OptParams {
-  float lr0, beta1, beta2, epsilon, clipvalue;
-  int schedule, steps_per_epoch, train_epochs;
-};
-
-// A captured graph holds several consecutive steps: step i of the graph works at
-// (st->fit_step + i, st->iterations + i) and one single-thread kernel advances the counters at
-// the end of the graph, so no kernel of the step needs a grid-wide "last CTA" handshake for it.
-__device__ __forceinline__ int resolve_rows(const FitDesc* desc, const TrainState* st, int rows_fixed,
-                                            int step_off) {
-  if (desc != nullptr && desc->batch_rows != nullptr) return desc->batch_rows[st->fit_step + step_off];
-  return rows_fixed;
-}
-
-// fit(): `train_inputs[shuffles_per_mlp]` (mlp_ensemble.py:175-176) is never materialised — the
-// kernels that read the batch follow the index
-__device__ __forceinline__ const int* batch_rows_of(const FitDesc* desc, const TrainState* st, int e,
-                                                    int ensemble, int step_off) {
-  return desc->batch_index + ((int64_t)(st->fit_step + step_off) * ensemble + e) * desc->bmax;
-}
 
 __global__ void advance_kernel(TrainState* st, int n) {
   st->iterations += n;
@@ -137,26 +102,6 @@ __device__ __forceinline__ void bulk_g2s(uint32_t dst, const void* src, uint32_t
       "cp.async.bulk.shared::cluster.global.mbarrier::complete_tx::bytes [%0], [%1], %2, [%3];" ::"r"(dst),
       "l"(src), "r"(bytes), "r"(bar)
       : "memory");
-}
-
-__device__ __forceinline__ float block_sum(float v, float* scratch) {
-  // fixed-order tree: shuffles inside the warp, then thread 0 adds the warp sums in order
-#pragma unroll
-  for (int o = 16; o > 0; o >>= 1) v += __shfl_down_sync(0xffffffffu, v, o);
-  const int w = threadIdx.x >> 5, l = threadIdx.x & 31;
-  __syncthreads();
-  if (l == 0) scratch[w] = v;
-  __syncthreads();
-  float s = 0.0f;
-  if (threadIdx.x == 0)
-    for (int i = 0; i < (int)(blockDim.x >> 5); ++i) s += scratch[i];
-  return s;   // valid in thread 0
-}
-
-__device__ float schedule_lr(const OptParams& o, int iterations) {
-  if (!o.schedule) return o.lr0;
-  const float epochs = floorf((float)(iterations / o.steps_per_epoch));
-  return fmaxf(o.lr0 * (1.0f - epochs / (float)o.train_epochs), 0.0f);
 }
 
 // ---------------------------------------------------------------------------------------------
@@ -435,17 +380,8 @@ train_chain_kernel(ChainArgs a, OptParams opt, const FitDesc* desc, TrainState* 
 #pragma unroll
             for (int j = 0; j < 4; j += 2) {
               float d_mu = 0.0f, d_pre = 0.0f;
-              if (c0 + j < p.n_dim && row_ok) {
-                const float mu = v[j] + pb[j];
-                const float pre = v[j + 1] + pb[j + 1];
-                const float var = softplus_tf(pre) + 1e-4f;
-                const float diff = mu - pm[i][j];
-                const float inv = 1.0f / var;
-                s_log += logf(6.28318530717958647692f * var);
-                s_sq += diff * diff * inv;
-                d_mu = c * diff * inv;
-                d_pre = 0.5f * c * (inv - diff * diff * inv * inv) * (1.0f / (1.0f + expf(-pre)));
-              }
+              if (c0 + j < p.n_dim && row_ok)
+                nll_terms(v[j] + pb[j], v[j + 1] + pb[j + 1], pm[i][j], c, s_log, s_sq, d_mu, d_pre);
               v[j] = d_mu;
               v[j + 1] = d_pre;
             }
@@ -454,14 +390,8 @@ train_chain_kernel(ChainArgs a, OptParams opt, const FitDesc* desc, TrainState* 
             float back = 1.0f;                                   // backward: the same 1 / (1 - rate)
             if (a.train && a.dropout_rate > 0.0f) {
               if (p.kind == kPassHidden) {
-                const uint4 bits = philox4x32_10(
-                    make_uint4((uint32_t)(c0 >> 2), (uint32_t)r, (uint32_t)(st->iterations + step_off),
-                               (uint32_t)e | ((uint32_t)cur.pass << 8) | (4u << 28)),
-                    philox_key(a.dropout_seed));
-                keep[0] = u01(bits.x) >= a.dropout_rate ? a.dropout_scale : 0.0f;
-                keep[1] = u01(bits.y) >= a.dropout_rate ? a.dropout_scale : 0.0f;
-                keep[2] = u01(bits.z) >= a.dropout_rate ? a.dropout_scale : 0.0f;
-                keep[3] = u01(bits.w) >= a.dropout_rate ? a.dropout_scale : 0.0f;
+                dropout_keep4(c0, r, (uint32_t)(st->iterations + step_off), e, cur.pass, a.dropout_rate,
+                              a.dropout_scale, a.dropout_seed, keep);
               } else {
                 back = a.dropout_scale;       // H > 0 <=> unit active AND kept (H is stored after dropout)
               }
@@ -663,14 +593,12 @@ train_update_kernel(UpdArgs a, OptParams opt, const FitDesc* desc, const TrainSt
 #pragma unroll
     for (int j = 0; j < 4; ++j) {
       if (tn0 + tx * 4 + j >= L.N) continue;
-      float g = acc[j];
-      a.grad[p0 + j] = g;
-      if (opt.clipvalue > 0.0f) g = fminf(fmaxf(g, -opt.clipvalue), opt.clipvalue);
-      const float m = mo[j] + (1.0f - opt.beta1) * (g - mo[j]);
-      const float v = ve[j] + (1.0f - opt.beta2) * (g * g - ve[j]);
+      float m, v;
+      a.grad[p0 + j] = acc[j];
+      adam_slots(acc[j], mo[j], ve[j], opt, m, v);
       a.m[p0 + j] = m;
       a.v[p0 + j] = v;
-      nw[j] = th[j] - lr_t * m / (sqrtf(v) + opt.epsilon);
+      nw[j] = adam_weight(th[j], m, v, opt, lr_t);
       a.theta[p0 + j] = nw[j];
     }
   }
@@ -720,6 +648,12 @@ struct simba_trainer {
   FitDesc* desc = nullptr;
   std::vector<int> tile_begin;       // update grid: first tile of each layer
   int n_upd_tiles = 0;
+  // bf16 tcgen05 path (trainer_tc.cu): per member the layers' UMMA weight images, rebuilt by every update
+  uint8_t* img = nullptr;
+  int64_t img_member_bytes = 0;
+  std::vector<TcLayer> tc;
+  std::vector<int> tc_tile_begin;
+  int tc_tiles = 0;
   cudaGraphExec_t fit_graph = nullptr;      // one training step
   cudaGraphExec_t fit_graph_n = nullptr;    // kGraphSteps consecutive steps (amortises the launch gap)
   cudaStream_t graph_stream = nullptr;
@@ -798,7 +732,7 @@ extern "C" int simba_trainer_destroy(simba_trainer_t* t) {
   if (t->fit_graph) cudaGraphExecDestroy(t->fit_graph);
   if (t->fit_graph_n) cudaGraphExecDestroy(t->fit_graph_n);
   if (t->graph_stream) cudaStreamDestroy(t->graph_stream);
-  cudaFree(t->theta); cudaFree(t->thetaT); cudaFree(t->m); cudaFree(t->v); cudaFree(t->grad);
+  cudaFree(t->theta); cudaFree(t->thetaT); cudaFree(t->img); cudaFree(t->m); cudaFree(t->v); cudaFree(t->grad);
   for (float* p : t->act) cudaFree(p);
   for (float* p : t->dz) cudaFree(p);
   cudaFree(t->partial); cudaFree(t->val_acc);
@@ -819,9 +753,19 @@ extern "C" int simba_trainer_create(simba_model_t* model, const simba_trainer_co
     return set_error(SIMBA_ERR_BAD_CONFIG, "Adam hyper-parameters out of range");
   if (!(cfg->dropout_rate >= 0.0f && cfg->dropout_rate < 1.0f))
     return set_error(SIMBA_ERR_BAD_CONFIG, "dropout_rate %g outside [0, 1)", cfg->dropout_rate);
+  if (cfg->precision != SIMBA_PREC_FP32 && cfg->precision != SIMBA_PREC_BF16_TC)
+    return set_error(SIMBA_ERR_BAD_CONFIG, "precision %d is neither SIMBA_PREC_FP32 nor SIMBA_PREC_BF16_TC",
+                     cfg->precision);
+  const simba_model_config_t* mc = model_config(model);
+  if (cfg->precision == SIMBA_PREC_BF16_TC &&
+      !train_tc_supported(mc->obs_dim + mc->act_dim, mc->obs_dim, mc->n_layers, mc->units))
+    return set_error(SIMBA_ERR_UNSUPPORTED,
+                     "bf16 tcgen05 training covers units <= 416, obs_dim + act_dim <= 126, obs_dim <= 124 and "
+                     "n_layers <= 6 (got units %d, obs_dim %d, act_dim %d, n_layers %d); precision fp32 trains "
+                     "this shape",
+                     mc->units, mc->obs_dim, mc->act_dim, mc->n_layers);
   int rc = simba_device_check();
   if (rc) return rc;
-  const simba_model_config_t* mc = model_config(model);
   if (mc->n_layers + 1 > kMaxTrainLayers)
     return set_error(SIMBA_ERR_UNSUPPORTED, "n_layers %d > %d", mc->n_layers, kMaxTrainLayers - 1);
   auto* t = new simba_trainer();
@@ -881,6 +825,19 @@ extern "C" int simba_trainer_create(simba_model_t* model, const simba_trainer_co
     TRY_OR_FREE(cudaMalloc(&t->thetaT, hostT.size() * sizeof(float)));
     TRY_OR_FREE(cudaMemcpy(t->thetaT, hostT.data(), hostT.size() * sizeof(float), cudaMemcpyHostToDevice));
   }
+  if (cfg->precision == SIMBA_PREC_BF16_TC) {
+    for (int l = 0; l <= t->L; ++l) t->tc.push_back(TcLayer{t->K[l], t->N[l], t->off[l], 0, 0});
+    t->img_member_bytes = train_tc_layout(t->tc.data(), t->L + 1);
+    std::vector<uint8_t> img((size_t)E * t->img_member_bytes, 0);
+    for (int e = 0; e < E; ++e)
+      train_tc_pack(t->tc.data(), t->L + 1, host.data() + (size_t)e * t->pn, img.data() + (size_t)e * t->img_member_bytes);
+    TRY_OR_FREE(cudaMalloc(&t->img, img.size()));
+    TRY_OR_FREE(cudaMemcpy(t->img, img.data(), img.size(), cudaMemcpyHostToDevice));
+    for (int l = 0; l <= t->L; ++l) {
+      t->tc_tile_begin.push_back(t->tc_tiles);
+      t->tc_tiles += train_tc_update_tiles(t->tc[l]);
+    }
+  }
   TRY_OR_FREE(cudaFuncSetAttribute(train_chain_kernel<4>, cudaFuncAttributeMaxDynamicSharedMemorySize,
                                    (int)chain_smem_bytes(4, t->ld_act)));
   TRY_OR_FREE(cudaFuncSetAttribute(train_chain_kernel<8>, cudaFuncAttributeMaxDynamicSharedMemorySize,
@@ -921,6 +878,26 @@ static int enqueue_chain(simba_trainer_t* t, const float* x, int64_t x_estride, 
                          const FitDesc* desc, int train, float* out_loss, int step_off,
                          cudaStream_t s) {
   const int64_t R = t->cap_rows, B = t->cfg.batch_size;
+  if (t->cfg.precision == SIMBA_PREC_BF16_TC) {
+    TcChainArgs a{};
+    for (int l = 0; l <= t->L; ++l) {
+      a.layer[l] = t->tc[l];
+      a.act[l] = t->act[l];
+      a.dz[l] = t->dz[l];
+    }
+    a.L = t->L;
+    a.act_estride = R; a.dz_estride = B;
+    a.x = x; a.x_estride = x_estride; a.gather = gather;
+    a.y = y; a.y_estride = y_estride;
+    a.img = t->img; a.img_member_bytes = t->img_member_bytes;
+    a.out_dim = t->O; a.ensemble = t->E;
+    a.partial = t->partial; a.tiles_cap = t->tiles_cap; a.train = train; a.out_loss = out_loss;
+    a.dropout_rate = t->cfg.dropout_rate;
+    a.dropout_scale = 1.0f / (1.0f - t->cfg.dropout_rate);
+    a.dropout_seed = t->cfg.dropout_seed;
+    SIMBA_CUDA_TRY(train_tc_chain(a, opt_params(t), desc, t->state, grid_rows, rows_fixed, step_off, s));
+    return SIMBA_OK;
+  }
   ChainArgs a{};
   int np = 0;
   for (int l = 0; l <= t->L; ++l) {
@@ -975,6 +952,24 @@ static int enqueue_step(simba_trainer_t* t, const float* x, int64_t x_estride, c
   int rc = enqueue_chain(t, x, x_estride, y, y_estride, gather, grid_rows, rows_fixed, desc, 1,
                          out_loss, step_off, s);
   if (rc) return rc;
+  if (t->cfg.precision == SIMBA_PREC_BF16_TC) {
+    TcUpdArgs u{};
+    for (int l = 0; l <= t->L; ++l) {
+      u.layer[l] = t->tc[l];
+      u.tile_begin[l] = t->tc_tile_begin[l];
+      u.n_tiles_n[l] = (t->N[l] + 127) / 128;
+      u.h[l] = l == 0 ? x : t->act[l];
+      u.h_estride[l] = l == 0 ? x_estride : R * t->K[l];
+      u.dz[l] = t->dz[l];
+    }
+    u.n_layers = t->L + 1;
+    u.gather0 = gather;
+    u.dz_estride = B;
+    u.theta = t->theta; u.m = t->m; u.v = t->v; u.grad = t->grad; u.pn = t->pn;
+    u.img = t->img; u.img_member_bytes = t->img_member_bytes; u.ensemble = t->E;
+    SIMBA_CUDA_TRY(train_tc_update(u, opt_params(t), desc, t->state, t->tc_tiles, rows_fixed, step_off, s));
+    return SIMBA_OK;
+  }
   UpdArgs u{};
   for (int l = 0; l <= t->L; ++l) {
     UpdLayer& U = u.layers[l];
@@ -1055,7 +1050,7 @@ extern "C" int simba_trainer_validation(simba_trainer_t* t, const float* x, cons
     const int nr = (int)((rows - r0) < t->cap_rows ? (rows - r0) : t->cap_rows);
     int rc = enqueue_chain(t, x + r0 * t->IN, 0, y + r0 * t->O, 0, 0, nr, nr, nullptr, 0, nullptr, 0, s);
     if (rc) return rc;
-    const int R = chain_tile_rows(t, nr);
+    const int R = t->cfg.precision == SIMBA_PREC_BF16_TC ? kTcRows : chain_tile_rows(t, nr);
     const int tiles = (nr + R - 1) / R;
     val_accumulate_kernel<<<1, 32, 0, s>>>(t->partial, t->tiles_cap, tiles, t->E, t->val_acc,
                                            r0 == 0 ? 1 : 0);

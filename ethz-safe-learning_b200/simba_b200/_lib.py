@@ -66,7 +66,8 @@ class TrainerConfig(C.Structure):
                 ('learning_rate', C.c_float), ('lr_schedule', C.c_int32),
                 ('steps_per_epoch', C.c_int32), ('train_epochs', C.c_int32),
                 ('beta1', C.c_float), ('beta2', C.c_float), ('epsilon', C.c_float),
-                ('clipvalue', C.c_float), ('dropout_rate', C.c_float), ('dropout_seed', C.c_uint64)]
+                ('clipvalue', C.c_float), ('dropout_rate', C.c_float), ('dropout_seed', C.c_uint64),
+                ('precision', C.c_int32)]
 
 
 _vp, _i32, _u64, _f = C.c_void_p, C.c_int32, C.c_uint64, C.c_float

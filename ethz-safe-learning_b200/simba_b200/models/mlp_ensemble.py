@@ -56,8 +56,15 @@ def glorot_uniform(rng, fan_in, fan_out):
 class MlpEnsemble(object):
     def __init__(self, inputs_dim, outputs_dim, ensemble_size, batch_size=64, validation_split=0.2,
                  learning_rate=0.00025, learning_rate_schedule=True, training_steps=5000,
-                 mlp_params=None, train_epochs=1, seed=0):
+                 mlp_params=None, train_epochs=1, seed=0, train_precision='fp32'):
+        if train_precision not in _lib.PRECISIONS:
+            raise ValueError("train_precision must be one of %s, got %r"
+                             % (sorted(_lib.PRECISIONS), train_precision))
         mlp_params = dict(mlp_params or {})
+        # 'fp32': the fp32 SIMT trainer; 'bf16': GEMMs on bf16 tcgen05 tensor cores with fp32 accumulation,
+        # NLL and Adam (DESIGN.md section 5, "bf16 training"). Shapes the bf16 trainer does not cover raise
+        # SimbaError SIMBA_ERR_UNSUPPORTED when the trainer is created.
+        self.train_precision = train_precision
         self.inputs_dim = inputs_dim
         self.outputs_dim = outputs_dim
         self.ensemble_size = ensemble_size
@@ -218,7 +225,8 @@ class MlpEnsemble(object):
             cfg = _lib.TrainerConfig(int(self.batch_size), self.EVAL_ROWS, float(self.learning_rate),
                                      int(self.learning_rate_schedule), int(self.training_steps),
                                      int(self.train_epochs), 0.9, 0.999, 1e-5, 1.0,
-                                     float(self.dropout_rate), int(self.dropout_seed))
+                                     float(self.dropout_rate), int(self.dropout_seed),
+                                     _lib.PRECISIONS[self.train_precision])
             t = C.c_void_p()
             _lib.check(self._lib.simba_trainer_create(h, C.byref(cfg), C.byref(t)))
             self._trainer = t

@@ -276,7 +276,8 @@ int simba_scorer_eval(const simba_scorer_t* sc, const float* obs, const float* n
  * Replaces MlpEnsemble.training_step / validation_step / fit (simba/models/mlp_ensemble.py:134-187):
  * forward (training=True, dropout 0), negative_log_likelihood (:64-67) summed over members / E,
  * backward, and tf.keras.optimizers.Adam(clipvalue, epsilon) with EpochLearningRateSchedule
- * (:70-88, :113-117) — all fp32 CUDA kernels on master weights that stay on the device. */
+ * (:70-88, :113-117) — CUDA kernels on fp32 master weights that stay on the device. The GEMMs run
+ * in fp32 (default) or, with precision = SIMBA_PREC_BF16_TC, on bf16 tcgen05 tensor cores. */
 typedef struct simba_trainer simba_trainer_t;
 typedef struct simba_trainer_config {
   int32_t batch_size;        /* models.yaml:4 — the largest training batch (rows per member)     */
@@ -290,6 +291,12 @@ typedef struct simba_trainer_config {
   float clipvalue;           /* mlp_ensemble.py:116 (1.0); <= 0 disables clipping               */
   float dropout_rate;        /* models.yaml:13 (0.0): Dropout after every hidden ReLU in training */
   uint64_t dropout_seed;     /* Philox key of the dropout masks (stream 4, see oracle/philox.py)  */
+  int32_t precision;         /* simba_precision. SIMBA_PREC_FP32 (0): the fp32 SIMT kernels, parity
+                                with the oracle. SIMBA_PREC_BF16_TC: bf16 tcgen05 GEMMs with fp32
+                                accumulation, NLL and Adam on fp32 master weights (DESIGN.md section 5,
+                                "bf16 training"); covers units <= 416, obs_dim + act_dim <= 126,
+                                obs_dim <= 124, n_layers <= 6 and returns SIMBA_ERR_UNSUPPORTED for
+                                any other shape (no fp32 fall-back)                               */
 } simba_trainer_config_t;
 
 /* Copies the model's current (set_layer) weights as fp32 master weights; Adam state zeroed. The
