@@ -27,7 +27,9 @@
 //     (after tcgen05.wait::st + fence) and moves on; the issuer warp bar.sync's on it, issues the
 //     layer, tcgen05.commit's onto the tile's mbarrier, waits for that (the only mbarrier poller of
 //     the tile) and bar.arrive's on the tile's "accumulator ready" barrier, on which the epilogue
-//     warps bar.sync;
+//     warps bar.sync. The one-tile variants split every layer into two 64-column halves on
+//     double-buffered accumulators and A operands, each half with its own pair of barriers, so one
+//     half drains while the other is still multiplied (see the issuer warp);
 //   * per hidden layer an epilogue thread reads its column slice of the fp32 accumulator row
 //     (tcgen05.ld 32x32b), applies ReLU, packs bf16 and writes the next layer's A operand
 //     (tcgen05.st); in the shadow of the following MMAs it produces one Philox block of the step's
@@ -69,7 +71,7 @@ namespace {
 constexpr int kU = 128;                 // hidden width this kernel covers
 constexpr int kMaxO = 60;               // observation dims (two Gaussian heads padded to 2 x 64 columns)
 constexpr int kAtomBytes = 128 * 128;   // one 64-wide K atom of a 128-row tile (bf16, SW128)
-constexpr int kBoundThreads = 640;      // launch bound: the hardware allocates warps in fours, so 17 / 18
+constexpr int kBoundThreads = 640;      // launch bound: the hardware allocates warps in fours, so 17 - 19
                                         // warps occupy 20 warp slots -> 96 registers per thread
 
 struct TileInfo {
@@ -155,13 +157,26 @@ __device__ __forceinline__ void rollout_tc_body(const RolloutParams& prm) {
   constexpr int NB = OW / 8;          // Philox blocks / 8-wide chunks per thread and step
   constexpr int HCOLS = 128 / Q;      // accumulator columns per thread and hidden layer
   // TMEM columns per tile: 128 fp32 accumulator columns, 64 fp32 state columns and 64 columns that
-  // hold the bf16 A operand (128 K-elements, two per 32-bit column). Layout:
-  // [NTILES x 128 acc][NTILES x 64 state][NTILES x 64 A]  ->  256 / 512 columns (power of two)
-  constexpr int kTmemCols = NTILES * 256;
+  // hold the bf16 A operand (128 K-elements, two per 32-bit column).
+  //   two tiles: [2 x 128 acc][2 x 64 state][2 x 64 A] = 512 columns
+  //   one tile (kDbl): [2 x 128 acc][64 state][2 x 64 A] = 448 of 512 allocated columns. The accumulator and
+  //   the A operand are double-buffered: consecutive GEMMs of a step alternate between buffers 0 and 1, so a
+  //   layer's two 64-column halves can drain while the other half is still being multiplied (see the issuer).
+  // Taking all 512 columns of the SM is safe only because no second CTA of these kernels can be resident on
+  // the SM and block in tcgen05.alloc: a CTA holds more than half of the SM's registers (576 or 640 threads
+  // under the 96-register bound) and, at C1 depth, of its shared memory.
+  constexpr bool kDbl = NTILES == 1;
+  static_assert(!kDbl || Q == 4, "the one-tile variants split the columns into halves of two column groups");
+  constexpr int kTmemCols = 512;
+  constexpr uint32_t kStateCol = kDbl ? 256 : NTILES * 128;
+  constexpr uint32_t kACol = kDbl ? 320 : NTILES * 192;
   // Throughput variant: the step's noise and the per-row running objective are parked in shared
   // memory to free registers. Latency variant (one tile): they stay in registers.
   constexpr bool kPark = NTILES > 1;
   constexpr int kBarAcc = 2, kBarA = 2 + NTILES, kBarPart = 2 + 2 * NTILES, kBarFree = 2 + 3 * NTILES;   // ids (+ tile)
+  // one tile: kBarAcc / kBarA are "accumulator ready" / "A ready" of the low column half (columns 0-63, the
+  // warps of column groups 0-1); these two are the high half's (column groups 2-3)
+  constexpr int kBarAccHi = 6, kBarAHi = 7;
   extern __shared__ __align__(1024) uint8_t smem_raw[];
   const RowGeom& g = prm.g;
   const int L = prm.L;
@@ -179,6 +194,7 @@ __device__ __forceinline__ void rollout_tc_body(const RolloutParams& prm) {
   const bool l0_pad_bias = (O + A + 2 <= 64);     // layer-0 bias rides in the K padding (see pack in api.cu)
   constexpr int n_quarters = 4;                   // TMEM lane quarters (= warps per column group) of a tile
   constexpr int tile_bar_threads = Q * 128 + 32;  // a tile's epilogue warps + one partner warp (issuer / scorer)
+  constexpr int half_bar_threads = Q * 64 + 32;   // one tile: the epilogue warps of a column half + the issuer or relay warp
 
   // ---- shared memory carve-up (base is 1024-aligned: required by SWIZZLE_128B) -------------------
   const uint32_t w_bytes = kAtomBytes + (uint32_t)L * 2 * kAtomBytes;     // layer 0: 1 atom; others: 2
@@ -198,7 +214,8 @@ __device__ __forceinline__ void rollout_tc_body(const RolloutParams& prm) {
   // bars[0] = weights landed; bars[1 + j] = MMAs of tile j committed. Named barriers: 0 = CTA, 1 = all
   // epilogue threads, 2 + j = "accumulator ready" of tile j, 2 + NTILES + j = "A ready"
   // PAIR: bars[1 + NTILES + p] = the peer's warps have sent their step-parity-p slices
-  uint32_t* tmem_slot = reinterpret_cast<uint32_t*>(bars + 1 + NTILES + 2);
+  // one tile: bars[1] = the low column half's MMAs committed, bars[3 + NTILES] = the high half's
+  uint32_t* tmem_slot = reinterpret_cast<uint32_t*>(bars + 1 + NTILES + 2 + (kDbl ? 1 : 0));
   TileInfo* tinfo = reinterpret_cast<TileInfo*>(tmem_slot + 2);
   uint64_t* seed_sh = reinterpret_cast<uint64_t*>(tinfo + NTILES);
   int32_t* w_state_sh = reinterpret_cast<int32_t*>(seed_sh + 1);     // [0] member whose weights are staged, [1] loads issued
@@ -245,6 +262,7 @@ __device__ __forceinline__ void rollout_tc_body(const RolloutParams& prm) {
     for (int j = 0; j < NTILES; ++j) {
       mbar_init(smem_u32(&bars[1 + j]), 1);                      // tcgen05.commit
     }
+    if (kDbl) mbar_init(smem_u32(&bars[3 + NTILES]), 1);         // tcgen05.commit of the high half
     if (PAIR) {                                                  // armed below, once the tile is known to be live
       mbar_init(smem_u32(&bars[1 + NTILES]), 1);
       mbar_init(smem_u32(&bars[2 + NTILES]), 1);
@@ -348,7 +366,29 @@ __device__ __forceinline__ void rollout_tc_body(const RolloutParams& prm) {
   __syncthreads();
 
   if (any_valid) {
-    if (warp >= kEpiWarps + NTILES) {
+    if (kDbl && warp == kEpiWarps + 2 * NTILES) {
+      // ====================== relay warp (one tile): commit 0 -> "accumulator low ready", commit 1 -> "high ready" ===
+      // The low half drains while the high half's last MMAs run. tcgen05.mma blocks the issuing thread at the
+      // pipe's rate, so the issuer itself would see commit 0 only after it has issued the high half's MMAs; this
+      // warp sleeps on the commit mbarriers instead (the tile's only mbarrier poller). The head pass reads both
+      // halves, so there the low half waits for commit 1 as well, which completes after every earlier MMA (commit
+      // 0's phase passes unobserved and is not waited for again). Neither barrier can run two phases ahead: the
+      // next commit onto it follows an "A ready" of the warps this relay releases.
+      if (tinfo[0].valid && late_gate(tinfo[0])) {
+        const uint32_t bar_lo = smem_u32(&bars[1]), bar_hi = smem_u32(&bars[3 + NTILES]);
+        for (int t = 0; t < H; ++t) {
+          for (int layer = 0; layer <= L; ++layer) {
+            mbar_wait(layer < L ? bar_lo : bar_hi, ph);
+            tc_fence_before();
+            named_bar_arrive_n(kBarAcc, half_bar_threads);
+            mbar_wait(bar_hi, ph);
+            ph ^= 1;
+            tc_fence_before();
+            named_bar_arrive_n(kBarAccHi, half_bar_threads);
+          }
+        }
+      }
+    } else if (warp >= kEpiWarps + NTILES) {
       // ====================== scorer warp of tile j: the per-row objective, off everybody's critical path ======
       // (mpc_policy.py:30-37 / safe_cem_mpc.py:82-93 on safety_gym.py:110-166). Lane i owns rows i, i + 32,
       // i + 64, i + 96 of the tile. After every head pass the epilogue warps bar.arrive on "partials
@@ -443,13 +483,104 @@ __device__ __forceinline__ void rollout_tc_body(const RolloutParams& prm) {
       if (tinfo[j].valid) {
         const uint32_t bar_acc = smem_u32(&bars[1 + j]);
         const uint32_t d_tmem = tmem_base + (uint32_t)j * 128;
-        const uint32_t a_tmem = tmem_base + (uint32_t)(NTILES * 192 + j * 64);       // lane 0, A columns
+        const uint32_t a_tmem = tmem_base + (uint32_t)(kACol + j * 64);              // lane 0, A columns
         const uint64_t ones_desc = umma_desc_k16_noswizzle(smem_u32(ones_smem));
         mbar_wait(bar_w, (uint32_t)(w_state_sh[1] - 1) & 1u);   // this member's weights have landed before the first MMA
 #ifdef SIMBA_TC_TIMELINE
         const int tl_who = (j == 0 && lane == 0) ? 2 : -1;
 #endif
         const bool live = late_gate(tinfo[j]);
+        if constexpr (kDbl) {
+          // One tile: every GEMM is issued as two N = 64 column halves, so that one half drains while the other
+          // is multiplied. Order: N0 x K[0,64) and N1 x K[0,64) (these read only A's low half), then, once the
+          // high half of A is in TMEM, N0 x K[64,128) + bias -> commit 0, N1 x K[64,128) + bias -> commit 1.
+          // Every output element still accumulates K-steps 0..7, then the bias, as the N = 128 MMAs of the
+          // two-tile kernel do (its rows are bit-identical). Layer 0 (K = 64): N0 (+ bias), commit 0, N1 (+ bias),
+          // commit 1. The pair's head GEMM multiplies only this CTA's columns: mu [32 c, 32 c + 32) and raw
+          // variance [64 + 32 c, ...), two N = 32 MMAs per K-step in place of the halves.
+          // Why no MMA reads or writes TMEM that an epilogue warp is still using: GEMM n reads A[n & 1] and
+          // accumulates into acc[n & 1];
+          //  * A[n & 1] is rewritten by the drain of GEMM n + 1 (or the head pass), which starts after a commit of
+          //    GEMM n + 1, and a commit completes only when every earlier MMA of this thread has, GEMM n included;
+          // The issuer waits for no commit: the relay warp below hands them to the epilogue warps.
+          //  * acc[n & 1] is next written by GEMM n + 2. Its low-half MMAs are issued after "A low ready" of
+          //    GEMM n + 2, its high-half MMAs after GEMM n + 1 was fully issued, i.e. after "A high ready" of
+          //    GEMM n + 1: each half's warps publish that only after their tcgen05.ld of acc[n & 1] was waited;
+          //  * the head pass -> layer 0 boundary stays a full synchronisation: the head pass reads both halves of
+          //    its accumulator (both commits), and layer 0 waits for the x slices of all warps (both "A ready").
+          const uint32_t bar_acc_hi = smem_u32(&bars[3 + NTILES]);
+          constexpr uint32_t kIdesc64 = umma_idesc_n(64u), kIdesc32 = umma_idesc_n(32u);
+          uint32_t par = 0;                                 // buffers of the next GEMM
+          // K-steps [kb, kb + 4) of one half: D columns d, B descriptor b (its rows = those columns)
+          auto mma4 = [&](uint32_t d, uint32_t a, uint64_t b, uint32_t idesc, int kb) {
+#pragma unroll
+            for (int k = 0; k < 4; ++k)
+              umma_bf16_ts(d, a + (uint32_t)(kb + k) * 8, b + (uint64_t)(((kb ? kAtomBytes : 0) + k * 32) >> 4), idesc,
+                           (kb + k) > 0 ? 1u : 0u);
+          };
+          // bias block rows from `col` (8-row groups of 256 bytes)
+          auto mma_bias = [&](uint32_t d, uint32_t bias_sm, uint32_t col, uint32_t idesc) {
+            umma_bf16(d, ones_desc, umma_desc_k16_noswizzle(bias_sm + col * 32), idesc, 1u);
+          };
+          for (int t = 0; live && t < H; ++t) {
+#ifdef SIMBA_TC_TIMELINE
+            const int tl_t = t;
+#endif
+            {                                               // layer 0 (K = 64): needs the x slices of all warps
+              const uint32_t d = d_tmem + par * 128, a = a_tmem + par * 64;
+              const uint64_t b = umma_desc_sw128(smem_u32(w_smem));
+              const uint32_t bias_sm = smem_u32(biask_smem);
+              named_bar_sync_n(kBarA, half_bar_threads);
+              named_bar_sync_n(kBarAHi, half_bar_threads);
+              tc_fence_after();
+              TL(0);
+              if (elect_one()) {
+                mma4(d, a, b, kIdesc64, 0);
+                if (!l0_pad_bias) mma_bias(d, bias_sm, 0u, kIdesc64);
+                umma_commit(bar_acc);
+                mma4(d + 64, a, b + (uint64_t)((64 * 128) >> 4), kIdesc64, 0);
+                if (!l0_pad_bias) mma_bias(d + 64, bias_sm, 64u, kIdesc64);
+                umma_commit(bar_acc_hi);
+              }
+              TL(1);
+              __syncwarp();
+              par ^= 1;                                     // the relay warp releases the epilogue warps
+            }
+            for (int layer = 1; layer <= L; ++layer) {
+              const uint32_t d = d_tmem + par * 128, a = a_tmem + par * 64;
+              const bool own_head = PAIR && layer == L;
+              const uint32_t c0 = own_head ? crank * 32 : 0u, c1 = own_head ? 64u + crank * 32 : 64u;   // columns = B rows
+              const uint32_t idesc = own_head ? kIdesc32 : kIdesc64;
+              // B rows c0 / c1 start whole 1024-byte swizzle groups (SW128)
+              const uint64_t bw = umma_desc_sw128(smem_u32(w_smem + kAtomBytes + (layer - 1) * 2 * kAtomBytes));
+              const uint64_t b0 = bw + (uint64_t)((c0 * 128) >> 4), b1 = bw + (uint64_t)((c1 * 128) >> 4);
+              const uint32_t bias_sm = smem_u32(biask_smem + layer * 4096);
+              named_bar_sync_n(kBarA, half_bar_threads);      // the low half of this GEMM's A is in TMEM
+              tc_fence_after();
+              TL(2 * layer);
+              if (elect_one()) {                              // K[0, 64) of both halves
+                mma4(d + c0, a, b0, idesc, 0);
+                mma4(d + c1, a, b1, idesc, 0);
+              }
+              TL(2 * layer + 1);
+              __syncwarp();
+              named_bar_sync_n(kBarAHi, half_bar_threads);    // the high half of A
+              tc_fence_after();
+              TL(20 + 2 * layer);
+              if (elect_one()) {                              // K[64, 128) + bias, one half after the other
+                mma4(d + c0, a, b0, idesc, 4);
+                mma_bias(d + c0, bias_sm, c0, idesc);
+                umma_commit(bar_acc);
+                mma4(d + c1, a, b1, idesc, 4);
+                mma_bias(d + c1, bias_sm, c1, idesc);
+                umma_commit(bar_acc_hi);
+              }
+              TL(21 + 2 * layer);
+              __syncwarp();
+              par ^= 1;
+            }
+          }
+        } else
         for (int t = 0; live && t < H; ++t) {
 #ifdef SIMBA_TC_TIMELINE
           const int tl_t = t;
@@ -498,13 +629,13 @@ __device__ __forceinline__ void rollout_tc_body(const RolloutParams& prm) {
         const RowId id = decode_row(g, ti.member, ti.k0 + (row_ok ? r : 0));
         const uint32_t lane_base = tmem_base + ((uint32_t)((wl & 3) * 32) << 16);
         const uint32_t t_acc = lane_base + (uint32_t)j * 128;
-        const uint32_t t_a = lane_base + (uint32_t)(NTILES * 192 + j * 64);   // this row's A-operand columns
+        const uint32_t t_a = lane_base + (uint32_t)(kACol + j * 64);          // this row's A-operand columns (one tile: buffer 0)
         const float* act_ptr = prm.actions + ((int64_t)id.s * g.N + id.i_global) * prm.action_stride;
         const simba_scorer_t& sc = prm.scorer;
 
         HeadCtx hc;
         hc.t_acc = t_acc;
-        hc.t_state = lane_base + (uint32_t)(NTILES * 128 + j * 64);
+        hc.t_state = lane_base + (uint32_t)(kStateCol + j * 64);
         hc.o_base = (PAIR ? (int)crank * 32 : 0) + cgp * OW;
         hc.O = O; hc.A = A;
         hc.slice_bits = TRAJ ? 0u : head_slice_bits<OW>(sc, hc.o_base);
@@ -538,7 +669,7 @@ __device__ __forceinline__ void rollout_tc_body(const RolloutParams& prm) {
               mbar_wait(my_xbar + 8u * b, (uint32_t)((t + 1) >> 1) & 1u);     // all of the peer's step-t stores have landed
               const uint4 v = xch_smem[(b * Q + cgp) * 128 + r];
               const uint32_t pk[4] = {v.x, v.y, v.z, v.w};
-              tmem_st<4>(t_a + (uint32_t)((((int)crank ^ 1) * 32 + cgp * 8) >> 1), pk);
+              tmem_st<4>(astore.t_a + (uint32_t)((((int)crank ^ 1) * 32 + cgp * 8) >> 1), pk);
             }
           }
         };
@@ -556,18 +687,25 @@ __device__ __forceinline__ void rollout_tc_body(const RolloutParams& prm) {
 #endif
         // this warp's slice of the tile's next A operand is complete: stores landed and ordered before
         // the issuer's MMAs; count the warp in on "A ready" without waiting
+        // one tile: the warps of column groups 0-1 hand off through the low half's barriers, 2-3 the high half's
+        static_assert(!kDbl || kBarAccHi - kBarAcc == kBarAHi - kBarA, "one offset selects both barriers of a half");
+        const int bar_off = kDbl ? (cgp >= Q / 2 ? kBarAHi - kBarA : 0) : j;
+        const int bar_acc_mine = kBarAcc + bar_off, bar_a_mine = kBarA + bar_off;
+        const int hand_off_threads = kDbl ? half_bar_threads : tile_bar_threads;
         auto publish_a = [&]() {
           tmem_st_wait();
           tc_fence_before();
-          named_bar_arrive_n(kBarA + j, tile_bar_threads);
+          named_bar_arrive_n(bar_a_mine, hand_off_threads);
         };
         auto wait_accumulator = [&]() {
           // released by the issuer warp's arrive. (Letting the sixteen epilogue warps sleep on the commit
           // mbarrier themselves is slower even in the one-tile variant: commit -> accumulator seen 496
           // cycles instead of 408 through the relay, measured.)
-          named_bar_sync_n(kBarAcc + j, tile_bar_threads);
+          named_bar_sync_n(bar_acc_mine, hand_off_threads);
           tc_fence_after();
         };
+        // one tile: buffers of GEMM l of step t (GEMM n of the item uses accumulator and A buffer n & 1)
+        auto gemm_par = [&](int t, int l) { return (uint32_t)(t * (L + 1) + l) & 1u; };
 
         // the thread whose column slice holds state column O prefetches a_{t+1} one step ahead (the L2
         // latency is off the critical path) and parks it in state columns [O, O + A) of its row
@@ -663,7 +801,7 @@ __device__ __forceinline__ void rollout_tc_body(const RolloutParams& prm) {
               constexpr int NLD = HCOLS / 32;                // 32-column loads per thread (2 at Q = 2)
               uint32_t v[NLD][32];
 #pragma unroll
-              for (int i = 0; i < NLD; ++i) tmem_ld<32>(t_acc + (uint32_t)(cgp * HCOLS + i * 32), v[i]);
+              for (int i = 0; i < NLD; ++i) tmem_ld<32>(t_acc + (kDbl ? gemm_par(t, l) * 128 : 0u) + (uint32_t)(cgp * HCOLS + i * 32), v[i]);
               tmem_ld_wait();
 #pragma unroll
               for (int i = 0; i < NLD; ++i) {
@@ -671,7 +809,7 @@ __device__ __forceinline__ void rollout_tc_body(const RolloutParams& prm) {
 #pragma unroll
                 for (int q = 0; q < 16; ++q)
                   pk[q] = pack_relu_bf16(__uint_as_float(v[i][2 * q]), __uint_as_float(v[i][2 * q + 1]));
-                tmem_st<16>(t_a + (uint32_t)((cgp * HCOLS + i * 32) / 2), pk);
+                tmem_st<16>(t_a + (kDbl ? (gemm_par(t, l) ^ 1u) * 64 : 0u) + (uint32_t)((cgp * HCOLS + i * 32) / 2), pk);
               }
             }
             TL(2 + l * 4);
@@ -718,6 +856,10 @@ __device__ __forceinline__ void rollout_tc_body(const RolloutParams& prm) {
           }
           if constexpr (TRAJ) {
             if (sink.row != nullptr) sink.row += O;
+          }
+          if constexpr (kDbl) {                             // the head GEMM's accumulator, x_{t+1} into the other A buffer
+            hc.t_acc = t_acc + gemm_par(t, L) * 128;
+            astore.t_a = t_a + (gemm_par(t, L) ^ 1u) * 64;
           }
           if (prm.sampling_propagation) head_step_pass<OW, true>(hc, noise, astore, t + 1 < H, sink);
           else head_step_pass<OW, false>(hc, noise, astore, t + 1 < H, sink);
@@ -772,7 +914,7 @@ static size_t tc_smem_bytes(int L, int ntiles, int q, int nparts, bool pair = fa
   if (ntiles > 1)                                                  // parking area of the two-tile variant:
     b += (size_t)(64 / q / 8) * (ntiles * q * 128) * sizeof(uint4);      // bf16x2 noise of the current step
   b += (size_t)8 * ntiles * 128 * sizeof(uint32_t);                      // per-row running objective
-  b += (3 + ntiles) * sizeof(uint64_t) + 2 * sizeof(uint32_t) + ntiles * sizeof(TileInfo) + sizeof(uint64_t) + 2 * sizeof(int32_t);
+  b += (3 + ntiles + (ntiles == 1 ? 1 : 0)) * sizeof(uint64_t) + 2 * sizeof(uint32_t) + ntiles * sizeof(TileInfo) + sizeof(uint64_t) + 2 * sizeof(int32_t);
   return b + 1024;                                                 // alignment slack
 }
 
@@ -805,8 +947,8 @@ static cudaError_t launch_variant(const RolloutParams& prm, cudaStream_t stream)
   if (sms <= 0) return cudaErrorInvalidValue;
   // persistent CTAs (one per SM, 1 CTA / SM by shared memory and TMEM); the pair variant runs one item per cluster
   const int grid = PAIR ? 2 * n_items : (n_items < sms ? n_items : sms);
-  // epilogue warps + an issuer and a scorer warp per tile
-  return launch_kernel(kern, grid, NTILES * Q * 128 + 64 * NTILES, smem, stream, PAIR ? 2 : 1, prm.pdl, prm);
+  // epilogue warps + an issuer and a scorer warp per tile (+ the one-tile variants' relay warp)
+  return launch_kernel(kern, grid, NTILES * Q * 128 + 64 * NTILES + (NTILES == 1 ? 32 : 0), smem, stream, PAIR ? 2 : 1, prm.pdl, prm);
 }
 
 cudaError_t launch_rollout_tc(const RolloutParams& prm, cudaStream_t stream) {

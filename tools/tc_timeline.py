@@ -66,8 +66,28 @@ for step in range(2, min(H - 1, 8)):
 k = t[3, 0]
 print("== launch anatomy, thread 0 of CTA 0 (cycles since kernel entry): setup done %d, PDL wait passed %d, first A published %d, "
       "all items done %d, exit %d" % tuple(int(k[i] - k[0]) for i in range(1, 6)))
-print("== issuer warp of tile 0 (cycles since epilogue warp 0's step start; layer: A-ready seen -> committed)")
+if wl == 'c4':
+    print("== issuer warp of tile 0 (cycles since epilogue warp 0's step start; layer: A-ready seen -> committed)")
+    for step in range(2, min(H - 1, 8)):
+        base = t[0, step][0]
+        ev = t[2, step]
+        print("step %2d " % step + ' | '.join("L%d %5d -> %5d" % (l, ev[2 * l] - base, ev[2 * l + 1] - base) for l in range(L + 1)))
+    sys.exit(0)
+# one-tile kernels: every layer is two 64-column halves. Epilogue warp 0 above drains the low half, the last warp the
+# high half. The issuer stamps 2l (A low half seen), 2l+1 (K[0,64) of both halves issued; layer 0: both halves
+# committed), 20+2l (A high half seen) and 21+2l (commits 0 and 1 issued) for hidden and head layers l >= 1.
+print("== issuer warp (cycles since epilogue warp 0's step start; layer: A low seen -> K[0,64) issued, "
+      "A high seen -> both halves committed)")
 for step in range(2, min(H - 1, 8)):
     base = t[0, step][0]
     ev = t[2, step]
-    print("step %2d " % step + ' | '.join("L%d %5d -> %5d" % (l, ev[2 * l] - base, ev[2 * l + 1] - base) for l in range(L + 1)))
+    parts = ["L0 %5d -> %5d" % (ev[0] - base, ev[1] - base)]
+    parts += ["L%d %5d -> %5d, %5d -> %5d" % (l, ev[2 * l] - base, ev[2 * l + 1] - base, ev[20 + 2 * l] - base,
+                                              ev[21 + 2 * l] - base) for l in range(1, L + 1)]
+    print("step %2d " % step + ' | '.join(parts))
+print("== per hidden layer: high half ready - low half ready / low half published - high half ready (cycles; the "
+      "low half drains while the high half's last MMAs run)")
+for step in range(2, min(H - 1, 8)):
+    lo, hi = t[0, step], t[1, step]
+    print("step %2d " % step + ' '.join("L%d %5d / %5d" % (l, hi[1 + 4 * l] - lo[1 + 4 * l], lo[3 + 4 * l] - hi[1 + 4 * l])
+                                        for l in range(L)))
