@@ -1,6 +1,7 @@
-// C-ABI of libsimba_b200.so (include/simba_b200.h): handles, weight packing, work lists, the
-// CUDA-graph planning call and the NCCL all-gather. Host-side C++; every compute step is a CUDA
-// kernel from rollout_f32.cu / rollout_tc.cu / cem_kernels.cu — there is no CPU path.
+// C-ABI of libsimba_b200.so (include/simba_b200.h): handles, device weight images (each packed by the
+// kernel file that reads it), work lists, the CUDA-graph planning call and the NCCL all-gather.
+// Host-side C++; every compute step is a CUDA kernel from rollout_f32.cu / rollout_tc.cu /
+// cem_kernels.cu — there is no CPU path.
 #include <dlfcn.h>
 
 #include <cmath>
@@ -46,26 +47,6 @@ extern "C" int simba_device_check(void) {
   return SIMBA_OK;
 }
 
-static inline int round_up(int x, int m) { return (x + m - 1) / m * m; }
-
-constexpr float kLog2e = 1.4426950408889634f;
-
-static float bf16_to_f32(uint16_t h) {
-  const uint32_t u = (uint32_t)h << 16;
-  float f;
-  memcpy(&f, &u, 4);
-  return f;
-}
-
-static uint16_t f32_to_bf16_rne(float f) {
-  uint32_t u;
-  memcpy(&u, &f, 4);
-  if ((u & 0x7fffffffu) > 0x7f800000u) return (uint16_t)((u >> 16) | 0x40);   // NaN
-  const uint32_t lsb = (u >> 16) & 1u;
-  u += 0x7fffu + lsb;
-  return (uint16_t)(u >> 16);
-}
-
 // ---------------------------------------------------------------------------------------------
 // model
 // ---------------------------------------------------------------------------------------------
@@ -81,15 +62,12 @@ struct simba_model {
   // device images
   float* d_w_f32 = nullptr;
   float* d_bias_f32 = nullptr;
-  void* d_w_bf16 = nullptr;
-  void* d_w_wide = nullptr;     // weight stream of rollout_tc_wide.cu (of the variant the shape selects)
-  int64_t w_wide_member_bytes = 0;
-  void* d_bias_k16 = nullptr;   // per member, per layer: UMMA B tile [128 n][16 k] (no swizzle) holding the bias as bf16 hi + lo
+  void* d_w_tc = nullptr;       // bf16 image of the tcgen05 family that runs the model (tc_family), if any
+  int64_t w_tc_member_bytes = 0;
   float tc_scale_a[128] = {0}, tc_scale_b[128] = {0};
   float* d_smin = nullptr;
   float* d_sdelta = nullptr;
   int n_chunks = 0, bias_stride = 0, act_rows = 0;
-  int64_t w_bf16_member_bytes = 0;
   // scratch for the model-level entry points (tile lists are rebuilt per call size)
   Tile* d_tiles = nullptr;
   int tiles_cap = 0;
@@ -123,10 +101,10 @@ extern "C" int simba_model_create(const simba_model_config_t* cfg, simba_model_t
 }
 
 static void model_free_device(simba_model* m) {
-  cudaFree(m->d_w_f32); cudaFree(m->d_bias_f32); cudaFree(m->d_w_bf16); cudaFree(m->d_bias_k16); cudaFree(m->d_w_wide);
+  cudaFree(m->d_w_f32); cudaFree(m->d_bias_f32); cudaFree(m->d_w_tc);
   cudaFree(m->d_smin); cudaFree(m->d_sdelta);
   m->d_w_f32 = m->d_bias_f32 = m->d_smin = m->d_sdelta = nullptr;
-  m->d_w_bf16 = m->d_bias_k16 = m->d_w_wide = nullptr;
+  m->d_w_tc = nullptr;
 }
 
 extern "C" int simba_model_destroy(simba_model_t* m) {
@@ -192,158 +170,12 @@ extern "C" int simba_model_set_scaler(simba_model_t* m, const float* mn, const f
   return SIMBA_OK;
 }
 
-// bf16 (hi, lo) split of a bias, hi = bf16(v), lo = bf16(v - hi): the kernels multiply both by a constant 1
-static void split_bf16(float v, uint16_t& hi, uint16_t& lo) {
-  hi = f32_to_bf16_rne(v);
-  lo = f32_to_bf16_rne(v - bf16_to_f32(hi));
-}
-
-// byte offset of element (n, k), 0 <= k < 64, in a K-major SWIZZLE_128B tile: row n is 128 bytes, and its
-// 16-byte chunk c is stored at chunk c ^ (n & 7)
-static int64_t sw128_offset(int n, int k) { return (int64_t)n * 128 + ((k / 8) ^ (n & 7)) * 16 + (k % 8) * 2; }
-
 // first commit: allocate; later commits overwrite in place (the sizes are fixed by the model config)
 template <class D, class T>
 static cudaError_t upload(D*& dst, const std::vector<T>& host) {
   const size_t bytes = host.size() * sizeof(T);
   const cudaError_t e = dst ? cudaSuccess : cudaMalloc(&dst, bytes);
   return e != cudaSuccess ? e : cudaMemcpy(dst, host.data(), bytes, cudaMemcpyHostToDevice);
-}
-
-// fp32 chunk stream of the fp32 kernel, per member: layer -> column block (128) -> k chunk (16), heads fused
-// as N = 2*O; the biases per layer, padded to whole column blocks (layout in m->n_chunks, m->bias_stride)
-static void pack_f32_image(const simba_model* m, std::vector<float>& w, std::vector<float>& b) {
-  const auto& c = m->cfg;
-  const int L = c.n_layers, E = c.ensemble_size, U = c.units, O = c.obs_dim, IN = c.obs_dim + c.act_dim;
-  const int KC = kF32ChunkRows, NB = kF32ChunkCols;
-  w.assign((size_t)E * m->n_chunks * KC * NB, 0.0f);
-  b.assign((size_t)E * m->bias_stride, 0.0f);
-  for (int e = 0; e < E; ++e) {
-    const std::vector<float>* kern = &m->kernels[e * (L + 2)];
-    const std::vector<float>* bias = &m->biases[e * (L + 2)];
-    size_t chunk = (size_t)e * m->n_chunks;
-    int boff = 0;
-    for (int l = 0; l <= L; ++l) {
-      const int K = l == 0 ? IN : U, N = l == L ? 2 * O : U;
-      const int Kp = round_up(K, KC), Np = round_up(N, NB);
-      auto weight = [&](int k, int n) -> float {
-        if (k >= K || n >= N) return 0.0f;
-        if (l < L) return kern[l][(size_t)k * U + n];
-        if (n < O) return kern[L][(size_t)k * O + n];            // mu head
-        return kern[L + 1][(size_t)k * O + (n - O)];             // var head
-      };
-      for (int nb = 0; nb < Np; nb += NB)
-        for (int kc = 0; kc < Kp; kc += KC, ++chunk)
-          for (int kk = 0; kk < KC; ++kk)
-            for (int n = 0; n < NB; ++n)
-              w[(chunk * KC + kk) * NB + n] = weight(kc + kk, nb + n);
-      for (int n = 0; n < N; ++n)
-        b[(size_t)e * m->bias_stride + boff + n] = l < L ? bias[l][n] : n < O ? bias[L][n] : bias[L + 1][n - O];
-      boff += Np;
-    }
-  }
-}
-
-static int64_t bf16_layer_bytes(int K) { return (int64_t)round_up(K, 64) / 64 * (128 * 128); }
-
-// bf16 image of the tcgen05 kernel, per member and layer the UMMA B operand B[n][k] = W[k][n], K-major SWIZZLE_128B:
-// one [128 rows][128 bytes] slab per 64-wide K atom; hidden and head layers occupy K = 128 (zero-padded). Heads: mu
-// -> rows [0, O), var -> rows [64, 64 + O), the raw-variance head pre-scaled by log2(e) (the kernels evaluate softplus
-// as ln2 * lg2(1 + ex2(x log2 e)) and get x log2 e out of the GEMM). Layer 0 carries its bias in the K padding (the
-// kernel feeds the constant 1 at k = IN, IN + 1). `bias_k16`: every layer's bias as one more K = 16 block of its GEMM,
-// B[n][0] = hi, B[n][1] = lo, K-major SWIZZLE_NONE: 8-row x 16-byte core matrices, the two K halves 128 B apart
-// (leading byte offset), 8-row groups 256 B apart (stride byte offset) -> 4 KB per layer. Returns a member's bytes.
-static int64_t pack_bf16_image(const simba_model* m, std::vector<uint16_t>& img, std::vector<uint16_t>& bias_k16) {
-  const auto& c = m->cfg;
-  const int L = c.n_layers, E = c.ensemble_size, U = c.units, O = c.obs_dim, IN = c.obs_dim + c.act_dim;
-  int64_t member_bytes = 0;
-  for (int l = 0; l <= L; ++l) member_bytes += bf16_layer_bytes(l == 0 ? IN : 128);
-  img.assign((size_t)E * member_bytes / 2, 0);
-  bias_k16.assign((size_t)E * (L + 1) * 2048, 0);
-  for (int e = 0; e < E; ++e) {
-    const std::vector<float>* kern = &m->kernels[e * (L + 2)];
-    const std::vector<float>* bias = &m->biases[e * (L + 2)];
-    int64_t off = (int64_t)e * member_bytes;
-    for (int l = 0; l <= L; ++l) {
-      const int K = l == 0 ? IN : U;
-      auto weight = [&](int k, int n) -> uint16_t {     // n = tile row (output feature)
-        if (l == 0 && IN + 2 <= 64 && (k == IN || k == IN + 1) && n < U) {
-          uint16_t hi, lo;
-          split_bf16(bias[0][n], hi, lo);
-          return k == IN ? hi : lo;
-        }
-        if (k >= K) return 0;
-        if (l < L) return n < U ? f32_to_bf16_rne(kern[l][(size_t)k * U + n]) : 0;
-        if (n < O) return f32_to_bf16_rne(kern[L][(size_t)k * O + n]);
-        if (n >= 64 && n < 64 + O) return f32_to_bf16_rne(kLog2e * kern[L + 1][(size_t)k * O + (n - 64)]);
-        return 0;
-      };
-      const int Kp = l == 0 ? IN : 128;
-      for (int at = 0; at < round_up(Kp, 64) / 64; ++at)
-        for (int n = 0; n < 128; ++n)
-          for (int kk = 0; kk < 64; ++kk)
-            img[(off + (int64_t)at * 128 * 128 + sw128_offset(n, kk)) / 2] = weight(at * 64 + kk, n);
-      off += bf16_layer_bytes(Kp);
-      for (int n = 0; n < 128; ++n) {
-        float bv = 0.0f;
-        if (l < L) bv = n < U ? bias[l][n] : 0.0f;
-        else if (n < O) bv = bias[L][n];
-        else if (n >= 64 && n < 64 + O) bv = kLog2e * bias[L + 1][n - 64];
-        uint16_t* bk = &bias_k16[((size_t)e * (L + 1) + l) * 2048 + (size_t)(n / 8) * 128 + (size_t)(n % 8) * 8];
-        split_bf16(bv, bk[0], bk[1]);
-      }
-    }
-  }
-  return member_bytes;
-}
-
-// weight stream of rollout_tc_wide.cu's variant with state width sw (64 or 128): per member the tiles of one
-// rollout step in consumption order — layer 0: sw / 64 tiles [UP x 64]; layers 1..L-1: KA tiles [UP x 64];
-// heads: KA tiles [2 sw x 64] (mu rows [0, O), var rows [sw, sw + O), var pre-scaled by log2(e) as above); each
-// tile K-major SWIZZLE_128B. UP is U zero-padded as rollout_tc_wide_units says. The bias of a layer sits in k
-// rows KB (hi) and KB + 1 (lo), which the kernel multiplies by constant ones in the A tile. Returns the bytes
-// of one member's stream.
-static int64_t pack_wide_image(const simba_model* m, int sw, std::vector<uint16_t>& img) {
-  const auto& c = m->cfg;
-  const int L = c.n_layers, E = c.ensemble_size, U = c.units, O = c.obs_dim, IN = c.obs_dim + c.act_dim;
-  const int UP = rollout_tc_wide_units(sw, U);
-  const int KA = (UP + 2 + 63) / 64;
-  const int64_t member_bytes = rollout_tc_wide_member_bytes(sw, L, UP);
-  img.assign((size_t)E * member_bytes / 2, 0);
-  for (int e = 0; e < E; ++e) {
-    int64_t off = (int64_t)e * member_bytes;
-    for (int l = 0; l <= L; ++l) {
-      const int K = l == 0 ? IN : U;                     // real input width
-      const int KB = l == 0 ? IN : UP;                   // the A tile holds the constant ones at k = KB, KB + 1
-      const int rows = l < L ? UP : 2 * sw;              // tile rows = output features
-      const int tiles = l == 0 ? sw / 64 : KA;
-      auto weight = [&](int k, int n) -> uint16_t {
-        int layer = l, col = n;                          // Keras layer index and output column
-        if (l == L) {
-          if (n < O) { layer = L; col = n; }
-          else if (n >= sw && n < sw + O) { layer = L + 1; col = n - sw; }
-          else return 0;
-        } else if (n >= U) {
-          return 0;                                      // padded hidden unit: weights and bias 0
-        }
-        const int width = l < L ? U : O;
-        const float pre = layer == L + 1 ? kLog2e : 1.0f;
-        if (k < K) return f32_to_bf16_rne(pre * m->kernels[e * (L + 2) + layer][(size_t)k * width + col]);
-        if (k == KB || k == KB + 1) {
-          uint16_t hi, lo;
-          split_bf16(pre * m->biases[e * (L + 2) + layer][col], hi, lo);
-          return k == KB ? hi : lo;
-        }
-        return 0;
-      };
-      for (int tI = 0; tI < tiles; ++tI) {
-        for (int n = 0; n < rows; ++n)
-          for (int kk = 0; kk < 64; ++kk) img[(off + sw128_offset(n, kk)) / 2] = weight(tI * 64 + kk, n);
-        off += (int64_t)rows * 128;
-      }
-    }
-  }
-  return member_bytes;
 }
 
 // scaler: delta = max - min, 1.01 where delta < 1e-5 (transition_model.py:85-86), for the fp32 kernel and
@@ -379,7 +211,7 @@ static RolloutKernel tc_family(const simba_model_config_t& c) {
 extern "C" int simba_model_commit(simba_model_t* m) {
   if (!m) return set_error(SIMBA_ERR_BAD_CONFIG, "null argument");
   const auto& c = m->cfg;
-  const int L = c.n_layers, U = c.units, O = c.obs_dim, IN = c.obs_dim + c.act_dim;
+  const int L = c.n_layers;
   for (size_t i = 0; i < m->layer_set.size(); ++i)
     if (!m->layer_set[i])
       return set_error(SIMBA_ERR_NOT_READY, "member %zu layer %zu has no weights", i / (L + 2),
@@ -391,45 +223,21 @@ extern "C" int simba_model_commit(simba_model_t* m) {
   // pointers when the weights or the scaler change (e.g. after every model.fit of the agent loop).
   // The copies below are synchronous, so they are ordered after earlier launches on any stream
   // only by the caller's own synchronisation (generate_action is synchronous).
-  const int KC = kF32ChunkRows, NB = kF32ChunkCols;
-  int n_chunks = 0, bias_stride = 0, act_rows = round_up(IN, KC);
-  for (int l = 0; l <= L; ++l) {
-    const int K = l == 0 ? IN : U, N = l == L ? 2 * O : U;
-    const int Kp = round_up(K, KC), Np = round_up(N, NB);
-    n_chunks += (Np / NB) * (Kp / KC);
-    bias_stride += Np;
-    act_rows = std::max(act_rows, std::max(Kp, Np));
-  }
-  m->n_chunks = n_chunks; m->bias_stride = bias_stride; m->act_rows = act_rows;
-  {
-    // the fp32 kernel keeps two activation tiles [act_rows x 32 rows] in shared memory: very wide
-    // layers (> ~780 units) do not fit and are rejected here rather than at the first launch
-    RolloutParams probe{};
-    probe.g.O = O; probe.g.A = c.act_dim; probe.act_rows = act_rows;
-    if (rollout_f32_smem_bytes(probe) > 227 * 1024)
-      return set_error(SIMBA_ERR_UNSUPPORTED, "units %d: the rollout kernels keep a row tile's activations in "
-                       "shared memory, which holds at most ~780 hidden units", U);
-  }
+  const ModelWeights mw{c, m->kernels, m->biases};
   std::vector<float> w, b;
-  pack_f32_image(m, w, b);
+  const int rc = rollout_f32_pack(mw, w, b, m->n_chunks, m->bias_stride, m->act_rows);
+  if (rc != SIMBA_OK) return rc;
   SIMBA_CUDA_TRY(cudaDeviceSynchronize());
   SIMBA_CUDA_TRY(upload(m->d_w_f32, w));
   SIMBA_CUDA_TRY(upload(m->d_bias_f32, b));
   // the bf16 image of the tcgen05 family that runs this shape, if any
   const RolloutKernel family = tc_family(c);
-  m->w_bf16_member_bytes = 0;
-  if (family == RolloutKernel::kTcOneCta) {
-    std::vector<uint16_t> img, bias_k16;
-    m->w_bf16_member_bytes = pack_bf16_image(m, img, bias_k16);
-    SIMBA_CUDA_TRY(upload(m->d_w_bf16, img));
-    SIMBA_CUDA_TRY(upload(m->d_bias_k16, bias_k16));
-  }
-  m->w_wide_member_bytes = 0;
-  if (family == RolloutKernel::kTcWide || family == RolloutKernel::kTcWideObs) {
-    std::vector<uint16_t> img;
-    m->w_wide_member_bytes = pack_wide_image(m, family == RolloutKernel::kTcWide ? 64 : 128, img);
-    SIMBA_CUDA_TRY(upload(m->d_w_wide, img));
-  }
+  std::vector<uint16_t> img;
+  m->w_tc_member_bytes = 0;
+  if (family == RolloutKernel::kTcOneCta) m->w_tc_member_bytes = rollout_tc_pack(mw, img);
+  if (family == RolloutKernel::kTcWide) m->w_tc_member_bytes = rollout_tc_wide_pack(64, mw, img);
+  if (family == RolloutKernel::kTcWideObs) m->w_tc_member_bytes = rollout_tc_wide_pack(128, mw, img);
+  if (family != RolloutKernel::kF32) SIMBA_CUDA_TRY(upload(m->d_w_tc, img));
   SIMBA_CUDA_TRY(upload(m->d_smin, m->smin));
   SIMBA_CUDA_TRY(upload(m->d_sdelta, pack_scaler(m)));
   m->committed = true;
@@ -445,11 +253,8 @@ static void fill_model_params(const simba_model* m, RolloutParams& prm) {
   prm.n_chunks = m->n_chunks;
   prm.bias_stride = m->bias_stride;
   prm.act_rows = m->act_rows;
-  prm.w_bf16 = m->d_w_bf16;
-  prm.w_bf16_member_bytes = m->w_bf16_member_bytes;
-  prm.w_wide = m->d_w_wide;
-  prm.w_wide_member_bytes = m->w_wide_member_bytes;
-  prm.bias_k16 = m->d_bias_k16;
+  prm.w_tc = m->d_w_tc;
+  prm.w_tc_member_bytes = m->w_tc_member_bytes;
   memcpy(prm.tc_scale_a, m->tc_scale_a, sizeof(prm.tc_scale_a));
   memcpy(prm.tc_scale_b, m->tc_scale_b, sizeof(prm.tc_scale_b));
   prm.smin = m->d_smin;

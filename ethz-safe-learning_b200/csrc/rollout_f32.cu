@@ -15,15 +15,18 @@
 // the order they are consumed, so the ring never drains across layers or steps. Each thread owns a
 // 4(row) x 4(col) register tile: per k one broadcast LDS.128 of activations and one LDS.128 of
 // weights feed 16 FFMAs (FMA-pipe bound, not LDS bound).
+#include <algorithm>
+
 #include "common.cuh"
+#include "internal.h"
 #include "rollout_params.cuh"
 
 namespace simba {
 
 namespace {
 constexpr int TM = kF32TileRows;      // rows per CTA
-constexpr int NB = kF32ChunkCols;     // output columns per pass
-constexpr int KC = kF32ChunkRows;     // k rows per weight chunk
+constexpr int NB = 128;               // output columns per pass: weight chunk = [KC k rows][NB cols] fp32
+constexpr int KC = 16;                // k rows per weight chunk
 constexpr int NT = 256;
 constexpr int WSTAGES = 3;
 constexpr int CHUNK = KC * NB;        // floats
@@ -264,16 +267,65 @@ __global__ void __launch_bounds__(NT) rollout_f32_kernel(const RolloutParams prm
   }
 }
 
-size_t rollout_f32_smem_bytes(const RolloutParams& prm) {
-  const int IN = prm.g.O + prm.g.A;
-  const int OS = prm.g.O | 1;
-  size_t floats = (size_t)WSTAGES * CHUNK + 2 * (size_t)prm.act_rows * TM + (size_t)TM * OS + 2 * IN;
+static size_t f32_smem_bytes(int O, int A, int act_rows) {
+  const int IN = O + A;
+  const int OS = O | 1;
+  size_t floats = (size_t)WSTAGES * CHUNK + 2 * (size_t)act_rows * TM + (size_t)TM * OS + 2 * IN;
   floats += (2 * IN) & 1;
   return floats * sizeof(float) + 5 * TM * sizeof(int64_t) + 16;
 }
 
+static int round_up(int x, int m) { return (x + m - 1) / m * m; }
+
+// The image the kernel streams, per member: layer -> column block (NB) -> k chunk (KC), the heads fused as N = 2 O
+// (mu columns [0, O), raw variance [O, 2 O)), zero-padded to n_chunks whole chunks; the biases per layer, padded
+// to whole column blocks (bias_stride floats). act_rows: rows of an activation buffer, the widest padded layer.
+int rollout_f32_pack(const ModelWeights& mw, std::vector<float>& w, std::vector<float>& b, int& n_chunks,
+                     int& bias_stride, int& act_rows) {
+  const auto& c = mw.cfg;
+  const int L = c.n_layers, E = c.ensemble_size, U = c.units, O = c.obs_dim, IN = c.obs_dim + c.act_dim;
+  n_chunks = 0; bias_stride = 0; act_rows = round_up(IN, KC);
+  for (int l = 0; l <= L; ++l) {
+    const int K = l == 0 ? IN : U, N = l == L ? 2 * O : U;
+    const int Kp = round_up(K, KC), Np = round_up(N, NB);
+    n_chunks += (Np / NB) * (Kp / KC);
+    bias_stride += Np;
+    act_rows = std::max(act_rows, std::max(Kp, Np));
+  }
+  // the kernel keeps two activation tiles [act_rows x 32 rows] in shared memory: very wide layers (> ~780 units)
+  // do not fit and are rejected here rather than at the first launch
+  if (f32_smem_bytes(O, c.act_dim, act_rows) > 227 * 1024)
+    return set_error(SIMBA_ERR_UNSUPPORTED, "units %d: the rollout kernels keep a row tile's activations in "
+                     "shared memory, which holds at most ~780 hidden units", U);
+  w.assign((size_t)E * n_chunks * CHUNK, 0.0f);
+  b.assign((size_t)E * bias_stride, 0.0f);
+  for (int e = 0; e < E; ++e) {
+    size_t chunk = (size_t)e * n_chunks;
+    int boff = 0;
+    for (int l = 0; l <= L; ++l) {
+      const int K = l == 0 ? IN : U, N = l == L ? 2 * O : U;
+      const int Kp = round_up(K, KC), Np = round_up(N, NB);
+      auto weight = [&](int k, int n) -> float {
+        if (k >= K || n >= N) return 0.0f;
+        if (l < L) return mw.kernel(e, l)[(size_t)k * U + n];
+        if (n < O) return mw.kernel(e, L)[(size_t)k * O + n];            // mu head
+        return mw.kernel(e, L + 1)[(size_t)k * O + (n - O)];             // var head
+      };
+      for (int nb = 0; nb < Np; nb += NB)
+        for (int kc = 0; kc < Kp; kc += KC, ++chunk)
+          for (int kk = 0; kk < KC; ++kk)
+            for (int n = 0; n < NB; ++n)
+              w[(chunk * KC + kk) * NB + n] = weight(kc + kk, nb + n);
+      for (int n = 0; n < N; ++n)
+        b[(size_t)e * bias_stride + boff + n] = l < L ? mw.bias(e, l)[n] : n < O ? mw.bias(e, L)[n] : mw.bias(e, L + 1)[n - O];
+      boff += Np;
+    }
+  }
+  return SIMBA_OK;
+}
+
 cudaError_t launch_rollout_f32(const RolloutParams& prm, cudaStream_t stream) {
-  const size_t smem = rollout_f32_smem_bytes(prm);
+  const size_t smem = f32_smem_bytes(prm.g.O, prm.g.A, prm.act_rows);
   // set on every launch: the attribute is per device and per function, and launches happen only at
   // graph capture or in the non-graph entry points, never on the replayed hot path
   {

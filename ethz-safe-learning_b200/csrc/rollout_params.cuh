@@ -1,12 +1,12 @@
 // Launch parameters shared by the fp32 and bf16-tcgen05 rollout kernels.
 #pragma once
+#include <vector>
+
 #include "common.cuh"
 
 namespace simba {
 
 constexpr int kF32TileRows = 32;     // rows per CTA of the fp32 kernel
-constexpr int kF32ChunkCols = 128;   // weight chunk = [16 k-rows][128 cols] fp32
-constexpr int kF32ChunkRows = 16;
 constexpr int kTcTileRows = 128;     // rows per tile of the tcgen05 kernel (UMMA_M)
 
 // The rollout kernel a planner launches; simba_planner_rollout_kernel reports it with these values.
@@ -26,17 +26,14 @@ struct RolloutParams {
   int32_t n_tiles;
   int32_t L, U;
   // fp32 image: per member, chunks [n_chunks][16][128] in consumption order; biases padded per layer
+  // (rollout_f32_pack)
   const float* w_f32;
   const float* bias_f32;
   int32_t n_chunks, bias_stride, act_rows;
-  // bf16 image: per member, per layer pre-swizzled UMMA B tiles (see pack_bf16_image in api.cu)
-  const void* w_bf16;
-  int64_t w_bf16_member_bytes;
-  // wide models (128 < units <= 440) and wide observations: per member the per-step stream of UMMA
-  // weight tiles in consumption order, biases in the K padding (see rollout_tc_wide.cu)
-  const void* w_wide;
-  int64_t w_wide_member_bytes;
-  const void* bias_k16;       // [E][L+1][4096 B] bias K-blocks (see pack_bf16_image in api.cu)
+  // bf16 image of the tcgen05 family that runs the model, w_tc_member_bytes per member, in the layout of that
+  // family's kernel file (rollout_tc_pack, rollout_tc_wide_pack)
+  const void* w_tc;
+  int64_t w_tc_member_bytes;
   RolloutKernel kernel;       // the kernel launch_rollout runs
   int32_t n_sms;              // SMs of the planner's device (grid of the persistent tcgen05 kernels)
   int32_t pdl;                // launch with programmatic stream serialization (fused plan path)
@@ -80,7 +77,6 @@ cudaError_t launch_rollout_f32(const RolloutParams& prm, cudaStream_t stream);
 cudaError_t launch_rollout_tc(const RolloutParams& prm, cudaStream_t stream);        // kTc{OneCta,Pair,TwoTile}
 cudaError_t launch_rollout_tc_wide(const RolloutParams& prm, cudaStream_t stream);   // kTcWide{,Obs}; prm.U: the model's units
 
-size_t rollout_f32_smem_bytes(const RolloutParams& prm);
 // Shape rules of the tcgen05 kernels, from the model alone (api.cu's tc_family combines them). rollout_tc.cu:
 bool rollout_tc_supported(int O, int A, int L, int U);
 bool rollout_tc_two_tiles_fit(int L, int n_constraints);
@@ -88,7 +84,25 @@ bool rollout_tc_pair_fits(int L, int n_constraints);
 // The weight-streaming kernel comes in two state widths `sw`: 64 (prm.kernel kTcWide) and 128 (kTcWideObs).
 bool rollout_tc_wide_supported(int sw, int O, int A, int L, int U);
 bool rollout_tc_wide_fits(int sw, int L, int U, int n_constraints);
-int rollout_tc_wide_units(int sw, int U);                     // the padded width the kernel runs
-int64_t rollout_tc_wide_member_bytes(int sw, int L, int UP);   // UP = padded units
+
+// What the weight packers read: the model's config and its Keras layers. Layer l of member e has the kernel
+// [K][N] (row-major) and the bias [N] at index e * (n_layers + 2) + l; layers n_layers and n_layers + 1 are the
+// mu and raw-variance heads.
+struct ModelWeights {
+  const simba_model_config_t& cfg;
+  const std::vector<std::vector<float>>& kernels;
+  const std::vector<std::vector<float>>& biases;
+  const float* kernel(int e, int l) const { return kernels[(size_t)e * (cfg.n_layers + 2) + l].data(); }
+  const float* bias(int e, int l) const { return biases[(size_t)e * (cfg.n_layers + 2) + l].data(); }
+};
+// Each kernel file packs the weight image its kernels read. The fp32 packer fills the image and its geometry
+// (RolloutParams::n_chunks, bias_stride, act_rows), or returns SIMBA_ERR_UNSUPPORTED for units the fp32 kernel's
+// shared memory cannot hold. The tcgen05 packers fill the image of all members and return a member's bytes
+// (RolloutParams::w_tc_member_bytes); they run only for shapes that rollout_tc_supported / rollout_tc_wide_supported
+// accept.
+int rollout_f32_pack(const ModelWeights& mw, std::vector<float>& w, std::vector<float>& b, int& n_chunks,
+                     int& bias_stride, int& act_rows);
+int64_t rollout_tc_pack(const ModelWeights& mw, std::vector<uint16_t>& img);
+int64_t rollout_tc_wide_pack(int sw, const ModelWeights& mw, std::vector<uint16_t>& img);
 
 }  // namespace simba

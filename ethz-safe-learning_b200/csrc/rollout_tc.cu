@@ -71,8 +71,19 @@ namespace {
 constexpr int kU = 128;                 // hidden width this kernel covers
 constexpr int kMaxO = 60;               // observation dims (two Gaussian heads padded to 2 x 64 columns)
 constexpr int kAtomBytes = 128 * 128;   // one 64-wide K atom of a 128-row tile (bf16, SW128)
+constexpr int kBiasBlockBytes = 4096;   // one layer's bias as a K = 16 B operand (rollout_tc_pack)
 constexpr int kBoundThreads = 640;      // launch bound: the hardware allocates warps in fours, so 17 - 19
                                         // warps occupy 20 warp slots -> 96 registers per thread
+
+// A member's image (rollout_tc_pack) is staged into shared memory as it is: the layers' weight atoms, layer 0
+// one and every later layer two (K = 128), then the L + 1 bias K-blocks.
+__host__ __device__ constexpr uint32_t tc_weight_bytes(int L) { return kAtomBytes + (uint32_t)L * 2 * kAtomBytes; }
+__host__ __device__ constexpr uint32_t tc_member_bytes(int L) {
+  return tc_weight_bytes(L) + (uint32_t)(L + 1) * kBiasBlockBytes;
+}
+// Layer 0 carries its bias in the K padding when the input of IN = O + A elements leaves room for the constant
+// ones at k = IN, IN + 1; otherwise it takes the bias K-step as every other layer does.
+__host__ __device__ constexpr bool tc_l0_pad_bias(int in_dim) { return in_dim + 2 <= 64; }
 
 struct TileInfo {
   int32_t member, k0, count, valid;
@@ -191,13 +202,13 @@ __device__ __forceinline__ void rollout_tc_body(const RolloutParams& prm) {
   const int n_items = (prm.n_tiles + NTILES - 1) / NTILES;
   const int cta_item0 = PAIR ? (int)(blockIdx.x >> 1) : (int)blockIdx.x;
   const int n_ctas = PAIR ? (int)(gridDim.x >> 1) : (int)gridDim.x;       // PAIR: one item per cluster (launch_variant)
-  const bool l0_pad_bias = (O + A + 2 <= 64);     // layer-0 bias rides in the K padding (see pack in api.cu)
+  const bool l0_pad_bias = tc_l0_pad_bias(O + A);
   constexpr int n_quarters = 4;                   // TMEM lane quarters (= warps per column group) of a tile
   constexpr int tile_bar_threads = Q * 128 + 32;  // a tile's epilogue warps + one partner warp (issuer / scorer)
   constexpr int half_bar_threads = Q * 64 + 32;   // one tile: the epilogue warps of a column half + the issuer or relay warp
 
   // ---- shared memory carve-up (base is 1024-aligned: required by SWIZZLE_128B) -------------------
-  const uint32_t w_bytes = kAtomBytes + (uint32_t)L * 2 * kAtomBytes;     // layer 0: 1 atom; others: 2
+  const uint32_t w_bytes = tc_weight_bytes(L);
   uint8_t* w_smem = smem_raw;
   uint8_t* biask_smem = w_smem + w_bytes;                                  // [(L+1)][4096]: bias K-blocks (B operand)
   uint8_t* ones_smem = biask_smem + (L + 1) * 4096;                        // [4096]: A operand of the bias K-step
@@ -240,9 +251,10 @@ __device__ __forceinline__ void rollout_tc_body(const RolloutParams& prm) {
       if (item * NTILES + q < prm.n_tiles && prm.tiles[item * NTILES + q].count > 0) wm = prm.tiles[item * NTILES + q].member;
     return wm;
   };
-  // one TMA bulk copy per layer, all onto bars[0] (thread 0 only; every MMA that read the previous set has completed)
+  // one TMA bulk copy per layer and one of the bias K-blocks, which end the member's image, all onto bars[0] (thread 0
+  // only; every MMA that read the previous set has completed)
   auto stage_weights = [&](int wm) {
-    const uint8_t* wsrc = reinterpret_cast<const uint8_t*>(prm.w_bf16) + (size_t)wm * prm.w_bf16_member_bytes;
+    const uint8_t* wsrc = reinterpret_cast<const uint8_t*>(prm.w_tc) + (size_t)wm * prm.w_tc_member_bytes;
     const uint32_t bk_bytes = (uint32_t)(L + 1) * 4096u;
     mbar_expect_tx(bar_w, w_bytes + bk_bytes);
     uint32_t off = 0;
@@ -251,8 +263,7 @@ __device__ __forceinline__ void rollout_tc_body(const RolloutParams& prm) {
       bulk_g2s(smem_u32(w_smem + off), wsrc + off, nb, bar_w);
       off += nb;
     }
-    bulk_g2s(smem_u32(biask_smem), reinterpret_cast<const uint8_t*>(prm.bias_k16) + (size_t)wm * bk_bytes,
-             bk_bytes, bar_w);
+    bulk_g2s(smem_u32(biask_smem), wsrc + (prm.w_tc_member_bytes - bk_bytes), bk_bytes, bar_w);
     w_state_sh[0] = wm;
     w_state_sh[1] += 1;
   };
@@ -905,8 +916,7 @@ __global__ void __launch_bounds__(kBoundThreads, 1) unfold_tc_kernel(const Rollo
 
 // ---- host side ------------------------------------------------------------------------------------
 static size_t tc_smem_bytes(int L, int ntiles, int q, int nparts, bool pair = false) {
-  size_t b = (size_t)kAtomBytes + (size_t)L * 2 * kAtomBytes;      // weights
-  b += (size_t)(L + 1) * 4096 + 4096;                              // bias K-blocks + ones tile
+  size_t b = tc_member_bytes(L) + 4096;                            // weights, bias K-blocks + ones tile
   b += 128 * sizeof(float);                                        // scaler
   b += kHeadParts * 64 * sizeof(float);                            // slice penalty table
   b += (size_t)ntiles * q * nparts * 128 * sizeof(float) * (pair ? 4 : 1);   // partial minima exchange (pair: 2 x 2 q slices)
@@ -921,10 +931,58 @@ static size_t tc_smem_bytes(int L, int ntiles, int q, int nparts, bool pair = fa
 constexpr size_t kMaxSmem = 227 * 1024;
 
 bool rollout_tc_supported(int O, int A, int L, int U) {
-  // narrower hidden layers run zero-padded to 128 units (simba_model_commit pads the images); the
+  // narrower hidden layers run zero-padded to 128 units (rollout_tc_pack pads the image); the
   // member's whole weight set must fit in shared memory next to the one-tile variant's buffers
   return U >= 1 && U <= kU && O >= 1 && O <= kMaxO && O + A <= 64 && A <= 4 && L >= 1 &&
          tc_smem_bytes(L, 1, 4, kHeadParts) + 1024 <= kMaxSmem;
+}
+
+// The image, per member, in the order stage_weights copies it into shared memory:
+//   * per layer the UMMA B operand B[n][k] = W[k][n], K-major SWIZZLE_128B: one [128 rows][128 bytes] slab per
+//     64-wide K atom, layer 0 one atom (K = O + A, zero-padded), every later layer two (K = units, zero-padded to
+//     128). Heads: mu -> rows [0, O), var -> rows [64, 64 + O), the raw-variance head pre-scaled by log2(e). When
+//     tc_l0_pad_bias, layer 0 carries its bias as bf16 hi / lo in k = IN, IN + 1, where the kernel feeds ones;
+//   * then per layer its bias as one more K = 16 block of its GEMM, B[n][0] = hi, B[n][1] = lo, K-major
+//     SWIZZLE_NONE: 8-row x 16-byte core matrices, the two K halves 128 B apart (leading byte offset), 8-row groups
+//     256 B apart (stride byte offset) -> kBiasBlockBytes per layer.
+int64_t rollout_tc_pack(const ModelWeights& mw, std::vector<uint16_t>& img) {
+  const auto& c = mw.cfg;
+  const int L = c.n_layers, E = c.ensemble_size, U = c.units, O = c.obs_dim, IN = c.obs_dim + c.act_dim;
+  const int64_t member_bytes = tc_member_bytes(L);
+  img.assign((size_t)E * member_bytes / 2, 0);
+  for (int e = 0; e < E; ++e) {
+    uint16_t* w = &img[(size_t)e * member_bytes / 2];
+    uint16_t* bias_k16 = w + tc_weight_bytes(L) / 2;
+    for (int l = 0; l <= L; ++l) {
+      const int K = l == 0 ? IN : U;
+      auto weight = [&](int k, int n) -> uint16_t {     // n = tile row (output feature)
+        if (l == 0 && tc_l0_pad_bias(IN) && (k == IN || k == IN + 1) && n < U) {
+          uint16_t hi, lo;
+          bf16_split(mw.bias(e, 0)[n], hi, lo);
+          return k == IN ? hi : lo;
+        }
+        if (k >= K) return 0;
+        if (l < L) return n < U ? bf16_bits(mw.kernel(e, l)[(size_t)k * U + n]) : 0;
+        if (n < O) return bf16_bits(mw.kernel(e, L)[(size_t)k * O + n]);
+        if (n >= 64 && n < 64 + O) return bf16_bits(kLog2e * mw.kernel(e, L + 1)[(size_t)k * O + (n - 64)]);
+        return 0;
+      };
+      const int atoms = l == 0 ? 1 : 2;
+      for (int at = 0; at < atoms; ++at)
+        for (int n = 0; n < 128; ++n)
+          for (int kk = 0; kk < 64; ++kk) w[(at * kAtomBytes + sw128_offset(n, kk)) / 2] = weight(at * 64 + kk, n);
+      w += atoms * kAtomBytes / 2;
+      for (int n = 0; n < 128; ++n) {
+        float bv = 0.0f;
+        if (l < L) bv = n < U ? mw.bias(e, l)[n] : 0.0f;
+        else if (n < O) bv = mw.bias(e, L)[n];
+        else if (n >= 64 && n < 64 + O) bv = kLog2e * mw.bias(e, L + 1)[n - 64];
+        uint16_t* bk = bias_k16 + l * kBiasBlockBytes / 2 + (n / 8) * 128 + (n % 8) * 8;
+        bf16_split(bv, bk[0], bk[1]);
+      }
+    }
+  }
+  return member_bytes;
 }
 
 // whether the two-tile throughput variant (and its shared-memory parking areas) fits for this depth

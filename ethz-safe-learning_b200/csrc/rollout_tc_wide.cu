@@ -200,8 +200,7 @@ __device__ __forceinline__ void rollout_tc_wide_body(const RolloutParams& prm) {
     if (warp == kEpiThreads / 32) {
       // ===================== producer warp: weight tiles through the TMA ring =====================
       if (elect_one()) {
-        const uint8_t* wsrc = reinterpret_cast<const uint8_t*>(prm.w_wide) +
-                              (size_t)ti.member * prm.w_wide_member_bytes;
+        const uint8_t* wsrc = reinterpret_cast<const uint8_t*>(prm.w_tc) + (size_t)ti.member * prm.w_tc_member_bytes;
         const int total = H * ws.tiles_per_step;
         int in_step = 0;
         for (int i = 0; i < total; ++i) {
@@ -558,7 +557,7 @@ static size_t wide_smem_bytes(int sw, int L, int UP, int nparts) {
 
 // widths that are not a multiple of 16 run zero-padded to the next one; the 128-column variant pads to at
 // least 128 (file comment)
-int rollout_tc_wide_units(int sw, int U) {
+static int rollout_tc_wide_units(int sw, int U) {
   const int UP = (U + 15) / 16 * 16;
   return sw == 64 ? UP : std::max(UP, WideCfg<128>::kMinUnits);
 }
@@ -579,9 +578,54 @@ bool rollout_tc_wide_fits(int sw, int L, int U, int n_constraints) {
   return wide_smem_bytes(sw, L, rollout_tc_wide_units(sw, U), 1 + n_constraints) <= 227 * 1024;
 }
 
-int64_t rollout_tc_wide_member_bytes(int sw, int L, int UP) {
+// The weight stream of the variant with state width sw, per member the tiles of one rollout step in consumption
+// order: layer 0: sw / 64 tiles [UP x 64]; layers 1..L-1: KA tiles [UP x 64]; heads: KA tiles [2 sw x 64] (mu rows
+// [0, O), var rows [sw, sw + O), the raw-variance head pre-scaled by log2(e)); each tile K-major SWIZZLE_128B. UP
+// is the width rollout_tc_wide_units pads to, its extra units have zero weights and bias. The bias of a layer
+// sits in k rows KB (hi) and KB + 1 (lo), which the kernel multiplies by constant ones in the A tile.
+int64_t rollout_tc_wide_pack(int sw, const ModelWeights& mw, std::vector<uint16_t>& img) {
+  const auto& c = mw.cfg;
+  const int L = c.n_layers, E = c.ensemble_size, U = c.units, O = c.obs_dim, IN = c.obs_dim + c.act_dim;
+  const int UP = rollout_tc_wide_units(sw, U);
   const WideShape ws = sw == 64 ? wide_shape<64>(UP, L) : wide_shape<128>(UP, L);
-  return (int64_t)(ws.tiles_per_step - ws.head_tiles) * ws.hid_tile_bytes + (int64_t)ws.KA * ws.head_tile_bytes;
+  const int KA = ws.KA;
+  const int64_t member_bytes =
+      (int64_t)(ws.tiles_per_step - ws.head_tiles) * ws.hid_tile_bytes + (int64_t)KA * ws.head_tile_bytes;
+  img.assign((size_t)E * member_bytes / 2, 0);
+  for (int e = 0; e < E; ++e) {
+    int64_t off = (int64_t)e * member_bytes;
+    for (int l = 0; l <= L; ++l) {
+      const int K = l == 0 ? IN : U;                     // real input width
+      const int KB = l == 0 ? IN : UP;                   // the A tile holds the constant ones at k = KB, KB + 1
+      const int rows = l < L ? UP : 2 * sw;              // tile rows = output features
+      const int tiles = l == 0 ? sw / 64 : KA;
+      auto weight = [&](int k, int n) -> uint16_t {
+        int layer = l, col = n;                          // Keras layer index and output column
+        if (l == L) {
+          if (n < O) { layer = L; col = n; }
+          else if (n >= sw && n < sw + O) { layer = L + 1; col = n - sw; }
+          else return 0;
+        } else if (n >= U) {
+          return 0;                                      // padded hidden unit: weights and bias 0
+        }
+        const int width = l < L ? U : O;
+        const float pre = layer == L + 1 ? kLog2e : 1.0f;
+        if (k < K) return bf16_bits(pre * mw.kernel(e, layer)[(size_t)k * width + col]);
+        if (k == KB || k == KB + 1) {
+          uint16_t hi, lo;
+          bf16_split(pre * mw.bias(e, layer)[col], hi, lo);
+          return k == KB ? hi : lo;
+        }
+        return 0;
+      };
+      for (int tI = 0; tI < tiles; ++tI) {
+        for (int n = 0; n < rows; ++n)
+          for (int kk = 0; kk < 64; ++kk) img[(off + sw128_offset(n, kk)) / 2] = weight(tI * 64 + kk, n);
+        off += (int64_t)rows * 128;
+      }
+    }
+  }
+  return member_bytes;
 }
 
 template <int kSW, bool TRAJ>

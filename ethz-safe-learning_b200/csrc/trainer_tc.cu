@@ -27,7 +27,6 @@
 // the trainer therefore uses the one descriptor form (`desc_kmajor`), and no kernel writes a second global
 // layout of the activations.
 #include <algorithm>
-#include <cstring>
 
 #include "common.cuh"
 #include "internal.h"
@@ -500,19 +499,6 @@ int64_t train_tc_layout(TcLayer* layers, int n) {
   return off;
 }
 
-static uint16_t host_bf16(float f) {          // round to nearest even (finite inputs)
-  uint32_t u;
-  memcpy(&u, &f, 4);
-  u += 0x7FFFu + ((u >> 16) & 1u);
-  return (uint16_t)(u >> 16);
-}
-static float host_bf16_value(uint16_t b) {
-  const uint32_t u = (uint32_t)b << 16;
-  float f;
-  memcpy(&f, &u, 4);
-  return f;
-}
-
 // element (row, col) of a K-major SWIZZLE_NONE image with `rows_p` padded rows, in bf16 units
 static size_t img_index(int row, int col, int rows_p) {
   return (size_t)(col >> 3) * rows_p * 8 + (size_t)(row >> 3) * 64 + (size_t)(row & 7) * 8 + (col & 7);
@@ -527,19 +513,14 @@ void train_tc_pack(const TcLayer* layers, int n, const float* theta, uint8_t* im
     for (int k = 0; k <= L.K; ++k)
       for (int c = 0; c < L.N; ++c) {
         const float w = W[(size_t)k * L.N + c];
-        if (k < L.K) {
-          fwd[img_index(c, k, npf)] = host_bf16(w);
-        } else {
-          const uint16_t hi = host_bf16(w);
-          fwd[img_index(c, k, npf)] = hi;
-          fwd[img_index(c, k + 1, npf)] = host_bf16(w - host_bf16_value(hi));
-        }
+        if (k < L.K) fwd[img_index(c, k, npf)] = bf16_bits(w);
+        else bf16_split(w, fwd[img_index(c, k, npf)], fwd[img_index(c, k + 1, npf)]);
       }
     if (L.bwd_off < 0) continue;
     uint16_t* bwd = reinterpret_cast<uint16_t*>(img + L.bwd_off);
     const int npb = r16(L.K);
     for (int k = 0; k < L.K; ++k)
-      for (int c = 0; c < L.N; ++c) bwd[img_index(k, c, npb)] = host_bf16(W[(size_t)k * L.N + c]);
+      for (int c = 0; c < L.N; ++c) bwd[img_index(k, c, npb)] = bf16_bits(W[(size_t)k * L.N + c]);
   }
 }
 
