@@ -1,7 +1,8 @@
-// Device pieces shared by the two ensemble trainers: the fp32 SIMT kernels (trainer.cu) and the bf16
+// Device pieces shared by the two ensemble trainers: the fp32 SIMT kernels (trainer_f32.cu) and the bf16
 // tcgen05 kernels (trainer_tc.cu). Both run the same step contract — batch gather through the fit
 // descriptor, Philox stream-4 dropout masks, the Gaussian negative log-likelihood with its gradient,
-// the fixed-order loss reduction and clip + Adam on the fp32 master weights — so these are written once.
+// the fixed-order loss reduction and clip + Adam on the fp32 master weights — so these are written once,
+// with the description of a training launch (TrainDesc) that the handle in trainer.cu passes to either.
 #pragma once
 #include <cstdint>
 
@@ -31,80 +32,77 @@ struct OptParams {
   int schedule, steps_per_epoch, train_epochs;
 };
 
-// ---- the bf16 tcgen05 trainer (trainer_tc.cu) ------------------------------------------------------
-constexpr int kTcMaxLayers = 7;        // n_layers <= 6 hidden layers + the merged Gaussian head
+constexpr int kMaxTrainLayers = 18;   // train layers: up to 16 hidden layers + the merged Gaussian head
 
-// Train layer l of the bf16 path: the fp32 master block [(K + 1) x N] of theta (trainer.cu) and the two
-// bf16 UMMA images the chain kernel reads, rebuilt by the update kernel after every Adam step:
-//   forward   B[n][k] = theta[k][n], rows N padded to 16, K + 2 columns padded to 16: k = K holds bf16(bias),
-//             k = K + 1 the residual bf16(bias - bf16(bias)) (the A tile carries ones there)
-//   backward  B[k][n] = theta[k][n] (k < K), rows K padded to 16, N columns padded to 16 (layers >= 1)
-// Both are K-major SWIZZLE_NONE: 8-row x 16-byte core matrices, row groups 128 B apart, 8-wide K groups
-// rows_padded * 16 B apart, so every 64-wide K chunk is one contiguous block.
-struct TcLayer {
+// Train layer l: the Keras kernel [K x N] and its bias as one [(K + 1) x N] row-major block of a member's theta, at
+// float offset `off` (the bias is the row that multiplies the constant 1). The Gaussian head's two Dense layers are
+// one block with N = 2 * O whose columns interleave (mu_0, var_0, mu_1, var_1, ...).
+struct TrainLayer {
   int K, N;
-  int64_t off;              // float offset of the block inside a member's theta
-  int64_t fwd_off, bwd_off; // byte offsets of the images inside a member's bf16 image (bwd_off < 0: layer 0)
+  int64_t off;
 };
 
-struct TcChainArgs {
-  TcLayer layer[kTcMaxLayers];
-  int L;                    // hidden layers (layer L is the head)
-  float* act[kTcMaxLayers]; // act[l], l >= 1: input of layer l [E][cap][K_l] (H_l after dropout)
-  int64_t act_estride;      // rows per member (cap)
-  float* dz[kTcMaxLayers];  // [E][batch][N_l]
-  int64_t dz_estride;       // rows per member (batch)
-  const float* x;           // [E][rows][K_0] (estride may be 0: validation shares its rows)
+// What the trainer handle (trainer.cu) owns, and the inputs of one call, in a form both precisions launch from. Each
+// launcher below translates it into its own kernels' arguments.
+struct TrainDesc {
+  int L;                              // hidden layers; layer L is the head
+  TrainLayer layer[kMaxTrainLayers];
+  float* act[kMaxTrainLayers];        // act[l], l >= 1: input of layer l [E][act_estride][K_l] (H_l after dropout)
+  int64_t act_estride;                // rows per member (cap)
+  float* dz[kMaxTrainLayers];         // dz[l]: gradient w.r.t. the pre-activation of layer l [E][dz_estride][N_l]
+  int64_t dz_estride;                 // rows per member (batch)
+  const float* x;                     // [E][rows][K_0] (estride may be 0: validation shares its rows)
   int64_t x_estride;
-  int gather;               // 1: batch rows follow the fit descriptor's index
-  const float* y;
+  int gather;                         // 1: batch rows follow the fit descriptor's index
+  const float* y;                     // [E][rows][O]
   int64_t y_estride;
-  const uint8_t* img;
-  int64_t img_member_bytes;
+  float *theta, *m, *v, *grad;        // fp32 master weights, Adam slots and last gradient, [E][pn]
+  int64_t pn;
+  uint8_t* img;                       // derived from theta, img_member_bytes per member, rewritten by every update:
+  int64_t img_member_bytes;           // theta^T for fp32, the UMMA images for bf16
   int out_dim, ensemble;
-  float* partial;
+  float* partial;                     // [E][tiles_cap][2]: NLL partials of the chain's row tiles
   int tiles_cap;
-  int train;
+  int train;                          // 0: forward and likelihood only (validation)
   float* out_loss;
   float dropout_rate, dropout_scale;
   uint64_t dropout_seed;
 };
 
-struct TcUpdArgs {
-  TcLayer layer[kTcMaxLayers];
-  int tile_begin[kTcMaxLayers];   // first CTA of each layer in the grid
-  int n_tiles_n[kTcMaxLayers];    // 128-column tiles of each layer
-  int n_layers;
-  const float* h[kTcMaxLayers];   // input of the layer (layer 0: x, or gathered through the fit descriptor)
-  int64_t h_estride[kTcMaxLayers];
-  int gather0;
-  const float* dz[kTcMaxLayers];
-  int64_t dz_estride;       // rows per member (batch)
-  float *theta, *m, *v, *grad;
-  int64_t pn;
-  uint8_t* img;
-  int64_t img_member_bytes;
-  int ensemble;
-};
-
-// shape coverage of the bf16 trainer (simba_trainer_create rejects everything else)
-bool train_tc_supported(int in_dim, int obs_dim, int n_layers, int units);
-// fills fwd_off / bwd_off, returns a member's image bytes
-int64_t train_tc_layout(TcLayer* layers, int n);
-// one member's images from its fp32 theta (host); `img` must be zeroed
-void train_tc_pack(const TcLayer* layers, int n, const float* theta, uint8_t* img);
-// 128-column tiles of the update grid, per layer
-int train_tc_update_tiles(const TcLayer& l);
-cudaError_t train_tc_chain(const TcChainArgs& a, const OptParams& opt, const FitDesc* desc, TrainState* st,
-                           int grid_rows, int rows_fixed, int step_off, cudaStream_t s);
-cudaError_t train_tc_update(const TcUpdArgs& a, const OptParams& opt, const FitDesc* desc, const TrainState* st,
-                            int n_tiles, int rows_fixed, int step_off, cudaStream_t s);
-constexpr int kTcRows = 128;      // batch rows per chain CTA (the MMA's M)
+// The host side of each precision: train_f32_* (trainer_f32.cu) and train_tc_* (trainer_tc.cu, bf16 tcgen05).
+//   check        SIMBA_OK, or SIMBA_ERR_UNSUPPORTED with its message for a shape the kernels cannot train
+//   image_bytes  a member's image
+//   pack         one member's image from its host theta; `img` must be zeroed
+//   chain        forward + likelihood (+ back-propagation of the activations when d.train) over `grid_rows` rows;
+//                `row_tiles` receives the CTAs per member, i.e. the partials it writes
+//   update       weight gradients, clip and Adam for every layer, and the image of the new weights
+int train_f32_check(const TrainDesc& d);
+int train_tc_check(const simba_model_config_t& mc);
+int64_t train_f32_image_bytes(const TrainDesc& d);
+int64_t train_tc_image_bytes(const TrainDesc& d);
+void train_f32_pack(const TrainDesc& d, const float* theta, uint8_t* img);
+void train_tc_pack(const TrainDesc& d, const float* theta, uint8_t* img);
+cudaError_t train_f32_chain(const TrainDesc& d, const OptParams& opt, const FitDesc* desc, TrainState* st,
+                            int grid_rows, int rows_fixed, int step_off, cudaStream_t s, int& row_tiles);
+cudaError_t train_tc_chain(const TrainDesc& d, const OptParams& opt, const FitDesc* desc, TrainState* st,
+                           int grid_rows, int rows_fixed, int step_off, cudaStream_t s, int& row_tiles);
+cudaError_t train_f32_update(const TrainDesc& d, const OptParams& opt, const FitDesc* desc, const TrainState* st,
+                             int rows_fixed, int step_off, cudaStream_t s);
+cudaError_t train_tc_update(const TrainDesc& d, const OptParams& opt, const FitDesc* desc, const TrainState* st,
+                            int rows_fixed, int step_off, cudaStream_t s);
 
 }  // namespace simba
 
 namespace {
-using namespace simba;
+// using-declarations, not `using namespace simba`: the directive would put simba's unnamed namespace (tc_ptx.cuh)
+// beside this one, and nvcc's host stubs for kernels kept in this one (trainer_f32.cu) would then be ambiguous
+using simba::FitDesc;
+using simba::OptParams;
+using simba::TrainState;
+using simba::philox4x32_10;
+using simba::philox_key;
+using simba::softplus_tf;
+using simba::u01;
 
 // A captured graph holds several consecutive steps: step i of the graph works at
 // (st->fit_step + i, st->iterations + i) and one single-thread kernel advances the counters at

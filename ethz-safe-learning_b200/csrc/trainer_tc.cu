@@ -1,5 +1,5 @@
 // bf16 tcgen05 ensemble training step (simba_trainer_config_t.precision = SIMBA_PREC_BF16_TC): the same
-// contract as trainer.cu's fp32 kernels — forward with dropout, Gaussian NLL and its gradient, activation
+// contract as trainer_f32.cu's fp32 kernels — forward with dropout, Gaussian NLL and its gradient, activation
 // back-propagation, weight gradients, clip and Adam on fp32 master weights — with every GEMM on the tensor
 // cores (bf16 operands, fp32 accumulation in tensor memory). Two launches per step, captured in the same
 // 16-step graphs as the fp32 path.
@@ -32,6 +32,68 @@
 #include "internal.h"
 #include "tc_ptx.cuh"
 #include "train_common.cuh"
+
+using namespace simba;
+
+namespace simba {
+
+constexpr int kTcMaxLayers = 7;        // n_layers <= 6 hidden layers + the merged Gaussian head
+constexpr int kTcRows = 128;           // batch rows per chain CTA (the MMA's M)
+
+// Train layer l (TrainLayer) with the two bf16 UMMA images of its block that the chain kernel reads, rebuilt by the
+// update kernel after every Adam step:
+//   forward   B[n][k] = theta[k][n], rows N padded to 16, K + 2 columns padded to 16: k = K holds bf16(bias),
+//             k = K + 1 the residual bf16(bias - bf16(bias)) (the A tile carries ones there)
+//   backward  B[k][n] = theta[k][n] (k < K), rows K padded to 16, N columns padded to 16 (layers >= 1)
+// Both are K-major SWIZZLE_NONE: 8-row x 16-byte core matrices, row groups 128 B apart, 8-wide K groups
+// rows_padded * 16 B apart, so every 64-wide K chunk is one contiguous block.
+struct TcLayer {
+  int K, N;
+  int64_t off;              // float offset of the block inside a member's theta
+  int64_t fwd_off, bwd_off; // byte offsets of the images inside a member's bf16 image (bwd_off < 0: layer 0)
+};
+
+struct TcChainArgs {
+  TcLayer layer[kTcMaxLayers];
+  int L;                    // hidden layers (layer L is the head)
+  float* act[kTcMaxLayers]; // act[l], l >= 1: input of layer l [E][cap][K_l] (H_l after dropout)
+  int64_t act_estride;      // rows per member (cap)
+  float* dz[kTcMaxLayers];  // [E][batch][N_l]
+  int64_t dz_estride;       // rows per member (batch)
+  const float* x;           // [E][rows][K_0] (estride may be 0: validation shares its rows)
+  int64_t x_estride;
+  int gather;               // 1: batch rows follow the fit descriptor's index
+  const float* y;
+  int64_t y_estride;
+  const uint8_t* img;
+  int64_t img_member_bytes;
+  int out_dim, ensemble;
+  float* partial;
+  int tiles_cap;
+  int train;
+  float* out_loss;
+  float dropout_rate, dropout_scale;
+  uint64_t dropout_seed;
+};
+
+struct TcUpdArgs {
+  TcLayer layer[kTcMaxLayers];
+  int tile_begin[kTcMaxLayers];   // first CTA of each layer in the grid
+  int n_tiles_n[kTcMaxLayers];    // 128-column tiles of each layer
+  int n_layers;
+  const float* h[kTcMaxLayers];   // input of the layer (layer 0: x, or gathered through the fit descriptor)
+  int64_t h_estride[kTcMaxLayers];
+  int gather0;
+  const float* dz[kTcMaxLayers];
+  int64_t dz_estride;       // rows per member (batch)
+  float *theta, *m, *v, *grad;
+  int64_t pn;
+  uint8_t* img;
+  int64_t img_member_bytes;
+  int ensemble;
+};
+
+}  // namespace simba
 
 namespace {
 
@@ -480,17 +542,24 @@ train_tc_update_kernel(const TcUpdArgs a, const OptParams opt, const FitDesc* de
 // Coverage: the shapes of both bf16 planner families. The chain kernel keeps a [128 x (units + 2)] bf16
 // A tile and two [units x 64] weight chunks in shared memory (217 KB at 416 units) and up to 416 fp32
 // accumulator columns in tensor memory; the heads (N = 2 obs_dim <= 248) are one MMA.
-bool train_tc_supported(int in_dim, int obs_dim, int n_layers, int units) {
-  return units >= 1 && units <= 416 && in_dim <= 126 && obs_dim >= 1 && obs_dim <= 124 && n_layers >= 1 &&
-         n_layers <= 6;
+int train_tc_check(const simba_model_config_t& mc) {
+  const int in_dim = mc.obs_dim + mc.act_dim;
+  if (mc.units >= 1 && mc.units <= 416 && in_dim <= 126 && mc.obs_dim >= 1 && mc.obs_dim <= 124 && mc.n_layers >= 1 &&
+      mc.n_layers <= 6)
+    return SIMBA_OK;
+  return set_error(SIMBA_ERR_UNSUPPORTED,
+                   "bf16 tcgen05 training covers units <= 416, obs_dim + act_dim <= 126, obs_dim <= 124 and "
+                   "n_layers <= 6 (got units %d, obs_dim %d, act_dim %d, n_layers %d); precision fp32 trains "
+                   "this shape",
+                   mc.units, mc.obs_dim, mc.act_dim, mc.n_layers);
 }
 
-int64_t train_tc_layout(TcLayer* layers, int n) {
+// the layers of `d` with the offsets of their images; returns a member's image bytes
+static int64_t layout(const TrainDesc& d, TcLayer* layers) {
   int64_t off = 0;
-  for (int l = 0; l < n; ++l) {
-    layers[l].fwd_off = off;
+  for (int l = 0; l <= d.L; ++l) {
+    layers[l] = TcLayer{d.layer[l].K, d.layer[l].N, d.layer[l].off, off, -1};
     off += (int64_t)r16(layers[l].N) * r16(layers[l].K + 2) * 2;
-    layers[l].bwd_off = -1;
     if (l > 0) {
       layers[l].bwd_off = off;
       off += (int64_t)r16(layers[l].K) * r16(layers[l].N) * 2;
@@ -499,13 +568,20 @@ int64_t train_tc_layout(TcLayer* layers, int n) {
   return off;
 }
 
+int64_t train_tc_image_bytes(const TrainDesc& d) {
+  TcLayer layers[kTcMaxLayers];
+  return layout(d, layers);
+}
+
 // element (row, col) of a K-major SWIZZLE_NONE image with `rows_p` padded rows, in bf16 units
 static size_t img_index(int row, int col, int rows_p) {
   return (size_t)(col >> 3) * rows_p * 8 + (size_t)(row >> 3) * 64 + (size_t)(row & 7) * 8 + (col & 7);
 }
 
-void train_tc_pack(const TcLayer* layers, int n, const float* theta, uint8_t* img) {
-  for (int l = 0; l < n; ++l) {
+void train_tc_pack(const TrainDesc& d, const float* theta, uint8_t* img) {
+  TcLayer layers[kTcMaxLayers];
+  layout(d, layers);
+  for (int l = 0; l <= d.L; ++l) {
     const TcLayer& L = layers[l];
     const float* W = theta + L.off;
     uint16_t* fwd = reinterpret_cast<uint16_t*>(img + L.fwd_off);
@@ -524,10 +600,6 @@ void train_tc_pack(const TcLayer* layers, int n, const float* theta, uint8_t* im
   }
 }
 
-int train_tc_update_tiles(const TcLayer& l) {
-  return ((l.K + 1 + kUpdTile - 1) / kUpdTile) * ((l.N + kUpdTile - 1) / kUpdTile);
-}
-
 // Each CTA allocates a power of two of TMEM columns (>= 32) and nothing else on the SM may then be short of
 // them: the dynamic shared memory request is raised until no more CTAs fit the SM than its 512 columns allow.
 static size_t smem_for_tmem(size_t smem, uint32_t tmem_cols) {
@@ -537,8 +609,22 @@ static size_t smem_for_tmem(size_t smem, uint32_t tmem_cols) {
   return std::max(smem, floor_bytes);
 }
 
-cudaError_t train_tc_chain(const TcChainArgs& a, const OptParams& opt, const FitDesc* desc, TrainState* st,
-                           int grid_rows, int rows_fixed, int step_off, cudaStream_t s) {
+cudaError_t train_tc_chain(const TrainDesc& d, const OptParams& opt, const FitDesc* desc, TrainState* st,
+                           int grid_rows, int rows_fixed, int step_off, cudaStream_t s, int& row_tiles) {
+  TcChainArgs a{};
+  layout(d, a.layer);
+  for (int l = 0; l <= d.L; ++l) {
+    a.act[l] = d.act[l];
+    a.dz[l] = d.dz[l];
+  }
+  a.L = d.L;
+  a.act_estride = d.act_estride; a.dz_estride = d.dz_estride;
+  a.x = d.x; a.x_estride = d.x_estride; a.gather = d.gather;
+  a.y = d.y; a.y_estride = d.y_estride;
+  a.img = d.img; a.img_member_bytes = d.img_member_bytes;
+  a.out_dim = d.out_dim; a.ensemble = d.ensemble;
+  a.partial = d.partial; a.tiles_cap = d.tiles_cap; a.train = d.train; a.out_loss = d.out_loss;
+  a.dropout_rate = d.dropout_rate; a.dropout_scale = d.dropout_scale; a.dropout_seed = d.dropout_seed;
   const int n_pass = a.train ? 2 * a.L + 1 : a.L + 1;
   int ka = r16(a.layer[0].K + 2), np_max = 0;
   for (int l = 0; l <= a.L; ++l) {
@@ -555,14 +641,31 @@ cudaError_t train_tc_chain(const TcChainArgs& a, const OptParams& opt, const Fit
   cudaError_t err = cudaFuncSetAttribute(train_tc_chain_kernel, cudaFuncAttributeMaxDynamicSharedMemorySize,
                                          (int)smem);
   if (err != cudaSuccess) return err;
-  dim3 grid((grid_rows + kTcRows - 1) / kTcRows, a.ensemble);
-  train_tc_chain_kernel<<<grid, kThreads, smem, s>>>(a, opt, desc, st, rows_fixed, step_off, n_pass, stage_bytes,
-                                                     a_bytes, tmem_cols);
+  row_tiles = (grid_rows + kTcRows - 1) / kTcRows;
+  train_tc_chain_kernel<<<dim3(row_tiles, a.ensemble), kThreads, smem, s>>>(a, opt, desc, st, rows_fixed, step_off,
+                                                                           n_pass, stage_bytes, a_bytes, tmem_cols);
   return cudaGetLastError();
 }
 
-cudaError_t train_tc_update(const TcUpdArgs& a, const OptParams& opt, const FitDesc* desc, const TrainState* st,
-                            int n_tiles, int rows_fixed, int step_off, cudaStream_t s) {
+cudaError_t train_tc_update(const TrainDesc& d, const OptParams& opt, const FitDesc* desc, const TrainState* st,
+                            int rows_fixed, int step_off, cudaStream_t s) {
+  TcUpdArgs a{};
+  layout(d, a.layer);
+  int n_tiles = 0;
+  for (int l = 0; l <= d.L; ++l) {
+    const int K = d.layer[l].K, N = d.layer[l].N;
+    a.tile_begin[l] = n_tiles;
+    a.n_tiles_n[l] = (N + kUpdTile - 1) / kUpdTile;
+    n_tiles += ((K + 1 + kUpdTile - 1) / kUpdTile) * a.n_tiles_n[l];
+    a.h[l] = l == 0 ? d.x : d.act[l];
+    a.h_estride[l] = l == 0 ? d.x_estride : d.act_estride * K;
+    a.dz[l] = d.dz[l];
+  }
+  a.n_layers = d.L + 1;
+  a.gather0 = d.gather;
+  a.dz_estride = d.dz_estride;
+  a.theta = d.theta; a.m = d.m; a.v = d.v; a.grad = d.grad; a.pn = d.pn;
+  a.img = d.img; a.img_member_bytes = d.img_member_bytes; a.ensemble = d.ensemble;
   const size_t smem = smem_for_tmem((size_t)2 * kUpdTile * kUpdRows * 2 + (size_t)kUpdTile * kGStride * 4, kUpdTile);
   cudaError_t err = cudaFuncSetAttribute(train_tc_update_kernel, cudaFuncAttributeMaxDynamicSharedMemorySize,
                                          (int)smem);

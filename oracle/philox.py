@@ -136,7 +136,7 @@ def final_normals(seed, act_dim, state_index=0):
 
 
 def dropout_keep(seed, iteration, member, layer, rows, units, rate):
-    """Dropout keep mask of the trainer (csrc/trainer.cu): [rows, units] bool, keep = u >= rate with
+    """Dropout keep mask of the trainer (csrc/train_common.cuh): [rows, units] bool, keep = u >= rate with
     u = uniform_from_bits(philox(column block j, batch row r, iteration, member | layer << 8 | 4 << 28))."""
     nblk = (units + 3) // 4
     ctr = np.empty((rows, nblk, 4), dtype=np.uint32)

@@ -105,7 +105,7 @@ def _library_choice(c, precision='bf16', switches=()):
 
 
 def _chain_tile_rows(E, rows):
-    """chain_tile_rows (csrc/trainer.cu): the smallest row tile that keeps E x row tiles within 160 CTAs."""
+    """chain_tile_rows (csrc/trainer_f32.cu): the smallest row tile that keeps E x row tiles within 160 CTAs."""
     for R in (4, 8):
         if E * -(-rows // R) <= 160:
             return R

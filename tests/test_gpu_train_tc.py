@@ -247,6 +247,31 @@ def test_wide_observation_fit_meets_the_fit_bound():
 
 
 @gpu
+def test_bf16_trainer_holds_no_fp32_back_propagation_copy():
+    """Both precisions keep the same master weights, Adam slots and buffers plus one image derived from the
+    weights: theta^T for fp32, the UMMA images for bf16 (about 21 and 22 MB at C5, E=10, 4x400). A bf16 trainer
+    must not also hold fp32's theta^T."""
+    import torch
+    ens = _ensemble(62, 60, 10, 64, 4, 400)
+    ens.build()                                          # the model handle and its commit are not the trainer's
+
+    def taken(precision):
+        ens.train_precision = precision
+        torch.cuda.synchronize()
+        free0, _ = torch.cuda.mem_get_info()
+        ens._ensure_trainer()
+        torch.cuda.synchronize()
+        free1, _ = torch.cuda.mem_get_info()
+        ens._drop_trainer()
+        return free0 - free1
+
+    taken('fp32'), taken('bf16')                         # warm-up: one-time allocations of the context
+    fp32 = taken('fp32')
+    bf16 = taken('bf16')
+    assert bf16 <= fp32 + 4 * 1024 * 1024, (fp32, bf16)
+
+
+@gpu
 def test_bf16_trained_weights_reach_the_model_handle():
     """After a bf16 fit, the model handle (through simba_trainer_sync_model) predicts exactly what a fresh
     model built on the trained weights predicts, on both rollout precisions."""

@@ -3,9 +3,10 @@ timeline stamps compiled in (the product build has none):
 
     cd ethz-safe-learning_b200/csrc && make && \
     nvcc -gencode arch=compute_100a,code=sm_100a -O3 -std=c++17 -lineinfo -Xcompiler -fPIC \
-         -DSIMBA_TRAIN_TIMELINE -c trainer.cu -o /tmp/trainer_tl.o && \
+         -DSIMBA_TRAIN_TIMELINE -c trainer_f32.cu -o /tmp/trainer_f32_tl.o && \
     nvcc -gencode arch=compute_100a,code=sm_100a -shared -o ../simba_b200/libsimba_b200_tl.so \
-         api.o cem_kernels.o rollout_f32.o rollout_tc.o rollout_tc_wide.o /tmp/trainer_tl.o -ldl
+         api.o cem_kernels.o rollout_f32.o rollout_tc.o rollout_tc_wide.o trainer.o trainer_tc.o \
+         /tmp/trainer_f32_tl.o -ldl
 """
 import ctypes as C
 import os
