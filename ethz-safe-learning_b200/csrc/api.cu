@@ -1184,15 +1184,29 @@ extern "C" int simba_unfold_tc_kernel(simba_model_t* m, int32_t batch, int32_t h
   return SIMBA_OK;
 }
 
-extern "C" int simba_ensemble_forward(simba_model_t* m, const float* x, const float* eps,
-                                      int32_t batch, float* out_mu, float* out_var,
-                                      float* out_sample, void* stream) {
+// The forward pass of the model's rows (mlp_ensemble.py:122-132, :189-193) as a one-step rollout whose state is x's
+// first O columns and whose action is the rest: a set prm.mu_out selects the forward form of the kernel.
+static int ensemble_forward(int precision, simba_model_t* m, const float* x, const float* eps, int32_t batch,
+                            float* out_mu, float* out_var, float* out_sample, void* stream) {
+  if (precision != SIMBA_PREC_FP32) {
+    int rc = unfold_tc_device_check(m);
+    if (rc != SIMBA_OK) return rc;
+  }
   if (!m || !x || !out_mu || !out_var) return set_error(SIMBA_ERR_BAD_CONFIG, "null argument");
   RolloutParams prm{};
-  int rc = model_rollout_params(m, SIMBA_PREC_FP32, batch, 1, prm);
+  int rc = model_rollout_params(m, precision, batch, 1, prm);
   if (rc != SIMBA_OK) return rc;
   const int O = m->cfg.obs_dim, IN = O + m->cfg.act_dim;
   prm.scale_on = 0;                               // x is used as given (mlp_ensemble.py:190)
+  if (precision != SIMBA_PREC_FP32) {
+    // the tcgen05 kernels scale through these tables alone: the identity of scale_on = 0 (pack_scaler), not the
+    // model's own
+    for (int k = 0; k < 128; ++k) {
+      prm.tc_scale_a[k] = k < IN ? 1.0f : 0.0f;
+      prm.tc_scale_b[k] = 0.0f;
+    }
+    prm.sampling_propagation = out_sample != nullptr;   // the draws enter the head pass only for a sample
+  }
   prm.states = x; prm.state_stride = IN; prm.state_per_row = 1;
   prm.actions = x + O; prm.action_stride = IN;
   prm.eps = eps;
@@ -1200,6 +1214,23 @@ extern "C" int simba_ensemble_forward(simba_model_t* m, const float* x, const fl
   if (out_sample && !eps) return set_error(SIMBA_ERR_BAD_CONFIG, "out_sample needs eps");
   SIMBA_CUDA_TRY(launch_rollout(prm, (cudaStream_t)stream));
   return SIMBA_OK;
+}
+
+extern "C" int simba_ensemble_forward(simba_model_t* m, const float* x, const float* eps,
+                                      int32_t batch, float* out_mu, float* out_var,
+                                      float* out_sample, void* stream) {
+  return ensemble_forward(SIMBA_PREC_FP32, m, x, eps, batch, out_mu, out_var, out_sample, stream);
+}
+
+extern "C" int simba_ensemble_forward_tc(simba_model_t* m, const float* x, const float* eps, int32_t batch,
+                                         float* out_mu, float* out_var, float* out_sample, void* stream) {
+  return ensemble_forward(SIMBA_PREC_BF16_TC, m, x, eps, batch, out_mu, out_var, out_sample, stream);
+}
+
+// the forward form runs the variant of the trajectory form at H = 1
+extern "C" int simba_ensemble_forward_tc_kernel(simba_model_t* m, int32_t batch, int32_t* kernel,
+                                                int32_t* work_items) {
+  return simba_unfold_tc_kernel(m, batch, 1, kernel, work_items);
 }
 
 extern "C" int simba_scale(simba_model_t* m, const float* x, int32_t batch, float* out, void* stream) {

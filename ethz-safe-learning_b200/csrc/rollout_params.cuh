@@ -68,9 +68,9 @@ struct RolloutParams {
   long long* timeline;        // clock64 stamps of CTA 0 (-DSIMBA_TC_TIMELINE builds only, else null)
 };
 
-// Launches the kernel prm.kernel names over prm.tiles: the trajectory form of a tcgen05 kernel when prm.traj_out is
-// set, its planning form otherwise (the fp32 kernel takes both from prm at run time). Defined in api.cu, next to
-// choose_rollout, which picks prm.kernel and the tile list.
+// Launches the kernel prm.kernel names over prm.tiles: the forward form of a tcgen05 kernel when prm.mu_out is set,
+// its trajectory form when prm.traj_out is, its planning form otherwise (the fp32 kernel takes all three from prm at
+// run time). Defined in api.cu, next to choose_rollout, which picks prm.kernel and the tile list.
 cudaError_t launch_rollout(const RolloutParams& prm, cudaStream_t stream);
 // the branches of launch_rollout, one per kernel file
 cudaError_t launch_rollout_f32(const RolloutParams& prm, cudaStream_t stream);

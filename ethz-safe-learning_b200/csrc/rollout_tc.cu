@@ -155,10 +155,16 @@ struct AStorePair {
 // idle, no partial minima are published, the scorer struct is not read. Each thread whose column slice
 // meets the action block stores its own action columns (head_store_own_actions). H is bounded only by
 // the 16 bits of the Philox step counter.
-template <int NTILES, int Q, bool PAIR, bool TRAJ>
+//
+// FWD (simba_ensemble_forward_tc): the forward form, a TRAJ form at H = 1 whose epilogue threads write, instead of
+// the state, the Gaussian head's mu, var and (with external draws) sample of their valid rows to prm.mu_out,
+// var_out and sample_out [B, O] (tc_head.cuh ForwardSink). Its head pass always forms the variance; without draws
+// the noise stays zero.
+template <int NTILES, int Q, bool PAIR, bool TRAJ, bool FWD = false>
 __device__ __forceinline__ void rollout_tc_body(const RolloutParams& prm) {
   static_assert(!PAIR || (NTILES == 1 && Q == 4), "the pair variant is the one-tile latency configuration");
   static_assert(!(PAIR && TRAJ), "the trajectory form has no pair variant");
+  static_assert(!FWD || TRAJ, "the forward form is a trajectory form");
   constexpr int kTileThreads = Q * 128;
   constexpr int kTileWarps = Q * 4;
   constexpr int kEpiThreads = NTILES * kTileThreads;
@@ -685,9 +691,11 @@ __device__ __forceinline__ void rollout_tc_body(const RolloutParams& prm) {
           }
         };
         const float* s0_ptr = prm.states + (prm.state_per_row ? id.r_global : (int64_t)id.s) * prm.state_stride;
-        // TRAJ: this row's s_t in traj_out, advanced by one step before every head pass
-        typename std::conditional<TRAJ, TrajSink, NoTraj>::type sink{};
-        if constexpr (TRAJ) {
+        // TRAJ: this row's s_t in traj_out, advanced by one step before every head pass; FWD: its outputs
+        typename std::conditional<FWD, ForwardSink, typename std::conditional<TRAJ, TrajSink, NoTraj>::type>::type sink{};
+        if constexpr (FWD) {
+          sink = ForwardSink{prm.mu_out, prm.var_out, prm.sample_out, row_ok ? (int)id.out : -1, O};
+        } else if constexpr (TRAJ) {
           sink.row = row_ok ? prm.traj_out + id.out * (int64_t)(H + 1) * O : nullptr;
           sink.O = O;
         }
@@ -755,7 +763,7 @@ __device__ __forceinline__ void rollout_tc_body(const RolloutParams& prm) {
           const int o0 = hc.o_base + b * 8;
           if (o0 >= O) return;                              // warp-uniform: nothing to draw
           uint4 z;
-          if (eps_row != nullptr) {
+          if (FWD || eps_row != nullptr) {                 // FWD: external draws only (sampling_propagation)
             z = external_noise8_bf16(eps_row + t * eps_step, o0, O);
           } else {
 #ifdef SIMBA_TC_TIMELINE
@@ -827,7 +835,7 @@ __device__ __forceinline__ void rollout_tc_body(const RolloutParams& prm) {
             publish_a();
             TL(3 + l * 4);
             if (prm.sampling_propagation) {
-              if (NTILES == 1 && L >= 2 * NB && eps_row == nullptr) {
+              if (!FWD && NTILES == 1 && L >= 2 * NB && eps_row == nullptr) {
                 // latency variant: a whole block (~1.3 k cycles for a lone warp: two serial dependency
                 // chains) is longer than one layer's MMA shadow, so it is split over two layers — the ten
                 // Philox rounds after an even layer, Box-Muller after the following odd one
@@ -865,14 +873,15 @@ __device__ __forceinline__ void rollout_tc_body(const RolloutParams& prm) {
               hc.part_mbar = astore.peer_bar;
             }
           }
-          if constexpr (TRAJ) {
+          if constexpr (TRAJ && !FWD) {
             if (sink.row != nullptr) sink.row += O;
           }
           if constexpr (kDbl) {                             // the head GEMM's accumulator, x_{t+1} into the other A buffer
             hc.t_acc = t_acc + gemm_par(t, L) * 128;
             astore.t_a = t_a + (gemm_par(t, L) ^ 1u) * 64;
           }
-          if (prm.sampling_propagation) head_step_pass<OW, true>(hc, noise, astore, t + 1 < H, sink);
+          if constexpr (FWD) head_step_pass<OW, true>(hc, noise, astore, false, sink);
+          else if (prm.sampling_propagation) head_step_pass<OW, true>(hc, noise, astore, t + 1 < H, sink);
           else head_step_pass<OW, false>(hc, noise, astore, t + 1 < H, sink);
           TL(41);
           exchange(t, t + 1 < H);
@@ -912,6 +921,12 @@ __global__ void __launch_bounds__(kBoundThreads, 1) rollout_tc_kernel(const Roll
 template <int NTILES, int Q>
 __global__ void __launch_bounds__(kBoundThreads, 1) unfold_tc_kernel(const RolloutParams prm) {
   rollout_tc_body<NTILES, Q, false, true>(prm);
+}
+
+// the forward form (simba_ensemble_forward_tc): the same two variants at H = 1
+template <int NTILES, int Q>
+__global__ void __launch_bounds__(kBoundThreads, 1) forward_tc_kernel(const RolloutParams prm) {
+  rollout_tc_body<NTILES, Q, false, true, true>(prm);
 }
 
 // ---- host side ------------------------------------------------------------------------------------
@@ -995,10 +1010,11 @@ bool rollout_tc_pair_fits(int L, int n_constraints) {
   return tc_smem_bytes(L, 1, 4, 1 + n_constraints, true) + 1024 <= kMaxSmem;
 }
 
-template <int NTILES, int Q, bool PAIR, bool TRAJ>
+template <int NTILES, int Q, bool PAIR, bool TRAJ, bool FWD = false>
 static cudaError_t launch_variant(const RolloutParams& prm, cudaStream_t stream) {
   void (*kern)(const RolloutParams) = rollout_tc_kernel<NTILES, Q, PAIR>;
-  if constexpr (TRAJ) kern = unfold_tc_kernel<NTILES, Q>;
+  if constexpr (FWD) kern = forward_tc_kernel<NTILES, Q>;
+  else if constexpr (TRAJ) kern = unfold_tc_kernel<NTILES, Q>;
   const size_t smem = tc_smem_bytes(prm.L, NTILES, Q, TRAJ ? 1 : 1 + prm.scorer.n_constraints, PAIR);
   const int n_items = (prm.n_tiles + NTILES - 1) / NTILES;
   const int sms = prm.n_sms;
@@ -1010,6 +1026,13 @@ static cudaError_t launch_variant(const RolloutParams& prm, cudaStream_t stream)
 }
 
 cudaError_t launch_rollout_tc(const RolloutParams& prm, cudaStream_t stream) {
+  if (prm.mu_out != nullptr) {
+    switch (prm.kernel) {   // the forward form: the trajectory form's variants
+      case RolloutKernel::kTcOneCta: return launch_variant<1, 4, false, true, true>(prm, stream);
+      case RolloutKernel::kTcTwoTile: return launch_variant<2, 2, false, true, true>(prm, stream);
+      default: return cudaErrorInvalidValue;
+    }
+  }
   if (prm.traj_out == nullptr) {
     switch (prm.kernel) {
       case RolloutKernel::kTcOneCta: return launch_variant<1, 4, false, false>(prm, stream);

@@ -134,8 +134,13 @@ struct TileInfoW {
 // rows to prm.traj_out [B, H + 1, O] (tc_head.cuh TrajSink) and score nothing (no partial minima, no objective,
 // no scorer struct read). Each thread whose column slice meets the action block stores its own action columns
 // (head_store_own_actions). H is bounded only by the 16 bits of the Philox step counter.
-template <int kSW, bool TRAJ>
+//
+// FWD (simba_ensemble_forward_tc): the forward form, a TRAJ form at H = 1 that writes the Gaussian head's mu, var
+// and (with external draws) sample of its valid rows to prm.mu_out, var_out and sample_out [B, O] instead of the
+// state (tc_head.cuh ForwardSink). Its head pass always forms the variance; without draws the noise stays zero.
+template <int kSW, bool TRAJ, bool FWD = false>
 __device__ __forceinline__ void rollout_tc_wide_body(const RolloutParams& prm) {
+  static_assert(!FWD || TRAJ, "the forward form is a trajectory form");
   using C = WideCfg<kSW>;
   constexpr int kStateCol = C::kStateCol, OW = C::OW, NB = C::NB, kHeadGroup = C::kHeadGroup;
   extern __shared__ __align__(1024) uint8_t smem_raw[];
@@ -309,9 +314,11 @@ __device__ __forceinline__ void rollout_tc_wide_body(const RolloutParams& prm) {
       const bool done_first = objective_done_first(prm.objective);
       const simba_scorer_t& sc = prm.scorer;
       const float* s0_ptr = prm.states + (prm.state_per_row ? id.r_global : (int64_t)id.s) * prm.state_stride;
-      // TRAJ: this row's s_t in traj_out, advanced by one step before every head pass
-      typename std::conditional<TRAJ, TrajSink, NoTraj>::type sink{};
-      if constexpr (TRAJ) {
+      // TRAJ: this row's s_t in traj_out, advanced by one step before every head pass; FWD: its outputs
+      typename std::conditional<FWD, ForwardSink, typename std::conditional<TRAJ, TrajSink, NoTraj>::type>::type sink{};
+      if constexpr (FWD) {
+        sink = ForwardSink{prm.mu_out, prm.var_out, prm.sample_out, row_ok ? (int)id.out : -1, O};
+      } else if constexpr (TRAJ) {
         sink.row = row_ok ? prm.traj_out + id.out * (int64_t)(H + 1) * O : nullptr;
         sink.O = O;
       }
@@ -384,7 +391,7 @@ __device__ __forceinline__ void rollout_tc_wide_body(const RolloutParams& prm) {
         const int o0 = hc.o_base + b * 8;
         if (o0 >= O) return;
         uint4 z;
-        if (prm.eps != nullptr) {
+        if (FWD || prm.eps != nullptr) {                   // FWD: external draws only (sampling_propagation)
           const float* ep = prm.eps + (((int64_t)id.s * H + t) * ((int64_t)g.P * g.N) + id.r_global) * O;
           z = external_noise8_bf16(ep, o0, O);
         } else {
@@ -483,10 +490,11 @@ __device__ __forceinline__ void rollout_tc_wide_body(const RolloutParams& prm) {
           // 96 registers: re-derive the slice predicates every step instead of holding them (no spills)
           asm volatile("mov.b32 %0, %0;" : "+r"(hc.slice_bits));
         }
-        if constexpr (TRAJ) {
+        if constexpr (TRAJ && !FWD) {
           if (sink.row != nullptr) sink.row += O;
         }
-        if (prm.sampling_propagation) head_step_pass<OW, true, kSW, kSW>(hc, noise, astore, t + 1 < H, sink);
+        if constexpr (FWD) head_step_pass<OW, true, kSW, kSW>(hc, noise, astore, false, sink);
+        else if (prm.sampling_propagation) head_step_pass<OW, true, kSW, kSW>(hc, noise, astore, t + 1 < H, sink);
         else head_step_pass<OW, false, kSW, kSW>(hc, noise, astore, t + 1 < H, sink);
         TLW(41);
         tmem_st_wait();
@@ -536,6 +544,12 @@ __global__ void __launch_bounds__(kWideThreads, 1) rollout_tc_wide_kernel(const 
 template <int kSW>
 __global__ void __launch_bounds__(kWideThreads, 1) unfold_tc_wide_kernel(const RolloutParams prm) {
   rollout_tc_wide_body<kSW, true>(prm);
+}
+
+// the forward form (simba_ensemble_forward_tc)
+template <int kSW>
+__global__ void __launch_bounds__(kWideThreads, 1) forward_tc_wide_kernel(const RolloutParams prm) {
+  rollout_tc_wide_body<kSW, true, true>(prm);
 }
 
 // ---- host side ------------------------------------------------------------------------------------
@@ -628,17 +642,25 @@ int64_t rollout_tc_wide_pack(int sw, const ModelWeights& mw, std::vector<uint16_
   return member_bytes;
 }
 
-template <int kSW, bool TRAJ>
+template <int kSW, bool TRAJ, bool FWD = false>
 static cudaError_t launch_wide(const RolloutParams& model_prm, cudaStream_t stream) {
   RolloutParams prm = model_prm;
   prm.U = rollout_tc_wide_units(kSW, prm.U);                       // the kernel runs the zero-padded width
   void (*kern)(const RolloutParams) = rollout_tc_wide_kernel<kSW>;
-  if constexpr (TRAJ) kern = unfold_tc_wide_kernel<kSW>;
+  if constexpr (FWD) kern = forward_tc_wide_kernel<kSW>;
+  else if constexpr (TRAJ) kern = unfold_tc_wide_kernel<kSW>;
   const size_t smem = wide_smem_bytes<kSW>(prm.L, prm.U, TRAJ ? 1 : 1 + prm.scorer.n_constraints);
   return launch_kernel(kern, prm.n_tiles, kWideThreads, smem, stream, 1, prm.pdl, prm);
 }
 
 cudaError_t launch_rollout_tc_wide(const RolloutParams& prm, cudaStream_t stream) {
+  if (prm.mu_out != nullptr) {
+    switch (prm.kernel) {
+      case RolloutKernel::kTcWide: return launch_wide<64, true, true>(prm, stream);
+      case RolloutKernel::kTcWideObs: return launch_wide<128, true, true>(prm, stream);
+      default: return cudaErrorInvalidValue;
+    }
+  }
   if (prm.traj_out == nullptr) {
     switch (prm.kernel) {
       case RolloutKernel::kTcWide: return launch_wide<64, false>(prm, stream);

@@ -1,6 +1,8 @@
 // The Gaussian-head / state / scoring pass shared by the two tcgen05 rollout kernels (rollout_tc.cu:
 // A operand in tensor memory; rollout_tc_wide.cu: A operand in a swizzled shared-memory tile), plus
-// the NOISE-stream generator they both use. One implementation, so a parity fix lands once.
+// the NOISE-stream generator they both use. One implementation, so a parity fix lands once. Where the
+// pass's values go besides tensor memory is its sink: nowhere (planning), the trajectory (simba_unfold_tc)
+// or the Gaussian head's mu, var and sample (simba_ensemble_forward_tc).
 //
 // What the pass replaces, per rollout row and step (SURVEY.md section 8 a6-a13):
 //   mlp_ensemble.py:28-34,189-193   mu, var = softplus(raw) + 1e-4, delta = mu + sqrt(var) * eps
@@ -214,15 +216,18 @@ __device__ __forceinline__ void head_publish(const HeadCtx& c, float gmin, const
     if (q < c.n_constraints) c.part[(1 + q) * 128] = cmin[q];
 }
 
-// Where the state values of a head pass go besides TMEM. The planning kernels keep nothing (NoTraj: the pass
-// scores the states). The trajectory form of the kernels (simba_unfold_tc) writes them to its row of
-// traj_out [B, H + 1, O] (TrajSink) and skips the scoring: no slice minima, nothing published.
+// Where the values of a head pass go besides TMEM. The planning kernels keep nothing (NoTraj: the pass
+// scores the states). The trajectory form of the kernels (simba_unfold_tc) writes the states to its row of
+// traj_out [B, H + 1, O] (TrajSink) and skips the scoring: no slice minima, nothing published. The forward
+// form (simba_ensemble_forward_tc) keeps the Gaussian head's per-element mu, var and sample instead of the
+// state (ForwardSink, kState = false: the sampling head pass hands each chunk to head8 and neither reads nor
+// writes the state columns).
 struct NoTraj {
-  static constexpr bool kScore = true;
+  static constexpr bool kScore = true, kState = true;
   __device__ __forceinline__ void put8(int, const float (&)[8]) const {}
 };
 struct TrajSink {
-  static constexpr bool kScore = false;
+  static constexpr bool kScore = false, kState = true;
   float* row;   // this row's state of the current step in traj_out, null for a padding row
   int O;
   // outputs [oc, oc + 8) below O: 16-byte stores where the address allows (row offsets are not 16-byte
@@ -242,6 +247,28 @@ struct TrajSink {
         if (oc + i < O) __stcs(p + i, v[i]);
     }
   }
+};
+struct ForwardSink {
+  static constexpr bool kScore = false, kState = false;
+  float* mu;       // mu_out / var_out / sample_out [B, O] (sample null when no sample is asked for)
+  float* var;
+  float* sample;
+  int row;         // this thread's row of them, -1 for a padding row
+  int O;
+  // mu: the fp32 accumulator; v: softplus(raw) + 1e-4 before its square root; smp: mu + sqrt(var) * eps.
+  // Stored as TrajSink stores a state chunk.
+  __device__ __forceinline__ void head8(int oc, const uint32_t (&mu_bits)[8], const float (&v)[8],
+                                        const float (&smp)[8]) const {
+    if (row < 0) return;
+    const int64_t off = (int64_t)row * O;
+    float m[8];
+#pragma unroll
+    for (int i = 0; i < 8; ++i) m[i] = __uint_as_float(mu_bits[i]);
+    TrajSink{mu + off, O}.put8(oc, m);
+    TrajSink{var + off, O}.put8(oc, v);
+    if (sample != nullptr) TrajSink{sample + off, O}.put8(oc, smp);
+  }
+  __device__ __forceinline__ void put8(int, const float (&)[8]) const {}
 };
 
 // Trajectory form: every thread whose slice [o_base, o_base + OW) meets the action columns [O, O + A) stores
@@ -320,10 +347,11 @@ __device__ __forceinline__ void head_step_pass(const HeadCtx& c, const Noise& no
   float gmin = INFINITY, cmin[SIMBA_MAX_CONSTRAINTS];
 #pragma unroll
   for (int q = 0; q < SIMBA_MAX_CONSTRAINTS; ++q) cmin[q] = INFINITY;
+  static_assert(Sink::kState || kSample, "the forward form forms the variance");
   uint32_t vm[2][8], vv[2][8], st[2][8];
   tmem_ld<8>(c.t_acc + c.o_base, vm[0]);
   if (kSample) tmem_ld<8>(c.t_acc + kVar + c.o_base, vv[0]);
-  tmem_ld<8>(c.t_state + c.o_base, st[0]);
+  if constexpr (Sink::kState) tmem_ld<8>(c.t_state + c.o_base, st[0]);
 #pragma unroll
   for (int ch = 0; ch < NCH; ++ch) {
     const int oc = c.o_base + ch * 8;
@@ -332,7 +360,7 @@ __device__ __forceinline__ void head_step_pass(const HeadCtx& c, const Noise& no
     if (ch + 1 < NCH) {                                    // next chunk's loads fly during this chunk's math
       tmem_ld<8>(c.t_acc + oc + 8, vm[nxt]);
       if (kSample) tmem_ld<8>(c.t_acc + kVar + oc + 8, vv[nxt]);
-      tmem_ld<8>(c.t_state + oc + 8, st[nxt]);
+      if constexpr (Sink::kState) tmem_ld<8>(c.t_state + oc + 8, st[nxt]);
     }
     float sv[8];
     if (kSample) {
@@ -341,6 +369,7 @@ __device__ __forceinline__ void head_step_pass(const HeadCtx& c, const Noise& no
       // two outputs per instruction wherever the op exists as fp32x2 (the MUFU ops and the clamp do not)
       const f32x2 kOne = f2_pack(1.0f, 1.0f);
       const f32x2 kLn2 = f2_pack(0.6931471805599453f, 0.6931471805599453f), kFloor = f2_pack(1e-4f, 1e-4f);
+      float hv[8], hd[8];                                  // !kState: var and mu + stddev * eps, for sink.head8
 #pragma unroll
       for (int q = 0; q < 8; q += 2) {
         float e0, e1, l0, l1, s0, s1;
@@ -351,26 +380,34 @@ __device__ __forceinline__ void head_step_pass(const HeadCtx& c, const Noise& no
         asm("lg2.approx.ftz.f32 %0, %1;" : "=f"(l0) : "f"(l0));
         asm("lg2.approx.ftz.f32 %0, %1;" : "=f"(l1) : "f"(l1));
         f2_unpack(f2_fma(f2_pack(l0, l1), kLn2, kFloor), s0, s1);
+        if constexpr (!Sink::kState) { hv[q] = s0; hv[q + 1] = s1; }
         asm("sqrt.approx.ftz.f32 %0, %1;" : "=f"(s0) : "f"(s0));
         asm("sqrt.approx.ftz.f32 %0, %1;" : "=f"(s1) : "f"(s1));
         const f32x2 eps = f2_pack(__uint_as_float(nw[q >> 1] << 16), __uint_as_float(nw[q >> 1] & 0xffff0000u));
         const f32x2 mu = f2_pack(__uint_as_float(vm[cur][q]), __uint_as_float(vm[cur][q + 1]));
-        const f32x2 old = f2_pack(__uint_as_float(st[cur][q]), __uint_as_float(st[cur][q + 1]));
-        f2_unpack(f2_add(old, f2_fma(f2_pack(s0, s1), eps, mu)), sv[q], sv[q + 1]);
+        if constexpr (Sink::kState) {
+          const f32x2 old = f2_pack(__uint_as_float(st[cur][q]), __uint_as_float(st[cur][q + 1]));
+          f2_unpack(f2_add(old, f2_fma(f2_pack(s0, s1), eps, mu)), sv[q], sv[q + 1]);
+        } else {
+          f2_unpack(f2_fma(f2_pack(s0, s1), eps, mu), hd[q], hd[q + 1]);
+        }
       }
+      if constexpr (!Sink::kState) sink.head8(oc, vm[cur], hv, hd);
     } else {
 #pragma unroll
       for (int q = 0; q < 8; ++q) sv[q] = __uint_as_float(st[cur][q]) + __uint_as_float(vm[cur][q]);
     }
-    {
-      uint32_t so[8];
+    if constexpr (Sink::kState) {
+      {
+        uint32_t so[8];
 #pragma unroll
-      for (int i = 0; i < 8; ++i) so[i] = __float_as_uint(sv[i]);
-      tmem_st<8>(c.t_state + oc, so);
+        for (int i = 0; i < 8; ++i) so[i] = __float_as_uint(sv[i]);
+        tmem_st<8>(c.t_state + oc, so);
+      }
+      sink.put8(oc, sv);                                   // s_{t+1} as stored to TMEM
+      head_chunk_tail<kTW>(c, astore, oc, Sink::kScore ? (c.slice_bits >> (ch * 5)) & 31u : 0u, sv, write_next,
+                           gmin, cmin);
     }
-    sink.put8(oc, sv);                                     // s_{t+1} as stored to TMEM
-    head_chunk_tail<kTW>(c, astore, oc, Sink::kScore ? (c.slice_bits >> (ch * 5)) & 31u : 0u, sv, write_next,
-                         gmin, cmin);
   }
   if constexpr (Sink::kScore) head_publish(c, gmin, cmin);
 }

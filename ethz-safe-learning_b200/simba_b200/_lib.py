@@ -104,6 +104,8 @@ _SIGNATURES = {
     'simba_unfold_tc': [_vp, _vp, _vp, _vp, _u64, _i32, _i32, _i32, _vp, _vp],
     'simba_unfold_tc_kernel': [_vp, _i32, _i32, _P(_i32), _P(_i32)],
     'simba_ensemble_forward': [_vp, _vp, _vp, _i32, _vp, _vp, _vp, _vp],
+    'simba_ensemble_forward_tc': [_vp, _vp, _vp, _i32, _vp, _vp, _vp, _vp],
+    'simba_ensemble_forward_tc_kernel': [_vp, _i32, _P(_i32), _P(_i32)],
     'simba_scale': [_vp, _vp, _i32, _vp, _vp],
     'simba_score_trajectories': [_vp, _vp, _vp, _vp, _vp],
     'simba_scorer_eval': [_P(Scorer), _vp, _vp, _i32, _i32, _vp, _vp, _vp, _vp],

@@ -2,7 +2,8 @@
 
 The E Gaussian MLPs (mlp_ensemble.py:37-61, :111-112) live as packed fp32 + bf16 images inside a
 `simba_model` handle of libsimba_b200.so; `forward` / `__call__` (mlp_ensemble.py:122-132,
-:189-193) run the fp32 CUDA kernel. Training (`training_step`, `validation_step`, `fit`,
+:189-193) run the fp32 CUDA kernel, or with precision='bf16' the bf16 tcgen05 kernels a bf16 planner
+rolls out on. Training (`training_step`, `validation_step`, `fit`,
 mlp_ensemble.py:134-187; SURVEY.md section 8 f1) runs on fp32 master weights inside a
 `simba_trainer` handle; the trained weights are handed back to the model handle (and to
 `ensemble[e].get_weights()`) the next time either is used.
@@ -147,7 +148,9 @@ class MlpEnsemble(object):
     def build(self):
         self._ensure_handle()
 
-    def _run(self, inputs, eps):
+    def _run(self, inputs, eps, precision):
+        if precision not in _lib.PRECISIONS:
+            raise ValueError("precision must be one of %s, got %r" % (sorted(_lib.PRECISIONS), precision))
         x, kind = _device.to_device(inputs)
         if x.dim() != 2 or x.shape[1] != self.inputs_dim:
             raise ValueError("inputs must be [B, %d]" % self.inputs_dim)
@@ -159,23 +162,29 @@ class MlpEnsemble(object):
         if eps is not None:
             e, _ = _device.to_device(eps)
             smp = torch.empty_like(mu)
-        _lib.check(self._lib.simba_ensemble_forward(h, _device.ptr(x), _device.ptr(e), b,
-                                                    _device.ptr(mu), _device.ptr(var),
-                                                    _device.ptr(smp), _device.stream_ptr()))
+        fn = self._lib.simba_ensemble_forward if precision == 'fp32' else self._lib.simba_ensemble_forward_tc
+        _lib.check(fn(h, _device.ptr(x), _device.ptr(e), b, _device.ptr(mu), _device.ptr(var),
+                      _device.ptr(smp), _device.stream_ptr()))
         return mu, var, smp, kind
 
-    def forward(self, inputs):
-        """mlp_ensemble.py:122-132: rows split into E contiguous chunks -> (cat_mus, cat_vars)."""
-        mu, var, _, kind = self._run(inputs, None)
+    def forward(self, inputs, *, precision='fp32'):
+        """mlp_ensemble.py:122-132: rows split into E contiguous chunks -> (cat_mus, cat_vars).
+        precision='bf16' runs the bf16 tcgen05 kernels of a bf16 planner (inputs, weights and
+        activations rounded to bf16, fp32 accumulation); shapes they do not cover raise SimbaError
+        SIMBA_ERR_UNSUPPORTED."""
+        mu, var, _, kind = self._run(inputs, None, precision)
         return _device.like_input(mu, kind), _device.like_input(var, kind)
 
-    def __call__(self, inputs, eps=None, *args, **kwargs):
+    def __call__(self, inputs, eps=None, *args, precision='fp32', **kwargs):
         """mlp_ensemble.py:189-193 -> (mean, stddev, sample). `eps` are the N(0,1) draws of
-        Normal.sample(); if omitted they are drawn with torch on the device."""
+        Normal.sample(); if omitted they are drawn with torch on the device. precision as in
+        `forward`; with 'bf16' the sample takes eps rounded to bf16, as a bf16 plan does."""
+        if precision not in _lib.PRECISIONS:
+            raise ValueError("precision must be one of %s, got %r" % (sorted(_lib.PRECISIONS), precision))
         x, _ = _device.to_device(inputs)
         if eps is None:
             eps = torch.randn((x.shape[0], self.outputs_dim), dtype=torch.float32, device=x.device)
-        mu, var, smp, kind = self._run(inputs, eps)
+        mu, var, smp, kind = self._run(inputs, eps, precision)
         return (_device.like_input(mu, kind), _device.like_input(torch.sqrt(var), kind),
                 _device.like_input(smp, kind))
 

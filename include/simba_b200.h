@@ -261,6 +261,16 @@ int simba_unfold_tc_kernel(simba_model_t* m, int32_t batch, int32_t horizon, int
 int simba_ensemble_forward(simba_model_t* m, const float* x, const float* eps_or_null,
                            int32_t batch, float* out_mu, float* out_var, float* out_sample_or_null,
                            void* stream);
+/* The same on the bf16 tcgen05 kernels of a bf16 planner (the forward form of the kernel
+ * simba_ensemble_forward_tc_kernel reports): same arguments, layouts and errors, with x, weights and activations
+ * rounded to bf16 as the planner's rollouts are, fp32 accumulators and eps rounded to bf16 in the sample. mu is the
+ * head's fp32 accumulator; var = softplus(raw) + 1e-4 on the MUFU path. SIMBA_ERR_UNSUPPORTED for shapes no
+ * tcgen05 kernel covers (no fp32 fall-back). */
+int simba_ensemble_forward_tc(simba_model_t* m, const float* x, const float* eps_or_null, int32_t batch,
+                              float* out_mu, float* out_var, float* out_sample_or_null, void* stream);
+/* -> *kernel (simba_rollout_kernel) and *work_items that simba_ensemble_forward_tc would launch for this batch on
+ * the current device: those of simba_unfold_tc_kernel at horizon 1 */
+int simba_ensemble_forward_tc_kernel(simba_model_t* m, int32_t batch, int32_t* kernel, int32_t* work_items);
 /* TransitionModel.scale — transition_model.py:79-87. x [B, O+A] -> out [B, O+A]. */
 int simba_scale(simba_model_t* m, const float* x, int32_t batch, float* out, void* stream);
 /* compute_objective on materialised trajectories — mpc_policy.py:26-39 / safe_cem_mpc.py:76-96.
