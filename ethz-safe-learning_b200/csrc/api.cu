@@ -584,7 +584,17 @@ extern "C" int simba_planner_create(simba_model_t* model, const simba_planner_co
   rc = choose_rollout(mc, cfg->precision, p->geom, cfg->scorer.n_constraints, false, p->n_sms, p->kernel, p->tiles);
   if (rc != SIMBA_OK) { delete p; return rc; }
 
-  p->fused_update = cfg->world_size == 1 && cfg->n_samples <= 1024 && getenv("SIMBA_B200_NO_FUSE") == nullptr;
+  // The fused update kernel (one CTA per state) takes a single rank's population of at most 1024 candidates and
+  // needs its shared memory (cem_update_smem_bytes: the staged rows when they fit under 200 KB, else the refit
+  // scratch and keys, at most ~25 KB within H * A <= 1024); a plan it does not fit runs the separate kernels.
+  int smem_optin = 0;
+  ce = cudaDeviceGetAttribute(&smem_optin, cudaDevAttrMaxSharedMemoryPerBlockOptin, p->device);
+  if (ce != cudaSuccess) { delete p; return set_error(SIMBA_ERR_CUDA, "shared memory size: %s", cudaGetErrorString(ce)); }
+  bool update_staged = false;
+  const size_t update_smem = cem_update_smem_bytes(cfg->particles, cfg->n_samples, cfg->n_elite, cfg->horizon,
+                                                   mc.act_dim, &update_staged);
+  p->fused_update = cfg->world_size == 1 && cfg->n_samples <= 1024 && update_smem <= (size_t)smem_optin &&
+                    getenv("SIMBA_B200_NO_FUSE") == nullptr;
   p->use_pdl = p->fused_update && cfg->precision == SIMBA_PREC_BF16_TC && getenv("SIMBA_B200_NO_PDL") == nullptr;
   p->c_max = beta_count_threshold(cfg->particles, cfg->posterior_mean_threshold, cfg->prior_mu,
                                   cfg->prior_sigma);
@@ -605,7 +615,7 @@ extern "C" int simba_planner_create(simba_model_t* model, const simba_planner_co
   PL_ALLOC(p->actions, S * N * HA * 4);
   PL_ALLOC(p->row_ret, S * P * Nl * 4);
   PL_ALLOC(p->row_csum, S * P * Nl * 4);
-  PL_ALLOC(p->row_cmask, S * P * Nl * 8);
+  PL_ALLOC(p->row_cmask, (size_t)cmask_planes(cfg->horizon) * S * P * Nl * 8);   // planes [W, S, P, N_local]
   PL_ALLOC(p->pairs_local, S * Nl * 8);
   PL_ALLOC(p->pairs_all, W * S * Nl * 8);
   PL_ALLOC(p->mu, S * HA * 4);
@@ -673,7 +683,7 @@ extern "C" int simba_planner_buffer(simba_planner_t* p, int32_t which, void** ou
   switch (which) {
     case SIMBA_BUF_ACTIONS: *out_ptr = p->actions; *out_bytes = S * N * HA * 4; break;
     case SIMBA_BUF_ROW_RETURN: *out_ptr = p->row_ret; *out_bytes = S * P * Nl * 4; break;
-    case SIMBA_BUF_ROW_COSTMASK: *out_ptr = p->row_cmask; *out_bytes = S * P * Nl * 8; break;
+    case SIMBA_BUF_ROW_COSTMASK: *out_ptr = p->row_cmask; *out_bytes = (uint64_t)cmask_planes(c.horizon) * S * P * Nl * 8; break;
     case SIMBA_BUF_ROW_COSTSUM: *out_ptr = p->row_csum; *out_bytes = S * P * Nl * 4; break;
     case SIMBA_BUF_PAIRS_LOCAL: *out_ptr = p->pairs_local; *out_bytes = S * Nl * 8; break;
     case SIMBA_BUF_PAIRS_ALL: *out_ptr = p->pairs_all; *out_bytes = W * S * Nl * 8; break;

@@ -132,12 +132,52 @@ cudaError_t launch_sample_actions(const SampleParams& p, cudaStream_t st) {
 // One thread per (state, local candidate); loads are coalesced across candidates for each
 // particle. Per-step counts use bit-sliced (carry-save) counters over the 64-bit cost masks, so
 // the H x P popcount costs ~3 logic ops per particle and plane. Summation order over particles
-// is fixed (p ascending) => bit-identical on every rank.
+// is fixed (p ascending) => bit-identical on every rank. Horizons beyond 64 steps run the
+// counters once more per further 64-step plane of the masks (cmask_planes).
 // =============================================================================================
-// rows of candidate i: element base + q * stride of each array, q = 0 .. P - 1
+// counter bits b = 0..7 of 64 steps: add one particle's mask word
+__device__ __forceinline__ void bitsliced_add(uint64_t (&plane)[8], uint64_t carry) {
+#pragma unroll
+  for (int b = 0; b < 8; ++b) {
+    const uint64_t t = plane[b] & carry;
+    plane[b] ^= carry;
+    carry = t;
+  }
+}
+// the largest count among the first `steps` (>= 1) steps of the counters
+__device__ __forceinline__ int bitsliced_max(const uint64_t (&plane)[8], int steps) {
+  uint64_t cand = (steps >= 64) ? ~0ull : ((1ull << steps) - 1ull);
+  int maxc = 0;
+#pragma unroll
+  for (int b = 7; b >= 0; --b) {
+    const uint64_t m = cand & plane[b];
+    if (m) { cand = m; maxc |= (1 << b); }
+  }
+  return maxc;
+}
+
+// H > 64: the largest per-step count of planes 1 .. W - 1 (steps [64, H)). Not inlined: the callers' H <= 64 code
+// stays as it was, and the fused update kernel, bound by the latency of its serial path, does not grow.
+__device__ __noinline__ int later_planes_max(const uint64_t* row_costmask, long base, int stride, int P, int H,
+                                             long plane_stride) {
+  int maxc = 0;
+  for (int w = 1; w < cmask_planes(H); ++w) {          // steps [64 w, 64 w + 64)
+    uint64_t plane[8];
+#pragma unroll
+    for (int b = 0; b < 8; ++b) plane[b] = 0ull;
+    const uint64_t* mw = row_costmask + w * plane_stride;
+#pragma unroll 4
+    for (int q = 0; q < P; ++q) bitsliced_add(plane, mw[base + (long)q * stride]);
+    maxc = max(maxc, bitsliced_max(plane, H - 64 * w));
+  }
+  return maxc;
+}
+
+// rows of candidate i: element base + q * stride of each array, q = 0 .. P - 1; mask plane w at
+// row_costmask + w * plane_stride
 __device__ __forceinline__ float2 reduce_rows(const float* row_return, const uint64_t* row_costmask,
                                               const float* row_costsum, long base, int stride, int P, int H,
-                                              int objective) {
+                                              long plane_stride, int objective) {
   float ret = 0.0f, csum = 0.0f;
   uint64_t plane[8];
 #pragma unroll
@@ -147,26 +187,15 @@ __device__ __forceinline__ float2 reduce_rows(const float* row_return, const uin
     const long r = base + (long)q * stride;
     ret = __fadd_rn(ret, row_return[r]);
     csum = __fadd_rn(csum, row_costsum[r]);
-    uint64_t carry = row_costmask[r];
-#pragma unroll
-    for (int b = 0; b < 8; ++b) {
-      const uint64_t t = plane[b] & carry;
-      plane[b] ^= carry;
-      carry = t;
-    }
+    bitsliced_add(plane, row_costmask[r]);
   }
   const float mean_ret = __fdiv_rn(ret, (float)P);
   float cost = 0.0f;
   if (objective == SIMBA_OBJ_LEAST_COST) {
     cost = __fdiv_rn(csum, (float)P);
   } else if (objective != SIMBA_OBJ_REWARD) {
-    uint64_t cand = (H >= 64) ? ~0ull : ((1ull << H) - 1ull);
-    int maxc = 0;
-#pragma unroll
-    for (int b = 7; b >= 0; --b) {
-      const uint64_t m = cand & plane[b];
-      if (m) { cand = m; maxc |= (1 << b); }
-    }
+    int maxc = bitsliced_max(plane, H);
+    if (H > 64) maxc = max(maxc, later_planes_max(row_costmask, base, stride, P, H, plane_stride));
     cost = (float)maxc;
   }
   return make_float2(mean_ret, cost);
@@ -174,7 +203,7 @@ __device__ __forceinline__ float2 reduce_rows(const float* row_return, const uin
 
 __device__ __forceinline__ float2 reduce_candidate(const ReduceParams& p, int s, int i) {
   return reduce_rows(p.row_return, p.row_costmask, p.row_costsum, (long)s * p.P * p.N_local + i, p.N_local, p.P, p.H,
-                     p.objective);
+                     (long)p.S * p.P * p.N_local, p.objective);
 }
 
 __global__ void __launch_bounds__(256) score_reduce_kernel(ReduceParams p) {
@@ -993,10 +1022,10 @@ cudaError_t launch_finalize(const FinalizeParams& p, cudaStream_t st) {
 #define UTL(k) do { } while (0)
 #endif
 // Particles gq, gq + G, ... of candidate i: per-step counts of set mask bits in byte lanes, W words of four
-// steps each (fully unrolled), added to the candidate's shared counters
+// steps each (fully unrolled), added to the candidate's shared counters cnt_sm[i * ld + w], w < W4
 template <int W>
 __device__ __forceinline__ void count_steps(const unsigned long long* st_mask, uint32_t* cnt_sm, int i, int gq, int G,
-                                            int P, int N, int W4) {
+                                            int P, int N, int W4, int ld) {
   uint32_t acc[W];
 #pragma unroll
   for (int w = 0; w < W; ++w) acc[w] = 0u;
@@ -1009,16 +1038,19 @@ __device__ __forceinline__ void count_steps(const unsigned long long* st_mask, u
   }
 #pragma unroll
   for (int w = 0; w < W; ++w)
-    if (w < W4 && acc[w] != 0u) atomicAdd(&cnt_sm[i * W4 + w], acc[w]);
+    if (w < W4 && acc[w] != 0u) atomicAdd(&cnt_sm[i * ld + w], acc[w]);
 }
 
 // Shared-memory staging of the fused update kernel (u.stage != 0), behind the elite list, 16-byte aligned:
-//   [rows] u64 cost masks, [rows] returns, [rows] cost sums   (rows = P * N: the rollout's per-row outputs)
-//   [N * HA] this state's current actions, [N * JB * 4] the next iteration's N(0,1) draws,
-//   [N] per-candidate maximum step count, [N] per-candidate rank
-__host__ __device__ inline size_t update_stage_bytes(int P, int N, int HA) {
+//   [W][rows] u64 cost-mask planes, [rows] returns, [rows] cost sums   (rows = P * N: the rollout's per-row
+//   outputs, W = cmask_planes(H)), [N * HA] this state's current actions, [N * JB * 4] the next iteration's
+//   N(0,1) draws, [N] per-candidate maximum step count, [N] per-candidate rank, the per-element action bounds,
+//   [N][max(16, ceil(H / 4))] per-step particle counters
+__host__ __device__ inline size_t update_stage_bytes(int P, int N, int H, int HA) {
   const size_t rows = (size_t)P * N, JB = (size_t)(HA + 3) / 4;
-  return rows * 16 + (size_t)N * HA * 4 + (size_t)N * JB * 16 + (size_t)N * 8 + (size_t)(HA + 4) * 8 + (size_t)N * 64 + 96;
+  const size_t W = (size_t)cmask_planes(H), W4 = (size_t)(H + 3) / 4;
+  return rows * (8 * W + 8) + (size_t)N * HA * 4 + (size_t)N * JB * 16 + (size_t)N * 8 + (size_t)(HA + 4) * 8 +
+         (size_t)N * 4 * (W4 > 16 ? W4 : 16) + 96;
 }
 
 // STAGED is a template parameter so that the kernel a single plan runs carries none of the fallback code
@@ -1052,10 +1084,11 @@ __global__ void __launch_bounds__(kRefitThreads) cem_update_kernel(UpdateParams 
   const int P = u.reduce.P;
   const int rows = P * N;
   const int JB = (HA + 3) >> 2;
+  const int n_planes = cmask_planes(u.reduce.H);                        // 64-step planes of the cost masks
   const int o_keys = (groups + 2) * HA + ((groups + 2) * HA & 1);       // float index, 8-byte aligned
   const int o_elite = o_keys + 2 * N;
   const int o_mask = (o_elite + K + 3) & ~3;                            // 16-byte aligned from here on
-  const int o_ret = o_mask + 2 * rows;
+  const int o_ret = o_mask + 2 * rows * n_planes;
   const int o_csum = o_ret + rows;
   const int o_act = (o_csum + rows + 3) & ~3;
   const int o_z = (o_act + N * HA + 3) & ~3;
@@ -1167,6 +1200,14 @@ __global__ void __launch_bounds__(kRefitThreads) cem_update_kernel(UpdateParams 
         if (idx < n_act) act_sm[idx] = av[q];
       }
     }
+    if (n_planes > 1) {
+      // H > 64: the later planes of the cost masks (global plane stride S * rows: one rank, N_local = N)
+#pragma unroll 1
+      for (int idx = tid; idx < (n_planes - 1) * rows; idx += kRefitThreads) {
+        const int w = 1 + idx / rows, r = idx - (w - 1) * rows;
+        st_mask[w * rows + r] = gmask[(long)w * u.reduce.S * rows + r];
+      }
+    }
   }
   __syncthreads();                                    // staged; everyone has read active[s] before refit clears it
   UTL(8);
@@ -1177,19 +1218,23 @@ __global__ void __launch_bounds__(kRefitThreads) cem_update_kernel(UpdateParams 
     unsigned long long key = 0ull;
     const int objective = u.reduce.objective;
     if (staged) {
-      const bool counts = objective != SIMBA_OBJ_LEAST_COST && objective != SIMBA_OBJ_REWARD && P < 256;
+      const bool counts = objective != SIMBA_OBJ_LEAST_COST && objective != SIMBA_OBJ_REWARD;
       if (counts) {
         // Number of particles whose done-masked cost bit is set, per step (safe_cem_mpc.py:110-120): every mask
         // is read once. Thread (i, gq) takes particles gq, gq + G, ... of candidate i and spreads each nibble
         // of the mask into four byte lanes (n * 0x00204081 & 0x01010101 puts bit k of n into byte k), so one
         // 32-bit add counts four steps; the G partial words per candidate are combined with shared-memory
-        // atomics (bytes cannot overflow: P < 256). Integer arithmetic: exact and order-free.
+        // atomics (bytes cannot overflow: P <= 255, checked at planner creation). Integer arithmetic: exact and
+        // order-free.
         const int G = u.chunks;
         const int gq = div_small(tid, N, inv_N), i = tid - gq * N;
         if (gq < G) {
-          if (W4 <= 4) count_steps<4>(st_mask, cnt_sm, i, gq, G, P, N, W4);        // H <= 16
-          else if (W4 <= 8) count_steps<8>(st_mask, cnt_sm, i, gq, G, P, N, W4);   // H <= 32
-          else count_steps<16>(st_mask, cnt_sm, i, gq, G, P, N, W4);
+          if (W4 <= 4) count_steps<4>(st_mask, cnt_sm, i, gq, G, P, N, W4, W4);        // H <= 16
+          else if (W4 <= 8) count_steps<8>(st_mask, cnt_sm, i, gq, G, P, N, W4, W4);   // H <= 32
+          else                                                                      // 64 steps per plane
+#pragma unroll 1
+            for (int w = 0; w < n_planes; ++w)
+              count_steps<16>(st_mask + w * rows, cnt_sm + 16 * w, i, gq, G, P, N, min(16, W4 - 16 * w), W4);
         }
       }
       float ret = 0.0f, csum = 0.0f;
@@ -1211,8 +1256,6 @@ __global__ void __launch_bounds__(kRefitThreads) cem_update_kernel(UpdateParams 
             mx = max(max(mx, c4 & 0xffu), max((c4 >> 8) & 0xffu, max((c4 >> 16) & 0xffu, c4 >> 24)));
           }
           cost = (float)mx;
-        } else if (objective != SIMBA_OBJ_REWARD) {
-          cost = reduce_rows(st_ret, reinterpret_cast<const uint64_t*>(st_mask), st_csum, tid, N, P, u.reduce.H, objective).y;
         }
         pr = make_float2(__fdiv_rn(ret, (float)P), cost);
       }
@@ -1331,21 +1374,28 @@ __global__ void __launch_bounds__(kRefitThreads) cem_update_kernel(UpdateParams 
   UTL(6);
 }
 
+size_t cem_update_smem_bytes(int P, int N, int K, int H, int A, bool* staged) {
+  const int HA = H * A;
+  const int groups = kRefitThreads / HA > 0 ? kRefitThreads / HA : 1;
+  size_t smem = (size_t)((groups + 2) * HA + 1) * sizeof(float);
+  smem = (smem + 7) / 8 * 8 + (size_t)N * 8 + (size_t)K * 4 + 16;
+  // the staging area (rows, actions, draws; see update_stage_bytes), when it fits
+  const size_t stage = update_stage_bytes(P, N, H, HA);
+  *staged = smem + stage + 1024 <= 200 * 1024 && N <= kRefitThreads;
+  return *staged ? smem + stage : smem;
+}
+
 cudaError_t launch_cem_update(const UpdateParams& u_in, cudaStream_t st) {
   UpdateParams u = u_in;
   const int HA = u.refit.H * u.refit.A;
-  const int groups = kRefitThreads / HA > 0 ? kRefitThreads / HA : 1;
-  u.refit.groups = groups;
+  u.refit.groups = kRefitThreads / HA > 0 ? kRefitThreads / HA : 1;
   u.chunks = kRefitThreads / u.select.N > 0 ? kRefitThreads / u.select.N : 1;
   u.per = (u.select.N + u.chunks - 1) / u.chunks;
   u.inv_N = 1.0f / (float)u.select.N;
   u.inv_JB = 1.0f / (float)((HA + 3) / 4);
-  size_t smem = (size_t)((groups + 2) * HA + 1) * sizeof(float);
-  smem = (smem + 7) / 8 * 8 + (size_t)u.select.N * 8 + (size_t)u.select.K * 4 + 16;
-  // the staging area (rows, actions, draws; see update_stage_bytes), when it fits
-  const size_t stage = update_stage_bytes(u.reduce.P, u.select.N, HA);
-  u.stage = (smem + stage + 1024 <= 200 * 1024 && u.select.N <= kRefitThreads) ? 1 : 0;
-  if (u.stage) smem += stage;
+  bool staged = false;
+  const size_t smem = cem_update_smem_bytes(u.reduce.P, u.select.N, u.select.K, u.refit.H, u.refit.A, &staged);
+  u.stage = staged ? 1 : 0;
   return launch_kernel(u.stage ? cem_update_kernel<true> : cem_update_kernel<false>, u.refit.S, kRefitThreads, smem, st,
                        1, u.pdl != 0, u);
 }
@@ -1494,9 +1544,13 @@ __global__ void score_traj_rows_kernel(simba_scorer_t sc, const float* traj, int
   for (int t = 0; t < H; ++t) {
     const float* nx = base + (long)(t + 1) * O;
     row_score_step(rs, sc, done_first, t, [&](int b) { return nx[b]; });
+    if (cmask_word_ends(t, H)) {                       // planes [W, rows]
+      row_costmask[(long)(t >> 6) * rows + r] = rs.cmask;
+      rs.cmask = 0ull;
+    }
   }
   row_return[r] = rs.cum;
-  row_costmask[r] = rs.cmask;
+  row_costmask[(long)((H - 1) >> 6) * rows + r] = rs.cmask;
   row_costsum[r] = rs.costsum;
 }
 

@@ -97,6 +97,10 @@ struct UpdateParams {                 // fused k8 + k9 + k10 (+ next k1 | k11): 
 };
 
 cudaError_t launch_cem_update(const UpdateParams& u, cudaStream_t st);
+// Dynamic shared memory of the fused update kernel at these sizes (P particles, N candidates, K elites, horizon H,
+// A action dims): the refit scratch and selection keys, plus the staging area of per-row outputs, actions and draws
+// when that fits under 200 KB (*staged)
+size_t cem_update_smem_bytes(int P, int N, int K, int H, int A, bool* staged);
 cudaError_t launch_plan_begin(const PlanInitParams& ip, const SampleParams& sp, cudaStream_t st);
 cudaError_t launch_sample_actions(const SampleParams& p, cudaStream_t st);
 cudaError_t launch_score_reduce(const ReduceParams& p, cudaStream_t st);

@@ -200,11 +200,22 @@ __device__ __forceinline__ float step_reward(const simba_scorer_t& c, float dist
 struct RowScore {
   float cum;        // cumulative masked reward
   float costsum;    // sum_t cost(s_t), no done mask (safe_cem_mpc.py:98-108)
-  uint64_t cmask;   // bit t = cost(s_t) * (1 - done) > 0
+  uint64_t cmask;   // the current word of the cost history: bit t & 63 = cost(s_t) * (1 - done) > 0
   float dist;       // goal distance of the current state s_t
   float cost;       // cost(s_t)
   bool done;
 };
+
+// A row's cost history is W = ceil(H / 64) 64-bit words, stored as planes [W, S, P, N_local] (plane stride
+// S * P * N_local rows): plane w holds steps [64 w, 64 w + 64), so with H <= 64 plane 0 is the whole history.
+__host__ __device__ __forceinline__ int cmask_planes(int H) { return (H + 63) >> 6; }
+// True after step t when the current word is complete and more steps follow: the caller stores it to plane
+// t >> 6 and starts a new word. The last word (plane W - 1) is stored after the last step, as with H <= 64,
+// where this is never true.
+__host__ __device__ __forceinline__ bool cmask_word_ends(int t, int H) { return (t & 63) == 63 && t + 1 < H; }
+__host__ __device__ __forceinline__ int64_t cmask_plane_stride(const RowGeom& g) {
+  return (int64_t)g.S * g.P * g.N_local;
+}
 
 template <class Load>
 __device__ __forceinline__ void row_score_init(RowScore& rs, const simba_scorer_t& c, Load ld) {
@@ -223,11 +234,11 @@ __device__ __forceinline__ void row_score_step(RowScore& rs, const simba_scorer_
   const float r = step_reward(c, rs.dist, next_dist, goal);
   if (done_first) {                                  // safe_cem_mpc.py:87-93
     rs.done = rs.done || goal;
-    if (!rs.done && rs.cost > 0.0f) rs.cmask |= (1ull << t);
+    if (!rs.done && rs.cost > 0.0f) rs.cmask |= (1ull << (t & 63));
     rs.cum = __fadd_rn(rs.cum, __fmul_rn(r, rs.done ? 0.0f : 1.0f));
   } else {                                           // mpc_policy.py:35-37
     rs.cum = __fadd_rn(rs.cum, __fmul_rn(r, rs.done ? 0.0f : 1.0f));
-    if (!rs.done && rs.cost > 0.0f) rs.cmask |= (1ull << t);
+    if (!rs.done && rs.cost > 0.0f) rs.cmask |= (1ull << (t & 63));
     rs.done = rs.done || goal;
   }
   rs.costsum = __fadd_rn(rs.costsum, rs.cost);

@@ -247,6 +247,10 @@ __global__ void __launch_bounds__(NT) rollout_f32_kernel(const RolloutParams prm
     if (my_valid) {
       const float* srow = state + tid * OS;
       row_score_step(rs, prm.scorer, done_first, t, [&](int b) { return srow[b]; });
+      if (cmask_word_ends(t, H)) {
+        if (prm.row_return != nullptr) prm.row_costmask[(t >> 6) * cmask_plane_stride(g) + my.out] = rs.cmask;
+        rs.cmask = 0ull;
+      }
     }
     if (prm.traj_out != nullptr) {
       for (int idx = tid; idx < TM * O; idx += NT) {
@@ -262,7 +266,7 @@ __global__ void __launch_bounds__(NT) rollout_f32_kernel(const RolloutParams prm
 
   if (my_valid && prm.row_return != nullptr) {
     prm.row_return[my.out] = rs.cum;
-    prm.row_costmask[my.out] = rs.cmask;
+    prm.row_costmask[((H - 1) >> 6) * cmask_plane_stride(g) + my.out] = rs.cmask;
     prm.row_costsum[my.out] = rs.costsum;
   }
 }

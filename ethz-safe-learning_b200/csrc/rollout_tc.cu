@@ -445,41 +445,56 @@ __device__ __forceinline__ void rollout_tc_body(const RolloutParams& prm) {
           my_rs[7 * 128 + 32 * i] = row < tis.count ? (uint32_t)decode_row(g, tis.member, tis.k0 + row).out : 0xffffffffu;
         }
         const bool live = late_gate(tis);
-        for (int ts = -1; live && ts < H; ++ts) {                          // ts = -1: distance / cost of s_0
-          named_bar_sync_n(kBarPart + j, tile_bar_threads);
-          const float* part_tile = part_tile0;
-          if (PAIR) {                                                      // + the peer CTA's slices of this step
-            mbar_wait(xbar + 8u * ((uint32_t)ts & 1u), (uint32_t)((ts + 1) >> 1) & 1u);
-            if (lane == 0 && ts + 2 < H) mbar_expect_tx(xbar + 8u * ((uint32_t)ts & 1u), xbytes(ts + 2));
-            part_tile += (ts & 1) * part_buf_floats;
-          }
+        // the steps of cost-history word w, then (H > 64, more steps follow) its store to plane w; ts = -1:
+        // distance / cost of s_0. The step loop is the same for every word.
+        for (int w = 0, ts = -1; live && ts < H; ++w) {
+          for (const int ts_end = min(H, 64 * w + 64); ts < ts_end; ++ts) {
+            named_bar_sync_n(kBarPart + j, tile_bar_threads);
+            const float* part_tile = part_tile0;
+            if (PAIR) {                                                      // + the peer CTA's slices of this step
+              mbar_wait(xbar + 8u * ((uint32_t)ts & 1u), (uint32_t)((ts + 1) >> 1) & 1u);
+              if (lane == 0 && ts + 2 < H) mbar_expect_tx(xbar + 8u * ((uint32_t)ts & 1u), xbytes(ts + 2));
+              part_tile += (ts & 1) * part_buf_floats;
+            }
 #pragma unroll 1
-          for (int i = 0; i < n_quarters; ++i) {
-            uint32_t* q = my_rs + 32 * i;
-            float nd, nc;
-            head_combine<NSL>(sc, part_tile + lane + 32 * i, nparts, nd, nc);
-            if (ts < 0) {
-              q[4 * 128] = __float_as_uint(nd);
-              q[5 * 128] = __float_as_uint(nc);
-            } else {
-              RowScore rs;
-              rs.cum = __uint_as_float(q[0]);
-              rs.costsum = __uint_as_float(q[128]);
-              rs.cmask = (uint64_t)q[2 * 128] | ((uint64_t)q[3 * 128] << 32);
-              rs.dist = __uint_as_float(q[4 * 128]);
-              rs.cost = __uint_as_float(q[5 * 128]);
-              rs.done = q[6 * 128] != 0u;
-              head_score_step(rs, sc, done_first, ts, nd, nc);
-              q[0] = __float_as_uint(rs.cum);
-              q[128] = __float_as_uint(rs.costsum);
-              q[2 * 128] = (uint32_t)rs.cmask;
-              q[3 * 128] = (uint32_t)(rs.cmask >> 32);
-              q[4 * 128] = __float_as_uint(rs.dist);
-              q[5 * 128] = __float_as_uint(rs.cost);
-              q[6 * 128] = rs.done ? 1u : 0u;
+            for (int i = 0; i < n_quarters; ++i) {
+              uint32_t* q = my_rs + 32 * i;
+              float nd, nc;
+              head_combine<NSL>(sc, part_tile + lane + 32 * i, nparts, nd, nc);
+              if (ts < 0) {
+                q[4 * 128] = __float_as_uint(nd);
+                q[5 * 128] = __float_as_uint(nc);
+              } else {
+                RowScore rs;
+                rs.cum = __uint_as_float(q[0]);
+                rs.costsum = __uint_as_float(q[128]);
+                rs.cmask = (uint64_t)q[2 * 128] | ((uint64_t)q[3 * 128] << 32);
+                rs.dist = __uint_as_float(q[4 * 128]);
+                rs.cost = __uint_as_float(q[5 * 128]);
+                rs.done = q[6 * 128] != 0u;
+                head_score_step(rs, sc, done_first, ts, nd, nc);
+                q[0] = __float_as_uint(rs.cum);
+                q[128] = __float_as_uint(rs.costsum);
+                q[2 * 128] = (uint32_t)rs.cmask;
+                q[3 * 128] = (uint32_t)(rs.cmask >> 32);
+                q[4 * 128] = __float_as_uint(rs.dist);
+                q[5 * 128] = __float_as_uint(rs.cost);
+                q[6 * 128] = rs.done ? 1u : 0u;
+              }
+            }
+            if (ts + 1 < H) named_bar_arrive_n(kBarFree + j, tile_bar_threads);
+          }
+          if (ts < H) {                                                    // word w is complete
+#pragma unroll 1
+            for (int i = 0; i < n_quarters; ++i) {
+              uint32_t* q = my_rs + 32 * i;
+              if (prm.row_return != nullptr && q[7 * 128] != 0xffffffffu)
+                prm.row_costmask[w * cmask_plane_stride(g) + q[7 * 128]] =
+                    (uint64_t)q[2 * 128] | ((uint64_t)q[3 * 128] << 32);
+              q[2 * 128] = 0u;
+              q[3 * 128] = 0u;
             }
           }
-          if (ts + 1 < H) named_bar_arrive_n(kBarFree + j, tile_bar_threads);
         }
         if (live && prm.row_return != nullptr) {
 #pragma unroll 1
@@ -488,7 +503,8 @@ __device__ __forceinline__ void rollout_tc_body(const RolloutParams& prm) {
             const uint32_t slot = q[7 * 128];
             if (slot != 0xffffffffu) {
               prm.row_return[slot] = __uint_as_float(q[0]);
-              prm.row_costmask[slot] = (uint64_t)q[2 * 128] | ((uint64_t)q[3 * 128] << 32);
+              prm.row_costmask[((H - 1) >> 6) * cmask_plane_stride(g) + slot] =
+                  (uint64_t)q[2 * 128] | ((uint64_t)q[3 * 128] << 32);
               prm.row_costsum[slot] = __uint_as_float(q[128]);
             }
           }

@@ -520,11 +520,17 @@ __device__ __forceinline__ void rollout_tc_wide_body(const RolloutParams& prm) {
           my_rs[640] = __float_as_uint(rs.cost);
           my_rs[768] = rs.done ? 1u : 0u;
         }
+        if (!TRAJ && cgp == 0 && cmask_word_ends(t, H)) {       // H > 64: word t >> 6 is complete
+          if (row_ok && prm.row_return != nullptr)
+            prm.row_costmask[(t >> 6) * cmask_plane_stride(g) + id.out] = (uint64_t)my_rs[256] | ((uint64_t)my_rs[384] << 32);
+          my_rs[256] = 0u;
+          my_rs[384] = 0u;
+        }
         TLW(43);
       }
       if (!TRAJ && cgp == 0 && row_ok && prm.row_return != nullptr) {
         prm.row_return[id.out] = __uint_as_float(my_rs[0]);
-        prm.row_costmask[id.out] = (uint64_t)my_rs[256] | ((uint64_t)my_rs[384] << 32);
+        prm.row_costmask[((H - 1) >> 6) * cmask_plane_stride(g) + id.out] = (uint64_t)my_rs[256] | ((uint64_t)my_rs[384] << 32);
         prm.row_costsum[id.out] = __uint_as_float(my_rs[128]);
       }
     }

@@ -446,11 +446,11 @@ __device__ __forceinline__ void head_score_step(RowScore& rs, const simba_scorer
   const float rew = step_reward(sc, rs.dist, next_dist, goal);
   if (done_first) {                                  // safe_cem_mpc.py:87-93
     rs.done = rs.done || goal;
-    if (!rs.done && rs.cost > 0.0f) rs.cmask |= (1ull << t);
+    if (!rs.done && rs.cost > 0.0f) rs.cmask |= (1ull << (t & 63));
     rs.cum += rs.done ? 0.0f : rew;
   } else {                                           // mpc_policy.py:35-37
     rs.cum += rs.done ? 0.0f : rew;
-    if (!rs.done && rs.cost > 0.0f) rs.cmask |= (1ull << t);
+    if (!rs.done && rs.cost > 0.0f) rs.cmask |= (1ull << (t & 63));
     rs.done = rs.done || goal;
   }
   rs.costsum += rs.cost;

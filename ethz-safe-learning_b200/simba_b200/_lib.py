@@ -10,7 +10,7 @@ import pathlib
 
 SIMBA_MAX_ACT = 16
 SIMBA_MAX_CONSTRAINTS = 4
-SIMBA_MAX_HORIZON = 64
+SIMBA_MAX_HORIZON = 1024   # and horizon * act_dim <= 1024
 
 OBJ_REWARD, OBJ_SAFE_PENALTY, OBJ_LEAST_COST, OBJ_FEASIBLE_FIRST = 0, 1, 2, 3
 PREC_FP32, PREC_BF16_TC = 0, 1

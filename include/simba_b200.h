@@ -31,7 +31,7 @@ extern "C" {
 
 #define SIMBA_MAX_ACT 16          /* action dims                                    */
 #define SIMBA_MAX_CONSTRAINTS 4   /* vases, hazards, pillars, gremlins (safety_gym.py:148-163) */
-#define SIMBA_MAX_HORIZON 64      /* per-row cost history is a 64-bit mask          */
+#define SIMBA_MAX_HORIZON 1024    /* and horizon * act_dim <= 1024                  */
 #define SIMBA_MAX_MEMBERS 64
 
 typedef enum simba_status {
@@ -155,14 +155,16 @@ int simba_sample_actions(simba_planner_t* p, const float* mu, const float* sigma
  * mlp_ensemble.py:122-132,189-193, safety_gym.py:110-166, the per-row part of
  * mpc_policy.py:26-37 / safe_cem_mpc.py:82-93. One launch per CEM iteration; trajectories
  * never reach HBM. states [S, O]; actions [S, N, H, A]; eps_or_null [S, H, P*N, O];
- * outputs per local row [S, P, N_local]: cumulative masked reward, bit t = cost(s_t)*(1-done_t)
- * (done order per objective), and the unmasked cost sum. DEVICE. */
+ * outputs per local row [S, P, N_local]: cumulative masked reward, the unmasked cost sum, and the cost
+ * history bit t = cost(s_t)*(1-done_t) (done order per objective) as W = ceil(H/64) 64-bit words in
+ * planes [W, S, P, N_local]: bit t & 63 of plane t >> 6 (W = 1 for H <= 64). DEVICE. */
 int simba_rollout_score(simba_planner_t* p, const float* states, const float* actions,
                         const float* eps_or_null, uint64_t seed, int32_t iteration,
                         const int32_t* active_or_null, float* out_row_return,
                         uint64_t* out_row_costmask, float* out_row_costsum, void* stream);
 
 /* k8  cross-particle reduction — mpc_policy.py:38-39, safe_cem_mpc.py:94-96,110-120,98-108.
+ * row_return, row_costsum [S, P, N_local]; row_costmask [W, S, P, N_local] as simba_rollout_score writes it.
  * -> per local candidate (return, cost) pairs [S, N_local, 2]: return = mean over particles;
  * cost = max_t count_t (SAFE_PENALTY / FEASIBLE_FIRST), mean cost sum (LEAST_COST), 0 (REWARD). */
 int simba_score_reduce(simba_planner_t* p, const float* row_return, const uint64_t* row_costmask,
