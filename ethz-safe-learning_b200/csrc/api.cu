@@ -57,6 +57,7 @@ struct simba_model {
   std::vector<char> layer_set;
   std::vector<float> smin, smax;
   int scale_on = 1;
+  int activation = SIMBA_ACT_RELU;
   bool scaler_set = false, committed = false;
   uint64_t generation = 0;     // bumped by every commit; planners re-capture their graph when it changes
   // device images
@@ -146,6 +147,19 @@ extern "C" int simba_model_get_layer(simba_model_t* m, int32_t member, int32_t l
 }
 
 const simba_model_config_t* simba::model_config(const simba_model_t* m) { return &m->cfg; }
+int simba::model_activation(const simba_model_t* m) { return m->activation; }
+
+// The activation is fixed before the first commit: planners and trainers built on the model keep the kernels they
+// chose, and a commit never re-selects them.
+extern "C" int simba_model_set_activation(simba_model_t* m, int32_t activation) {
+  if (!m) return set_error(SIMBA_ERR_BAD_CONFIG, "null argument");
+  if (activation != SIMBA_ACT_RELU && activation != SIMBA_ACT_SWISH)
+    return set_error(SIMBA_ERR_BAD_CONFIG, "activation %d unknown", activation);
+  if (m->generation > 0)
+    return set_error(SIMBA_ERR_BAD_CONFIG, "the activation is set before the model's first commit");
+  m->activation = activation;
+  return SIMBA_OK;
+}
 
 extern "C" int simba_model_set_scaler(simba_model_t* m, const float* mn, const float* mx,
                                       int32_t scale_features) {
@@ -260,6 +274,7 @@ static void fill_model_params(const simba_model* m, RolloutParams& prm) {
   prm.smin = m->d_smin;
   prm.sdelta = m->d_sdelta;
   prm.scale_on = m->scale_on;
+  prm.act = m->activation;
 }
 
 // ---------------------------------------------------------------------------------------------

@@ -144,6 +144,19 @@ __device__ __forceinline__ float softplus_tf(float x) {
   return log1pf(e);
 }
 
+// Hidden-layer activation (simba_model_set_activation), a compile-time parameter of the kernel bodies.
+constexpr int kActRelu = SIMBA_ACT_RELU, kActSwish = SIMBA_ACT_SWISH;
+
+// fp32 swish (tf.nn.swish) and its derivative, accurate libm expf and explicit round-to-nearest operations in the
+// order of the oracle's float32 numpy: sigmoid(z) = 1 / (1 + exp(-z)), swish(z) = z * sigmoid(z),
+// swish'(z) = sigmoid(z) * (1 + z * (1 - sigmoid(z)))
+__device__ __forceinline__ float sigmoid_f32(float z) { return __fdiv_rn(1.0f, __fadd_rn(1.0f, expf(-z))); }
+__device__ __forceinline__ float swish_f32(float z) { return __fmul_rn(z, sigmoid_f32(z)); }
+__device__ __forceinline__ float swish_grad_f32(float z) {
+  const float s = sigmoid_f32(z);
+  return __fmul_rn(s, __fadd_rn(1.0f, __fmul_rn(z, __fsub_rn(1.0f, s))));
+}
+
 // ---------------------------------------------------------------------------------------------
 // SafetyGymStateScorer pieces (simba/environment_utils/safety_gym.py:110-192). Arithmetic is
 // written with explicit round-to-nearest ops so nvcc cannot contract it into FMAs: the scoring

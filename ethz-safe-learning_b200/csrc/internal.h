@@ -11,6 +11,7 @@ namespace simba {
 // records the message behind simba_last_error() and returns `code`
 int set_error(int code, const char* fmt, ...) __attribute__((format(printf, 2, 3)));
 const simba_model_config_t* model_config(const simba_model_t* m);
+int model_activation(const simba_model_t* m);   // simba_activation of the hidden layers
 
 // Host side of the bf16 weight images. bf16_bits rounds to nearest even and keeps a NaN a (quiet) NaN.
 inline uint16_t bf16_bits(float f) {

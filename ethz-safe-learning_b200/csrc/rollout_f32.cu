@@ -42,7 +42,9 @@ __device__ __forceinline__ void cp_async_wait() {
 }
 }  // namespace
 
-__global__ void __launch_bounds__(NT) rollout_f32_kernel(const RolloutParams prm) {
+// ACT: the hidden layers' activation (kActRelu, kActSwish)
+template <int ACT>
+__device__ __forceinline__ void rollout_f32_body(const RolloutParams prm) {
   extern __shared__ float4 smem_f4[];
   float* smem = reinterpret_cast<float*>(smem_f4);
   const RowGeom& g = prm.g;
@@ -182,7 +184,7 @@ __global__ void __launch_bounds__(NT) rollout_f32_kernel(const RolloutParams prm
           }
           ++a;
         }
-        // epilogue: bias (+ ReLU for hidden layers, mlp_ensemble.py:19-20) -> out[n][row]
+        // epilogue: bias (+ the activation for hidden layers, mlp_ensemble.py:19-20) -> out[n][row]
 #pragma unroll
         for (int j = 0; j < 4; ++j) {
           const int n = nb + 4 * cg + j;
@@ -190,8 +192,13 @@ __global__ void __launch_bounds__(NT) rollout_f32_kernel(const RolloutParams prm
           float4 v;
           v.x = acc[0][j] + b; v.y = acc[1][j] + b; v.z = acc[2][j] + b; v.w = acc[3][j] + b;
           if (l < L) {
-            v.x = fmaxf(v.x, 0.0f); v.y = fmaxf(v.y, 0.0f);
-            v.z = fmaxf(v.z, 0.0f); v.w = fmaxf(v.w, 0.0f);
+            if constexpr (ACT == kActSwish) {
+              v.x = swish_f32(v.x); v.y = swish_f32(v.y);
+              v.z = swish_f32(v.z); v.w = swish_f32(v.w);
+            } else {
+              v.x = fmaxf(v.x, 0.0f); v.y = fmaxf(v.y, 0.0f);
+              v.z = fmaxf(v.z, 0.0f); v.w = fmaxf(v.w, 0.0f);
+            }
           }
           *reinterpret_cast<float4*>(out + n * TM + 4 * rg) = v;
         }
@@ -271,6 +278,11 @@ __global__ void __launch_bounds__(NT) rollout_f32_kernel(const RolloutParams prm
   }
 }
 
+__global__ void __launch_bounds__(NT) rollout_f32_kernel(const RolloutParams prm) { rollout_f32_body<kActRelu>(prm); }
+__global__ void __launch_bounds__(NT) rollout_swish_f32_kernel(const RolloutParams prm) {
+  rollout_f32_body<kActSwish>(prm);
+}
+
 static size_t f32_smem_bytes(int O, int A, int act_rows) {
   const int IN = O + A;
   const int OS = O | 1;
@@ -330,14 +342,14 @@ int rollout_f32_pack(const ModelWeights& mw, std::vector<float>& w, std::vector<
 
 cudaError_t launch_rollout_f32(const RolloutParams& prm, cudaStream_t stream) {
   const size_t smem = f32_smem_bytes(prm.g.O, prm.g.A, prm.act_rows);
+  void (*kern)(const RolloutParams) = prm.act == kActSwish ? rollout_swish_f32_kernel : rollout_f32_kernel;
   // set on every launch: the attribute is per device and per function, and launches happen only at
   // graph capture or in the non-graph entry points, never on the replayed hot path
   {
-    cudaError_t e = cudaFuncSetAttribute(rollout_f32_kernel,
-                                         cudaFuncAttributeMaxDynamicSharedMemorySize, (int)smem);
+    cudaError_t e = cudaFuncSetAttribute(kern, cudaFuncAttributeMaxDynamicSharedMemorySize, (int)smem);
     if (e != cudaSuccess) return e;
   }
-  rollout_f32_kernel<<<prm.n_tiles, NT, smem, stream>>>(prm);
+  kern<<<prm.n_tiles, NT, smem, stream>>>(prm);
   return cudaGetLastError();
 }
 

@@ -160,7 +160,10 @@ struct AStorePair {
 // the state, the Gaussian head's mu, var and (with external draws) sample of their valid rows to prm.mu_out,
 // var_out and sample_out [B, O] (tc_head.cuh ForwardSink). Its head pass always forms the variance; without draws
 // the noise stays zero.
-template <int NTILES, int Q, bool PAIR, bool TRAJ, bool FWD = false>
+//
+// ACT: the hidden layers' activation, applied where the drain packs the fp32 accumulator to bf16 (kActRelu:
+// cvt.rn.relu; kActSwish: swish_approx, tc_ptx.cuh).
+template <int NTILES, int Q, bool PAIR, bool TRAJ, bool FWD = false, int ACT = kActRelu>
 __device__ __forceinline__ void rollout_tc_body(const RolloutParams& prm) {
   static_assert(!PAIR || (NTILES == 1 && Q == 4), "the pair variant is the one-tile latency configuration");
   static_assert(!(PAIR && TRAJ), "the trajectory form has no pair variant");
@@ -828,7 +831,7 @@ __device__ __forceinline__ void rollout_tc_body(const RolloutParams& prm) {
             else head_store_actions(hc, act_pf);
           }
           prefetch_actions(t + 2);
-          // ---- hidden layers: TMEM accumulator (bias included) -> ReLU -> bf16 -> next A operand ------
+          // ---- hidden layers: TMEM accumulator (bias included) -> activation -> bf16 -> next A operand -
           for (int l = 0; l < L; ++l) {
             wait_accumulator();
             TL(1 + l * 4);
@@ -843,7 +846,7 @@ __device__ __forceinline__ void rollout_tc_body(const RolloutParams& prm) {
                 uint32_t pk[16];
 #pragma unroll
                 for (int q = 0; q < 16; ++q)
-                  pk[q] = pack_relu_bf16(__uint_as_float(v[i][2 * q]), __uint_as_float(v[i][2 * q + 1]));
+                  pk[q] = pack_act_bf16<ACT>(__uint_as_float(v[i][2 * q]), __uint_as_float(v[i][2 * q + 1]));
                 tmem_st<16>(t_a + (kDbl ? (gemm_par(t, l) ^ 1u) * 64 : 0u) + (uint32_t)((cgp * HCOLS + i * 32) / 2), pk);
               }
             }
@@ -945,6 +948,20 @@ __global__ void __launch_bounds__(kBoundThreads, 1) forward_tc_kernel(const Roll
   rollout_tc_body<NTILES, Q, false, true, true>(prm);
 }
 
+// the swish forms of the three above (kActSwish)
+template <int NTILES, int Q, bool PAIR>
+__global__ void __launch_bounds__(kBoundThreads, 1) rollout_swish_tc_kernel(const RolloutParams prm) {
+  rollout_tc_body<NTILES, Q, PAIR, false, false, kActSwish>(prm);
+}
+template <int NTILES, int Q>
+__global__ void __launch_bounds__(kBoundThreads, 1) unfold_swish_tc_kernel(const RolloutParams prm) {
+  rollout_tc_body<NTILES, Q, false, true, false, kActSwish>(prm);
+}
+template <int NTILES, int Q>
+__global__ void __launch_bounds__(kBoundThreads, 1) forward_swish_tc_kernel(const RolloutParams prm) {
+  rollout_tc_body<NTILES, Q, false, true, true, kActSwish>(prm);
+}
+
 // ---- host side ------------------------------------------------------------------------------------
 static size_t tc_smem_bytes(int L, int ntiles, int q, int nparts, bool pair = false) {
   size_t b = tc_member_bytes(L) + 4096;                            // weights, bias K-blocks + ones tile
@@ -1028,9 +1045,10 @@ bool rollout_tc_pair_fits(int L, int n_constraints) {
 
 template <int NTILES, int Q, bool PAIR, bool TRAJ, bool FWD = false>
 static cudaError_t launch_variant(const RolloutParams& prm, cudaStream_t stream) {
-  void (*kern)(const RolloutParams) = rollout_tc_kernel<NTILES, Q, PAIR>;
-  if constexpr (FWD) kern = forward_tc_kernel<NTILES, Q>;
-  else if constexpr (TRAJ) kern = unfold_tc_kernel<NTILES, Q>;
+  const bool swish = prm.act == kActSwish;
+  void (*kern)(const RolloutParams) = swish ? rollout_swish_tc_kernel<NTILES, Q, PAIR> : rollout_tc_kernel<NTILES, Q, PAIR>;
+  if constexpr (FWD) kern = swish ? forward_swish_tc_kernel<NTILES, Q> : forward_tc_kernel<NTILES, Q>;
+  else if constexpr (TRAJ) kern = swish ? unfold_swish_tc_kernel<NTILES, Q> : unfold_tc_kernel<NTILES, Q>;
   const size_t smem = tc_smem_bytes(prm.L, NTILES, Q, TRAJ ? 1 : 1 + prm.scorer.n_constraints, PAIR);
   const int n_items = (prm.n_tiles + NTILES - 1) / NTILES;
   const int sms = prm.n_sms;

@@ -138,7 +138,8 @@ struct TileInfoW {
 // FWD (simba_ensemble_forward_tc): the forward form, a TRAJ form at H = 1 that writes the Gaussian head's mu, var
 // and (with external draws) sample of its valid rows to prm.mu_out, var_out and sample_out [B, O] instead of the
 // state (tc_head.cuh ForwardSink). Its head pass always forms the variance; without draws the noise stays zero.
-template <int kSW, bool TRAJ, bool FWD = false>
+// ACT: the hidden layers' activation, applied where drain_chunks packs the accumulator to bf16 (rollout_tc.cu)
+template <int kSW, bool TRAJ, bool FWD = false, int ACT = kActRelu>
 __device__ __forceinline__ void rollout_tc_wide_body(const RolloutParams& prm) {
   static_assert(!FWD || TRAJ, "the forward form is a trajectory form");
   using C = WideCfg<kSW>;
@@ -443,7 +444,7 @@ __device__ __forceinline__ void rollout_tc_wide_body(const RolloutParams& prm) {
           else head_store_actions(hc, act_pf);
         }
         prefetch_actions(t + 2, owns_actions);
-        // ---- hidden layers: TMEM -> ReLU -> bf16 -> swizzled A tile (bias is in the accumulator) ----
+        // ---- hidden layers: TMEM -> activation -> bf16 -> swizzled A tile (bias is in the accumulator) ----
         for (int l = 0; l < L; ++l) {
           wait_accumulator();
           TLW(1 + l * 4);
@@ -458,10 +459,10 @@ __device__ __forceinline__ void rollout_tc_wide_body(const RolloutParams& prm) {
 #pragma unroll
               for (int u = 0; u < NC; ++u)
                 st_shared_v4(a_chunk(c + u),
-                             pack_relu_bf16(__uint_as_float(v[u * 8 + 0]), __uint_as_float(v[u * 8 + 1])),
-                             pack_relu_bf16(__uint_as_float(v[u * 8 + 2]), __uint_as_float(v[u * 8 + 3])),
-                             pack_relu_bf16(__uint_as_float(v[u * 8 + 4]), __uint_as_float(v[u * 8 + 5])),
-                             pack_relu_bf16(__uint_as_float(v[u * 8 + 6]), __uint_as_float(v[u * 8 + 7])));
+                             pack_act_bf16<ACT>(__uint_as_float(v[u * 8 + 0]), __uint_as_float(v[u * 8 + 1])),
+                             pack_act_bf16<ACT>(__uint_as_float(v[u * 8 + 2]), __uint_as_float(v[u * 8 + 3])),
+                             pack_act_bf16<ACT>(__uint_as_float(v[u * 8 + 4]), __uint_as_float(v[u * 8 + 5])),
+                             pack_act_bf16<ACT>(__uint_as_float(v[u * 8 + 6]), __uint_as_float(v[u * 8 + 7])));
             };
             int c = my_c0;
             for (; c + 4 <= my_c1; c += 4) drain_chunks(std::integral_constant<int, 4>{}, c);
@@ -558,6 +559,20 @@ __global__ void __launch_bounds__(kWideThreads, 1) forward_tc_wide_kernel(const 
   rollout_tc_wide_body<kSW, true, true>(prm);
 }
 
+// the swish forms of the three above (kActSwish)
+template <int kSW>
+__global__ void __launch_bounds__(kWideThreads, 1) rollout_swish_tc_wide_kernel(const RolloutParams prm) {
+  rollout_tc_wide_body<kSW, false, false, kActSwish>(prm);
+}
+template <int kSW>
+__global__ void __launch_bounds__(kWideThreads, 1) unfold_swish_tc_wide_kernel(const RolloutParams prm) {
+  rollout_tc_wide_body<kSW, true, false, kActSwish>(prm);
+}
+template <int kSW>
+__global__ void __launch_bounds__(kWideThreads, 1) forward_swish_tc_wide_kernel(const RolloutParams prm) {
+  rollout_tc_wide_body<kSW, true, true, kActSwish>(prm);
+}
+
 // ---- host side ------------------------------------------------------------------------------------
 template <int kSW>
 static size_t wide_smem_bytes(int L, int U, int nparts) {
@@ -652,9 +667,10 @@ template <int kSW, bool TRAJ, bool FWD = false>
 static cudaError_t launch_wide(const RolloutParams& model_prm, cudaStream_t stream) {
   RolloutParams prm = model_prm;
   prm.U = rollout_tc_wide_units(kSW, prm.U);                       // the kernel runs the zero-padded width
-  void (*kern)(const RolloutParams) = rollout_tc_wide_kernel<kSW>;
-  if constexpr (FWD) kern = forward_tc_wide_kernel<kSW>;
-  else if constexpr (TRAJ) kern = unfold_tc_wide_kernel<kSW>;
+  const bool swish = prm.act == kActSwish;
+  void (*kern)(const RolloutParams) = swish ? rollout_swish_tc_wide_kernel<kSW> : rollout_tc_wide_kernel<kSW>;
+  if constexpr (FWD) kern = swish ? forward_swish_tc_wide_kernel<kSW> : forward_tc_wide_kernel<kSW>;
+  else if constexpr (TRAJ) kern = swish ? unfold_swish_tc_wide_kernel<kSW> : unfold_tc_wide_kernel<kSW>;
   const size_t smem = wide_smem_bytes<kSW>(prm.L, prm.U, TRAJ ? 1 : 1 + prm.scorer.n_constraints);
   return launch_kernel(kern, prm.n_tiles, kWideThreads, smem, stream, 1, prm.pdl, prm);
 }

@@ -5,6 +5,8 @@
 
 #include <cstdint>
 
+#include "common.cuh"
+
 namespace simba {
 namespace {
 
@@ -149,6 +151,19 @@ __device__ __forceinline__ uint32_t pack_bf16(float a, float b) {
   uint32_t r;
   asm("cvt.rn.bf16x2.f32 %0, %1, %2;" : "=r"(r) : "f"(b), "f"(a));
   return r;
+}
+// swish(z) = z sigmoid(z) = h + h tanh(h) with h = z / 2: one MUFU op (tanh.approx.f32) per element
+__device__ __forceinline__ float swish_approx(float z) {
+  const float h = 0.5f * z;
+  float t;
+  asm("tanh.approx.f32 %0, %1;" : "=f"(t) : "f"(h));
+  return fmaf(h, t, h);
+}
+// act(a), act(b) -> packed bf16x2 (a in the low half), for the activation ACT (kActRelu, kActSwish)
+template <int ACT>
+__device__ __forceinline__ uint32_t pack_act_bf16(float a, float b) {
+  if constexpr (ACT == kActSwish) return pack_bf16(swish_approx(a), swish_approx(b));
+  else return pack_relu_bf16(a, b);
 }
 // packed fp32x2 add (FADD2): one issue slot for two bias adds
 __device__ __forceinline__ float2 add2(uint32_t lo, uint32_t hi, float2 b) {

@@ -42,6 +42,14 @@ struct TrainLayer {
   int64_t off;
 };
 
+// Swish training (SIMBA_ACT_SWISH): the backward pass cannot recover swish'(Z) from H, so the training forward pass
+// stores, per hidden layer, the multiplier M_l = keep * swish'(Z_l) of dZ_{l-1} = M_l * (dZ_l . theta_l^T). m[l],
+// 1 <= l <= L: [E][estride][N_{l-1}], the layout of dz[l - 1].
+struct SwishMult {
+  float* m[kMaxTrainLayers];
+  int64_t estride;                    // rows per member (batch)
+};
+
 // What the trainer handle (trainer.cu) owns, and the inputs of one call, in a form both precisions launch from. Each
 // launcher below translates it into its own kernels' arguments.
 struct TrainDesc {
@@ -67,6 +75,8 @@ struct TrainDesc {
   float* out_loss;
   float dropout_rate, dropout_scale;
   uint64_t dropout_seed;
+  int activation;                     // simba_activation of the hidden layers
+  SwishMult mult;                     // swish models only (else null)
 };
 
 // The host side of each precision: train_f32_* (trainer_f32.cu) and train_tc_* (trainer_tc.cu, bf16 tcgen05).
@@ -103,6 +113,10 @@ using simba::philox4x32_10;
 using simba::philox_key;
 using simba::softplus_tf;
 using simba::u01;
+using simba::SwishMult;
+using simba::kActSwish;
+using simba::swish_f32;
+using simba::swish_grad_f32;
 
 // A captured graph holds several consecutive steps: step i of the graph works at
 // (st->fit_step + i, st->iterations + i) and one single-thread kernel advances the counters at
@@ -140,7 +154,7 @@ __device__ float schedule_lr(const OptParams& o, int iterations) {
   return fmaxf(o.lr0 * (1.0f - epochs / (float)o.train_epochs), 0.0f);
 }
 
-// Dropout after every hidden ReLU in training (mlp_ensemble.py:17-22): keep = u01(philox) >= rate,
+// Dropout after every hidden activation in training (mlp_ensemble.py:17-22): keep = u01(philox) >= rate,
 // kept activations scaled by 1 / (1 - rate). One Philox block covers columns col .. col + 3 (col a
 // multiple of 4). Counter (column block, batch row, iteration, member | layer << 8 | stream 4 << 28),
 // key = dropout_seed — restated in oracle/philox.py.

@@ -148,6 +148,7 @@ extern "C" int simba_trainer_destroy(simba_trainer_t* t) {
   for (int l = 0; l <= t->L; ++l) {
     cudaFree(d.act[l]);
     cudaFree(d.dz[l]);
+    cudaFree(d.mult.m[l]);
   }
   cudaFree(d.partial); cudaFree(t->val_acc);
   cudaFree(t->state); cudaFree(t->desc);
@@ -232,6 +233,12 @@ extern "C" int simba_trainer_create(simba_model_t* model, const simba_trainer_co
   for (int l = 0; l <= t->L; ++l) {
     TRY_OR_FREE(cudaMalloc(&d.act[l], (size_t)E * R * d.layer[l].K * sizeof(float)));
     TRY_OR_FREE(cudaMalloc(&d.dz[l], (size_t)E * cfg->batch_size * d.layer[l].N * sizeof(float)));
+  }
+  d.activation = model_activation(model);
+  if (d.activation == SIMBA_ACT_SWISH) {             // the backward multipliers of the hidden layers
+    d.mult.estride = cfg->batch_size;
+    for (int l = 1; l <= t->L; ++l)
+      TRY_OR_FREE(cudaMalloc(&d.mult.m[l], (size_t)E * cfg->batch_size * d.layer[l].K * sizeof(float)));
   }
   d.tiles_cap = (int)((R + 3) / 4);                    // the smallest row tile of either chain kernel
   TRY_OR_FREE(cudaMalloc(&d.partial, (size_t)E * d.tiles_cap * 2 * sizeof(float)));

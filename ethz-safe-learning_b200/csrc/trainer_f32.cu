@@ -95,8 +95,8 @@ struct ChainPass {
   int kind;
   float* out;             // hidden: H_{l+1} [E][cap][n]; head: dZ_L [E][B][n]; backward: dZ_{l-1}
   int64_t out_estride;
-  const float* mask;      // backward: H_l [E][cap][n_dim of this pass]; > 0 <=> the unit was active
-  int64_t mask_estride;
+  const float* mask;      // backward: ReLU: H_l [E][cap][n_dim of this pass], > 0 <=> the unit was active;
+  int64_t mask_estride;   // swish: M_l [E][batch][n_dim], the multiplier of dZ (SwishMult)
 };
 
 struct ChainArgs {
@@ -188,10 +188,12 @@ __device__ __forceinline__ void issue_chunk(const ChainArgs& a, const ChunkCurso
 // FMA chains, and the operands of a k-group (4 weight float4s + kGroupRows broadcast activation
 // float4s) sit in registers ahead of their use. The partial tiles are added in a fixed order
 // through shared memory when the layer's last chunk is done.
-template <int kRows>
-__global__ void __launch_bounds__(kChainThreads)
-train_chain_kernel(ChainArgs a, OptParams opt, const FitDesc* desc, TrainState* st, int rows_fixed,
-                   int step_off) {
+//
+// ACT = kActSwish: a hidden pass applies swish and, in training, stores M = keep * swish'(Z) to mult.m[l + 1];
+// a backward pass multiplies by M, read through p.mask. ReLU (kActRelu) ignores `mult`.
+template <int kRows, int ACT>
+__device__ __forceinline__ void train_chain_body(const ChainArgs& a, const OptParams& opt, const FitDesc* desc,
+                                                 TrainState* st, int rows_fixed, int step_off, const SwishMult& mult) {
   constexpr int kRowGroups = chain_row_groups(kRows);   // the 8 warps: kRowGroups row groups x kSplitK k-slices
   constexpr int kSplitK = kChainWarps / kRowGroups;
   constexpr int kGroupRows = kRows / kRowGroups;
@@ -366,11 +368,32 @@ train_chain_kernel(ChainArgs a, OptParams opt, const FitDesc* desc, TrainState* 
                 back = a.dropout_scale;       // H > 0 <=> unit active AND kept (H is stored after dropout)
               }
             }
+            if constexpr (ACT == kActSwish) {
+              float mv[4];                                       // M = keep * swish'(Z); dropout is folded in
 #pragma unroll
-            for (int j = 0; j < 4; ++j) {
-              const bool ok = c0 + j < p.n_dim;
-              if (p.kind == kPassHidden) v[j] = ok ? fmaxf(v[j] + pb[j], 0.0f) * keep[j] : 0.0f;
-              else v[j] = (ok && row_ok && pm[i][j] > 0.0f) ? v[j] * back : 0.0f;
+              for (int j = 0; j < 4; ++j) {
+                const bool ok = c0 + j < p.n_dim;
+                if (p.kind == kPassHidden) {
+                  const float z = v[j] + pb[j];
+                  v[j] = ok ? swish_f32(z) * keep[j] : 0.0f;
+                  mv[j] = ok ? keep[j] * swish_grad_f32(z) : 0.0f;
+                } else {
+                  v[j] = (ok && row_ok) ? v[j] * pm[i][j] : 0.0f;
+                }
+              }
+              if (p.kind == kPassHidden && a.train && row_ok) {
+                float* mo = mult.m[cur.pass + 1] + e * mult.estride * p.n_dim + (int64_t)r * p.n_dim + c0;
+#pragma unroll
+                for (int j = 0; j < 4; ++j)
+                  if (c0 + j < p.n_dim) mo[j] = mv[j];
+              }
+            } else {
+#pragma unroll
+              for (int j = 0; j < 4; ++j) {
+                const bool ok = c0 + j < p.n_dim;
+                if (p.kind == kPassHidden) v[j] = ok ? fmaxf(v[j] + pb[j], 0.0f) * keep[j] : 0.0f;
+                else v[j] = (ok && row_ok && pm[i][j] > 0.0f) ? v[j] * back : 0.0f;
+              }
             }
           }
           // columns past n_dim are written as zeros so that the next pass can consume k in groups of 4
@@ -444,6 +467,20 @@ train_chain_kernel(ChainArgs a, OptParams opt, const FitDesc* desc, TrainState* 
   if (a.out_loss) *a.out_loss = loss;
   if (desc != nullptr && desc->losses != nullptr) desc->losses[st->fit_step + step_off] = loss;
   st->nll_ticket = 0;
+}
+
+template <int kRows>
+__global__ void __launch_bounds__(kChainThreads)
+train_chain_kernel(ChainArgs a, OptParams opt, const FitDesc* desc, TrainState* st, int rows_fixed,
+                   int step_off) {
+  train_chain_body<kRows, simba::kActRelu>(a, opt, desc, st, rows_fixed, step_off, SwishMult{});
+}
+
+template <int kRows>
+__global__ void __launch_bounds__(kChainThreads)
+train_swish_chain_kernel(ChainArgs a, OptParams opt, const FitDesc* desc, TrainState* st, int rows_fixed,
+                         int step_off, SwishMult mult) {
+  train_chain_body<kRows, kActSwish>(a, opt, desc, st, rows_fixed, step_off, mult);
 }
 
 // ---------------------------------------------------------------------------------------------
@@ -639,7 +676,11 @@ cudaError_t train_f32_chain(const TrainDesc& d, const OptParams& opt, const FitD
       p.k_dim = ly.N; p.n_dim = ly.K;
       p.kind = kPassBackward;
       p.out = d.dz[l - 1]; p.out_estride = d.dz_estride * ly.K;      // K_l == N_{l-1}
-      p.mask = d.act[l]; p.mask_estride = d.act_estride * ly.K;
+      if (d.activation == kActSwish) {
+        p.mask = d.mult.m[l]; p.mask_estride = d.mult.estride * ly.K;
+      } else {
+        p.mask = d.act[l]; p.mask_estride = d.act_estride * ly.K;
+      }
     }
   a.n_pass = np;
   a.x = d.x; a.x_estride = d.x_estride; a.gather = d.gather;
@@ -654,12 +695,21 @@ cudaError_t train_f32_chain(const TrainDesc& d, const OptParams& opt, const FitD
   a.partial = d.partial; a.tiles_cap = d.tiles_cap; a.train = d.train; a.out_loss = d.out_loss;
   a.dropout_rate = d.dropout_rate; a.dropout_scale = d.dropout_scale; a.dropout_seed = d.dropout_seed;
   const int TR = chain_tile_rows(d.ensemble, grid_rows);
-  auto kernel = TR == 4 ? train_chain_kernel<4> : TR == 8 ? train_chain_kernel<8> : train_chain_kernel<16>;
   const size_t smem = chain_smem_bytes(TR, a.ld_act);
+  row_tiles = (grid_rows + TR - 1) / TR;
+  const dim3 grid(row_tiles, d.ensemble);
+  if (d.activation == kActSwish) {
+    auto kernel = TR == 4 ? train_swish_chain_kernel<4> : TR == 8 ? train_swish_chain_kernel<8>
+                                                                    : train_swish_chain_kernel<16>;
+    const cudaError_t err = cudaFuncSetAttribute(kernel, cudaFuncAttributeMaxDynamicSharedMemorySize, (int)smem);
+    if (err != cudaSuccess) return err;
+    kernel<<<grid, kChainThreads, smem, s>>>(a, opt, desc, st, rows_fixed, step_off, d.mult);
+    return cudaGetLastError();
+  }
+  auto kernel = TR == 4 ? train_chain_kernel<4> : TR == 8 ? train_chain_kernel<8> : train_chain_kernel<16>;
   const cudaError_t err = cudaFuncSetAttribute(kernel, cudaFuncAttributeMaxDynamicSharedMemorySize, (int)smem);
   if (err != cudaSuccess) return err;
-  row_tiles = (grid_rows + TR - 1) / TR;
-  kernel<<<dim3(row_tiles, d.ensemble), kChainThreads, smem, s>>>(a, opt, desc, st, rows_fixed, step_off);
+  kernel<<<grid, kChainThreads, smem, s>>>(a, opt, desc, st, rows_fixed, step_off);
   return cudaGetLastError();
 }
 

@@ -151,10 +151,13 @@ __device__ __forceinline__ void store_a8(uint32_t a_base, int kg, int r, const f
 namespace simba {
 namespace {
 
-__global__ void __launch_bounds__(kThreads, 1)
-train_tc_chain_kernel(const TcChainArgs a, const OptParams opt, const FitDesc* desc, TrainState* st,
-                      int rows_fixed, int step_off, int n_pass, uint32_t stage_bytes, uint32_t a_bytes,
-                      uint32_t tmem_cols) {
+// ACT = kActSwish: the hidden epilogue applies swish and, in training, stores M = keep * swish'(Z) to mult.m[l + 1];
+// back-propagation multiplies by M. ReLU (kActRelu) ignores `mult`.
+template <int ACT>
+__device__ __forceinline__ void train_tc_chain_body(const TcChainArgs& a, const OptParams& opt, const FitDesc* desc,
+                                                    TrainState* st, int rows_fixed, int step_off, int n_pass,
+                                                    uint32_t stage_bytes, uint32_t a_bytes, uint32_t tmem_cols,
+                                                    const SwishMult& mult) {
   extern __shared__ __align__(1024) uint8_t smem[];
   __shared__ __align__(8) uint64_t bars[5];      // full[2], empty[2], accumulator
   __shared__ uint32_t tmem_slot;
@@ -259,7 +262,7 @@ train_tc_chain_kernel(const TcChainArgs a, const OptParams opt, const FitDesc* d
 
       const TcLayer& ly = a.layer[pg.layer];
       if (pg.kind == 0) {
-        // ---- hidden layer: relu, dropout, H_{l+1} out, bf16 A tile (ones at N, N + 1) ----
+        // ---- hidden layer: activation, dropout, H_{l+1} out, bf16 A tile (ones at N, N + 1) ----
         const int N = ly.N, kp_next = r16(N + 2);
         float* hout = a.act[pg.layer + 1] + ((int64_t)e * a.act_estride + rg) * N;
         for (int c0 = 0; c0 < kp_next; c0 += 16) {
@@ -269,8 +272,18 @@ train_tc_chain_kernel(const TcChainArgs a, const OptParams opt, const FitDesc* d
             tmem_ld_wait();
           }
           float h[16];
+          [[maybe_unused]] float gm[16];                // swish: M = keep * swish'(Z)
+          if constexpr (ACT == kActSwish) {
 #pragma unroll
-          for (int j = 0; j < 16; ++j) h[j] = (c0 + j < N) ? fmaxf(__uint_as_float(v[j]), 0.0f) : 0.0f;
+            for (int j = 0; j < 16; ++j) {
+              const float z = __uint_as_float(v[j]);
+              h[j] = (c0 + j < N) ? swish_f32(z) : 0.0f;
+              gm[j] = (c0 + j < N) ? swish_grad_f32(z) : 0.0f;
+            }
+          } else {
+#pragma unroll
+            for (int j = 0; j < 16; ++j) h[j] = (c0 + j < N) ? fmaxf(__uint_as_float(v[j]), 0.0f) : 0.0f;
+          }
           if (dropout) {
 #pragma unroll
             for (int q = 0; q < 4; ++q) {
@@ -279,13 +292,22 @@ train_tc_chain_kernel(const TcChainArgs a, const OptParams opt, const FitDesc* d
               dropout_keep4(c0 + 4 * q, rg, iteration, e, pg.layer, a.dropout_rate, a.dropout_scale,
                             a.dropout_seed, keep);
 #pragma unroll
-              for (int i = 0; i < 4; ++i) h[4 * q + i] *= keep[i];
+              for (int i = 0; i < 4; ++i) {
+                h[4 * q + i] *= keep[i];
+                if constexpr (ACT == kActSwish) gm[4 * q + i] = keep[i] * gm[4 * q + i];
+              }
             }
           }
           if (a.train && row_ok) {
 #pragma unroll
             for (int j = 0; j < 16; ++j)
               if (c0 + j < N) hout[c0 + j] = h[j];
+            if constexpr (ACT == kActSwish) {
+              float* mout = mult.m[pg.layer + 1] + ((int64_t)e * mult.estride + rg) * N;
+#pragma unroll
+              for (int j = 0; j < 16; ++j)
+                if (c0 + j < N) mout[c0 + j] = gm[j];
+            }
           }
 #pragma unroll
           for (int j = 0; j < 16; ++j)
@@ -325,10 +347,11 @@ train_tc_chain_kernel(const TcChainArgs a, const OptParams opt, const FitDesc* d
           }
         }
       } else {
-        // ---- back-propagation through layer l >= 1: dZ_{l-1} = relu'(H_l) * (dZ_l . theta_l^T) ----
+        // ---- back-propagation through layer l >= 1: dZ_{l-1} = relu'(H_l) * (dZ_l . theta_l^T) (swish: M_l * ..) --
         const int K = ly.K, l = pg.layer;
         const float back = dropout ? a.dropout_scale : 1.0f;  // H > 0 <=> active AND kept (stored after dropout)
-        const float* hm = a.act[l] + ((int64_t)e * a.act_estride + rg) * K;
+        const float* hm = ACT == kActSwish ? mult.m[l] + ((int64_t)e * mult.estride + rg) * K
+                                           : a.act[l] + ((int64_t)e * a.act_estride + rg) * K;
         float* dzo = a.dz[l - 1] + ((int64_t)e * a.dz_estride + rg) * K;
         for (int c0 = 0; c0 < pg.np; c0 += 16) {
           uint32_t v[16];
@@ -338,7 +361,8 @@ train_tc_chain_kernel(const TcChainArgs a, const OptParams opt, const FitDesc* d
 #pragma unroll
           for (int j = 0; j < 16; ++j) {
             const int k = c0 + j;
-            d[j] = (k < K && row_ok && hm[k] > 0.0f) ? __uint_as_float(v[j]) * back : 0.0f;
+            if constexpr (ACT == kActSwish) d[j] = (k < K && row_ok) ? __uint_as_float(v[j]) * hm[k] : 0.0f;
+            else d[j] = (k < K && row_ok && hm[k] > 0.0f) ? __uint_as_float(v[j]) * back : 0.0f;
           }
           if (row_ok) {
 #pragma unroll
@@ -360,6 +384,23 @@ train_tc_chain_kernel(const TcChainArgs a, const OptParams opt, const FitDesc* d
   }
   finish_chain_loss(s_log, s_sq, scratch, last, a.partial, a.tiles_cap, (rows + kTcRows - 1) / kTcRows, rows,
                     a.out_dim, a.ensemble, a.train, a.out_loss, opt, desc, st, step_off);
+}
+
+__global__ void __launch_bounds__(kThreads, 1)
+train_tc_chain_kernel(const TcChainArgs a, const OptParams opt, const FitDesc* desc, TrainState* st,
+                      int rows_fixed, int step_off, int n_pass, uint32_t stage_bytes, uint32_t a_bytes,
+                      uint32_t tmem_cols) {
+  train_tc_chain_body<kActRelu>(a, opt, desc, st, rows_fixed, step_off, n_pass, stage_bytes, a_bytes, tmem_cols,
+                                SwishMult{});
+}
+
+// (not train_tc_swish_...: the name keeps the ReLU kernels' spill check to the two it names)
+__global__ void __launch_bounds__(kThreads, 1)
+train_swish_tc_chain_kernel(const TcChainArgs a, const OptParams opt, const FitDesc* desc, TrainState* st,
+                            int rows_fixed, int step_off, int n_pass, uint32_t stage_bytes, uint32_t a_bytes,
+                            uint32_t tmem_cols, const SwishMult mult) {
+  train_tc_chain_body<kActSwish>(a, opt, desc, st, rows_fixed, step_off, n_pass, stage_bytes, a_bytes, tmem_cols,
+                                 mult);
 }
 
 // dtheta tile [128 k] x [128 n] of one layer = [H, 1]^T . dZ over every batch row, then clip + Adam and the
@@ -638,12 +679,20 @@ cudaError_t train_tc_chain(const TrainDesc& d, const OptParams& opt, const FitDe
   uint32_t tmem_cols = 32;
   while ((int)tmem_cols < np_max) tmem_cols <<= 1;
   const size_t smem = smem_for_tmem((size_t)a_bytes + 2 * stage_bytes, tmem_cols);
-  cudaError_t err = cudaFuncSetAttribute(train_tc_chain_kernel, cudaFuncAttributeMaxDynamicSharedMemorySize,
-                                         (int)smem);
+  const bool swish = d.activation == kActSwish;
+  cudaError_t err = swish ? cudaFuncSetAttribute(train_swish_tc_chain_kernel,
+                                                 cudaFuncAttributeMaxDynamicSharedMemorySize, (int)smem)
+                          : cudaFuncSetAttribute(train_tc_chain_kernel, cudaFuncAttributeMaxDynamicSharedMemorySize,
+                                                 (int)smem);
   if (err != cudaSuccess) return err;
   row_tiles = (grid_rows + kTcRows - 1) / kTcRows;
-  train_tc_chain_kernel<<<dim3(row_tiles, a.ensemble), kThreads, smem, s>>>(a, opt, desc, st, rows_fixed, step_off,
-                                                                           n_pass, stage_bytes, a_bytes, tmem_cols);
+  const dim3 grid(row_tiles, a.ensemble);
+  if (swish)
+    train_swish_tc_chain_kernel<<<grid, kThreads, smem, s>>>(a, opt, desc, st, rows_fixed, step_off, n_pass,
+                                                             stage_bytes, a_bytes, tmem_cols, d.mult);
+  else
+    train_tc_chain_kernel<<<grid, kThreads, smem, s>>>(a, opt, desc, st, rows_fixed, step_off, n_pass, stage_bytes,
+                                                       a_bytes, tmem_cols);
   return cudaGetLastError();
 }
 

@@ -14,6 +14,7 @@ SIMBA_MAX_HORIZON = 1024   # and horizon * act_dim <= 1024
 
 OBJ_REWARD, OBJ_SAFE_PENALTY, OBJ_LEAST_COST, OBJ_FEASIBLE_FIRST = 0, 1, 2, 3
 PREC_FP32, PREC_BF16_TC = 0, 1
+ACT_RELU, ACT_SWISH = 0, 1
 MAP_SPLIT, MAP_PARTICLE = 0, 1
 (BUF_ACTIONS, BUF_ROW_RETURN, BUF_ROW_COSTMASK, BUF_ROW_COSTSUM, BUF_PAIRS_LOCAL, BUF_PAIRS_ALL,
  BUF_ELITE, BUF_MU, BUF_SIGMA, BUF_BEST_ACTION, BUF_BEST_SCORE, BUF_ACTIVE, BUF_SCORES) = range(13)
@@ -81,6 +82,7 @@ _SIGNATURES = {
     'simba_model_set_layer': [_vp, _i32, _i32, _vp, _vp],
     'simba_model_set_scaler': [_vp, _vp, _vp, _i32],
     'simba_model_commit': [_vp],
+    'simba_model_set_activation': [_vp, _i32],
     'simba_planner_create': [_vp, _P(PlannerConfig), _P(_vp)],
     'simba_planner_destroy': [_vp],
     'simba_planner_set_external_draws': [_vp, _vp, _vp, _vp],

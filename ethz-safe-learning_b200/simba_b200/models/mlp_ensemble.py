@@ -48,6 +48,12 @@ class MemberWeights(object):
         return self.get_weights()
 
 
+# mlp_params['activation'] spellings -> simba_activation
+ACTIVATIONS = {'tf.nn.relu': _lib.ACT_RELU, 'relu': _lib.ACT_RELU,
+               'tf.nn.swish': _lib.ACT_SWISH, 'tf.nn.silu': _lib.ACT_SWISH, 'swish': _lib.ACT_SWISH,
+               'silu': _lib.ACT_SWISH}
+
+
 def glorot_uniform(rng, fan_in, fan_out):
     """Keras Dense default initialiser (mlp_ensemble.py:13, :28-30)."""
     limit = np.sqrt(6.0 / (fan_in + fan_out))
@@ -79,10 +85,12 @@ class MlpEnsemble(object):
         self.n_layers = int(mlp_params.get('n_layers', 4))
         self.units = int(mlp_params.get('units', 128))
         activation = mlp_params.get('activation', 'tf.nn.relu')
-        if activation not in ('tf.nn.relu', 'relu'):
-            raise _lib.SimbaError(-6, "only ReLU hidden activations are fused (got %r)" % (activation,))
+        if activation not in ACTIVATIONS:
+            raise _lib.SimbaError(-6, "only ReLU and swish hidden activations are fused (got %r)" % (activation,))
+        # the reference eval()s the string (mlp_ensemble.py:14): tf.nn.silu is tf.nn.swish
+        self.activation = ACTIVATIONS[activation]
         # inference runs with training=False, so dropout is the identity there; training_step applies
-        # it after every hidden ReLU (mlp_ensemble.py:17-22) with Philox masks keyed by dropout_seed
+        # it after every hidden activation (mlp_ensemble.py:17-22) with Philox masks keyed by dropout_seed
         self.dropout_rate = float(mlp_params.get('dropout_rate', 0.0))
         self.dropout_seed = int(seed)
         rng = np.random.default_rng(seed)
@@ -114,6 +122,7 @@ class MlpEnsemble(object):
             h = C.c_void_p()
             _lib.check(self._lib.simba_model_create(C.byref(cfg), C.byref(h)))
             self._handle = h
+            _lib.check(self._lib.simba_model_set_activation(h, self.activation))
             self._dirty = True
         if self._dirty:
             for e, member in enumerate(self.ensemble):

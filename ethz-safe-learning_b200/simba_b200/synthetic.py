@@ -109,17 +109,17 @@ def make_workload(cfg_name='c1', sensors=None, seed=0, mu_scale=0.05, var_bias=-
 
 def build_policy(c, objective='penalty', precision='bf16', member_map='split', threshold=0.15,
                  smoothing=0.0, stddev_threshold=0.0, noise_stddev=0.01, sampling_propagation=True,
-                 scorer_config=None, seed=0, n_states=None, rank=0, world_size=1):
+                 scorer_config=None, seed=0, n_states=None, rank=0, world_size=1, activation='tf.nn.relu'):
     """The reference's construction sequence (mbrl_agent.py:103-118) on the B200 classes:
     environment -> TransitionModel(MlpEnsemble) -> CemMpc / SafeCemMpc, with the workload's
-    weights and scaler statistics loaded."""
+    weights and scaler statistics loaded. `activation`: mlp_params['activation'] of the ensemble."""
     from .environment_utils import ScorerEnvironment
     from .models import TransitionModel
     from .policies import CemMpc, SafeCemMpc
     env = ScorerEnvironment(c['sensors'], scorer_config, action_low=[-1.0] * c['A'], action_high=[1.0] * c['A'])
     tm = TransitionModel('mlp_ensemble', env.observation_space, env.action_space, True,
                          sampling_propagation, ensemble_size=c['E'],
-                         mlp_params=dict(n_layers=c['L'], units=c['U'], activation='tf.nn.relu',
+                         mlp_params=dict(n_layers=c['L'], units=c['U'], activation=activation,
                                          dropout_rate=0.0))
     for e in range(c['E']):
         tm.model.ensemble[e].set_weights(c['weights'][e])

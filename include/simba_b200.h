@@ -59,6 +59,11 @@ typedef enum simba_precision {
   SIMBA_PREC_BF16_TC = 1         /* bf16 tcgen05 rollout, fp32 accumulate: separately stated tolerance */
 } simba_precision;
 
+typedef enum simba_activation {
+  SIMBA_ACT_RELU = 0,            /* tf.nn.relu after every hidden Dense layer (mlp_ensemble.py:17-22), the default */
+  SIMBA_ACT_SWISH = 1            /* tf.nn.swish: z * sigmoid(z)                                        */
+} simba_activation;
+
 typedef enum simba_member_map {
   SIMBA_MAP_SPLIT = 0,           /* tf.split: member(r) = r / (P*N/E), r = p*N + i (mlp_ensemble.py:123) */
   SIMBA_MAP_PARTICLE = 1         /* member(p) = floor(p*E/P); equals SPLIT whenever E divides P      */
@@ -90,6 +95,10 @@ int simba_model_set_scaler(simba_model_t* m, const float* inputs_min, const floa
                            int32_t scale_features);
 /* pack + upload the fp32 and bf16 weight images; must follow set_layer / set_scaler changes */
 int simba_model_commit(simba_model_t* m);
+/* the hidden layers' activation, simba_activation (SIMBA_ACT_RELU unless set). Planners, trainers and the
+ * unfold / forward calls of the model all apply it. Allowed only before the model's first
+ * simba_model_commit; after it, or for an unknown value, SIMBA_ERR_BAD_CONFIG. */
+int simba_model_set_activation(simba_model_t* m, int32_t activation);
 
 /* ---- reward / cost scorer: replaces SafetyGymStateScorer (simba/environment_utils/safety_gym.py
  *      :104-192, goal task) as a parameter struct ------------------------------------------- */
