@@ -466,6 +466,10 @@ struct simba_planner {
 
   bool use_pdl = false;        // programmatic dependent launch between rollout and fused update kernels
   bool fused_update = false;   // one rank, N <= 1024: reduce+select+refit(+next sample | finalize) in one kernel
+  int32_t update_rule = SIMBA_UPDATE_CEM;
+  float temperature = 0.0f;    // MPPI
+  bool captured = false;       // a plan's graph has been captured: the update rule is fixed
+  int smem_optin = 0;
   int c_max = -1;
   // workspace
   float *actions = nullptr, *row_ret = nullptr, *row_csum = nullptr, *pairs_local = nullptr,
@@ -556,6 +560,14 @@ extern "C" int simba_planner_destroy(simba_planner_t* p) {
   return SIMBA_OK;
 }
 
+// fused update kernel (one CTA per state) for a single rank's population of at most 1024 candidates whose update
+// needs `update_smem` bytes of shared memory; otherwise the separate kernels
+static void choose_update_path(simba_planner* p, size_t update_smem) {
+  p->fused_update = p->cfg.world_size == 1 && p->cfg.n_samples <= 1024 && update_smem <= (size_t)p->smem_optin &&
+                    getenv("SIMBA_B200_NO_FUSE") == nullptr;
+  p->use_pdl = p->fused_update && p->cfg.precision == SIMBA_PREC_BF16_TC && getenv("SIMBA_B200_NO_PDL") == nullptr;
+}
+
 extern "C" int simba_planner_create(simba_model_t* model, const simba_planner_config_t* cfg,
                                     simba_planner_t** out) {
   if (!model || !cfg || !out) return set_error(SIMBA_ERR_BAD_CONFIG, "null argument");
@@ -605,12 +617,11 @@ extern "C" int simba_planner_create(simba_model_t* model, const simba_planner_co
   int smem_optin = 0;
   ce = cudaDeviceGetAttribute(&smem_optin, cudaDevAttrMaxSharedMemoryPerBlockOptin, p->device);
   if (ce != cudaSuccess) { delete p; return set_error(SIMBA_ERR_CUDA, "shared memory size: %s", cudaGetErrorString(ce)); }
+  p->smem_optin = smem_optin;
   bool update_staged = false;
   const size_t update_smem = cem_update_smem_bytes(cfg->particles, cfg->n_samples, cfg->n_elite, cfg->horizon,
                                                    mc.act_dim, &update_staged);
-  p->fused_update = cfg->world_size == 1 && cfg->n_samples <= 1024 && update_smem <= (size_t)smem_optin &&
-                    getenv("SIMBA_B200_NO_FUSE") == nullptr;
-  p->use_pdl = p->fused_update && cfg->precision == SIMBA_PREC_BF16_TC && getenv("SIMBA_B200_NO_PDL") == nullptr;
+  choose_update_path(p, update_smem);
   p->c_max = beta_count_threshold(cfg->particles, cfg->posterior_mean_threshold, cfg->prior_mu,
                                   cfg->prior_sigma);
 
@@ -664,6 +675,33 @@ extern "C" int simba_planner_create(simba_model_t* model, const simba_planner_co
                      cudaGetErrorString(cudaGetLastError()));
   }
   *out = p;
+  return SIMBA_OK;
+}
+
+extern "C" int simba_planner_set_update_rule(simba_planner_t* p, int32_t rule, float temperature) {
+  if (!p) return set_error(SIMBA_ERR_BAD_CONFIG, "null argument");
+  if (rule != SIMBA_UPDATE_CEM && rule != SIMBA_UPDATE_MPPI) return set_error(SIMBA_ERR_BAD_CONFIG, "update rule %d unknown", rule);
+  if (p->captured) return set_error(SIMBA_ERR_BAD_CONFIG, "the update rule is fixed once the planner has planned");
+  const auto& c = p->cfg;
+  const int A = p->model->cfg.act_dim;
+  bool staged = false;
+  if (rule == SIMBA_UPDATE_CEM) {
+    p->update_rule = rule;
+    choose_update_path(p, cem_update_smem_bytes(c.particles, c.n_samples, c.n_elite, c.horizon, A, &staged));
+    return SIMBA_OK;
+  }
+  if (!(temperature > 0.0f) || !std::isfinite(temperature))
+    return set_error(SIMBA_ERR_BAD_CONFIG, "MPPI temperature %g must be finite and > 0", (double)temperature);
+  if (c.objective == SIMBA_OBJ_FEASIBLE_FIRST)
+    return set_error(SIMBA_ERR_UNSUPPORTED, "MPPI needs a scalar score: FEASIBLE_FIRST is an order");
+  if (c.world_size > 1)
+    return set_error(SIMBA_ERR_UNSUPPORTED, "MPPI runs on one rank (world_size %d): shard states instead", c.world_size);
+  if (mppi_refit_smem_bytes(c.n_samples, c.horizon, A) > (size_t)p->smem_optin)
+    return set_error(SIMBA_ERR_UNSUPPORTED, "MPPI update of %d candidates x %d values does not fit shared memory",
+                     c.n_samples, c.horizon * A);
+  p->update_rule = rule;
+  p->temperature = temperature;
+  choose_update_path(p, mppi_update_smem_bytes(c.particles, c.n_samples, c.horizon, A, &staged));
   return SIMBA_OK;
 }
 
@@ -898,24 +936,114 @@ extern "C" int simba_finalize_action(simba_planner_t* p, const float* best_actio
   return do_finalize_action(p, best_action, z, seed, nullptr, out_action, stream);
 }
 
+static MppiParams make_mppi_params(simba_planner_t* p, const float* pairs, const float* actions, const int32_t* active,
+                                   float* mu, float* best_action, float* best_score, int32_t* iterations_run) {
+  MppiParams mp{};
+  mp.S = p->cfg.n_states; mp.N = p->cfg.n_samples; mp.H = p->cfg.horizon; mp.A = p->model->cfg.act_dim;
+  mp.objective = p->cfg.objective; mp.c_max = (float)p->c_max;
+  mp.temperature = p->temperature;
+  mp.smoothing = p->cfg.smoothing;
+  mp.one_minus_smoothing = (float)(1.0 - (double)p->cfg.smoothing);
+  mp.pairs = pairs; mp.actions = actions; mp.active = active; mp.mu = mu;
+  mp.best_action = best_action; mp.best_score = best_score; mp.iterations_run = iterations_run;
+  return mp;
+}
+
+extern "C" int simba_mppi_update(simba_planner_t* p, const float* pairs, const float* actions,
+                                 const int32_t* active, float* mu, float* best_action, float* best_score,
+                                 void* stream) {
+  if (!p || !pairs || !actions || !mu || !best_action || !best_score)
+    return set_error(SIMBA_ERR_BAD_CONFIG, "null argument");
+  if (p->update_rule != SIMBA_UPDATE_MPPI)
+    return set_error(SIMBA_ERR_BAD_CONFIG, "the planner's update rule is not SIMBA_UPDATE_MPPI");
+  const MppiParams mp = make_mppi_params(p, pairs, actions, active, mu, best_action, best_score, nullptr);
+  SIMBA_CUDA_TRY(launch_mppi_refit(mp, (cudaStream_t)stream));
+  return SIMBA_OK;
+}
+
 // ---- the planning call ---------------------------------------------------------------------------
+static PlanInitParams make_plan_init_params(simba_planner* p) {
+  PlanInitParams ip{};
+  ip.S = p->cfg.n_states; ip.H = p->cfg.horizon; ip.A = p->model->cfg.act_dim;
+  memcpy(ip.init_mean, p->cfg.init_mean, sizeof(ip.init_mean));
+  memcpy(ip.init_stddev, p->cfg.init_stddev, sizeof(ip.init_stddev));
+  ip.mu = p->mu; ip.sigma = p->sigma; ip.best_action = p->best_action; ip.best_score = p->best_score;
+  ip.active = p->active; ip.iterations_run = p->iters;
+  return ip;
+}
+
+// An MPPI plan: CEM's init, sampling, rollout and reduction, the MPPI update in place of selection and refit, and the
+// final noise on mu[s, 0, :]. One rank. Fused: init + sample(0), then per iteration the rollout and one
+// mppi_update_kernel (reduce + update + next sampling | finalize + outputs).
+static int enqueue_mppi_plan(simba_planner* p, cudaStream_t st, int* n_launches) {
+  const uint64_t* sp = p->d_seed;
+  const auto& c = p->cfg;
+  const size_t S = c.n_states, N = c.n_samples, HA = (size_t)c.horizon * p->model->cfg.act_dim;
+  const size_t B = (size_t)c.particles * N, O = p->model->cfg.obs_dim;
+  const PlanInitParams ip = make_plan_init_params(p);
+  const MppiParams mp = make_mppi_params(p, p->pairs_local, p->actions, p->active, p->mu, p->best_action,
+                                         p->best_score, p->iters);
+  const FinalizeParams fp = make_finalize_params(p, p->mu, p->ext_z_final, 0, sp, p->d_out_action);   // on mu[s, 0, :]
+  int launches = 0;
+  if (p->fused_update) {
+    const SampleParams sp0 = make_sample_params(p, p->mu, p->sigma, p->ext_z_actions, 0, sp, 0, p->active, p->actions);
+    SIMBA_CUDA_TRY(launch_plan_begin(ip, sp0, st)); ++launches;
+  } else {
+    SIMBA_CUDA_TRY(launch_plan_init(ip, st)); ++launches;
+  }
+  for (int it = 0; it < c.iterations; ++it) {
+    const float* eps = p->ext_eps ? p->ext_eps + (size_t)it * S * c.horizon * B * O : nullptr;
+    int rc;
+    if (p->fused_update) {
+      rc = do_rollout_score(p, p->d_states, p->actions, eps, 0, sp, it, p->active, p->row_ret, p->row_cmask,
+                            p->row_csum, st, p->use_pdl);
+      if (rc) return rc; ++launches;
+      MppiUpdateParams u{};
+      u.pdl = p->use_pdl ? 1 : 0;
+      u.reduce = make_reduce_params(p, p->row_ret, p->row_cmask, p->row_csum, p->active, p->pairs_local);
+      u.mppi = mp;
+      const float* zn = (p->ext_z_actions && it + 1 < c.iterations)
+                            ? p->ext_z_actions + (size_t)(it + 1) * S * N * HA : nullptr;
+      u.sample = make_sample_params(p, p->mu, p->sigma, zn, 0, sp, it + 1, p->active, p->actions);
+      u.finalize = fp;
+      u.last = (it + 1 == c.iterations) ? 1 : 0;
+      u.out_score = p->d_out_score;
+      u.out_iters = p->d_out_iters;
+      SIMBA_CUDA_TRY(launch_mppi_update(u, st)); ++launches;
+      continue;
+    }
+    const float* z = p->ext_z_actions ? p->ext_z_actions + (size_t)it * S * N * HA : nullptr;
+    const SampleParams smp = make_sample_params(p, p->mu, p->sigma, z, 0, sp, it, p->active, p->actions);
+    SIMBA_CUDA_TRY(launch_sample_actions(smp, st)); ++launches;
+    rc = do_rollout_score(p, p->d_states, p->actions, eps, 0, sp, it, p->active, p->row_ret, p->row_cmask,
+                          p->row_csum, st);
+    if (rc) return rc; ++launches;
+    rc = simba_score_reduce(p, p->row_ret, p->row_cmask, p->row_csum, p->active, p->pairs_local, st);
+    if (rc) return rc; ++launches;
+    SIMBA_CUDA_TRY(launch_mppi_refit(mp, st)); ++launches;
+  }
+  if (!p->fused_update) {
+    SIMBA_CUDA_TRY(launch_mppi_finalize(fp, (int)HA, st)); ++launches;
+    SIMBA_CUDA_TRY(launch_plan_output(p->best_score, p->iters, p->d_out_score, p->d_out_iters, c.n_states, st));
+    ++launches;
+  }
+  if (n_launches) *n_launches = launches;
+  return SIMBA_OK;
+}
+
 // One plan = init + I x (sample, rollout, reduce, [all-gather], select, refit) + finalize + output,
 // captured once as a CUDA graph. The graph reads the states from p->d_states and the Philox seed from
 // p->d_seed (device memory), so neither a new state nor a new seed needs a re-capture; the early
 // exit of cem_mpc.py:66-67 is the device-side active[] flag that turns later nodes into no-ops.
 static int enqueue_plan(simba_planner* p, cudaStream_t st, int* n_launches) {
+  if (p->update_rule == SIMBA_UPDATE_MPPI) return enqueue_mppi_plan(p, st, n_launches);
   const uint64_t* sp = p->d_seed;
   const auto& c = p->cfg;
   const auto& mc = p->model->cfg;
   const size_t S = c.n_states, N = c.n_samples, HA = (size_t)c.horizon * mc.act_dim;
   const size_t B = (size_t)c.particles * N, O = mc.obs_dim;
   int launches = 0;
-  PlanInitParams ip{};
-  ip.S = c.n_states; ip.H = c.horizon; ip.A = mc.act_dim;
-  memcpy(ip.init_mean, c.init_mean, sizeof(ip.init_mean));
-  memcpy(ip.init_stddev, c.init_stddev, sizeof(ip.init_stddev));
-  ip.mu = p->mu; ip.sigma = p->sigma; ip.best_action = p->best_action; ip.best_score = p->best_score;
-  ip.active = p->active; ip.iterations_run = p->iters;
+  const PlanInitParams ip = make_plan_init_params(p);
   const bool multi = c.world_size > 1;
   float* pairs_all = multi ? p->pairs_all : p->pairs_local;
   if (!p->fused_update) { SIMBA_CUDA_TRY(launch_plan_init(ip, st)); ++launches; }
@@ -1002,6 +1130,7 @@ static int ensure_graph(simba_planner* p) {
   if (rc != SIMBA_OK) { if (g) cudaGraphDestroy(g); return rc; }
   if (ce != cudaSuccess) return set_error(SIMBA_ERR_CUDA, "graph capture failed: %s", cudaGetErrorString(ce));
   p->graph = g;
+  p->captured = true;
   SIMBA_CUDA_TRY(cudaGraphInstantiate(&p->graph_exec, p->graph, 0));
   p->launches_per_plan = launches;
   p->graph_generation = p->model->generation;
@@ -1020,6 +1149,10 @@ static int upload_seed(simba_planner* p, uint64_t seed, cudaStream_t st) {
 
 extern "C" int simba_planner_launches_per_plan(simba_planner_t* p, int32_t* out) {
   if (!p || !out) return set_error(SIMBA_ERR_BAD_CONFIG, "null argument");
+  if (p->update_rule == SIMBA_UPDATE_MPPI) {        // init, I x (sample, rollout, reduce, update), finalize, output
+    *out = p->fused_update ? 1 + 2 * p->cfg.iterations : 1 + 4 * p->cfg.iterations + 2;
+    return SIMBA_OK;
+  }
   const int per_iter = 5 + (p->cfg.world_size > 1 ? 1 : 0);
   *out = p->fused_update ? 1 + 2 * p->cfg.iterations : 1 + per_iter * p->cfg.iterations + 2;
   return SIMBA_OK;

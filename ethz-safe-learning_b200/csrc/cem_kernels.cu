@@ -983,7 +983,8 @@ cudaError_t launch_refit(const RefitParams& p_in, cudaStream_t st) {
 // =============================================================================================
 // k11  final noise — simba/policies/cem_mpc.py:68 : best + z * noise_stddev (not re-clipped)
 // =============================================================================================
-__device__ __forceinline__ void finalize_element(const FinalizeParams& p, int idx) {
+// z * noise_stddev of element idx = s * A + a of the [S, A] action
+__device__ __forceinline__ float final_noise(const FinalizeParams& p, int idx) {
   const int s = idx / p.A, a = idx - s * p.A;
   float z;
   if (p.z != nullptr) z = p.z[idx];
@@ -993,7 +994,11 @@ __device__ __forceinline__ void finalize_element(const FinalizeParams& p, int id
     const float zz[4] = {n.x, n.y, n.z, n.w};
     z = zz[a & 3];
   }
-  p.out[idx] = __fadd_rn(p.best[idx], __fadd_rn(__fmul_rn(z, p.noise_stddev), 0.0f));
+  return __fadd_rn(__fmul_rn(z, p.noise_stddev), 0.0f);
+}
+
+__device__ __forceinline__ void finalize_element(const FinalizeParams& p, int idx) {
+  p.out[idx] = __fadd_rn(p.best[idx], final_noise(p, idx));
 }
 
 __global__ void finalize_kernel(FinalizeParams p) {
@@ -1397,6 +1402,300 @@ cudaError_t launch_cem_update(const UpdateParams& u_in, cudaStream_t st) {
   const size_t smem = cem_update_smem_bytes(u.reduce.P, u.select.N, u.select.K, u.refit.H, u.refit.A, &staged);
   u.stage = staged ? 1 : 0;
   return launch_kernel(u.stage ? cem_update_kernel<true> : cem_update_kernel<false>, u.refit.S, kRefitThreads, smem, st,
+                       1, u.pdl != 0, u);
+}
+
+// =============================================================================================
+// MPPI update — Williams et al., "Information theoretic MPC for model-based reinforcement learning"
+// (ICRA 2017), the update PDDM (Nagabandi et al., 2019) plans with: every candidate contributes to the
+// new mean, weighted by exp((score - max score) / temperature); sigma stays fixed. Sampling, rollout,
+// scoring and the final noise are CEM's code. Both sums of the weighted mean run in one fixed order on
+// every path: ascending within blocks of 32 candidates, blocks folded in ascending order into
+// superblocks of 1024 candidates, superblocks folded in ascending order. The fused kernel (N <= 1024,
+// one superblock) and the separate refit kernel therefore give the same bits.
+// =============================================================================================
+constexpr int kMppiThreads = 1024;
+constexpr int kMppiSuper = 1024;          // candidates per superblock
+constexpr int kMppiBlock = 32;            // candidates per block
+constexpr int kMppiClusterSize = 8;       // CTAs per state of the refit when N > kMppiSuper
+
+// weight of a score against the largest non-NaN score m; a NaN score (a diverged rollout) weighs 0
+__device__ __forceinline__ float mppi_weight(float score, float m, float temperature) {
+  return score != score ? 0.0f : expf(__fdiv_rn(__fsub_rn(score, m), temperature));
+}
+
+// order key of the best candidate: larger score first, the lower index among ties. A key whose upper half is 0
+// belongs to a NaN score, so a maximum of 0 means every score was NaN.
+__device__ __forceinline__ unsigned long long mppi_key(float score, int i) {
+  return ((unsigned long long)ordered_u32(score) << 32) | (unsigned long long)(0xffffffffu - (uint32_t)i);
+}
+__device__ __forceinline__ int mppi_key_index(unsigned long long k) { return (int)(0xffffffffu - (uint32_t)k); }
+__device__ __forceinline__ float mppi_key_score(unsigned long long k) {     // inverse of ordered_u32 (-0 reads +0)
+  const uint32_t u = (uint32_t)(k >> 32);
+  return __uint_as_float((u & 0x80000000u) ? (u & 0x7fffffffu) : ~u);
+}
+
+// the largest key over the CTA, returned to every thread; called once per kernel (slot: a shared word)
+__device__ __forceinline__ unsigned long long mppi_block_max(unsigned long long k, unsigned long long* slot) {
+#pragma unroll
+  for (int d = 16; d > 0; d >>= 1) {
+    const unsigned long long o = __shfl_xor_sync(0xffffffffu, k, d);
+    k = o > k ? o : k;
+  }
+  if (threadIdx.x == 0) *slot = 0ull;
+  __syncthreads();
+  if ((threadIdx.x & 31) == 0) atomicMax(slot, k);
+  __syncthreads();
+  return *slot;
+}
+
+// One superblock's column sums: out[c] = sum_i w[i] * acts[i * HA + c] for c < HA and out[HA] = sum_i w[i], over
+// i < n <= kMppiSuper, in the fixed block order. acts: global or shared memory. blk: [ceil(n / 32)][HA + 1] shared
+// partials. Called by all kMppiThreads threads; ends with a CTA barrier.
+__device__ __forceinline__ void mppi_superblock(const float* w, const float* acts, int n, int HA, float* blk,
+                                                float* out) {
+  const int C = HA + 1, nb = (n + kMppiBlock - 1) / kMppiBlock;
+  for (int it = threadIdx.x; it < nb * C; it += kMppiThreads) {
+    const int b = it / C, c = it - b * C;
+    const int i0 = b * kMppiBlock, i1 = min(n, i0 + kMppiBlock);
+    float acc = 0.0f;
+    if (c < HA) {
+#pragma unroll 8
+      for (int i = i0; i < i1; ++i) acc = __fadd_rn(acc, __fmul_rn(w[i], acts[(long)i * HA + c]));
+    } else {
+      for (int i = i0; i < i1; ++i) acc = __fadd_rn(acc, w[i]);
+    }
+    blk[it] = acc;
+  }
+  __syncthreads();
+  for (int c = threadIdx.x; c < C; c += kMppiThreads) {
+    float acc = blk[c];
+    for (int b = 1; b < nb; ++b) acc = __fadd_rn(acc, blk[b * C + c]);
+    out[c] = acc;
+  }
+  __syncthreads();
+}
+
+// mu <- smoothing mu + (1 - smoothing) tot[c] / tot[HA], in the CEM refit's operation order; left unchanged when
+// every score was NaN. Best-so-far with strict '>' from the top key (acts_top: that candidate's row), and one more
+// iteration run. mu_sm (or null) receives this state's mean after the update. Called by every thread of one CTA.
+__device__ __forceinline__ void mppi_finish(const MppiParams& p, int s, unsigned long long top, const float* tot,
+                                            const float* acts_top, float* mu_sm) {
+  const int HA = p.H * p.A;
+  const bool valid = (top >> 32) != 0ull;
+  const float best_prev = p.best_score[s];
+  for (int c = threadIdx.x; c < HA; c += kMppiThreads) {
+    float v = p.mu[s * HA + c];
+    if (valid) {
+      v = __fadd_rn(__fmul_rn(p.smoothing, v), __fmul_rn(p.one_minus_smoothing, __fdiv_rn(tot[c], tot[HA])));
+      p.mu[s * HA + c] = v;
+    }
+    if (mu_sm != nullptr) mu_sm[c] = v;
+  }
+  __syncthreads();                                     // best_score[s] has been read by every thread
+  const float top_score = mppi_key_score(top);
+  if (valid && top_score > best_prev) {                // cem_mpc.py:58 strict '>'
+    if (threadIdx.x < p.A) p.best_action[s * p.A + threadIdx.x] = acts_top[threadIdx.x];
+    if (threadIdx.x == 0) p.best_score[s] = top_score;
+  }
+  if (threadIdx.x == 0 && p.iterations_run != nullptr) p.iterations_run[s] += 1;
+}
+
+// The separate refit: `ctas` CTAs per state (a cluster of kMppiClusterSize when N > kMppiSuper, one CTA otherwise),
+// CTA r taking superblocks [r per, r per + per). The maximum is combined over the cluster (exact); rank 0 folds every
+// superblock's sums in ascending order through distributed shared memory.
+__global__ void __launch_bounds__(kMppiThreads) mppi_refit_kernel(MppiParams p, int ctas, int per) {
+  const int s = blockIdx.x / ctas, rank = blockIdx.x - s * ctas;
+  if (p.active != nullptr && p.active[s] == 0) return;      // uniform over the cluster
+  extern __shared__ __align__(16) float sh[];
+  const int HA = p.H * p.A, C = HA + 1, N = p.N;
+  float* w = sh;                                             // [kMppiSuper] weights of one superblock
+  float* blk = w + kMppiSuper;                               // [32][C] block partials
+  float* sbp = blk + kMppiBlock * C;                         // [per][C] this CTA's superblock sums
+  float* tot = sbp + per * C;                                // [C]
+  __shared__ unsigned long long sh_key;
+  const float2* pairs = reinterpret_cast<const float2*>(p.pairs) + (long)s * N;
+  const int lo = min(N, rank * per * kMppiSuper), hi = min(N, lo + per * kMppiSuper);
+  unsigned long long k = 0ull;
+  for (int i = lo + threadIdx.x; i < hi; i += kMppiThreads) {
+    const float2 pr = pairs[i];
+    const unsigned long long ki = mppi_key(pair_score(p.objective, pr.x, pr.y, p.c_max), i);
+    k = ki > k ? ki : k;
+  }
+  unsigned long long top = mppi_block_max(k, &sh_key);
+  cg::cluster_group cluster = cg::this_cluster();
+  if (ctas > 1) {
+    cluster.sync();                                          // every CTA's maximum is in its sh_key
+    for (int r = 0; r < ctas; ++r) {
+      const unsigned long long o = *cluster.map_shared_rank(&sh_key, r);
+      top = o > top ? o : top;
+    }
+  }
+  const float m = mppi_key_score(top);
+  const float* acts = p.actions + (long)s * N * HA;
+  for (int q = 0; lo + q * kMppiSuper < hi; ++q) {
+    const int i0 = lo + q * kMppiSuper, n = min(kMppiSuper, hi - i0);
+    for (int j = threadIdx.x; j < n; j += kMppiThreads) {
+      const float2 pr = pairs[i0 + j];
+      w[j] = mppi_weight(pair_score(p.objective, pr.x, pr.y, p.c_max), m, p.temperature);
+    }
+    __syncthreads();
+    mppi_superblock(w, acts + (long)i0 * HA, n, HA, blk, sbp + q * C);
+  }
+  if (ctas > 1) cluster.sync();                              // every superblock's sums are complete
+  if (rank == 0) {
+    const int n_super = (N + kMppiSuper - 1) / kMppiSuper;
+    for (int c = threadIdx.x; c < C; c += kMppiThreads) {
+      float acc = sbp[c];
+#pragma unroll 8
+      for (int g = 1; g < n_super; ++g) {
+        const int r = g / per;
+        const float* src = r == 0 ? sbp : cluster.map_shared_rank(sbp, r);
+        acc = __fadd_rn(acc, src[(g - r * per) * C + c]);
+      }
+      tot[c] = acc;
+    }
+    __syncthreads();
+    mppi_finish(p, s, top, tot, acts + (long)mppi_key_index(top) * HA, nullptr);
+  }
+  if (ctas > 1) cluster.sync();                              // no CTA exits while rank 0 reads its shared memory
+}
+
+static void mppi_refit_geometry(int N, int* ctas, int* per) {
+  const int n_super = (N + kMppiSuper - 1) / kMppiSuper;
+  *ctas = n_super > 1 ? kMppiClusterSize : 1;
+  *per = (n_super + *ctas - 1) / *ctas;
+}
+
+size_t mppi_refit_smem_bytes(int N, int H, int A) {
+  int ctas = 1, per = 1;
+  mppi_refit_geometry(N, &ctas, &per);
+  const size_t C = (size_t)H * A + 1;
+  return (kMppiSuper + (kMppiBlock + per + 1) * C) * sizeof(float);
+}
+
+cudaError_t launch_mppi_refit(const MppiParams& p, cudaStream_t st) {
+  int ctas = 1, per = 1;
+  mppi_refit_geometry(p.N, &ctas, &per);
+  return launch_kernel(mppi_refit_kernel, p.S * ctas, kMppiThreads, mppi_refit_smem_bytes(p.N, p.H, p.A), st, ctas,
+                       false, p, ctas, per);
+}
+
+// Fused MPPI update for one rank's population of at most 1024 candidates, one CTA per state: k8 of this iteration
+// (the rows staged in shared memory when they fit, reduced by reduce_rows), the update, then k1 of the NEXT iteration
+// from the new mean, or k11 on mu[s, 0, :] and the plan outputs after the last one. Launched behind the rollout as a
+// programmatic dependent, like cem_update_kernel. The same device functions as score_reduce_kernel, mppi_refit_kernel,
+// sample_actions_kernel and finalize_kernel: the same bits.
+template <bool STAGED>
+__global__ void __launch_bounds__(kMppiThreads) mppi_update_kernel(MppiUpdateParams u) {
+  asm volatile("griddepcontrol.launch_dependents;" ::: "memory");
+  asm volatile("griddepcontrol.wait;" ::: "memory");
+  const MppiParams& p = u.mppi;
+  const int s = blockIdx.x, tid = threadIdx.x;
+  const int HA = p.H * p.A, C = HA + 1, N = p.N, P = u.reduce.P, rows = P * N;
+  const int n_planes = cmask_planes(u.reduce.H);
+  extern __shared__ __align__(16) float sh[];
+  float* w = sh;                                             // [N] weights
+  float* blk = w + kMppiSuper;                               // [32][C] block partials
+  float* tot = blk + kMppiBlock * C;                         // [C]
+  float* mu_sm = tot + C;                                    // [HA] the new mean
+  float* sg_sm = mu_sm + HA;                                 // [HA] sigma
+  const int o_stage = (kMppiSuper + (kMppiBlock + 1) * C + 2 * HA + 3) & ~3;
+  uint64_t* st_mask = reinterpret_cast<uint64_t*>(sh + o_stage);             // [W][rows]
+  float* st_ret = sh + o_stage + 2 * n_planes * rows;        // [rows]
+  float* st_csum = st_ret + rows;                            // [rows]
+  float* act_sm = st_csum + rows;                            // [N][HA]
+  __shared__ unsigned long long sh_key;
+  const bool active = p.active == nullptr || p.active[s] != 0;
+  if (active) {
+    if (STAGED) {
+      const float* gret = u.reduce.row_return + (long)s * rows;
+      const float* gcsum = u.reduce.row_costsum + (long)s * rows;
+      const uint64_t* gmask = u.reduce.row_costmask + (long)s * rows;
+      const float* gact = p.actions + (long)s * N * HA;
+      for (int idx = tid; idx < rows; idx += kMppiThreads) { st_ret[idx] = gret[idx]; st_csum[idx] = gcsum[idx]; }
+      for (int idx = tid; idx < n_planes * rows; idx += kMppiThreads) {   // plane stride S * rows in global memory
+        const int pl = idx / rows;
+        st_mask[idx] = gmask[(long)pl * u.reduce.S * rows + (idx - pl * rows)];
+      }
+      for (int idx = tid; idx < N * HA; idx += kMppiThreads) act_sm[idx] = gact[idx];
+      __syncthreads();
+    }
+    float score = 0.0f;
+    unsigned long long k = 0ull;
+    if (tid < N) {
+      const float2 pr = STAGED ? reduce_rows(st_ret, st_mask, st_csum, tid, N, P, u.reduce.H, rows, u.reduce.objective)
+                               : reduce_candidate(u.reduce, s, tid);
+      if (u.reduce.out_pairs != nullptr) reinterpret_cast<float2*>(u.reduce.out_pairs)[(long)s * N + tid] = pr;
+      score = pair_score(p.objective, pr.x, pr.y, p.c_max);
+      k = mppi_key(score, tid);
+    }
+    const unsigned long long top = mppi_block_max(k, &sh_key);
+    if (tid < N) w[tid] = mppi_weight(score, mppi_key_score(top), p.temperature);
+    __syncthreads();
+    const float* acts = STAGED ? act_sm : p.actions + (long)s * N * HA;
+    mppi_superblock(w, acts, N, HA, blk, tot);
+    mppi_finish(p, s, top, tot, acts + (long)mppi_key_index(top) * HA, mu_sm);
+    __syncthreads();
+  }
+  if (!u.last) {
+    if (active) {                                            // k1 of the next iteration, from the new mean
+      for (int c = tid; c < HA; c += kMppiThreads) sg_sm[c] = u.sample.sigma[s * HA + c];
+      __syncthreads();
+      const uint64_t seed = u.sample.seed_ptr ? *u.sample.seed_ptr : u.sample.seed;
+      const int JB = (HA + 3) >> 2;
+      for (int idx = tid; idx < N * JB; idx += kMppiThreads) {
+        const int i = idx / JB, j = idx - i * JB;
+        float out[4];
+        sample_values4_from(u.sample, mu_sm, sg_sm, seed, s, i, j, out);
+        store_block4(u.sample, s, i, j, out, u.sample.out);
+      }
+    }
+  } else {
+    // ---- k11 on mu[s, 0, :] + plan outputs ----------------------------------------------------------
+    __threadfence_block();
+    __syncthreads();
+    if (tid < u.finalize.A) {
+      const int idx = s * u.finalize.A + tid;
+      u.finalize.out[idx] = __fadd_rn(mu_sm[tid], final_noise(u.finalize, idx));     // mu[s, 0, a] + noise
+    }
+    if (tid == 0) {
+      u.out_score[s] = p.best_score[s];
+      if (u.out_iters != nullptr) u.out_iters[s] = p.iterations_run[s];
+    }
+  }
+}
+
+// k11 of an MPPI plan: mu[s, 0, :] + noise (p.best = mu [S, H, A])
+__global__ void mppi_finalize_kernel(FinalizeParams p, int HA) {
+  const int idx = blockIdx.x * blockDim.x + threadIdx.x;
+  if (idx >= p.S * p.A) return;
+  const int s = idx / p.A;
+  p.out[idx] = __fadd_rn(p.best[s * HA + (idx - s * p.A)], final_noise(p, idx));
+}
+
+cudaError_t launch_mppi_finalize(const FinalizeParams& p, int HA, cudaStream_t st) {
+  const int n = p.S * p.A;
+  mppi_finalize_kernel<<<(n + 127) / 128, 128, 0, st>>>(p, HA);
+  return cudaGetLastError();
+}
+
+size_t mppi_update_smem_bytes(int P, int N, int H, int A, bool* staged) {
+  const int HA = H * A, C = HA + 1;
+  const size_t base = (size_t)((kMppiSuper + (kMppiBlock + 1) * C + 2 * HA + 3) & ~3) * sizeof(float);
+  const size_t rows = (size_t)P * N;
+  const size_t stage = rows * (8 * (size_t)cmask_planes(H) + 8) + (size_t)N * HA * 4;
+  *staged = base + stage + 1024 <= 200 * 1024;
+  return *staged ? base + stage : base;
+}
+
+cudaError_t launch_mppi_update(const MppiUpdateParams& u_in, cudaStream_t st) {
+  MppiUpdateParams u = u_in;
+  if (u.mppi.N > kMppiSuper) return cudaErrorInvalidValue;
+  bool staged = false;
+  const size_t smem = mppi_update_smem_bytes(u.reduce.P, u.mppi.N, u.mppi.H, u.mppi.A, &staged);
+  u.stage = staged ? 1 : 0;
+  return launch_kernel(staged ? mppi_update_kernel<true> : mppi_update_kernel<false>, u.mppi.S, kMppiThreads, smem, st,
                        1, u.pdl != 0, u);
 }
 

@@ -96,7 +96,41 @@ struct UpdateParams {                 // fused k8 + k9 + k10 (+ next k1 | k11): 
   long long* timeline;                // -DSIMBA_TC_TIMELINE builds: clock64 stamps of the phases (tools/tc_timeline.py)
 };
 
+// MPPI update (Williams et al., "Information theoretic MPC for model-based reinforcement learning", ICRA 2017):
+// w_i = exp((score_i - max score) / temperature), 0 for a NaN score; mu <- smoothing mu + (1 - smoothing) sum w a / sum w;
+// sigma stays fixed. One rank: pairs hold all N candidates.
+struct MppiParams {
+  int32_t S, N, H, A, objective;
+  float c_max, temperature, smoothing, one_minus_smoothing;
+  const float* pairs;                 // [S, N, 2]
+  const float* actions;               // [S, N, H, A]
+  const int32_t* active;
+  float* mu;                          // [S, H, A], updated in place
+  float* best_action;                 // [S, A]   best-so-far (strict '>'), as CEM's selection keeps it
+  float* best_score;                  // [S]
+  int32_t* iterations_run;            // [S] or null
+};
+
+struct MppiUpdateParams {             // fused k8 + MPPI update (+ next k1 | k11): one rank, N <= 1024
+  ReduceParams reduce;
+  MppiParams mppi;
+  SampleParams sample;                // next iteration's sampling (ignored when last)
+  FinalizeParams finalize;            // used when last, on mu[s, 0, :]
+  int32_t last;
+  int32_t pdl;
+  int32_t stage;                      // set by launch_mppi_update: rows and actions of a state fit in shared memory
+  float* out_score;
+  int32_t* out_iters;
+};
+
 cudaError_t launch_cem_update(const UpdateParams& u, cudaStream_t st);
+cudaError_t launch_mppi_refit(const MppiParams& p, cudaStream_t st);
+cudaError_t launch_mppi_update(const MppiUpdateParams& u, cudaStream_t st);
+cudaError_t launch_mppi_finalize(const FinalizeParams& p, int HA, cudaStream_t st);   // p.best = mu [S, H, A]
+// Dynamic shared memory of the MPPI kernels: the fused update without its optional staging area (P particles, N <= 1024
+// candidates), and the separate refit at any N. A plan whose refit does not fit the device is rejected.
+size_t mppi_update_smem_bytes(int P, int N, int H, int A, bool* staged);
+size_t mppi_refit_smem_bytes(int N, int H, int A);
 // Dynamic shared memory of the fused update kernel at these sizes (P particles, N candidates, K elites, horizon H,
 // A action dims): the refit scratch and selection keys, plus the staging area of per-row outputs, actions and draws
 // when that fits under 200 KB (*staged)

@@ -15,6 +15,7 @@ SIMBA_MAX_HORIZON = 1024   # and horizon * act_dim <= 1024
 OBJ_REWARD, OBJ_SAFE_PENALTY, OBJ_LEAST_COST, OBJ_FEASIBLE_FIRST = 0, 1, 2, 3
 PREC_FP32, PREC_BF16_TC = 0, 1
 ACT_RELU, ACT_SWISH = 0, 1
+UPDATE_CEM, UPDATE_MPPI = 0, 1
 MAP_SPLIT, MAP_PARTICLE = 0, 1
 (BUF_ACTIONS, BUF_ROW_RETURN, BUF_ROW_COSTMASK, BUF_ROW_COSTSUM, BUF_PAIRS_LOCAL, BUF_PAIRS_ALL,
  BUF_ELITE, BUF_MU, BUF_SIGMA, BUF_BEST_ACTION, BUF_BEST_SCORE, BUF_ACTIVE, BUF_SCORES) = range(13)
@@ -93,6 +94,8 @@ _SIGNATURES = {
     'simba_select_elites': [_vp, _vp, _vp, _vp, _vp, _vp, _vp, _vp, _vp],
     'simba_refit': [_vp, _vp, _vp, _vp, _vp, _vp, _vp, _vp],
     'simba_finalize_action': [_vp, _vp, _vp, _u64, _vp, _vp],
+    'simba_planner_set_update_rule': [_vp, _i32, _f],
+    'simba_mppi_update': [_vp, _vp, _vp, _vp, _vp, _vp, _vp, _vp],
     'simba_plan': [_vp, _vp, _u64, _vp, _vp, _vp, _vp],
     'simba_plan_host': [_vp, _vp, _u64, _vp, _vp, _vp],
     'simba_planner_buffer': [_vp, _i32, _P(_vp), _P(_u64)],

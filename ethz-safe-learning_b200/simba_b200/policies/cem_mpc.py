@@ -99,6 +99,11 @@ class CemMpc(MpcPolicy):
             cfg = self._config()
             h = C.c_void_p()
             _lib.check(self._lib.simba_planner_create(model_handle, C.byref(cfg), C.byref(h)))
+            try:
+                self._configure_planner(h)
+            except BaseException:
+                self._lib.simba_planner_destroy(h)
+                raise
             self._planner = h
             self._cfg = cfg
             if self._external is not None:
@@ -106,6 +111,9 @@ class CemMpc(MpcPolicy):
         else:
             self.model.model._ensure_handle()        # re-commit if weights / scaler changed
         return self._planner
+
+    def _configure_planner(self, handle):
+        """Settings made right after simba_planner_create, before the first plan (none for CEM)."""
 
     def __del__(self):
         try:

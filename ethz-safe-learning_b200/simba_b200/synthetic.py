@@ -109,13 +109,15 @@ def make_workload(cfg_name='c1', sensors=None, seed=0, mu_scale=0.05, var_bias=-
 
 def build_policy(c, objective='penalty', precision='bf16', member_map='split', threshold=0.15,
                  smoothing=0.0, stddev_threshold=0.0, noise_stddev=0.01, sampling_propagation=True,
-                 scorer_config=None, seed=0, n_states=None, rank=0, world_size=1, activation='tf.nn.relu'):
+                 scorer_config=None, seed=0, n_states=None, rank=0, world_size=1, activation='tf.nn.relu',
+                 temperature=None):
     """The reference's construction sequence (mbrl_agent.py:103-118) on the B200 classes:
     environment -> TransitionModel(MlpEnsemble) -> CemMpc / SafeCemMpc, with the workload's
-    weights and scaler statistics loaded. `activation`: mlp_params['activation'] of the ensemble."""
+    weights and scaler statistics loaded. `activation`: mlp_params['activation'] of the ensemble.
+    With a `temperature`, MppiMpc / SafeMppiMpc instead (no n_elite, no stddev_threshold)."""
     from .environment_utils import ScorerEnvironment
     from .models import TransitionModel
-    from .policies import CemMpc, SafeCemMpc
+    from .policies import CemMpc, MppiMpc, SafeCemMpc, SafeMppiMpc
     env = ScorerEnvironment(c['sensors'], scorer_config, action_low=[-1.0] * c['A'], action_high=[1.0] * c['A'])
     tm = TransitionModel('mlp_ensemble', env.observation_space, env.action_space, True,
                          sampling_propagation, ensemble_size=c['E'],
@@ -124,6 +126,14 @@ def build_policy(c, objective='penalty', precision='bf16', member_map='split', t
     for e in range(c['E']):
         tm.model.ensemble[e].set_weights(c['weights'][e])
     tm.set_statistics(c['smin'], c['smax'])
+    if temperature is not None:
+        common = dict(horizon=c['H'], iterations=c['I'], smoothing=smoothing, n_samples=c['N'], particles=c['P'],
+                      noise_stddev=noise_stddev, temperature=temperature, precision=precision,
+                      member_map=member_map, seed=seed, n_states=c['S'] if n_states is None else n_states,
+                      rank=rank, world_size=world_size)
+        if objective == 'reward':
+            return MppiMpc(tm, env, **common)
+        return SafeMppiMpc(tm, env, posterior_mean_threashold=threshold, selection=objective, **common)
     common = dict(horizon=c['H'], iterations=c['I'], smoothing=smoothing, n_samples=c['N'],
                   n_elite=c['K'], particles=c['P'], stddev_threshold=stddev_threshold,
                   noise_stddev=noise_stddev, precision=precision, member_map=member_map, seed=seed,

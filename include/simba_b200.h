@@ -64,6 +64,13 @@ typedef enum simba_activation {
   SIMBA_ACT_SWISH = 1            /* tf.nn.swish: z * sigmoid(z)                                        */
 } simba_activation;
 
+typedef enum simba_update_rule {
+  SIMBA_UPDATE_CEM = 0,          /* elite selection and refit, cem_mpc.py:56-67, the default            */
+  SIMBA_UPDATE_MPPI = 1          /* softmax-weighted mean of all candidates, sigma fixed (Williams et al.,
+                                    "Information theoretic MPC for model-based reinforcement learning",
+                                    ICRA 2017; the update PDDM, Nagabandi et al. 2019, plans with)   */
+} simba_update_rule;
+
 typedef enum simba_member_map {
   SIMBA_MAP_SPLIT = 0,           /* tf.split: member(r) = r / (P*N/E), r = p*N + i (mlp_ensemble.py:123) */
   SIMBA_MAP_PARTICLE = 1         /* member(p) = floor(p*E/P); equals SPLIT whenever E divides P      */
@@ -199,6 +206,26 @@ int simba_select_elites(simba_planner_t* p, const float* pairs_all, const float*
 int simba_refit(simba_planner_t* p, const float* actions, const int32_t* elite, float* mu,
                 float* sigma, int32_t* active_or_null, int32_t* iterations_run_or_null,
                 void* stream);
+
+/* The planner's update rule, simba_update_rule (SIMBA_UPDATE_CEM unless set). SIMBA_UPDATE_MPPI keeps the sampling
+ * (k1), the rollout and scoring (k2-k8) and the final noise of CEM and replaces k9 + k10 with the MPPI update of
+ * Williams et al. (ICRA 2017): per state and iteration, with scores S_i of the planner's objective,
+ *   m = max_i S_i over non-NaN scores,  w_i = exp((S_i - m) / temperature)  (0 for a NaN score),
+ *   mu <- smoothing * mu + (1 - smoothing) * sum_i w_i a_i / sum_i w_i    (mu unchanged if every score is NaN),
+ * sigma fixed, no early exit (iterations_run = I), best_score = the largest score seen (strict '>'), and the action
+ * mu[0, :] + noise_stddev * z_final (not re-clipped). n_elite and stddev_threshold are not used. `temperature` is
+ * ignored for SIMBA_UPDATE_CEM. Allowed only before the planner's first plan. Returns SIMBA_ERR_BAD_CONFIG for an
+ * unknown rule, a temperature that is not finite and > 0, or a call after the first plan; SIMBA_ERR_UNSUPPORTED for
+ * SIMBA_OBJ_FEASIBLE_FIRST (an order with no scalar score), world_size > 1, or a population whose update does not fit
+ * the device's shared memory. */
+int simba_planner_set_update_rule(simba_planner_t* p, int32_t rule, float temperature);
+
+/* MPPI update of one iteration (the rule above), the kernel an MPPI plan runs after k8 when its update is not fused.
+ * pairs [S, N, 2] as simba_score_reduce writes them; actions [S, N, H, A]; mu [S, H, A] is updated in place;
+ * best_action [S, A] (the best candidate's first action) and best_score [S] are read-modify-write. The planner's
+ * rule must be SIMBA_UPDATE_MPPI. DEVICE. */
+int simba_mppi_update(simba_planner_t* p, const float* pairs, const float* actions, const int32_t* active_or_null,
+                      float* mu, float* best_action, float* best_score, void* stream);
 
 /* k11  final exploration noise — cem_mpc.py:68 (not re-clipped). */
 int simba_finalize_action(simba_planner_t* p, const float* best_action, const float* z_or_null,
